@@ -10,11 +10,14 @@ the timed step (fused into the update kernel over NVLink peer memory; `collectiv
 A "step" is one such forward+backward over one batch of synthetic latents.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2|cfg3]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the reference's own CPU implementation of the
 path (the oracle port, pinned bit-for-bit to the reference source) on the host cores.
 Only this file's cpu_baseline / `--impl reference` legs execute anything under oracle/.
+`--dump-outputs DIR` writes rank 0's results of the last timed step as DIR/<name>.npy (see dump_outputs()); the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -75,6 +78,23 @@ def synth(N, K, D, seed):
     x = E[pi] + 0.5 * E.std() * torch.randn(N, D, generator=g)
     gz = torch.randn(N, D, generator=g)
     return x.to(torch.bfloat16), E, gz
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each tensor as out_dir/<name>.npy: floating-point results as float32, code indices as float64 (exact
+    for every index).  Every workload's outputs fit DUMP_LIMIT_BYTES whole (cfg4, the largest, is ~40 MB)."""
+    import numpy as np
+    host = {name: (t.float() if t.is_floating_point() else t.double()).detach().cpu().numpy()
+            for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_LIMIT_BYTES, f'--dump-outputs: {total} bytes exceed {DUMP_LIMIT_BYTES}'
+    out = pathlib.Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in host.items():
+        np.save(out / f'{name}.npy', a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -145,7 +165,7 @@ def run_reference(args, wl, budget_s: float = 150.0):
         xo = x[:n].float().requires_grad_(True)
         out = O.quantizer_forward(spec, [xo], E, prob)
         torch.autograd.backward((out['z_ste'][0], out['loss'][0]), (gz[:n], torch.ones([])))
-        return out
+        return dict(z=out['z_ste'][0], loss=out['loss'][0], quant=out['quant'][0], gx=xo.grad, codebook=out['weight'])
 
     t0 = time.perf_counter()
     step(N)                                    # untimed probe: sizes the per-step sample
@@ -158,12 +178,13 @@ def run_reference(args, wl, budget_s: float = 150.0):
         step(n)
     t0 = time.perf_counter()
     for _ in range(steps):
-        step(n)
+        last = step(n)
     dt = (time.perf_counter() - t0) / steps
     value = n / dt
     sample = (f'{"full batch" if n == N else f"first {n} of {N} tokens"} of {wl["name"]} per step x {steps} timed steps '
               f'after {warmup} warm-ups, fp32, torch {torch.__version__} CPU, {threads} threads')
-    return dict(value=value, ms=dt * 1e3, cores=threads, kind='port', sample=sample, steps=steps, warmup=warmup)
+    return dict(value=value, ms=dt * 1e3, cores=threads, kind='port', sample=sample, steps=steps, warmup=warmup,
+                outputs=last)
 
 
 def run_gpu_eager(wl, dev, x0, E, gz0, autocast: bool, steps: int = 10):
@@ -225,7 +246,7 @@ def run_cfg5(args, rank, world, local_rank):
         dist.barrier()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    steps = min(args.steps, 20)
+    steps = args.steps
     e0.record()
     for _ in range(steps):
         quant = step()
@@ -233,6 +254,8 @@ def run_cfg5(args, rank, world, local_rank):
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(quant=quant))
     ms = e0.elapsed_time(e1) / steps
     if world > 1:
         t = torch.tensor([ms], device=dev)
@@ -262,7 +285,9 @@ def run_cfg5(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=200)
+    ap.add_argument('--steps', type=int, default=200,
+                    help='timed steps of the metric (every workload and --impl); the secondary legs time fewer: '
+                         'the end-to-end leg min(K, 100) steps, the isolated assign-kernel timing min(K, 30) launches')
     ap.add_argument('--warmup', type=int, default=10)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--workload', default='cfg2', choices=sorted(WORKLOADS) + ['cfg5'])
@@ -275,7 +300,12 @@ def main():
                          "'all' also ships the bf16 token gradient, which in a training loop stays on the device")
     ap.add_argument('--breakdown', action='store_true',
                     help='also time CUDA graphs of step prefixes (encode only / + gather+loss / + backward)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="after the timed steps, write rank 0's results of the last one (z, loss, code indices, token "
+                         'gradient, updated codebook; cfg5: code indices) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
@@ -290,6 +320,8 @@ def main():
         if rank != 0:
             return
         r = run_reference(args, wl)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r['outputs'])
         print(json.dumps(dict(
             metric=metric, value=r['value'], unit=unit, n_gpus=args.gpus, steps=r['steps'], warmup=r['warmup'],
             ms_per_step=r['ms'], higher_is_better=True, scaling='weak', vs_baseline=None, dtype='f32', data='synthetic',
@@ -389,9 +421,12 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        run(i)
+        last = run(i)
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:   # before any later leg runs another step (training updates the codebook)
+        dump_outputs(args.dump_outputs, dict(z=last['z'], loss=last['loss'], quant=last['quant'], gx=last['gx'],
+                                             codebook=q.embedding.weight))
     ms = e0.elapsed_time(e1) / args.steps
     if world > 1:
         t = torch.tensor([ms], device=dev)
@@ -663,7 +698,7 @@ def main():
                         launch='CUDA graph replay' if graphs else 'eager', kernels_per_step=launches_per_step),
             clocks=clocks, roofline=roofline, collective=collective, cpu_baseline=cpu_baseline,
             gpu_eager_baseline=gpu_eager, breakdown_ms=breakdown,
-            e2e=dict(value=N * world / (e2e_ms * 1e-3), unit=unit, ms_per_step=e2e_ms, h2d_bytes_per_step=h2d,
+            e2e=dict(value=N * world / (e2e_ms * 1e-3), unit=unit, ms_per_step=e2e_ms, steps=k2, h2d_bytes_per_step=h2d,
                      d2h_bytes_per_step=d2h, cpu_affinity=numa,
                      readback=args.e2e_readback,
                      note='per step: bf16 tokens + bf16 upstream gradient host->device (widened to fp32 on the device), '

@@ -190,6 +190,53 @@ def run_lazy_init(N, K, D, iters):
                 quant=memo['quant'].clone(), W_after=q.embedding.weight.detach().clone(), loss=loss.detach().clone())
 
 
+ANCHOR_GOLDEN = 'anchors_entropy.pt'
+CACHED_ANCHOR_SHAPES = [(200, 64), (64, 64), (40, 64)]   # N > K, N == K, N < K (cache and noise top-up)
+
+
+def run_anchor_cases(ref=None):
+    """CachedAnchor over three consecutive steps per (N, K), EntropyLoss and MultinomialAnchor on seeded inputs: from
+    the reference's own classes when `ref` (`ref_loader.load()`) is given, else from the restatements
+    (`anchors.cached_rows_and_indices`, `O.entropy_loss`, `O.multinomial_anchor`) that
+    tests/test_oracle_vs_reference.py pins to those classes bit for bit."""
+    from vector_quantization_b200.anchors import cached_rows_and_indices
+    D = 8
+    cached = {}
+    for N, K in CACHED_ANCHOR_SHAPES:
+        g = torch.Generator().manual_seed(N)
+        ref_anchor = ref.cvqvae.anchors.CachedAnchor() if ref is not None else None
+        cache = torch.empty(0)
+        xs, anchors = [], []
+        for step in range(3):
+            x = torch.randn(N, D, generator=g)
+            torch.manual_seed(100 + step)
+            random.seed(100 + step)
+            if ref_anchor is not None:
+                got, _ = ref_anchor(x, None, torch.zeros(N, K), None, torch.zeros(K))   # only d's shape is read
+            else:
+                rows, idx = cached_rows_and_indices(x, K, cache)
+                got = rows[idx]
+            cache = got
+            xs.append(x)
+            anchors.append(got.clone())
+        cached[(N, K)] = dict(x=xs, anchors=anchors)
+    x, E = O.synthetic_latents(96, 24, 8, seed=3)
+    d = O.distance('L2', x, E)
+    temperature = 0.7
+    if ref is not None:
+        entropy = ref.vq.losses.EntropyLoss(temperature=temperature)(None, None, dict(distance=d))
+        torch.manual_seed(5)
+        mn_anchors, _ = ref.cvqvae.anchors.MultinomialAnchor()(x, E, d, None, torch.zeros(24))
+    else:
+        entropy = O.entropy_loss(d, temperature)
+        torch.manual_seed(5)
+        mn_anchors, _ = O.multinomial_anchor(x, d)
+    source = ('reference source' if ref is not None else
+              'restatements pinned bit for bit to the reference source by tests/test_oracle_vs_reference.py')
+    return dict(source=source, D=D, cached_anchor=cached, x=x, E=E, d=d, temperature=temperature,
+                entropy=entropy.detach().clone(), multinomial_seed=5, multinomial_anchors=mn_anchors.clone())
+
+
 def main():
     OUT.mkdir(parents=True, exist_ok=True)
     ref = R.load()
@@ -207,7 +254,14 @@ def main():
         rec = run_lazy_init(*args)
         torch.save(rec, OUT / f'vqkd_lazy_init_{tag}.pt')
         print(f'vqkd_lazy_init_{tag}: oracle == reference source bit-for-bit (N={args[0]} K={args[1]} iters={args[3]})')
+    torch.save(run_anchor_cases(ref), OUT / ANCHOR_GOLDEN)
+    print(f'{ANCHOR_GOLDEN}: written from the reference source')
 
 
 if __name__ == '__main__':
-    main()
+    if sys.argv[1:] == ['anchors']:   # that file alone, from the pinned restatements when the reference is absent
+        rec = run_anchor_cases(R.load() if R.available() else None)
+        torch.save(rec, OUT / ANCHOR_GOLDEN)
+        print(f'{ANCHOR_GOLDEN}: written from the {rec["source"]}')
+    else:
+        main()

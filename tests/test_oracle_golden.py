@@ -70,3 +70,32 @@ def test_oracle_kmeans_lazy_init_matches_golden(tag):
     W = O.vqkd_lazy_init(rec['x'], rec['W0'], rec['iters'])
     close = torch.isclose(W, rec['W_init'], rtol=1e-5, atol=1e-6).all(1)
     assert close.float().mean() >= (0.95 if tag == 'iters10' else 1.0)
+
+
+@pytest.mark.parametrize('N,K', [(200, 64), (64, 64), (40, 64)])
+def test_cached_anchor_sampling_rule_matches_golden(N, K):
+    """`cached_rows_and_indices` (the product's CachedAnchor rule) against the stored anchors of the reference's
+    CachedAnchor under the same seeds, bit for bit, over three consecutive steps (cache top-up) for N > K, N == K and
+    N < K."""
+    import random
+    from vector_quantization_b200.anchors import cached_rows_and_indices
+    rec = torch.load(GOLDEN / 'anchors_entropy.pt', weights_only=False)['cached_anchor'][(N, K)]
+    cache = torch.empty(0)
+    for step, (x, want) in enumerate(zip(rec['x'], rec['anchors'])):
+        torch.manual_seed(100 + step); random.seed(100 + step)
+        rows, idx = cached_rows_and_indices(x, K, cache)
+        cache = rows[idx]
+        assert torch.equal(cache, want), step
+
+
+def test_entropy_loss_and_multinomial_anchor_match_golden():
+    """`O.entropy_loss` and `O.multinomial_anchor` (the oracle of the compat-mode GPU tests) against the stored outputs
+    of the reference's EntropyLoss and MultinomialAnchor on the stored distance matrix.  The anchors are compared bit
+    for bit under the same torch seed; the entropy to fp32 rounding, since its softmax/log reductions may be summed in
+    a different order on another CPU."""
+    rec = torch.load(GOLDEN / 'anchors_entropy.pt', weights_only=False)
+    x, d = rec['x'], rec['d']
+    torch.testing.assert_close(O.entropy_loss(d, rec['temperature']), rec['entropy'], rtol=1e-6, atol=1e-7)
+    torch.manual_seed(rec['multinomial_seed'])
+    anchors, _ = O.multinomial_anchor(x, d)
+    assert torch.equal(anchors, rec['multinomial_anchors'])

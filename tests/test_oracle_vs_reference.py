@@ -22,6 +22,13 @@ def test_restatement_equals_reference_source_and_golden_is_reproducible():
             assert torch.equal(a['W_after'], b['W_after']) and torch.equal(a['loss'], b['loss'])
     for levels in ([8, 8, 5, 5, 5], [8, 8, 8, 5, 5, 5]):
         M.run_fsq(levels)
+    rec = M.run_anchor_cases(ref_loader.load())
+    disk = torch.load(GOLDEN / M.ANCHOR_GOLDEN, weights_only=False)
+    for key, case in rec['cached_anchor'].items():
+        for a, b in zip(case['anchors'], disk['cached_anchor'][key]['anchors']):
+            assert torch.equal(a, b), key
+    assert torch.equal(rec['entropy'], disk['entropy'])
+    assert torch.equal(rec['multinomial_anchors'], disk['multinomial_anchors'])
 
 
 def test_plugin_force_registers_into_reference_registries():
