@@ -28,7 +28,8 @@
 extern "C" {
 #endif
 
-#define VQB200_ABI_VERSION 3 /* 2: fp16 plane formats, vqb_row_inv_norm(f16_rows), vqb_transpose_last2, vqb_compact_tokens; 3: vqb_comm_*, g_dtype of vqb_quantize_backward */
+#define VQB200_ABI_VERSION 3 /* 2: fp16 plane formats, vqb_row_inv_norm(f16_rows), vqb_transpose_last2, vqb_compact_tokens; 3: vqb_comm_*, g_dtype of vqb_quantize_backward;
+                                3 (additive): vqb_segment_chunk, vqb_code_sort*, vqb_segment_sum_*, vqb_quantize_backward_rows */
 
 typedef enum { VQB_OK = 0, VQB_ERR_ARG = -1, VQB_ERR_CUDA = -2, VQB_ERR_UNSUPPORTED = -3 } vqb_status;
 typedef enum { VQB_F32 = 0, VQB_BF16 = 1 } vqb_dtype;
@@ -234,6 +235,13 @@ int vqb_quantize_backward(const void* g_zste, int g_dtype /* VQB_F32, or VQB_BF1
                           void* gx_out /* x dtype */, float* gW_accum,
                           int64_t g_hw /* 0: g_zste and gx token-major; h*w > 0: both NCHW [N/hw, D, hw] (x stays token-major) */,
                           void* stream);
+/* The same backward with each token's codebook-gradient row STORED to gW_rows fp32 [N, D] instead of atomically added
+ * into gW (gx bit-identical to vqb_quantize_backward).  vqb_segment_sum_rows over those rows gives a deterministic gW. */
+int vqb_quantize_backward_rows(const void* g_zste, int g_dtype, const void* x, int x_dtype, int normalize_x,
+                               const float* W, int64_t K, const int64_t* quant, int64_t N, int D,
+                               const float* g_codebook, const float* g_commitment,
+                               const float* g_codebook_norm, const float* g_commitment_norm,
+                               int want_norm_mse, void* gx_out, float* gW_rows, int64_t g_hw, void* stream);
 
 /* ---- row l2-normalisation (NormalizeCallback.before_encode on x) ------------------------ *
  * vq/algorithms/vq/callbacks/normalize.py:24  — forward y = x / max(||x||, 1e-12); backward
@@ -255,6 +263,36 @@ int vqb_scatter_stats(const void* x, int x_dtype, int64_t N, int D, int normaliz
 int vqb_bincount_accumulate(const int64_t* quant, int64_t n, int64_t* counts, int64_t K,
                             int add_total, /* 1: counts[K] += n (numel slot of the fused [K | 1] all-reduce buffer) */
                             void* stream);
+
+/* ---- deterministic per-code reductions (torch.use_deterministic_algorithms) --------------- *
+ * The atomic scatters above (vqb_scatter_stats, the gW of vqb_quantize_backward) are order-dependent in the last
+ * bits.  These entry points give the same sums with a fixed association:
+ *   for code k with tokens t_1 < ... < t_m (tokens whose code is outside [0, K) are skipped; packed keys resolve
+ *   as in vqb_scatter_stats), cut the list into consecutive chunks of VQB_SEGMENT_CHUNK tokens; sum each chunk
+ *   serially in ascending token order from +0.0f, add the chunk sums serially in chunk order from +0.0f, and add
+ *   that total ONCE to the output element (a plain read-modify-write: a zero-filled output keeps the accumulate
+ *   semantics of vqb_scatter_stats).  Codes without tokens leave their output untouched.
+ * VQB_SEGMENT_CHUNK = 256: the longest serial chain is max(C, m / C) additions, so a collapsed codebook (all N tokens
+ * on one code) costs ~2 sqrt(N) dependent additions at N = 65 536 instead of N; a smaller C mostly adds chunk
+ * partials (scratch traffic) for codes of a few tokens, the common case. */
+#define VQB_SEGMENT_CHUNK 256
+int64_t vqb_segment_chunk(void);
+/* Stable sort of the tokens by code (LSD radix, 8-bit digits: ceil(bits(K) / 8) passes of 3 launches + 2 launches; no
+ * host synchronisation, no spinning).  order: int32 [N] token indices grouped by code, ascending within a code, the
+ * tokens with an out-of-range code last; offsets: int32 [K+1], code k owns order[offsets[k] .. offsets[k+1]).
+ * N < 2^31.  `scratch` needs vqb_code_sort_scratch_bytes(N, K) bytes. */
+size_t vqb_code_sort_scratch_bytes(int64_t N, int64_t K);
+int vqb_code_sort(const int64_t* quant,                /* [N] indices, or NULL when `keys` is given */
+                  const unsigned long long* keys, int64_t key_index_offset, int64_t N, int64_t K,
+                  int32_t* order, int32_t* offsets, void* scratch, size_t scratch_bytes, void* stream);
+/* out_sums fp32 [K, D] (+)= the contract sums of rows (fp32 or bf16 [N, D]; normalize_rows: F.normalize of each row,
+ * its norm computed with the lane geometry of vqb_scatter_stats, so each row's value depends on that row alone);
+ * out_counts (optional) fp32 [K] (+)= offsets[k+1] - offsets[k].  (order, offsets) from vqb_code_sort.  No float
+ * atomics.  `scratch` needs vqb_segment_sum_scratch_bytes(N, K, D) bytes (chunk partials, N / C + K + 1 rows). */
+size_t vqb_segment_sum_scratch_bytes(int64_t N, int64_t K, int D);
+int vqb_segment_sum_rows(const void* rows, int rows_dtype, int64_t N, int D, int normalize_rows,
+                         const int32_t* order, const int32_t* offsets, int64_t K,
+                         float* out_sums, float* out_counts, void* scratch, size_t scratch_bytes, void* stream);
 
 /* VQKDCallback._kmeans tail + after_encode:  callbacks.py:66-71,126-128,73-75
  *   C = cnt>0 ? S/max(cnt,1) : E ;  W <- normalize( E*decay + normalize(C)*(1-decay) )   (in place) */

@@ -71,6 +71,16 @@ SIGNATURES = {
                                     c_void_p]),
     'vqb_quantize_backward': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p, c_int64, c_int,
                                       c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p]),
+    'vqb_quantize_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p, c_int64,
+                                           c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64,
+                                           c_void_p]),
+    'vqb_segment_chunk': (c_int64, []),
+    'vqb_code_sort_scratch_bytes': (c_size_t, [c_int64, c_int64]),
+    'vqb_code_sort': (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_size_t,
+                              c_void_p]),
+    'vqb_segment_sum_scratch_bytes': (c_size_t, [c_int64, c_int64, c_int]),
+    'vqb_segment_sum_rows': (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p,
+                                     c_void_p, c_void_p, c_size_t, c_void_p]),
     'vqb_l2norm_forward': (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_int, c_void_p]),
     'vqb_l2norm_backward': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_int, c_void_p, c_int, c_void_p]),
     'vqb_scatter_stats': (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_int64,

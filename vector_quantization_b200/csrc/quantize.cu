@@ -220,7 +220,8 @@ __global__ void __launch_bounds__(256) quantize_forward_kernel(
 //   g_y = g_zste + c_cm (y - z) + J_n(y)^T [c_cmn (u - v)]         c_* = g4[*] * 2 / (N D)
 //   g_z = c_cb (z - y) + J_n(z)^T [c_cbn (v - u)]                   -> atomically added to gW[q]
 //   g_x_in = J_n(x_in)^T g_y  when normalize_x, else g_y            J_n(a)^T g = (g - (g.n(a)) n(a)) / |a|
-template <typename TX, typename TG, int G, int V, int NV>
+// kRowsOut: store each token's g_z row to gW + n*D ([N, D] rows for the deterministic segment sum) instead of the atomics
+template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut = false>
 __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
     const TG* __restrict__ gz, const TX* __restrict__ x, int normalize_x, const float* __restrict__ W, int64_t K,
     const int64_t* __restrict__ quant, int64_t N, int D, const float* __restrict__ g_cb,
@@ -320,7 +321,9 @@ __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
         gy_dot_y = fmaf(g_y, yv, gy_dot_y);
         gw[i] = g_w;
       }
-      if (gW && valid && d0 < D) {
+      if constexpr (kRowsOut) {
+        if (valid && d0 < D) store_slice<float, V>(gW + n * D, d0, D, gw);
+      } else if (gW && valid && d0 < D) {
         float* dst = gW + q * D + d0;
         if constexpr (V == 8) {   // two red.global.add.v4.f32 instead of eight scalar atomics (the slice is 32-byte aligned)
           atomicAdd(reinterpret_cast<float4*>(dst), make_float4(gw[0], gw[1], gw[2], gw[3]));
@@ -465,12 +468,17 @@ int vqb_gather_ste_loss(const void* x, int x_dtype, int64_t N, int D, int normal
   return VQB_OK;
 }
 
-int vqb_quantize_backward(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x, const float* W, int64_t K,
-                          const int64_t* quant, int64_t N, int D, const float* g_cb, const float* g_cm,
-                          const float* g_cbn, const float* g_cmn, int want_norm, void* gx, float* gW, int64_t g_hw,
-                          void* stream) {
+}  // extern "C"
+
+// kRowsOut selects the per-token-row variant (gW then points at fp32 [N, D] rows)
+template <bool kRowsOut>
+static int quantize_backward_launch(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x, const float* W,
+                                    int64_t K, const int64_t* quant, int64_t N, int D, const float* g_cb, const float* g_cm,
+                                    const float* g_cbn, const float* g_cmn, int want_norm, void* gx, float* gW,
+                                    int64_t g_hw, void* stream) {
   VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "vqb_quantize_backward: g_hw must divide N");
   VQB_REQUIRE(gz && x && W && quant && gx, "vqb_quantize_backward: null pointer");
+  VQB_REQUIRE(!kRowsOut || gW, "vqb_quantize_backward_rows: null gW_rows");
   VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "vqb_quantize_backward: bad shape");
   RowGeom geom;
   VQB_REQUIRE(row_geom(D, N, &geom), "vqb_quantize_backward: D=%d unsupported", D);
@@ -478,20 +486,38 @@ int vqb_quantize_backward(const void* gz, int g_dtype, const void* x, int x_dtyp
   const int blocks = grid_for(N, 256 / geom.G);
   bool launched = false;
   if (x_dtype == VQB_F32 && g_dtype == VQB_F32) {
-    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<float, float, G, V, NV>, blocks, 256, 0, st,
+    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<float, float, G, V, NV, kRowsOut>, blocks, 256, 0, st,
         (const float*)gz, (const float*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn, want_norm, (float*)gx, gW, g_hw)))
   } else if (x_dtype == VQB_BF16 && g_dtype == VQB_F32) {
-    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<__nv_bfloat16, float, G, V, NV>, blocks, 256, 0, st,
+    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<__nv_bfloat16, float, G, V, NV, kRowsOut>, blocks, 256, 0, st,
         (const float*)gz, (const __nv_bfloat16*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn, want_norm,
         (__nv_bfloat16*)gx, gW, g_hw)))
   } else if (x_dtype == VQB_BF16 && g_dtype == VQB_BF16) {   // bf16 upstream gradient (autocast training): read as is
-    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<__nv_bfloat16, __nv_bfloat16, G, V, NV>, blocks, 256, 0, st,
+    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<__nv_bfloat16, __nv_bfloat16, G, V, NV, kRowsOut>, blocks, 256, 0, st,
         (const __nv_bfloat16*)gz, (const __nv_bfloat16*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn,
         want_norm, (__nv_bfloat16*)gx, gW, g_hw)))
   }
   VQB_REQUIRE(launched, "vqb_quantize_backward: unsupported dtype/geometry");
   VQB_LAUNCH_OK();
   return VQB_OK;
+}
+
+extern "C" {
+
+int vqb_quantize_backward(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x, const float* W, int64_t K,
+                          const int64_t* quant, int64_t N, int D, const float* g_cb, const float* g_cm,
+                          const float* g_cbn, const float* g_cmn, int want_norm, void* gx, float* gW, int64_t g_hw,
+                          void* stream) {
+  return quantize_backward_launch<false>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn,
+                                         want_norm, gx, gW, g_hw, stream);
+}
+
+int vqb_quantize_backward_rows(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x, const float* W,
+                               int64_t K, const int64_t* quant, int64_t N, int D, const float* g_cb, const float* g_cm,
+                               const float* g_cbn, const float* g_cmn, int want_norm, void* gx, float* gW_rows,
+                               int64_t g_hw, void* stream) {
+  return quantize_backward_launch<true>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn,
+                                        want_norm, gx, gW_rows, g_hw, stream);
 }
 
 int vqb_unpack_keys(const unsigned long long* keys, int64_t n, int64_t offset, int64_t* idx, float* score,

@@ -18,6 +18,7 @@ from ._lib import BACKEND_SIMT, BACKEND_TCGEN05, PLANES_F16, PLANES_F16X2, VQB_B
 __all__ = [
     'Operand', 'as_operand', 'pack_rows', 'fold_l2_side', 'can_fold_l2', 'assign', 'certify', 'cvq_needy_codes', 'gather_operand_rows', 'scatter_keys', 'row_inv_norm', 'new_keys', 'unpack_keys', 'keys_flip_sign', 'gather_ste_loss',
     'quantize_backward', 'l2norm_forward', 'l2norm_backward', 'scatter_stats', 'bincount_accumulate',
+    'deterministic_enabled', 'segment_chunk', 'code_sort', 'segment_sum_rows',
     'kmeans_ema_update', 'gather_rows_by_key', 'cvq_update', 'embedding_gather', 'fsq_params', 'fsq_forward', 'fsq_backward',
     'fsq_decode', 'transpose_last2', 'compact_tokens', 'distance_matrix', 'comm_kmeans_ema_update', 'comm_cvq_update',
     'comm_allreduce_min_keys', 'comm_allreduce_sum_f32', 'BACKEND_TCGEN05', 'BACKEND_SIMT',
@@ -383,9 +384,12 @@ def gather_ste_loss(x: torch.Tensor, W: torch.Tensor, *, quant: torch.Tensor | N
 
 
 def quantize_backward(g_z: torch.Tensor, x: torch.Tensor, W: torch.Tensor, quant: torch.Tensor, g4, *,
-                      normalize_x: bool = False, want_norm: bool, need_gW: bool, g_hw: int = 0):
+                      normalize_x: bool = False, want_norm: bool, need_gW: bool, g_hw: int = 0,
+                      deterministic: bool | None = None):
     """g4: a float32 [4] tensor or a sequence of four 0-dim device tensors / None
-    (codebook, commitment, codebook-norm, commitment-norm upstream gradients)."""
+    (codebook, commitment, codebook-norm, commitment-norm upstream gradients).
+    deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, gW is the segment sum of the
+    per-token gradient rows (fixed association, see vqb_segment_sum_rows) instead of fp32 atomics.  gx is the same."""
     lib = _lib.load()
     if isinstance(g4, torch.Tensor):
         g4 = [g4[i] for i in range(4)]
@@ -394,10 +398,19 @@ def quantize_backward(g_z: torch.Tensor, x: torch.Tensor, W: torch.Tensor, quant
     if not (g_z.dtype == torch.float32 or (g_z.dtype == torch.bfloat16 and x.dtype == torch.bfloat16)):
         g_z = g_z.float()
     N, D = x.shape
+    K = W.shape[0]
     gx = torch.empty_like(x)
     gW = torch.zeros_like(W) if need_gW else None
+    if need_gW and deterministic_enabled(deterministic):
+        rows = _det_ws(x.device, 'gw_rows', N * D, torch.float32)
+        _call('vqb_quantize_backward_rows', lib.vqb_quantize_backward_rows, dev, _p(g_z), _dt(g_z), _p(x), _dt(x),
+              int(normalize_x), _p(W), K, _p(quant), N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm),
+              _p(gx), _p(rows), g_hw, _S)
+        order, offsets = _code_sort_ws(dev, N, K, quant, None, 0)
+        _segment_sum(dev, rows, N, D, False, order, offsets, K, gW, None)
+        return gx, gW
     _call('vqb_quantize_backward', lib.vqb_quantize_backward, dev, _p(g_z), _dt(g_z), _p(x), _dt(x), int(normalize_x), _p(W),
-          W.shape[0], _p(quant), N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm), _p(gx), _p(gW),
+          K, _p(quant), N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm), _p(gx), _p(gW),
           g_hw, _S)
     return gx, gW
 
@@ -420,17 +433,108 @@ def l2norm_backward(gy: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
 
 
 def scatter_stats(x: torch.Tensor, quant: torch.Tensor | None, K: int, *, normalize_x: bool = False,
-                  out: torch.Tensor | None = None, keys: torch.Tensor | None = None, key_offset: int = 0) -> torch.Tensor:
+                  out: torch.Tensor | None = None, keys: torch.Tensor | None = None, key_offset: int = 0,
+                  deterministic: bool | None = None) -> torch.Tensor:
     """fp32 [K*D + K] = per-code feature sums followed by per-code counts (one all-reduce buffer).  The code of a
-    token comes from `quant` (int64 indices) or straight from the packed `keys` of the assignment."""
+    token comes from `quant` (int64 indices) or straight from the packed `keys` of the assignment.
+    deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, the sums are formed by the code
+    sort + chunked segment sum (fixed association, see vqb_segment_sum_rows) instead of fp32 atomics."""
     lib = _lib.load()
     dev = _cuda(x, quant, out, keys)
     assert (quant is None) != (keys is None)
     N, D = x.shape
     stats = out if out is not None else torch.zeros((K * D + K,), dtype=torch.float32, device=x.device)
+    if deterministic_enabled(deterministic):
+        assert stats.dtype == torch.float32 and stats.numel() >= K * D + K
+        order, offsets = _code_sort_ws(dev, N, K, quant, keys, key_offset)
+        _segment_sum(dev, x, N, D, normalize_x, order, offsets, K, stats, stats[K * D:])
+        return stats
     _call('vqb_scatter_stats', lib.vqb_scatter_stats, dev, _p(x), _dt(x), N, D, int(normalize_x), _p(quant), _p(keys),
           key_offset, _p(stats), K, _S)
     return stats
+
+
+# ---- deterministic per-code reductions (csrc/segment.cu) ---------------------------------------------------------
+
+
+def deterministic_enabled(deterministic: bool | None = None) -> bool:
+    """The switch of the deterministic reductions: an explicit argument, else torch's own flag, read at call time."""
+    return torch.are_deterministic_algorithms_enabled() if deterministic is None else bool(deterministic)
+
+
+def segment_chunk() -> int:
+    """C of the segment-sum association contract (VQB_SEGMENT_CHUNK)."""
+    return int(_lib.load().vqb_segment_chunk())
+
+
+_DET_WS: dict = {}
+_DET_RETIRED: list = []
+
+
+def _det_ws(device, name: str, numel: int, dtype: torch.dtype) -> torch.Tensor:
+    """Scratch of the deterministic path, cached per (device, stream, name) like `_loss_ws`, so a captured CUDA graph
+    replays the same buffers.  Grows in powers of two; an outgrown buffer stays referenced because a graph captured
+    earlier may still read it."""
+    key = (device.index, torch.cuda.current_stream(device).cuda_stream, name)
+    buf = _DET_WS.get(key)
+    if buf is None or buf.numel() < numel:
+        if buf is not None:
+            _DET_RETIRED.append(buf)
+        buf = _DET_WS[key] = torch.empty((1 << max(numel - 1, 0).bit_length(),), dtype=dtype, device=device)
+    return buf[:numel]
+
+
+def _code_sort_call(dev, N: int, K: int, quant, keys, key_offset: int, order, offsets) -> None:
+    lib = _lib.load()
+    scratch = _det_ws(dev, 'sort', int(lib.vqb_code_sort_scratch_bytes(N, K)), torch.uint8)
+    _call('vqb_code_sort', lib.vqb_code_sort, dev, _p(quant), _p(keys), key_offset, N, K, _p(order), _p(offsets),
+          _p(scratch), scratch.numel(), _S)
+
+
+def _code_sort_ws(dev, N: int, K: int, quant, keys, key_offset: int):
+    order = _det_ws(dev, 'order', N, torch.int32)
+    offsets = _det_ws(dev, 'offsets', K + 1, torch.int32)
+    _code_sort_call(dev, N, K, quant, keys, key_offset, order, offsets)
+    return order, offsets
+
+
+def _segment_sum(dev, rows, N: int, D: int, normalize: bool, order, offsets, K: int, out_sums, out_counts) -> None:
+    lib = _lib.load()
+    scratch = _det_ws(dev, 'segment', int(lib.vqb_segment_sum_scratch_bytes(N, K, D)), torch.uint8)
+    _call('vqb_segment_sum_rows', lib.vqb_segment_sum_rows, dev, _p(rows), _dt(rows), N, D, int(normalize), _p(order),
+          _p(offsets), K, _p(out_sums), _p(out_counts), _p(scratch), scratch.numel(), _S)
+
+
+def code_sort(K: int, *, quant: torch.Tensor | None = None, keys: torch.Tensor | None = None,
+              key_offset: int = 0) -> tuple[torch.Tensor, torch.Tensor]:
+    """Stable sort of the tokens by code (vqb_code_sort) -> (order int32 [N], offsets int32 [K+1]): code k owns
+    order[offsets[k]:offsets[k+1]] in ascending token order; tokens whose code is outside [0, K) come last."""
+    dev = _cuda(quant, keys)
+    assert (quant is None) != (keys is None)
+    idx = quant if quant is not None else keys
+    assert idx.dtype == torch.int64
+    N = idx.numel()
+    order = torch.empty((N,), dtype=torch.int32, device=idx.device)
+    offsets = torch.empty((K + 1,), dtype=torch.int32, device=idx.device)
+    _code_sort_call(dev, N, K, quant, keys, key_offset, order, offsets)
+    return order, offsets
+
+
+def segment_sum_rows(rows: torch.Tensor, order: torch.Tensor, offsets: torch.Tensor, *, normalize: bool = False,
+                     out_sums: torch.Tensor | None = None, out_counts: torch.Tensor | None = None) -> torch.Tensor:
+    """out_sums fp32 [K, D] (+)= the per-code sums of `rows` (fp32 / bf16 [N, D]) in the fixed association of
+    vqb_segment_sum_rows; out_counts fp32 [K] (+)= the token counts.  Zero-filled outputs are allocated when omitted."""
+    dev = _cuda(rows, order, offsets, out_sums, out_counts)
+    assert order.dtype == torch.int32 and offsets.dtype == torch.int32 and rows.dim() == 2
+    N, D = rows.shape
+    K = offsets.numel() - 1
+    assert order.numel() == N
+    if out_sums is None:
+        out_sums = torch.zeros((K, D), dtype=torch.float32, device=rows.device)
+    assert out_sums.dtype == torch.float32 and out_sums.numel() == K * D
+    assert out_counts is None or (out_counts.dtype == torch.float32 and out_counts.numel() == K)
+    _segment_sum(dev, rows, N, D, normalize, order, offsets, K, out_sums, out_counts)
+    return out_sums
 
 
 def bincount_accumulate(quant: torch.Tensor, counts: torch.Tensor, K: int | None = None,
