@@ -29,7 +29,8 @@ extern "C" {
 #endif
 
 #define VQB200_ABI_VERSION 3 /* 2: fp16 plane formats, vqb_row_inv_norm(f16_rows), vqb_transpose_last2, vqb_compact_tokens; 3: vqb_comm_*, g_dtype of vqb_quantize_backward;
-                                3 (additive): vqb_segment_chunk, vqb_code_sort*, vqb_segment_sum_*, vqb_quantize_backward_rows */
+                                3 (additive): vqb_segment_chunk, vqb_code_sort*, vqb_segment_sum_*, vqb_quantize_backward_rows,
+                                vqb_decode_tokens, vqb_fsq_decode_tokens */
 
 typedef enum { VQB_OK = 0, VQB_ERR_ARG = -1, VQB_ERR_CUDA = -2, VQB_ERR_UNSUPPORTED = -3 } vqb_status;
 typedef enum { VQB_F32 = 0, VQB_BF16 = 1 } vqb_dtype;
@@ -333,6 +334,20 @@ int vqb_fsq_forward(const void* x, int x_dtype, int64_t N, const vqb_fsq_params*
 int vqb_fsq_backward(const void* gz, int g_dtype, const void* x, int x_dtype, int64_t N,
                      const vqb_fsq_params* p_host, void* gx, int gx_dtype, void* stream);
 int vqb_fsq_decode(const int32_t* index, int64_t N, const vqb_fsq_params* p_host, float* z_out, void* stream);
+
+/* ---- token ids -> NCHW latents ---------------------------------------------------------------- *
+ * Decode-only path of the tokenizer (decode_from_quant, vq/tasks/image_reconstruction/models.py:97-108):
+ * z[b][d][s] = W[id[b*hw + s]][d], written straight into the caller's NCHW layout ('b h w c -> b c h w' fused).
+ * ids: [batch * hw], id_bytes 2 (uint16), 4 (int32) or 8 (int64).  out_dtype VQB_F32 or VQB_BF16 (round to nearest even).
+ * An id outside [0, K) gives a NaN row (every channel); if bad_count is given (a device int, zeroed by the caller),
+ * it is incremented by the number of such tokens.  No fault, no clamping.  (vqb_embedding_gather and vqb_fsq_decode
+ * keep their clamp / wrap behaviour.) */
+int vqb_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const float* W, int64_t K, int D,
+                      void* z_out, int out_dtype, int* bad_count, void* stream);
+/* The same for FSQ's implicit codebook (fsq/quantizers.py:59-63,136-137): digits of the mixed-radix id, value
+ * digit / half - 1 evaluated exactly as vqb_fsq_decode does; valid ids are [0, prod(levels)). */
+int vqb_fsq_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_fsq_params* p_host,
+                          void* z_out, int out_dtype, int* bad_count, void* stream);
 
 /* ---- compatibility mode: the materialised distance matrix ---------------------------------- *
  * out[n, k] = torch.cdist(x, W)[n, k]  (cosine = 0)         vq/algorithms/vq/distances.py:28-32

@@ -96,6 +96,10 @@ SIGNATURES = {
     'vqb_fsq_backward': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, POINTER(FSQParams), c_void_p, c_int,
                                  c_void_p]),
     'vqb_fsq_decode': (c_int, [c_void_p, c_int64, POINTER(FSQParams), c_void_p, c_void_p]),
+    'vqb_decode_tokens': (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_int64, c_int, c_void_p, c_int, c_void_p,
+                                  c_void_p]),
+    'vqb_fsq_decode_tokens': (c_int, [c_void_p, c_int, c_int64, c_int64, POINTER(FSQParams), c_void_p, c_int, c_void_p,
+                                      c_void_p]),
     'vqb_distance_matrix': (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     'vqb_comm_alloc': (c_int, [c_size_t, POINTER(c_void_p), POINTER(c_ubyte)]),
     'vqb_comm_open': (c_int, [POINTER(c_ubyte), POINTER(c_void_p)]),

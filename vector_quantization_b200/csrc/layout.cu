@@ -80,6 +80,154 @@ __global__ void __launch_bounds__(256) transpose_last2_vec_kernel(const T* __res
   }
 }
 
+// ---- token ids -> NCHW latents (decode_from_quant, vq/tasks/image_reconstruction/models.py:97-108) ----------------
+// The transpose above with a different load stage: the "source row" of spatial position s is the codebook row of its
+// token id.  A row source provides
+//   int64_t code(int64_t n)    the id of token n if it is in [0, size), else -1
+//   float4 quad(code, c)       channels c .. c+3 of that code's row (channels >= D: any value; code -1: NaN)
+constexpr float kNaN = __builtin_nanf("");
+
+template <typename TI>
+__device__ __forceinline__ int64_t checked_id(const TI* __restrict__ ids, int64_t n, int64_t size) {
+  const int64_t id = (int64_t)ids[n];
+  return id >= 0 && id < size ? id : -1;
+}
+
+template <typename TI>
+struct VqRowSource {     // nn.Embedding: row = W[id] (fp32 [K, D])
+  const TI* __restrict__ ids;
+  const float* __restrict__ W;
+  int64_t K;
+  int D;
+  bool vec;              // D % 4 == 0 and W 16-byte aligned: every quad is one 16-byte load
+  __device__ __forceinline__ int64_t code(int64_t n) const { return checked_id(ids, n, K); }
+  __device__ __forceinline__ float4 quad(int64_t code, int c) const {
+    if (code < 0) return make_float4(kNaN, kNaN, kNaN, kNaN);
+    const float* row = W + code * D + c;
+    if (vec) return __ldg(reinterpret_cast<const float4*>(row));
+    float4 q;
+    q.x = __ldg(row);
+    q.y = c + 1 < D ? __ldg(row + 1) : 0.f;
+    q.z = c + 2 < D ? __ldg(row + 2) : 0.f;
+    q.w = c + 3 < D ? __ldg(row + 3) : 0.f;
+    return q;
+  }
+};
+
+template <typename TI>
+struct FsqRowSource {    // implicit FSQ codebook: digit d of the mixed-radix id, digit / half - 1 (as fsq_decode_kernel)
+  const TI* __restrict__ ids;
+  vqb_fsq_params p;
+  int64_t size;          // prod(levels)
+  __device__ __forceinline__ int64_t code(int64_t n) const { return checked_id(ids, n, size); }
+  __device__ __forceinline__ float value(int id, int d) const {
+    if (d >= p.D) return 0.f;
+    const int digit = (id / p.cumprod[d]) % p.levels[d];                 // fsq/quantizers.py:59-63
+    return __fsub_rn(__fdiv_rn((float)digit, p.half[d]), 1.f);           // :137
+  }
+  __device__ __forceinline__ float4 quad(int64_t code, int c) const {
+    if (code < 0) return make_float4(kNaN, kNaN, kNaN, kNaN);
+    const int id = (int)code;                                              // size < 2^31
+    return make_float4(value(id, c), value(id, c + 1), value(id, c + 2), value(id, c + 3));
+  }
+};
+
+// z[b][d][s] = row(id[b * hw + s])[d].  Block = one band of TS spatial positions of one image (blockIdx.x) and a
+// stride over the channel tiles of TD channels (blockIdx.y, gridDim.y); the rows go through an fp32 shared tile
+// and leave as 16-byte stores along hw.  Stores fall back to scalar ones where hw is not a multiple of the vector
+// (or z is not 16-byte aligned).  Each block reads its band's ids once; blockIdx.y == 0 counts the bad ones.
+template <class Src, typename TO, int TS, int TD>
+__global__ void __launch_bounds__(256) decode_tokens_kernel(const Src src, int64_t hw, int64_t bands_per_image, int D,
+                                                            TO* __restrict__ z, bool vec_store, int* __restrict__ bad_count) {
+  constexpr int VE = 16 / sizeof(TO);          // output elements per 16-byte store
+  constexpr int QPR = TD / 4;                  // quads per tile row
+  constexpr int VPC = TS / VE;                 // vectors per output row of the tile
+  static_assert(TD % 4 == 0 && TS % VE == 0, "tile shape");
+  static_assert(TS <= 256, "one id per thread: __syncthreads_count then sums the bad ids");
+  __shared__ float tile[TS][TD + 1];           // +1: conflict-free column reads in the store stage
+  __shared__ int64_t codes[TS];
+  const int64_t b = (int64_t)blockIdx.x / bands_per_image;
+  const int64_t s0 = ((int64_t)blockIdx.x - b * bands_per_image) * TS;
+  const int ns = (int)min((int64_t)TS, hw - s0);
+  int bad = 0;
+  for (int r = threadIdx.x; r < TS; r += 256) {
+    const int64_t c = r < ns ? src.code(b * hw + s0 + r) : 0;
+    codes[r] = c;
+    bad += c < 0;
+  }
+  bad = __syncthreads_count(bad);              // also publishes codes[]
+  if (bad && blockIdx.y == 0 && threadIdx.x == 0 && bad_count) atomicAdd(bad_count, bad);
+  TO* __restrict__ zb = z + b * D * hw;
+  for (int c0 = blockIdx.y * TD; c0 < D; c0 += gridDim.y * TD) {
+    for (int v = threadIdx.x; v < TS * QPR; v += 256) {
+      const int r = v / QPR, cq = (v % QPR) * 4;
+      if (r < ns && c0 + cq < D) {
+        const float4 q = src.quad(codes[r], c0 + cq);
+        tile[r][cq] = q.x;
+        tile[r][cq + 1] = q.y;
+        tile[r][cq + 2] = q.z;
+        tile[r][cq + 3] = q.w;
+      }
+    }
+    __syncthreads();
+    // same store order as transpose_last2_vec_kernel: lanes along one output row when it is short (VPC <= 8)
+    for (int v = threadIdx.x; v < TD * VPC; v += 256) {
+      const int rv = (VPC <= 8 ? v % VPC : v / TD) * VE, c = VPC <= 8 ? v / VPC : v % TD;
+      if (c0 + c < D && rv < ns) {
+        TO* out = zb + (int64_t)(c0 + c) * hw + s0 + rv;
+        if (vec_store && rv + VE <= ns) {
+          uint4 raw;
+          TO* e = reinterpret_cast<TO*>(&raw);
+#pragma unroll
+          for (int i = 0; i < VE; ++i) e[i] = from_f32<TO>(tile[rv + i][c]);
+          *reinterpret_cast<uint4*>(out) = raw;
+        } else {
+          for (int i = 0; i < VE && rv + i < ns; ++i) out[i] = from_f32<TO>(tile[rv + i][c]);
+        }
+      }
+    }
+    __syncthreads();
+  }
+}
+
+template <int TS, int TD, class Src>
+static int launch_decode_tokens(const Src& src, int64_t batch, int64_t hw, int D, void* z, int out_dtype, int* bad,
+                                cudaStream_t st) {
+  const int64_t per_image = (hw + TS - 1) / TS, bands = per_image * batch;
+  VQB_REQUIRE(bands <= 0x7fffffff, "decode_tokens: too many tokens (batch * ceil(hw / %d) must be < 2^31)", TS);
+  const int64_t ct = (D + TD - 1) / TD;
+  int64_t gy = ((int64_t)sm_count() * 16 + bands - 1) / bands;   // enough blocks for ~2 waves, as the transpose
+  gy = gy > ct ? ct : (gy < 1 ? 1 : gy);
+  const dim3 grid((unsigned)bands, (unsigned)gy);
+  const int ve = out_dtype == VQB_F32 ? 4 : 8;
+  const bool vec_store = hw % ve == 0 && (uintptr_t)z % 16 == 0;
+  if (out_dtype == VQB_F32)
+    decode_tokens_kernel<Src, float, TS, TD><<<grid, 256, 0, st>>>(src, hw, per_image, D, (float*)z, vec_store, bad);
+  else
+    decode_tokens_kernel<Src, __nv_bfloat16, TS, TD><<<grid, 256, 0, st>>>(src, hw, per_image, D, (__nv_bfloat16*)z,
+                                                                           vec_store, bad);
+  VQB_LAUNCH_OK();
+  return VQB_OK;
+}
+
+// tile shape follows the row width, as in vqb_transpose_last2: narrow rows (LlamaGen's 8, FSQ's 5-6) get a narrow tile
+template <class Src>
+static int launch_decode_tokens_for_width(const Src& src, int64_t batch, int64_t hw, int D, void* z, int out_dtype,
+                                          int* bad, cudaStream_t st) {
+  if (D <= 16) return launch_decode_tokens<128, 16>(src, batch, hw, D, z, out_dtype, bad, st);
+  if (D <= 32) return launch_decode_tokens<64, 32>(src, batch, hw, D, z, out_dtype, bad, st);
+  return launch_decode_tokens<32, 64>(src, batch, hw, D, z, out_dtype, bad, st);
+}
+
+static int check_decode_args(const char* fn, const void* ids, int id_bytes, int64_t batch, int64_t hw, const void* z,
+                             int out_dtype) {
+  VQB_REQUIRE(ids && z, "%s: null pointer", fn);
+  VQB_REQUIRE(id_bytes == 2 || id_bytes == 4 || id_bytes == 8, "%s: id_bytes must be 2 (uint16), 4 (int32) or 8 (int64)", fn);
+  VQB_REQUIRE(out_dtype == VQB_F32 || out_dtype == VQB_BF16, "%s: out_dtype must be VQB_F32 or VQB_BF16", fn);
+  VQB_REQUIRE(batch >= 0 && hw >= 0, "%s: bad shape", fn);
+  return VQB_OK;
+}
+
 template <typename TO>
 __global__ void compact_tokens_kernel(const unsigned long long* __restrict__ keys, int64_t n, int64_t offset,
                                       TO* __restrict__ out) {
@@ -177,6 +325,48 @@ int vqb_compact_tokens(const unsigned long long* keys, int64_t n, int64_t index_
   else compact_tokens_kernel<int32_t><<<blocks, 256, 0, st>>>(keys, n, index_offset, (int32_t*)out);
   VQB_LAUNCH_OK();
   return VQB_OK;
+}
+
+int vqb_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const float* W, int64_t K, int D,
+                      void* z_out, int out_dtype, int* bad_count, void* stream) {
+  if (int e = check_decode_args("vqb_decode_tokens", ids, id_bytes, batch, hw, z_out, out_dtype)) return e;
+  VQB_REQUIRE(W, "vqb_decode_tokens: null pointer");
+  VQB_REQUIRE(K >= 1 && D >= 1, "vqb_decode_tokens: bad codebook shape");
+  if (batch == 0 || hw == 0) return VQB_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool vec = D % 4 == 0 && (uintptr_t)W % 16 == 0;
+  if (id_bytes == 2)
+    return launch_decode_tokens_for_width(VqRowSource<uint16_t>{(const uint16_t*)ids, W, K, D, vec}, batch, hw, D, z_out,
+                                          out_dtype, bad_count, st);
+  if (id_bytes == 4)
+    return launch_decode_tokens_for_width(VqRowSource<int32_t>{(const int32_t*)ids, W, K, D, vec}, batch, hw, D, z_out,
+                                          out_dtype, bad_count, st);
+  return launch_decode_tokens_for_width(VqRowSource<int64_t>{(const int64_t*)ids, W, K, D, vec}, batch, hw, D, z_out,
+                                        out_dtype, bad_count, st);
+}
+
+int vqb_fsq_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_fsq_params* p_host,
+                          void* z_out, int out_dtype, int* bad_count, void* stream) {
+  if (int e = check_decode_args("vqb_fsq_decode_tokens", ids, id_bytes, batch, hw, z_out, out_dtype)) return e;
+  VQB_REQUIRE(p_host, "vqb_fsq_decode_tokens: null params");
+  VQB_REQUIRE(p_host->D >= 1 && p_host->D <= 16, "vqb_fsq_decode_tokens: D must be in 1..16 (got %d)", p_host->D);
+  int64_t size = 1;
+  for (int d = 0; d < p_host->D && size <= 0x7fffffff; ++d) {
+    VQB_REQUIRE(p_host->levels[d] >= 1, "vqb_fsq_decode_tokens: levels must be >= 1");
+    size *= p_host->levels[d];
+  }
+  VQB_REQUIRE(size <= 0x7fffffff, "vqb_fsq_decode_tokens: codebook size must be below 2^31");
+  if (batch == 0 || hw == 0) return VQB_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = p_host->D;    // <= 16: one 128 x 16 tile shape
+  if (id_bytes == 2)
+    return launch_decode_tokens<128, 16>(FsqRowSource<uint16_t>{(const uint16_t*)ids, *p_host, size}, batch, hw, D, z_out,
+                                         out_dtype, bad_count, st);
+  if (id_bytes == 4)
+    return launch_decode_tokens<128, 16>(FsqRowSource<int32_t>{(const int32_t*)ids, *p_host, size}, batch, hw, D, z_out,
+                                         out_dtype, bad_count, st);
+  return launch_decode_tokens<128, 16>(FsqRowSource<int64_t>{(const int64_t*)ids, *p_host, size}, batch, hw, D, z_out,
+                                       out_dtype, bad_count, st);
 }
 
 }  // extern "C"

@@ -20,7 +20,7 @@ __all__ = [
     'quantize_backward', 'l2norm_forward', 'l2norm_backward', 'scatter_stats', 'bincount_accumulate',
     'deterministic_enabled', 'segment_chunk', 'code_sort', 'segment_sum_rows',
     'kmeans_ema_update', 'gather_rows_by_key', 'cvq_update', 'embedding_gather', 'fsq_params', 'fsq_forward', 'fsq_backward',
-    'fsq_decode', 'transpose_last2', 'compact_tokens', 'distance_matrix', 'comm_kmeans_ema_update', 'comm_cvq_update',
+    'fsq_decode', 'decode_tokens', 'fsq_decode_tokens', 'transpose_last2', 'compact_tokens', 'distance_matrix', 'comm_kmeans_ema_update', 'comm_cvq_update',
     'comm_allreduce_min_keys', 'comm_allreduce_sum_f32', 'BACKEND_TCGEN05', 'BACKEND_SIMT',
 ]
 
@@ -707,3 +707,50 @@ def fsq_decode(index: torch.Tensor, p: FSQParams) -> torch.Tensor:
     z = torch.empty((flat.numel(), p.D), dtype=torch.float32, device=index.device)
     _call('vqb_fsq_decode', lib.vqb_fsq_decode, dev, _p(flat), flat.numel(), ctypes.byref(p), _p(z), _S)
     return z.reshape(*index.shape, p.D)
+
+
+# ---- token ids -> NCHW latents (csrc/layout.cu) -------------------------------------------------------------------
+_ID_BYTES = {torch.uint16: 2, torch.int32: 4, torch.int64: 8}
+
+
+def _decode_out(ids: torch.Tensor, hw: int, D: int, out_dtype: torch.dtype, bad_count: torch.Tensor | None):
+    """Checks the ids / counter of a decode_tokens call; returns (b, id_bytes, z) with z = empty [b, D, *spatial]."""
+    if ids.dtype not in _ID_BYTES:
+        raise TypeError(f'token ids must be uint16, int32 or int64, got {ids.dtype}')
+    if out_dtype not in (torch.float32, torch.bfloat16):
+        raise TypeError(f'out_dtype must be float32 or bfloat16, got {out_dtype}')
+    if bad_count is not None and (bad_count.dtype != torch.int32 or bad_count.numel() != 1):
+        raise TypeError('bad_count must be a one-element int32 tensor')
+    n = ids.numel()
+    if hw <= 0 or n % hw:
+        raise ValueError(f'{n} token ids do not split into images of hw = {hw} tokens')
+    b = n // hw
+    spatial = tuple(ids.shape[1:]) if ids.dim() >= 2 and ids.shape[0] == b else (hw,)
+    return b, _ID_BYTES[ids.dtype], torch.empty((b, D) + spatial, dtype=out_dtype, device=ids.device)
+
+
+def decode_tokens(W: torch.Tensor, ids: torch.Tensor, hw: int, out_dtype: torch.dtype = torch.float32,
+                  bad_count: torch.Tensor | None = None) -> torch.Tensor:
+    """Token ids [b, h, w] (uint16 / int32 / int64, b * hw in all) -> z = W[ids] as [b, D, h, w] of `out_dtype`, in one
+    launch (vqb_decode_tokens).  An id outside [0, K) gives a NaN row and is counted into `bad_count` (a zeroed
+    one-element int32 device tensor) when one is given."""
+    lib = _lib.load()
+    dev = _cuda(W, ids, bad_count)
+    if W.dtype != torch.float32 or W.dim() != 2:
+        raise TypeError('the codebook must be a float32 [K, D] tensor')
+    K, D = W.shape
+    b, id_bytes, z = _decode_out(ids, hw, D, out_dtype, bad_count)
+    _call('vqb_decode_tokens', lib.vqb_decode_tokens, dev, _p(ids), id_bytes, b, hw, _p(W), K, D, _p(z), _dt(z),
+          _p(bad_count), _S)
+    return z
+
+
+def fsq_decode_tokens(ids: torch.Tensor, p: FSQParams, hw: int, out_dtype: torch.dtype = torch.float32,
+                      bad_count: torch.Tensor | None = None) -> torch.Tensor:
+    """decode_tokens for FSQ's implicit codebook: valid ids are [0, prod(levels)) (vqb_fsq_decode_tokens)."""
+    lib = _lib.load()
+    dev = _cuda(ids, bad_count)
+    b, id_bytes, z = _decode_out(ids, hw, p.D, out_dtype, bad_count)
+    _call('vqb_fsq_decode_tokens', lib.vqb_fsq_decode_tokens, dev, _p(ids), id_bytes, b, hw, ctypes.byref(p), _p(z),
+          _dt(z), _p(bad_count), _S)
+    return z

@@ -1,7 +1,8 @@
 """The callers and data formats either side of the quantizer (SURVEY.md §8f items 1 and 3).
 
 Reference: `BaseModel.quantize` / `encode_to_quant` (vq/tasks/image_tokenization/models/base.py:116-146) hand
-the quantizer NCHW encoder features; `TokenizeCallback` (runners/callbacks.py:29-53) and
+the quantizer NCHW encoder features; `decode_from_quant` (vq/tasks/image_reconstruction/models.py:97-108) turns
+token grids back into NCHW decoder input; `TokenizeCallback` (runners/callbacks.py:29-53) and
 `tools/tokenize_llamagen.py:93-103` write the resulting token grids to disk.  The functions here take the
 quantizer (not a whole tokenizer model: encoders/decoders are out of scope) and reproduce those contracts —
 memo keys, shapes, dtypes, file formats — with the layout changes done by the transpose kernel of the C-ABI
@@ -16,9 +17,10 @@ import torch
 
 from . import functional as Fq
 from . import ops
-from .quantizers import VectorQuantizer, get_memo
+from ._lib import VQBError
+from .quantizers import FiniteScalarQuantizer, VectorQuantizer, get_memo
 
-__all__ = ['quantize', 'encode_to_quant', 'save_tokens', 'load_tokens', 'save_llamagen_codes', 'TokenStreamWriter']
+__all__ = ['quantize', 'encode_to_quant', 'decode_from_quant', 'save_tokens', 'load_tokens', 'save_llamagen_codes', 'TokenStreamWriter']
 
 
 def quantize(quantizer, x: torch.Tensor, memo: dict):
@@ -61,6 +63,64 @@ def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = F
         quant = quant.to(torch.int32)
     quantizer_memo.update(x=rows, quant=quant)
     return quant.view(b, h, w), memo
+
+
+def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torch.dtype = torch.float32,
+                      check: bool = True):
+    """`decode_from_quant` before the decoder (vq/tasks/image_reconstruction/models.py:97-108): token ids
+    quant [b, h, w] -> (z [b, c, h, w] contiguous of `dtype`, memo) with memo['quantizer'] = the quantizer's memo as
+    `quantizer.decode` leaves it.  quant is uint16, int32 or int64 on the GPU: what `encode_to_quant` (compact or not)
+    and FSQ produce, or a `load_tokens` dump moved to the device.  The codebook is used as stored (no before_encode).
+
+    A VectorQuantizer or FiniteScalarQuantizer without before_decode / after_decode hooks decodes in ONE launch that
+    reads the ids as they are and writes NCHW `dtype` directly.  Hooks, or a codebook that requires grad with grad
+    enabled, take `quantizer.decode` (hooks honoured, differentiable gather) + the transpose + a cast instead; on
+    valid ids both give the same values.
+
+    An id outside [0, codebook_size) is an error: with check=True (one 4-byte device-to-host read) it raises
+    IndexError with the number of such tokens.  check=False does not synchronise (safe inside a CUDA graph capture)
+    and, on the one-launch path, decodes such tokens to NaN in every channel."""
+    if quant.dim() != 3:
+        raise ValueError(f'expected token ids of shape [b, h, w], got {tuple(quant.shape)}')
+    if not quant.is_cuda:
+        raise VQBError('vector_quantization_b200 decodes CUDA (sm_100a) token ids only; there is no CPU fallback')
+    if dtype not in (torch.float32, torch.bfloat16):
+        raise TypeError(f'dtype must be float32 or bfloat16, got {dtype}')
+    b, h, w = quant.shape
+    quantizer_memo = get_memo(memo, 'quantizer')
+    fsq = isinstance(quantizer, FiniteScalarQuantizer)
+    hooked = any(quantizer._callbacks.overrides(hook) for hook in ('before_decode', 'after_decode'))
+    if isinstance(quantizer, VectorQuantizer):
+        W = quantizer._weight()
+        fused = not hooked and not (torch.is_grad_enabled() and W.requires_grad)
+    else:
+        # FiniteScalarQuantizer.decode returns the encode memo's z when there is one: leave that case to it
+        fused = fsq and not hooked and 'z' not in quantizer_memo.get('encode', {})
+    quant = quant.contiguous()
+    if fused:
+        bad = torch.zeros(1, dtype=torch.int32, device=quant.device) if check else None
+        if fsq:
+            get_memo(quantizer_memo, 'encode')
+            z = ops.fsq_decode_tokens(quant, quantizer._params, h * w, dtype, bad)
+        else:
+            z = ops.decode_tokens(W.detach(), quant, h * w, dtype, bad)
+        get_memo(quantizer_memo, 'decode')
+        if check:
+            _raise_bad_ids(int(bad.item()), quantizer.codebook_size)
+        return z, memo
+    wide = quant.to(torch.int32) if quant.dtype == torch.uint16 else quant     # uint16 has no CUDA comparisons
+    wide = wide.to(torch.int32 if fsq else torch.int64)
+    if check:
+        K = quantizer.codebook_size
+        _raise_bad_ids(int(((wide < 0) | (wide >= K)).sum()), K)
+    z, memo['quantizer'] = quantizer.decode(wide, quantizer_memo)
+    z = Fq.rows_to_nchw(z, b, z.shape[-1], h, w)
+    return (z if z.dtype == dtype else z.to(dtype)), memo
+
+
+def _raise_bad_ids(count: int, codebook_size: int) -> None:
+    if count:
+        raise IndexError(f'{count} token id(s) outside [0, {codebook_size}): not in the codebook')
 
 
 def save_tokens(path: str | pathlib.Path, id_: Sequence[Any], category: torch.Tensor, quant: torch.Tensor,
