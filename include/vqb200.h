@@ -244,6 +244,45 @@ int vqb_quantize_backward_rows(const void* g_zste, int g_dtype, const void* x, i
                                const float* g_codebook_norm, const float* g_commitment_norm,
                                int want_norm_mse, void* gx_out, float* gW_rows, int64_t g_hw, void* stream);
 
+/* ---- residual quantization (RQ-VAE: L codebooks, level l quantizes what levels 1..l-1 left over) ------------ *
+ *   r_0 = x;  e_l = W_l[q_l];  zhat_1 = e_1, zhat_l = zhat_{l-1} + e_l;  r_l = r_{l-1} - e_l   (fp32 add / subtract,
+ *   never fused into an FMA);  z = x + (zhat_L - x) (straight-through to x over the whole depth).
+ * Level l's four MSE terms compare e_l with r_{l-1} exactly as vqb_gather_ste_loss compares W[q] with x, so L = 1
+ * gives bit for bit the results of vqb_gather_ste_loss / vqb_quantize_backward.  The per-level pointers travel BY
+ * VALUE (the struct is copied into the kernel parameters): no device pointer table, no host-to-device copy. */
+#define VQB_MAX_LEVELS 16
+typedef struct {
+  int L;                                   /* 1 .. VQB_MAX_LEVELS */
+  const float* W[VQB_MAX_LEVELS];          /* level codebooks, fp32 [K, D] each (the same K and D at every level) */
+  float* gW[VQB_MAX_LEVELS];               /* backward: gW_l accumulators (pre-zeroed; NULL = not wanted), or the
+                                              level's fp32 [N, D] rows of the _rows variant */
+  const float* g[VQB_MAX_LEVELS][4];       /* backward: DEVICE scalars g_codebook, g_commitment, g_codebook_norm,
+                                              g_commitment_norm of level l (NULL = 0) */
+} vqb_residual_levels;
+/* One level: reads r_{l-1} (r_dtype: x's dtype at level 0, VQB_F32 after), the level's keys or indices and W_l[q];
+ * writes quant_out[n*L + level] (optional; the [N, L] code layout), and
+ *   level < L-1 (r_out != NULL): zhat (fp32 [N, D], written at level 0, updated in place after) and r_out = r_l;
+ *   level = L-1 (r_out == NULL): z_out = x + (zhat_L - x) (optional; token-major, or NCHW with z_hw > 0 as in
+ *                                vqb_gather_ste_loss); zhat is read, not written.
+ * mse4_out: this level's four terms (deterministic two-stage sum; partials / ticket as for vqb_gather_ste_loss). */
+int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N, int D,
+                      const float* W, int64_t K, const int64_t* quant, const unsigned long long* keys,
+                      int64_t key_index_offset, int64_t* quant_out, int L, int level, float* zhat, float* r_out,
+                      float* z_out, int64_t z_hw, int want_norm_mse, float* mse4_out, float* partials,
+                      unsigned int* ticket, void* stream);
+/* The whole depth's backward in ONE launch.  Per token r_{l-1} is recomputed with the forward's operations (bit
+ * identical), then  gx = g_z + sum_l [commitment-role terms of level l]  (x dtype) and  gW_l[q_l] += [codebook-role
+ * row of level l]  (fp32 vector atomics), each term as in vqb_quantize_backward with (x, W) = (r_{l-1}, W_l).
+ * quant: int64 [N, L].  g_hw as in vqb_quantize_backward. */
+int vqb_residual_backward(const void* g_z, int g_dtype, const void* x, int x_dtype, const vqb_residual_levels* levels,
+                          int64_t K, const int64_t* quant, int64_t N, int D, int want_norm_mse, void* gx_out,
+                          int64_t g_hw, void* stream);
+/* The same with level l's codebook-gradient rows STORED to levels->gW[l] (fp32 [N, D] each; gx identical): their
+ * vqb_segment_sum_rows, level by level, is a deterministic gW_l. */
+int vqb_residual_backward_rows(const void* g_z, int g_dtype, const void* x, int x_dtype,
+                               const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
+                               int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
+
 /* ---- row l2-normalisation (NormalizeCallback.before_encode on x) ------------------------ *
  * vq/algorithms/vq/callbacks/normalize.py:24  — forward y = x / max(||x||, 1e-12); backward
  * gx = (gy - (gy.y) y) / max(||x||, 1e-12). */
@@ -348,6 +387,12 @@ int vqb_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, 
  * digit / half - 1 evaluated exactly as vqb_fsq_decode does; valid ids are [0, prod(levels)). */
 int vqb_fsq_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_fsq_params* p_host,
                           void* z_out, int out_dtype, int* bad_count, void* stream);
+/* The same for residual codes: ids [batch * hw, L] (a token's L ids contiguous), z[b][d][s] = sum_l W_l[id_l][d]
+ * with the fp32 adds of zhat in vqb_residual_step (level order).  An id outside [0, K) at ANY level gives a NaN row
+ * and counts the token once.  Only levels->L and levels->W are read. */
+int vqb_decode_residual_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw,
+                               const vqb_residual_levels* levels, int64_t K, int D, void* z_out, int out_dtype,
+                               int* bad_count, void* stream);
 
 /* ---- compatibility mode: the materialised distance matrix ---------------------------------- *
  * out[n, k] = torch.cdist(x, W)[n, k]  (cosine = 0)         vq/algorithms/vq/distances.py:28-32

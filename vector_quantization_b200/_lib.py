@@ -33,6 +33,15 @@ class FSQParams(Structure):
                 ('half', c_float * 16), ('cumprod', c_int * 16), ('levels', c_int * 16)]
 
 
+MAX_LEVELS = 16   # VQB_MAX_LEVELS
+
+
+class ResidualLevels(Structure):
+    """vqb_residual_levels: the per-level device pointers, passed by value into the kernels."""
+    _fields_ = [('L', c_int), ('W', c_void_p * MAX_LEVELS), ('gW', c_void_p * MAX_LEVELS),
+                ('g', (c_void_p * 4) * MAX_LEVELS)]
+
+
 # name -> (restype, argtypes); must list EVERY symbol declared in include/vqb200.h
 # (tests/test_abi.py parses the header and checks this table and the .so against it).
 SIGNATURES = {
@@ -74,6 +83,13 @@ SIGNATURES = {
     'vqb_quantize_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p, c_int64,
                                            c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64,
                                            c_void_p]),
+    'vqb_residual_step': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_int, c_void_p, c_int64, c_void_p, c_void_p,
+                                  c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p,
+                                  c_void_p, c_void_p, c_void_p]),
+    'vqb_residual_backward': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
+                                      c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_residual_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
+                                           c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_segment_chunk': (c_int64, []),
     'vqb_code_sort_scratch_bytes': (c_size_t, [c_int64, c_int64]),
     'vqb_code_sort': (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_size_t,
@@ -100,6 +116,8 @@ SIGNATURES = {
                                   c_void_p]),
     'vqb_fsq_decode_tokens': (c_int, [c_void_p, c_int, c_int64, c_int64, POINTER(FSQParams), c_void_p, c_int, c_void_p,
                                       c_void_p]),
+    'vqb_decode_residual_tokens': (c_int, [c_void_p, c_int, c_int64, c_int64, POINTER(ResidualLevels), c_int64, c_int,
+                                           c_void_p, c_int, c_void_p, c_void_p]),
     'vqb_distance_matrix': (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     'vqb_comm_alloc': (c_int, [c_size_t, POINTER(c_void_p), POINTER(c_ubyte)]),
     'vqb_comm_open': (c_int, [POINTER(c_ubyte), POINTER(c_void_p)]),

@@ -132,6 +132,51 @@ struct FsqRowSource {    // implicit FSQ codebook: digit d of the mixed-radix id
   }
 };
 
+template <typename TI>
+struct ResidualRowSource {   // RQ-VAE codes: token n's ids are ids[n*L .. n*L + L); row = sum_l W_l[id_l], level order
+  const TI* __restrict__ ids;
+  const float* W[VQB_MAX_LEVELS];   // indexed with unrolled constants only: the struct stays in the parameter bank
+  int L;
+  int64_t K;
+  int D;
+  bool vec;                  // D % 4 == 0 and every W_l 16-byte aligned
+  __device__ __forceinline__ int64_t code(int64_t n) const {   // n when all L ids are in [0, K), else -1
+    bool ok = true;
+#pragma unroll
+    for (int l = 0; l < VQB_MAX_LEVELS; ++l)
+      if (l < L) ok = ok && checked_id(ids, n * L + l, K) >= 0;
+    return ok ? n : -1;
+  }
+  __device__ __forceinline__ float4 quad(int64_t code, int c) const {
+    if (code < 0) return make_float4(kNaN, kNaN, kNaN, kNaN);
+    float4 s;
+#pragma unroll
+    for (int l = 0; l < VQB_MAX_LEVELS; ++l) {
+      if (l < L) {
+        const float* row = W[l] + (int64_t)ids[code * L + l] * D + c;
+        float4 q;
+        if (vec) {
+          q = __ldg(reinterpret_cast<const float4*>(row));
+        } else {
+          q.x = __ldg(row);
+          q.y = c + 1 < D ? __ldg(row + 1) : 0.f;
+          q.z = c + 2 < D ? __ldg(row + 2) : 0.f;
+          q.w = c + 3 < D ? __ldg(row + 3) : 0.f;
+        }
+        if (l == 0) {
+          s = q;
+        } else {    // the running sum of vqb_residual_step: one round-to-nearest add per level
+          s.x = __fadd_rn(s.x, q.x);
+          s.y = __fadd_rn(s.y, q.y);
+          s.z = __fadd_rn(s.z, q.z);
+          s.w = __fadd_rn(s.w, q.w);
+        }
+      }
+    }
+    return s;
+  }
+};
+
 // z[b][d][s] = row(id[b * hw + s])[d].  Block = one band of TS spatial positions of one image (blockIdx.x) and a
 // stride over the channel tiles of TD channels (blockIdx.y, gridDim.y); the rows go through an fp32 shared tile
 // and leave as 16-byte stores along hw.  Stores fall back to scalar ones where hw is not a multiple of the vector
@@ -343,6 +388,35 @@ int vqb_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, 
                                           out_dtype, bad_count, st);
   return launch_decode_tokens_for_width(VqRowSource<int64_t>{(const int64_t*)ids, W, K, D, vec}, batch, hw, D, z_out,
                                         out_dtype, bad_count, st);
+}
+
+int vqb_decode_residual_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_residual_levels* lv,
+                               int64_t K, int D, void* z_out, int out_dtype, int* bad_count, void* stream) {
+  if (int e = check_decode_args("vqb_decode_residual_tokens", ids, id_bytes, batch, hw, z_out, out_dtype)) return e;
+  VQB_REQUIRE(lv, "vqb_decode_residual_tokens: null levels");
+  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "vqb_decode_residual_tokens: L=%d outside [1, %d]", lv->L,
+              VQB_MAX_LEVELS);
+  VQB_REQUIRE(K >= 1 && D >= 1, "vqb_decode_residual_tokens: bad codebook shape");
+  bool aligned = true;
+  for (int l = 0; l < lv->L; ++l) {
+    VQB_REQUIRE(lv->W[l], "vqb_decode_residual_tokens: null codebook at level %d", l);
+    aligned = aligned && (uintptr_t)lv->W[l] % 16 == 0;
+  }
+  if (batch == 0 || hw == 0) return VQB_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool vec = D % 4 == 0 && aligned;
+#define VQB_RESIDUAL_SRC(TI_) \
+  ResidualRowSource<TI_> src{(const TI_*)ids, {}, lv->L, K, D, vec};                                                  \
+  for (int l = 0; l < lv->L; ++l) src.W[l] = lv->W[l];                                                               \
+  return launch_decode_tokens_for_width(src, batch, hw, D, z_out, out_dtype, bad_count, st);
+  if (id_bytes == 2) {
+    VQB_RESIDUAL_SRC(uint16_t)
+  }
+  if (id_bytes == 4) {
+    VQB_RESIDUAL_SRC(int32_t)
+  }
+  VQB_RESIDUAL_SRC(int64_t)
+#undef VQB_RESIDUAL_SRC
 }
 
 int vqb_fsq_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_fsq_params* p_host,

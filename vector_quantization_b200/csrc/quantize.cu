@@ -90,6 +90,43 @@ __device__ __forceinline__ void block_sum2(float& a, float& b, float* sh /* >= 2
   }
 }
 
+// ---- the loss tail shared by the forward kernels -----------------------------------------------------------------
+// Block sums of (sse, sse_n), then the deterministic two-stage fold into mse4[0..3].
+__device__ __forceinline__ void finish_mse4(float sse, float sse_n, int64_t N, int D, float* __restrict__ mse4,
+                                            float* __restrict__ partials, unsigned int* __restrict__ ticket,
+                                            float* sh) {
+  block_sum2(sse, sse_n, sh);
+  // Only warp 0 stays for the ticket: the other warps retire without waiting for the fence, and the last
+  // block's warp 0 alone folds the per-block partials (fixed assignment and tree order -> deterministic).
+  if (threadIdx.x >= 32) return;
+  unsigned int t = 0;
+  if (threadIdx.x == 0) {
+    partials[blockIdx.x] = sse;
+    partials[kMaxPartials + blockIdx.x] = sse_n;
+    __threadfence();
+    t = atomicAdd(ticket, 1u);
+  }
+  t = __shfl_sync(0xffffffffu, t, 0);
+  if (t == gridDim.x - 1) {
+    __threadfence();
+    float a = 0.f, b = 0.f;
+    for (int i = threadIdx.x; i < (int)gridDim.x; i += 32) {
+      a += __ldcg(partials + i);
+      b += __ldcg(partials + kMaxPartials + i);
+    }
+    a = warp_sum(a);
+    b = warp_sum(b);
+    if (threadIdx.x == 0) {
+      const float inv = 1.f / ((float)N * (float)D);
+      mse4[0] = a * inv;
+      mse4[1] = a * inv;
+      mse4[2] = b * inv;
+      mse4[3] = b * inv;
+      *ticket = 0u;  // self-reset for the next launch
+    }
+  }
+}
+
 __device__ __forceinline__ int64_t row_index(const int64_t* __restrict__ quant,
                                              const unsigned long long* __restrict__ keys, int64_t n,
                                              int64_t key_offset, int64_t K) {
@@ -183,36 +220,7 @@ __global__ void __launch_bounds__(256) quantize_forward_kernel(
     }
     if (quant_out && valid && lane == 0) quant_out[n] = q;
   }
-  block_sum2(sse, sse_n, sh);
-  // Only warp 0 stays for the ticket: the other warps retire without waiting for the fence, and the last
-  // block's warp 0 alone folds the per-block partials (fixed assignment and tree order -> deterministic).
-  if (threadIdx.x >= 32) return;
-  unsigned int t = 0;
-  if (threadIdx.x == 0) {
-    partials[blockIdx.x] = sse;
-    partials[kMaxPartials + blockIdx.x] = sse_n;
-    __threadfence();
-    t = atomicAdd(ticket, 1u);
-  }
-  t = __shfl_sync(0xffffffffu, t, 0);
-  if (t == gridDim.x - 1) {
-    __threadfence();
-    float a = 0.f, b = 0.f;
-    for (int i = threadIdx.x; i < (int)gridDim.x; i += 32) {
-      a += __ldcg(partials + i);
-      b += __ldcg(partials + kMaxPartials + i);
-    }
-    a = warp_sum(a);
-    b = warp_sum(b);
-    if (threadIdx.x == 0) {
-      const float inv = 1.f / ((float)N * (float)D);
-      mse4[0] = a * inv;
-      mse4[1] = a * inv;
-      mse4[2] = b * inv;
-      mse4[3] = b * inv;
-      *ticket = 0u;  // self-reset for the next launch
-    }
-  }
+  finish_mse4(sse, sse_n, N, D, mse4, partials, ticket, sh);
 }
 
 // ---- backward ----------------------------------------------------------------------------------
@@ -343,6 +351,229 @@ __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
       for (int it = 0; it < NV; ++it)
 #pragma unroll
         for (int i = 0; i < V; ++i) gr[it][i] = (gr[it][i] - proj * yr[it][i]) * inv;
+    }
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      if (valid && d0 < D) {
+        if (g_hw > 0) store_slice_nchw<TX, V>(gx, n, g_hw, d0, D, gr[it]);
+        else store_slice<TX, V>(gx + n * D, d0, D, gr[it]);
+      }
+    }
+  }
+}
+
+// ---- residual quantization -----------------------------------------------------------------------------------------
+// One level of the residual chain (see vqb_residual_step): the per-token work of quantize_forward_kernel with (x, W[q])
+// = (r_{l-1}, W_l[q_l]), plus the running sum zhat and the next residual.  Every sum is an explicit round-to-nearest
+// add / subtract, so the backward can recompute r_{l-1} bit for bit.  TR: the dtype of r_{l-1} (TX at level 0).
+template <typename TX, typename TR, int G, int V, int NV>
+__global__ void __launch_bounds__(256) residual_step_kernel(
+    const TR* __restrict__ r_in, const TX* __restrict__ x, int64_t N, int D, const float* __restrict__ W, int64_t K,
+    const int64_t* __restrict__ quant, const unsigned long long* __restrict__ keys, int64_t key_offset,
+    int64_t* __restrict__ quant_out, int L, int level, float* __restrict__ zhat, float* __restrict__ r_out,
+    float* __restrict__ z_out, int64_t z_hw, int want_norm, float* __restrict__ mse4, float* __restrict__ partials,
+    unsigned int* __restrict__ ticket) {
+  __shared__ float sh[16];
+  pdl_wait();               // keys / codebook / previous level come from the preceding launches
+  pdl_launch_dependents();
+  const int lane = threadIdx.x % G;
+  const int64_t rows_per_block = blockDim.x / G;
+  const bool last = r_out == nullptr;
+  float sse = 0.f, sse_n = 0.f;
+  for (int64_t base = blockIdx.x * rows_per_block; base < N; base += (int64_t)gridDim.x * rows_per_block) {
+    const int64_t n_raw = base + threadIdx.x / G;  // warp-uniform trip count: shuffles need every lane
+    const bool valid = n_raw < N;
+    const int64_t n = valid ? n_raw : N - 1;
+    const int64_t q = row_index(quant, keys, n, key_offset, K);
+    const float* __restrict__ wrow = W + q * D;
+    const TR* __restrict__ rrow = r_in + n * D;
+    float rr[NV][V], wr[NV][V];
+    float srr = 0.f, sww = 0.f;
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      if (d0 < D) {
+        load_slice<TR, V>(rrow, d0, D, rr[it]);
+        load_slice<float, V>(wrow, d0, D, wr[it]);
+      } else {
+#pragma unroll
+        for (int i = 0; i < V; ++i) rr[it][i] = wr[it][i] = 0.f;
+      }
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        srr = fmaf(rr[it][i], rr[it][i], srr);
+        sww = fmaf(wr[it][i], wr[it][i], sww);
+      }
+    }
+    float rdr = 1.f, rdw = 1.f;
+    if (want_norm) {
+      srr = group_sum<G>(srr);
+      sww = group_sum<G>(sww);
+      rdr = 1.f / fmaxf(sqrtf(srr), kNormEps);
+      rdw = 1.f / fmaxf(sqrtf(sww), kNormEps);
+    }
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        const float diff = __fsub_rn(wr[it][i], rr[it][i]);
+        if (valid) sse = fmaf(diff, diff, sse);
+        if (want_norm) {
+          const float dn = wr[it][i] * rdw - rr[it][i] * rdr;
+          if (valid) sse_n = fmaf(dn, dn, sse_n);
+        }
+      }
+      if (valid && d0 < D) {
+        float h[V];   // zhat_l
+        if (level > 0 && zhat) {
+          load_slice<float, V>(zhat + n * D, d0, D, h);
+#pragma unroll
+          for (int i = 0; i < V; ++i) h[i] = __fadd_rn(h[i], wr[it][i]);
+        } else {
+#pragma unroll
+          for (int i = 0; i < V; ++i) h[i] = wr[it][i];
+        }
+        if (!last) {
+          float rn[V];
+#pragma unroll
+          for (int i = 0; i < V; ++i) rn[i] = __fsub_rn(rr[it][i], wr[it][i]);
+          if (zhat) store_slice<float, V>(zhat + n * D, d0, D, h);
+          store_slice<float, V>(r_out + n * D, d0, D, rn);
+        } else if (z_out) {
+          float xv[V], zr[V];
+          if (level == 0) {     // r_0 is x itself
+#pragma unroll
+            for (int i = 0; i < V; ++i) xv[i] = rr[it][i];
+          } else {
+            load_slice<TX, V>(x + n * D, d0, D, xv);
+          }
+#pragma unroll
+          for (int i = 0; i < V; ++i) zr[i] = __fadd_rn(xv[i], __fsub_rn(h[i], xv[i]));   // ste value: x + (zhat - x)
+          if (z_hw > 0) store_slice_nchw<float, V>(z_out, n, z_hw, d0, D, zr);
+          else store_slice<float, V>(z_out + n * D, d0, D, zr);
+        }
+      }
+    }
+    if (quant_out && valid && lane == 0) quant_out[n * L + level] = q;
+  }
+  finish_mse4(sse, sse_n, N, D, mse4, partials, ticket, sh);
+}
+
+// All L levels of the backward in one pass per token: r_{l-1} is rebuilt with the forward's subtractions, each level
+// contributes quantize_backward_kernel's terms with (y, z) = (r_{l-1}, W_l[q_l]) (no token normalisation): its
+// commitment-role terms accumulate onto g_z in level order, its codebook-role row goes to gW_l (atomics, or the level's
+// [N, D] rows with kRowsOut).  The level table is a __grid_constant__ parameter: indexed in place, never copied.
+template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut>
+__global__ void __launch_bounds__(256) residual_backward_kernel(
+    const TG* __restrict__ gz, const TX* __restrict__ x, const __grid_constant__ vqb_residual_levels lv, int64_t K,
+    const int64_t* __restrict__ quant, int64_t N, int D, int want_norm, TX* __restrict__ gx, int64_t g_hw) {
+  pdl_wait();               // upstream gradients / indices come from the preceding launches
+  pdl_launch_dependents();
+  const int lane = threadIdx.x % G;
+  const int64_t rows_per_block = blockDim.x / G;
+  const float scale = 2.f / ((float)N * (float)D);
+  const int L = lv.L;
+  for (int64_t base = blockIdx.x * rows_per_block; base < N; base += (int64_t)gridDim.x * rows_per_block) {
+    const int64_t n_raw = base + threadIdx.x / G;
+    const bool valid = n_raw < N;
+    const int64_t n = valid ? n_raw : N - 1;
+    const TX* __restrict__ xrow = x + n * D;
+    float yr[NV][V], wr[NV][V], gr[NV][V];   // r_{l-1}, W_l[q_l], the running token gradient
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      if (d0 < D) {
+        load_slice<TX, V>(xrow, d0, D, yr[it]);
+        if (g_hw > 0) load_slice_nchw<TG, V>(gz, n, g_hw, d0, D, gr[it]);
+        else load_slice<TG, V>(gz + n * D, d0, D, gr[it]);
+      } else {
+#pragma unroll
+        for (int i = 0; i < V; ++i) yr[it][i] = gr[it][i] = 0.f;
+      }
+    }
+#pragma unroll 1
+    for (int l = 0; l < L; ++l) {
+      const float* __restrict__ g_cb = lv.g[l][0];
+      const float* __restrict__ g_cm = lv.g[l][1];
+      const float* __restrict__ g_cbn = lv.g[l][2];
+      const float* __restrict__ g_cmn = lv.g[l][3];
+      const float c_cb = g_cb ? *g_cb * scale : 0.f, c_cm = g_cm ? *g_cm * scale : 0.f;
+      const float c_cbn = (want_norm && g_cbn) ? *g_cbn * scale : 0.f, c_cmn = (want_norm && g_cmn) ? *g_cmn * scale : 0.f;
+      const int64_t q = row_index(quant, nullptr, n * L + l, 0, K);
+      const float* __restrict__ wrow = lv.W[l] + q * D;
+      float* __restrict__ gW = lv.gW[l];
+      float sxx = 0.f, sww = 0.f;
+#pragma unroll
+      for (int it = 0; it < NV; ++it) {
+        const int d0 = (it * G + lane) * V;
+        if (d0 < D) {
+          load_slice<float, V>(wrow, d0, D, wr[it]);
+        } else {
+#pragma unroll
+          for (int i = 0; i < V; ++i) wr[it][i] = 0.f;
+        }
+#pragma unroll
+        for (int i = 0; i < V; ++i) {
+          sxx = fmaf(yr[it][i], yr[it][i], sxx);
+          sww = fmaf(wr[it][i], wr[it][i], sww);
+        }
+      }
+      float dy = 1.f, dw = 1.f, uu = 0.f, vv = 0.f, uv = 0.f;
+      bool cy = false, cw = false;
+      if (want_norm) {
+        float syw = 0.f;
+#pragma unroll
+        for (int it = 0; it < NV; ++it)
+#pragma unroll
+          for (int i = 0; i < V; ++i) syw = fmaf(yr[it][i], wr[it][i], syw);
+        sxx = group_sum<G>(sxx);
+        sww = group_sum<G>(sww);
+        syw = group_sum<G>(syw);
+        const float ny = sqrtf(sxx), nw = sqrtf(sww);
+        cy = ny < kNormEps;
+        cw = nw < kNormEps;
+        dy = 1.f / fmaxf(ny, kNormEps);   // reciprocal norms
+        dw = 1.f / fmaxf(nw, kNormEps);
+        uu = sxx * dy * dy;
+        vv = sww * dw * dw;
+        uv = syw * dy * dw;
+      }
+#pragma unroll
+      for (int it = 0; it < NV; ++it) {
+        const int d0 = (it * G + lane) * V;
+        float gw[V];
+#pragma unroll
+        for (int i = 0; i < V; ++i) {
+          const float yv = yr[it][i], wv = wr[it][i];
+          float g_y = gr[it][i] + c_cm * (yv - wv);
+          float g_w = c_cb * (wv - yv);
+          if (want_norm) {
+            const float u = yv * dy, v = wv * dw;
+            const float gu = c_cmn * (u - v), gu_dot_u = c_cmn * (uu - uv);
+            g_y += (gu - (cy ? 0.f : gu_dot_u * u)) * dy;
+            const float gv = c_cbn * (v - u), gv_dot_v = c_cbn * (vv - uv);
+            g_w += (gv - (cw ? 0.f : gv_dot_v * v)) * dw;
+          }
+          gr[it][i] = g_y;
+          gw[i] = g_w;
+          yr[it][i] = __fsub_rn(yv, wv);    // r_l
+        }
+        if constexpr (kRowsOut) {
+          if (valid && d0 < D) store_slice<float, V>(gW + n * D, d0, D, gw);
+        } else if (gW && valid && d0 < D) {
+          float* dst = gW + q * D + d0;
+          if constexpr (V == 8) {
+            atomicAdd(reinterpret_cast<float4*>(dst), make_float4(gw[0], gw[1], gw[2], gw[3]));
+            atomicAdd(reinterpret_cast<float4*>(dst + 4), make_float4(gw[4], gw[5], gw[6], gw[7]));
+          } else {
+#pragma unroll
+            for (int i = 0; i < V; ++i)
+              if (d0 + i < D) atomicAdd(dst + i, gw[i]);
+          }
+        }
+      }
     }
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
@@ -518,6 +749,95 @@ int vqb_quantize_backward_rows(const void* gz, int g_dtype, const void* x, int x
                                int64_t g_hw, void* stream) {
   return quantize_backward_launch<true>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn,
                                         want_norm, gx, gW_rows, g_hw, stream);
+}
+
+int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N, int D, const float* W,
+                      int64_t K, const int64_t* quant, const unsigned long long* keys, int64_t key_index_offset,
+                      int64_t* quant_out, int L, int level, float* zhat, float* r_out, float* z_out, int64_t z_hw,
+                      int want_norm, float* mse4, float* partials, unsigned int* ticket, void* stream) {
+  VQB_REQUIRE(z_hw >= 0 && (z_hw == 0 || N % z_hw == 0), "vqb_residual_step: z_hw must divide N (tokens = images x h*w)");
+  VQB_REQUIRE(r_in && x && W && mse4 && partials && ticket, "vqb_residual_step: null pointer");
+  VQB_REQUIRE((quant != nullptr) != (keys != nullptr), "vqb_residual_step: pass exactly one of quant / keys");
+  VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "vqb_residual_step: bad shape N=%lld D=%d K=%lld", (long long)N, D, (long long)K);
+  VQB_REQUIRE(L >= 1 && L <= VQB_MAX_LEVELS && level >= 0 && level < L, "vqb_residual_step: level %d of L=%d (L <= %d)",
+              level, L, VQB_MAX_LEVELS);
+  VQB_REQUIRE((r_out != nullptr) == (level < L - 1), "vqb_residual_step: r_out is required below the last level, and "
+              "must be NULL at the last one");
+  VQB_REQUIRE(level == 0 ? (r_in == x && r_dtype == x_dtype) : r_dtype == VQB_F32,
+              "vqb_residual_step: r_in is x at level 0 and an fp32 residual after");
+  VQB_REQUIRE(z_out == nullptr || level == 0 || zhat, "vqb_residual_step: z needs zhat (the levels' running sum)");
+  RowGeom geom;
+  VQB_REQUIRE(row_geom(D, N, &geom), "vqb_residual_step: D=%d unsupported (multiple of 8 up to 2048, or any D <= 256)", D);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int blocks = grid_for(N, 256 / geom.G);
+  VQB_REQUIRE(blocks <= kMaxPartials, "vqb_residual_step: grid too large");
+  bool launched = false;
+#define VQB_RESIDUAL_STEP(TX_, TR_)                                                                                   \
+  VQB_DISPATCH_GEOM((launch_pdl(residual_step_kernel<TX_, TR_, G, V, NV>, blocks, 256, 0, st, (const TR_*)r_in,        \
+      (const TX_*)x, N, D, W, K, quant, keys, key_index_offset, quant_out, L, level, zhat, r_out, z_out, z_hw,        \
+      want_norm, mse4, partials, ticket)))
+  if (x_dtype == VQB_F32 && r_dtype == VQB_F32) {
+    VQB_RESIDUAL_STEP(float, float)
+  } else if (x_dtype == VQB_BF16 && r_dtype == VQB_BF16) {
+    VQB_RESIDUAL_STEP(__nv_bfloat16, __nv_bfloat16)
+  } else if (x_dtype == VQB_BF16 && r_dtype == VQB_F32) {
+    VQB_RESIDUAL_STEP(__nv_bfloat16, float)
+  }
+#undef VQB_RESIDUAL_STEP
+  VQB_REQUIRE(launched, "vqb_residual_step: unsupported dtype/geometry");
+  VQB_LAUNCH_OK();
+  return VQB_OK;
+}
+
+}  // extern "C"
+
+template <bool kRowsOut>
+static int residual_backward_launch(const char* fn, const void* gz, int g_dtype, const void* x, int x_dtype,
+                                    const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int D,
+                                    int want_norm, void* gx, int64_t g_hw, void* stream) {
+  VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
+  VQB_REQUIRE(gz && x && lv && quant && gx, "%s: null pointer", fn);
+  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "%s: L=%d outside [1, %d]", fn, lv->L, VQB_MAX_LEVELS);
+  for (int l = 0; l < lv->L; ++l) {
+    VQB_REQUIRE(lv->W[l], "%s: null codebook at level %d", fn, l);
+    VQB_REQUIRE(!kRowsOut || lv->gW[l], "%s: null gradient rows at level %d", fn, l);
+  }
+  VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "%s: bad shape", fn);
+  RowGeom geom;
+  VQB_REQUIRE(row_geom(D, N, &geom), "%s: D=%d unsupported", fn, D);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int blocks = grid_for(N, 256 / geom.G);
+  bool launched = false;
+#define VQB_RESIDUAL_BWD(TX_, TG_)                                                                                      \
+  VQB_DISPATCH_GEOM((launch_pdl(residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>, blocks, 256, 0, st,             \
+      (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw)))
+  if (x_dtype == VQB_F32 && g_dtype == VQB_F32) {
+    VQB_RESIDUAL_BWD(float, float)
+  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_F32) {
+    VQB_RESIDUAL_BWD(__nv_bfloat16, float)
+  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_BF16) {
+    VQB_RESIDUAL_BWD(__nv_bfloat16, __nv_bfloat16)
+  }
+#undef VQB_RESIDUAL_BWD
+  VQB_REQUIRE(launched, "%s: unsupported dtype/geometry", fn);
+  VQB_LAUNCH_OK();
+  return VQB_OK;
+}
+
+extern "C" {
+
+int vqb_residual_backward(const void* gz, int g_dtype, const void* x, int x_dtype, const vqb_residual_levels* levels,
+                          int64_t K, const int64_t* quant, int64_t N, int D, int want_norm, void* gx, int64_t g_hw,
+                          void* stream) {
+  return residual_backward_launch<false>("vqb_residual_backward", gz, g_dtype, x, x_dtype, levels, K, quant, N, D,
+                                         want_norm, gx, g_hw, stream);
+}
+
+int vqb_residual_backward_rows(const void* gz, int g_dtype, const void* x, int x_dtype,
+                               const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
+                               int want_norm, void* gx, int64_t g_hw, void* stream) {
+  return residual_backward_launch<true>("vqb_residual_backward_rows", gz, g_dtype, x, x_dtype, levels, K, quant, N, D,
+                                        want_norm, gx, g_hw, stream);
 }
 
 int vqb_unpack_keys(const unsigned long long* keys, int64_t n, int64_t offset, int64_t* idx, float* score,

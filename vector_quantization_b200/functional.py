@@ -349,6 +349,100 @@ def quantize_ste_loss(x: torch.Tensor, W: torch.Tensor, index: torch.Tensor, wan
     return z, (m0, m1, m2, m3), quant, xn
 
 
+@torch.no_grad()
+def residual_levels(levels, x: torch.Tensor, memos, want_norm: bool, *, quant_out: torch.Tensor | None = None,
+                    z_out: torch.Tensor | None = None, z_hw: int = 0, compact_out: torch.Tensor | None = None,
+                    track_codebooks: bool = False):
+    """The level loop of a residual quantizer: level l runs its own `encode` (before_encode -> assignment ->
+    after_encode, codebook updates included) on r_{l-1}, then ONE `vqb_residual_step` launch gathers W_l[q_l] from the
+    codebook as that encode left it, writes the [N, L] indices, the running sum and r_l, and at the last level
+    z = x + (zhat_L - x).  memos[l] becomes level l's memo (x = r_{l-1}, quant = its indices).
+    compact_out: uint16 / int32 [L, N]: the compact ids of every level, straight from its packed assignment keys (every
+    level must then accept packed keys: no training callback reads the indices).
+    -> (mse fp32 [L, 4], [CodebookRef per level] (registered with the level when track_codebooks))"""
+    N, D = x.shape
+    L = len(levels)
+    mse = torch.empty((L, 4), dtype=torch.float32, device=x.device)
+    zhat = torch.empty((N, D), dtype=torch.float32, device=x.device) if (L > 1 and z_out is not None) else None
+    refs = []
+    r = x
+    for l, level in enumerate(levels):
+        memo = memos[l]
+        lazy = level._callbacks.packed_keys_ok()
+        memo['_lazy_unpack'] = lazy
+        _, index, memo = level.encode(r, memo)
+        W = level._weight().detach()
+        ref = CodebookRef(W)
+        if track_codebooks:
+            level._pending.add(ref)
+        refs.append(ref)
+        last = l == L - 1
+        if compact_out is not None:
+            assert lazy, 'compact ids need the packed assignment keys'
+            ops.compact_tokens(index, level.codebook_size, out=compact_out[l])
+        r_out = None if last else torch.empty((N, D), dtype=torch.float32, device=x.device)
+        if not (last and z_out is None and quant_out is None):
+            ops.residual_step(r, x, W, mse[l], level=l, L=L, quant=None if lazy else index, keys=index if lazy else None,
+                              quant_out=quant_out, zhat=zhat, r_out=r_out, z_out=z_out if last else None, z_hw=z_hw,
+                              want_norm=want_norm)
+        memo['x'] = r
+        memo['quant'] = quant_out[:, l] if quant_out is not None else index
+        r = r_out
+    return mse, refs
+
+
+class _ResidualQuantize(torch.autograd.Function):
+    """The whole depth of a residual quantizer as ONE node: forward = the level loop (`residual_levels`), backward = one
+    `vqb_residual_backward` launch for all levels (+ per-level code sort / segment sum under the deterministic flag).
+    Outputs z, quant [N, L] and the 4 L MSE terms as separate 0-dim tensors (their upstream gradients arrive as
+    device scalars)."""
+
+    @staticmethod
+    def forward(ctx, x, x_nchw, levels, memos, want_norm, track, *Ws):
+        N, D = x.shape
+        L = len(levels)
+        hw = 0 if x_nchw is None else x_nchw.shape[2] * x_nchw.shape[3]
+        z = torch.empty(tuple(x_nchw.shape) if x_nchw is not None else (N, D), dtype=torch.float32, device=x.device)
+        quant = torch.empty((N, L), dtype=torch.int64, device=x.device)
+        mse, refs = residual_levels(levels, x, memos, want_norm, quant_out=quant, z_out=z, z_hw=hw,
+                                    track_codebooks=track)
+        ctx.save_for_backward(x, quant)
+        ctx.refs = refs
+        ctx.nchw = None if x_nchw is None else tuple(x_nchw.shape)
+        ctx.want_norm = want_norm
+        ctx.set_materialize_grads(False)
+        ctx.mark_non_differentiable(quant)
+        return (z, quant) + tuple(mse.view(-1).unbind(0))
+
+    @staticmethod
+    def backward(ctx, gz, _gq, *g):
+        x, quant = ctx.saved_tensors
+        L = quant.shape[1]
+        if gz is None:
+            gz = torch.zeros(ctx.nchw or x.shape, dtype=torch.float32, device=x.device)
+        g4s = [[None if t is None else t.contiguous().float() for t in g[4 * l:4 * l + 4]] for l in range(L)]
+        need_gW = list(ctx.needs_input_grad[6:6 + L])
+        hw = 0 if ctx.nchw is None else ctx.nchw[2] * ctx.nchw[3]
+        gx, gWs = ops.residual_backward(gz.contiguous(), x, [r.tensor for r in ctx.refs], quant, g4s,
+                                        want_norm=ctx.want_norm, need_gW=need_gW, g_hw=hw)
+        if ctx.nchw is not None:     # the gradient belongs to the NCHW latents
+            return (None, gx.view(ctx.nchw) if ctx.needs_input_grad[1] else None, None, None, None, None, *gWs)
+        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, None, *gWs)
+
+
+def residual_quantize(levels, x: torch.Tensor, memos, want_norm: bool, *, nchw: torch.Tensor | None = None):
+    """Residual quantization of x [N, D] (fp32 / bf16) through `levels` (VectorQuantizer modules sharing K and D).
+    -> (z fp32 [N, D] (or NCHW like `nchw`): value x + (zhat_L - x), gradient straight to x;
+        quant int64 [N, L];  mse: per level the four MSE terms (codebook, commitment, codebook-norm,
+        commitment-norm) of e_l against r_{l-1}, 0-dim tensors whose gradients reach W_l and, through r_{l-1}, x)"""
+    Ws = [level._weight() for level in levels]
+    track = torch.is_grad_enabled() and (x.requires_grad or (nchw is not None and nchw.requires_grad)
+                                         or any(W.requires_grad for W in Ws))
+    out = _ResidualQuantize.apply(x.contiguous(), nchw, list(levels), memos, bool(want_norm), track, *Ws)
+    z, quant, flat = out[0], out[1], out[2:]
+    return z, quant, [tuple(flat[4 * l:4 * l + 4]) for l in range(len(levels))]
+
+
 class _FSQ(torch.autograd.Function):
 
     @staticmethod

@@ -13,14 +13,16 @@ from dataclasses import dataclass
 import torch
 
 from . import _lib
-from ._lib import BACKEND_SIMT, BACKEND_TCGEN05, PLANES_F16, PLANES_F16X2, VQB_BF16, VQB_F32, FSQParams, check
+from ._lib import (BACKEND_SIMT, BACKEND_TCGEN05, MAX_LEVELS, PLANES_F16, PLANES_F16X2, VQB_BF16, VQB_F32, FSQParams,
+                   ResidualLevels, check)
 
 __all__ = [
     'Operand', 'as_operand', 'pack_rows', 'fold_l2_side', 'can_fold_l2', 'assign', 'certify', 'cvq_needy_codes', 'gather_operand_rows', 'scatter_keys', 'row_inv_norm', 'new_keys', 'unpack_keys', 'keys_flip_sign', 'gather_ste_loss',
     'quantize_backward', 'l2norm_forward', 'l2norm_backward', 'scatter_stats', 'bincount_accumulate',
     'deterministic_enabled', 'segment_chunk', 'code_sort', 'segment_sum_rows',
     'kmeans_ema_update', 'gather_rows_by_key', 'cvq_update', 'embedding_gather', 'fsq_params', 'fsq_forward', 'fsq_backward',
-    'fsq_decode', 'decode_tokens', 'fsq_decode_tokens', 'transpose_last2', 'compact_tokens', 'distance_matrix', 'comm_kmeans_ema_update', 'comm_cvq_update',
+    'fsq_decode', 'decode_tokens', 'fsq_decode_tokens', 'residual_step', 'residual_backward', 'decode_residual_tokens',
+    'transpose_last2', 'compact_tokens', 'distance_matrix', 'comm_kmeans_ema_update', 'comm_cvq_update',
     'comm_allreduce_min_keys', 'comm_allreduce_sum_f32', 'BACKEND_TCGEN05', 'BACKEND_SIMT',
 ]
 
@@ -210,13 +212,17 @@ def transpose_last2(src: torch.Tensor) -> torch.Tensor:
     return dst
 
 
-def compact_tokens(keys: torch.Tensor, codebook_size: int, index_offset: int = 0) -> torch.Tensor:
-    """Packed keys -> compact token ids: uint16 for codebooks of at most 65 536 codes, int32 otherwise."""
+def compact_tokens(keys: torch.Tensor, codebook_size: int, index_offset: int = 0,
+                   out: torch.Tensor | None = None) -> torch.Tensor:
+    """Packed keys -> compact token ids: uint16 for codebooks of at most 65 536 codes, int32 otherwise (written into
+    `out` when given: a contiguous tensor of that dtype and the keys' size)."""
     lib = _lib.load()
-    dev = _cuda(keys)
+    dev = _cuda(keys, out)
     assert keys.dtype == torch.int64
     small = codebook_size <= 65536
-    out = torch.empty(keys.shape, dtype=torch.uint16 if small else torch.int32, device=keys.device)
+    if out is None:
+        out = torch.empty(keys.shape, dtype=torch.uint16 if small else torch.int32, device=keys.device)
+    assert out.dtype == (torch.uint16 if small else torch.int32) and out.numel() == keys.numel()
     _call('vqb_compact_tokens', lib.vqb_compact_tokens, dev, _p(keys), keys.numel(), index_offset, _p(out), 2 if small else 4,
           _S)
     return out
@@ -753,4 +759,105 @@ def fsq_decode_tokens(ids: torch.Tensor, p: FSQParams, hw: int, out_dtype: torch
     b, id_bytes, z = _decode_out(ids, hw, p.D, out_dtype, bad_count)
     _call('vqb_fsq_decode_tokens', lib.vqb_fsq_decode_tokens, dev, _p(ids), id_bytes, b, hw, ctypes.byref(p), _p(z),
           _dt(z), _p(bad_count), _S)
+    return z
+
+
+# ---- residual quantization (csrc/quantize.cu, csrc/layout.cu) ------------------------------------------------------
+
+
+def _residual_levels(Ws, gWs=None, g4s=None) -> ResidualLevels:
+    """The vqb_residual_levels struct (host memory, copied by value into the kernel parameters)."""
+    if not 1 <= len(Ws) <= MAX_LEVELS:
+        raise ValueError(f'residual quantization takes 1..{MAX_LEVELS} levels, got {len(Ws)}')
+    p = ResidualLevels()
+    p.L = len(Ws)
+    for l, W in enumerate(Ws):
+        p.W[l] = W.data_ptr()
+        if gWs is not None and gWs[l] is not None:
+            p.gW[l] = gWs[l].data_ptr()
+        if g4s is not None:
+            for k, g in enumerate(g4s[l]):
+                if g is not None:
+                    p.g[l][k] = g.data_ptr()
+    return p
+
+
+def _codebooks(Ws) -> tuple[int, int]:
+    K, D = Ws[0].shape
+    for W in Ws:
+        if W.dtype != torch.float32 or tuple(W.shape) != (K, D):
+            raise TypeError(f'every level codebook must be a float32 [{K}, {D}] tensor, got {W.dtype} {tuple(W.shape)}')
+    return K, D
+
+
+def residual_step(r: torch.Tensor, x: torch.Tensor, W: torch.Tensor, mse4: torch.Tensor, *, level: int, L: int,
+                  quant: torch.Tensor | None = None, keys: torch.Tensor | None = None, key_offset: int = 0,
+                  quant_out: torch.Tensor | None = None, zhat: torch.Tensor | None = None,
+                  r_out: torch.Tensor | None = None, z_out: torch.Tensor | None = None, z_hw: int = 0,
+                  want_norm: bool = False) -> None:
+    """One level of the residual chain (vqb_residual_step), into the caller's buffers: quant_out int64 [N, L]
+    (column `level`), zhat fp32 [N, D], r_out fp32 [N, D] (None at the last level), z_out fp32 [N, D] or NCHW
+    (last level only), mse4 fp32 [4] (this level's terms).  r is x at level 0 and the previous r_out after."""
+    lib = _lib.load()
+    dev = _cuda(r, x, W, mse4, quant, keys, quant_out, zhat, r_out, z_out)
+    assert W.dtype == torch.float32 and (quant is None) != (keys is None) and mse4.dtype == torch.float32
+    assert quant_out is None or (quant_out.dtype == torch.int64 and quant_out.shape == (x.shape[0], L))
+    N, D = x.shape
+    partials, ticket = _loss_ws(x.device)
+    _call('vqb_residual_step', lib.vqb_residual_step, dev, _p(r), _dt(r), _p(x), _dt(x), N, D, _p(W), W.shape[0],
+          _p(quant), _p(keys), key_offset, _p(quant_out), L, level, _p(zhat), _p(r_out), _p(z_out), z_hw,
+          int(want_norm), _p(mse4), _p(partials), _p(ticket), _S)
+
+
+def residual_backward(g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tensor, g4s, *, want_norm: bool,
+                      need_gW, g_hw: int = 0, deterministic: bool | None = None):
+    """Backward of the whole residual depth in one launch (vqb_residual_backward).  Ws: the L codebooks as used by the
+    forward; quant: int64 [N, L]; g4s: per level four 0-dim fp32 device tensors / None (codebook, commitment,
+    codebook-norm, commitment-norm upstream gradients); need_gW: per level bool.
+    deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, each gW_l is the segment sum of
+    the level's per-token rows (vqb_residual_backward_rows + vqb_code_sort + vqb_segment_sum_rows, the contract of
+    quantize_backward).  -> (gx in x's dtype, [gW_l fp32 [K, D] or None])"""
+    lib = _lib.load()
+    L = len(Ws)
+    dev = _cuda(g_z, x, quant, *Ws, *[g for g4 in g4s for g in g4])
+    K, D = _codebooks(Ws)
+    N = x.shape[0]
+    assert x.shape[1] == D and quant.dtype == torch.int64 and quant.shape == (N, L) and len(g4s) == L
+    assert all(g is None or g.dtype == torch.float32 for g4 in g4s for g in g4)
+    if not (g_z.dtype == torch.float32 or (g_z.dtype == torch.bfloat16 and x.dtype == torch.bfloat16)):
+        g_z = g_z.float()
+    gx = torch.empty_like(x)
+    gWs = [torch.zeros_like(W) if need else None for W, need in zip(Ws, need_gW)]
+    if any(need_gW) and deterministic_enabled(deterministic):
+        rows = _det_ws(x.device, 'gw_rows', L * N * D, torch.float32).view(L, N, D)
+        p = _residual_levels(Ws, list(rows), g4s)
+        _call('vqb_residual_backward_rows', lib.vqb_residual_backward_rows, dev, _p(g_z), _dt(g_z), _p(x), _dt(x),
+              ctypes.byref(p), K, _p(quant), N, D, int(want_norm), _p(gx), g_hw, _S)
+        by_level = quant.view(L, N) if L == 1 else transpose_last2(quant.view(1, N, L)).view(L, N)
+        for l, gW in enumerate(gWs):
+            if gW is not None:
+                order, offsets = _code_sort_ws(dev, N, K, by_level[l], None, 0)
+                _segment_sum(dev, rows[l], N, D, False, order, offsets, K, gW, None)
+        return gx, gWs
+    p = _residual_levels(Ws, gWs, g4s)
+    _call('vqb_residual_backward', lib.vqb_residual_backward, dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K,
+          _p(quant), N, D, int(want_norm), _p(gx), g_hw, _S)
+    return gx, gWs
+
+
+def decode_residual_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtype = torch.float32,
+                           bad_count: torch.Tensor | None = None) -> torch.Tensor:
+    """Residual token ids [b, h, w, L] (uint16 / int32 / int64; a token's L ids contiguous) -> z = sum_l W_l[id_l]
+    (level order, fp32 adds) as [b, D, h, w] of `out_dtype`, in one launch (vqb_decode_residual_tokens).  A token with
+    an id outside [0, K) at any level gives a NaN row and is counted once into `bad_count`."""
+    lib = _lib.load()
+    dev = _cuda(ids, bad_count, *Ws)
+    K, D = _codebooks(Ws)
+    L = len(Ws)
+    if ids.dim() < 2 or ids.shape[-1] != L:
+        raise ValueError(f'expected residual token ids with a trailing depth axis of {L}, got {tuple(ids.shape)}')
+    b, id_bytes, z = _decode_out(ids.select(-1, 0), hw, D, out_dtype, bad_count)
+    p = _residual_levels(Ws)
+    _call('vqb_decode_residual_tokens', lib.vqb_decode_residual_tokens, dev, _p(ids), id_bytes, b, hw, ctypes.byref(p),
+          K, D, _p(z), _dt(z), _p(bad_count), _S)
     return z

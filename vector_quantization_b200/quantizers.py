@@ -14,6 +14,7 @@ library must be present — there is no CPU or eager-PyTorch fallback.
 """
 from __future__ import annotations
 
+import copy
 import weakref
 from typing import Mapping, Sequence
 
@@ -30,7 +31,7 @@ from .registry import (Config, InitRegistry, ModelRegistry, ModuleDict, VQITQuan
                        build_module_dict, get_config)
 
 __all__ = ['BaseQuantizer', 'VectorQuantizer', 'VQGANQuantizer', 'VQKDQuantizer', 'ScalarQuantizer',
-           'FiniteScalarQuantizer']
+           'FiniteScalarQuantizer', 'ResidualVectorQuantizer']
 
 
 def get_memo(memo: dict, key: str) -> dict:
@@ -445,3 +446,168 @@ class FiniteScalarQuantizer(ScalarQuantizer):
         z, memo = self.decode(quant, memo)
         memo['loss'] = get_memo(memo, 'loss')
         return z, x.new_zeros([]), memo
+
+
+@VQITQuantizerRegistry.register_()
+class ResidualVectorQuantizer(BaseQuantizer):
+    """Residual quantization (RQ-VAE): L codebooks code every token in turn, level l quantizing what the earlier levels
+    left over.  Levels are ordinary VectorQuantizer / VQGANQuantizer modules built from ONE config node (`quantizer`),
+    stored as `_quantizers.{l}`; level l runs its own `encode` (before_encode -> assignment -> after_encode, codebook
+    update included) on its input r_{l-1}:
+
+        r_0 = x                       (fp32 view of the tokens; x is fp32 or bf16)
+        q_l = level_l.encode(r_{l-1});  e_l = W_l[q_l]   (the codebook after this step's update)
+        zhat_l = e_l (l = 1) or zhat_{l-1} + e_l;  r_l = r_{l-1} - e_l        (level order, fp32, no FMA)
+        z = x + (zhat_L - x)          (one straight-through estimator over the whole depth: the gradient goes to x)
+        loss = sum_l sum_name loss_{l,name}(e_l, r_{l-1}),  r_{l-1} = x - sum_{j<l} sg(e_j)
+
+    so level l's CodebookLoss trains W_l against sg(r_{l-1}) and its CommitmentLoss reaches x through r_{l-1}.  With
+    L = 1 this is VectorQuantizer.forward bit for bit.  memo: 'x' (the tokens), 'quant' (int64 [N, L]), 'levels'
+    (level l's own memo: x = r_{l-1}, encode, decode, loss), 'loss' (per loss name, the sum over the levels).
+
+    Accepted: 1 <= L <= 16, L2 or Cosine distance, no callback or CVQVAECallback (NearestAnchor / CachedAnchor),
+    CodebookLoss / CommitmentLoss / VQGANLoss with or without mse.norm.  Rejected with a ValueError: callbacks that
+    rewrite the tokens (NormalizeCallback and its subclasses), callbacks that hook decode or loss, and compatibility
+    mode (EntropyLoss, MultinomialAnchor, materialize_distance).  `init_weights` is applied to every level."""
+
+    MAX_LEVELS = 16
+
+    def __init__(self, *args, num_quantizers: int, quantizer: Mapping, **kwargs) -> None:
+        super().__init__(*args, **kwargs)
+        if isinstance(num_quantizers, bool) or not isinstance(num_quantizers, int) or \
+                not 1 <= num_quantizers <= self.MAX_LEVELS:
+            raise ValueError(f'ResidualVectorQuantizer: num_quantizers={num_quantizers!r} is outside [1, {self.MAX_LEVELS}]')
+        if list(self._callbacks) or len(self._losses):
+            raise ValueError('ResidualVectorQuantizer: callbacks and losses belong to the level config (`quantizer`), '
+                             'not to the residual quantizer itself')
+        levels = []
+        for _ in range(num_quantizers):
+            cfg = Config(copy.deepcopy(dict(quantizer)))
+            cfg['init_weights'] = None       # applied per level by init_weights (after the train / eval mode is set)
+            levels.append(VQITQuantizerRegistry.build(cfg))
+        for level in levels:
+            self._check_level(level)
+        self._quantizers = nn.ModuleList(levels)
+
+    @staticmethod
+    def _check_level(level) -> None:
+        from .callbacks import BaseCallback, CVQVAECallback, NormalizeCallback
+        from .losses import CodebookLoss, CommitmentLoss, VQGANLoss
+        name = type(level).__name__
+        if not isinstance(level, VectorQuantizer):
+            raise ValueError(f'ResidualVectorQuantizer: the levels must be VectorQuantizer modules, got {name}')
+        if level.materialize_distance:
+            raise ValueError('ResidualVectorQuantizer: materialize_distance (compatibility mode) is not supported')
+        for c in level._callbacks:
+            cname = type(c).__name__
+            if isinstance(c, NormalizeCallback):
+                raise ValueError(f'ResidualVectorQuantizer: callback {cname} rewrites the tokens; a residual of '
+                                 'normalised levels is not supported')
+            hooks = [h for h in ('before_decode', 'after_decode', 'before_loss', 'after_loss')
+                     if getattr(type(c), h) is not getattr(BaseCallback, h)]
+            if hooks:
+                raise ValueError(f'ResidualVectorQuantizer: callback {cname} hooks {", ".join(hooks)}; callbacks that '
+                                 'hook decode or loss are not supported')
+            if not isinstance(c, CVQVAECallback):
+                raise ValueError(f'ResidualVectorQuantizer: callback {cname} is not supported (levels take no callback '
+                                 'or CVQVAECallback)')
+            if c._anchor.needs_distance:
+                raise ValueError(f'ResidualVectorQuantizer: {type(c._anchor).__name__} of {cname} reads the [N, K] '
+                                 'distance matrix (compatibility mode), which is not supported')
+        for lname, loss in level._losses.items():
+            if not isinstance(loss, (CodebookLoss, CommitmentLoss, VQGANLoss)):
+                raise ValueError(f'ResidualVectorQuantizer: loss {lname!r} ({type(loss).__name__}) is not supported '
+                                 '(CodebookLoss, CommitmentLoss and VQGANLoss are)')
+
+    @property
+    def quantizers(self) -> nn.ModuleList:
+        return self._quantizers
+
+    @property
+    def num_quantizers(self) -> int:
+        return len(self._quantizers)
+
+    @property
+    def embedding_dim(self) -> int:
+        return self._quantizers[0].embedding_dim
+
+    @property
+    def codebook_size(self) -> int:
+        """Codes per level."""
+        return self._quantizers[0].codebook_size
+
+    @property
+    def embeddings(self) -> torch.Tensor:
+        """[L, K, D] copy of the level codebooks."""
+        return torch.stack([level.embedding.weight.detach() for level in self._quantizers]).clone()
+
+    def _init_weights(self, config) -> bool:
+        for level in self._quantizers:
+            level.init_weights(Config(copy.deepcopy(dict(config))))
+        return False
+
+    def _weights(self) -> list:
+        return [level._weight() for level in self._quantizers]
+
+    def _want_norm(self) -> bool:
+        return self._quantizers[0]._loss_terms()
+
+    def _level_memos(self, memo: dict) -> list:
+        memo['levels'] = [dict() for _ in self._quantizers]
+        return memo['levels']
+
+    @torch.no_grad()
+    def encode(self, x: torch.Tensor, memo: dict):
+        """-> (x, quant int64 [N, L], memo); every level's callbacks run as in forward (codebook updates included)."""
+        x = _check_tokens(x, self.embedding_dim)
+        quant = torch.empty((x.shape[0], self.num_quantizers), dtype=torch.int64, device=x.device)
+        Fq.residual_levels(list(self._quantizers), x, self._level_memos(memo), self._want_norm(), quant_out=quant)
+        return x, quant, memo
+
+    @torch.no_grad()
+    def encode_compact(self, x: torch.Tensor, memo: dict) -> torch.Tensor:
+        """Tokenise-only encode: [L, N'] uint16 (K <= 65 536) or int32 ids straight from the packed assignment keys (N' = N
+        rounded up to 8; the first N columns are the ids); None when a level's training callback needs int64 indices
+        (then `encode` is the way)."""
+        if not all(level._callbacks.packed_keys_ok() for level in self._quantizers):
+            return None
+        x = _check_tokens(x, self.embedding_dim)
+        N = x.shape[0]
+        # rows padded to 8 ids: every row starts 16-byte aligned, as vqb_compact_tokens stores 16 bytes at a time
+        out = torch.empty((self.num_quantizers, (N + 7) // 8 * 8),
+                          dtype=torch.uint16 if self.codebook_size <= 65536 else torch.int32, device=x.device)
+        Fq.residual_levels(list(self._quantizers), x, self._level_memos(memo), self._want_norm(), compact_out=out[:, :N])
+        return out
+
+    def decode(self, quant: torch.Tensor, memo: dict):
+        """quant [N, L] (or [..., L]; uint16 / int32 / int64) -> (zhat fp32 [..., D], memo): sum_l W_l[q_l] in level order,
+        one launch.  A token with an id outside [0, codebook_size) at any level decodes to NaN."""
+        if not quant.is_cuda:
+            raise VQBError('ResidualVectorQuantizer decodes CUDA tensors only; there is no CPU fallback')
+        lead = tuple(quant.shape[:-1])
+        flat = quant.contiguous().view(-1, quant.shape[-1])
+        z = ops.decode_residual_tokens([W.detach() for W in self._weights()], flat, 1)
+        get_memo(memo, 'decode')
+        return z.view(*lead, self.embedding_dim), memo
+
+    def forward(self, x: torch.Tensor, memo: dict):
+        x = _check_tokens(x, self.embedding_dim)
+        nchw = memo.pop('_nchw', None)     # tokenizer.quantize: x is the token-major copy of these [b, c, h, w] latents
+        levels = list(self._quantizers)
+        memos = self._level_memos(memo)
+        z, quant, mse = Fq.residual_quantize(levels, x, memos, self._want_norm(), nchw=nchw)
+        memo.update(x=x, quant=quant)
+        loss_memo = get_memo(memo, 'loss')
+        loss = None
+        for l, (level, level_memo) in enumerate(zip(levels, memos)):
+            level_memo['decode'] = get_memo(level_memo, 'decode')
+            level_loss = get_memo(level_memo, 'loss')
+            for name, module in level._losses.items():
+                value = module.from_mse4(mse[l])
+                level_loss[name] = value
+                loss_memo[name] = value if l == 0 else loss_memo[name] + value
+        for name in levels[0]._losses:
+            loss = loss_memo[name] if loss is None else loss + loss_memo[name]
+        if loss is None:
+            loss = mse[0][0].new_zeros([])
+        return z, loss, memo

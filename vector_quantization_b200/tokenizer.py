@@ -18,17 +18,20 @@ import torch
 from . import functional as Fq
 from . import ops
 from ._lib import VQBError
-from .quantizers import FiniteScalarQuantizer, VectorQuantizer, get_memo
+from .quantizers import FiniteScalarQuantizer, ResidualVectorQuantizer, VectorQuantizer, get_memo
 
 __all__ = ['quantize', 'encode_to_quant', 'decode_from_quant', 'save_tokens', 'load_tokens', 'save_llamagen_codes', 'TokenStreamWriter']
 
 
 def quantize(quantizer, x: torch.Tensor, memo: dict):
     """`BaseModel.quantize` (base.py:116-129): x [b, c, h, w] -> (z [b, c, h, w] contiguous, q_loss, memo) with
-    memo['quantizer'] = the quantizer's memo (+ 'x_shape')."""
+    memo['quantizer'] = the quantizer's memo (+ 'x_shape').  A ResidualVectorQuantizer always takes the fused layout: its
+    last residual step writes z NCHW."""
     quantizer_memo = get_memo(memo, 'quantizer')
     quantizer_memo['x_shape'] = (b, c, h, w) = tuple(x.shape)
-    if isinstance(quantizer, VectorQuantizer) and quantizer.can_fuse_nchw() and x.is_cuda:
+    fusable = isinstance(quantizer, ResidualVectorQuantizer) or (isinstance(quantizer, VectorQuantizer)
+                                                                  and quantizer.can_fuse_nchw())
+    if fusable and x.is_cuda:
         # Layout fusion: ONE transposed copy of the latents feeds the assignment, the callbacks and the kernels' token
         # reads; z is written NCHW by the gather kernel, and the backward reads the NCHW upstream gradient and writes
         # the NCHW token gradient directly — no transpose after the quantizer, none in the backward.
@@ -47,10 +50,23 @@ def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = F
     """`BaseModel.encode_to_quant` after the encoder (base.py:131-146): x [b, c, h, w] -> (quant [b, h, w], memo);
     memo['quantizer'] gets 'x_shape', 'x' (token-major, after the callbacks) and 'quant' ([b*h*w] int64).
     compact=True is the tokenise-only variant: token ids come back as uint16 (K <= 65 536) or int32 straight
-    from the packed assignment keys and memo['quantizer']['quant'] holds that compact tensor."""
+    from the packed assignment keys and memo['quantizer']['quant'] holds that compact tensor.
+    A ResidualVectorQuantizer gives quant [b, h, w, L] (a token's L ids contiguous); with compact=True each level's
+    ids are compacted into a row of an [L, N] buffer and one transpose makes the [N, L] layout."""
     quantizer_memo = get_memo(memo, 'quantizer')
     quantizer_memo['x_shape'] = (b, _, h, w) = tuple(x.shape)
     rows = Fq.nchw_to_rows(x)
+    if isinstance(quantizer, ResidualVectorQuantizer):
+        L = quantizer.num_quantizers
+        by_level = quantizer.encode_compact(rows, quantizer_memo) if compact else None
+        if by_level is not None:
+            quant = ops.transpose_last2(by_level.view(1, L, -1)).view(-1, L)[:b * h * w]
+        else:
+            rows, quant, _ = quantizer.encode(rows, quantizer_memo)
+            if compact:
+                quant = quant.to(torch.int32)
+        quantizer_memo.update(x=rows, quant=quant)
+        return quant.view(b, h, w, L), memo
     # keep the packed keys (no int64 unpack launch) unless a training callback consumes the indices in after_encode
     lazy = compact and isinstance(quantizer, VectorQuantizer) and quantizer._callbacks.packed_keys_ok()
     if lazy:
@@ -71,6 +87,7 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     quant [b, h, w] -> (z [b, c, h, w] contiguous of `dtype`, memo) with memo['quantizer'] = the quantizer's memo as
     `quantizer.decode` leaves it.  quant is uint16, int32 or int64 on the GPU: what `encode_to_quant` (compact or not)
     and FSQ produce, or a `load_tokens` dump moved to the device.  The codebook is used as stored (no before_encode).
+    A ResidualVectorQuantizer takes quant [b, h, w, L] and decodes sum_l W_l[id_l] in one launch.
 
     A VectorQuantizer or FiniteScalarQuantizer without before_decode / after_decode hooks decodes in ONE launch that
     reads the ids as they are and writes NCHW `dtype` directly.  Hooks, or a codebook that requires grad with grad
@@ -80,14 +97,25 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     An id outside [0, codebook_size) is an error: with check=True (one 4-byte device-to-host read) it raises
     IndexError with the number of such tokens.  check=False does not synchronise (safe inside a CUDA graph capture)
     and, on the one-launch path, decodes such tokens to NaN in every channel."""
-    if quant.dim() != 3:
+    residual = isinstance(quantizer, ResidualVectorQuantizer)
+    if residual and (quant.dim() != 4 or quant.shape[-1] != quantizer.num_quantizers):
+        raise ValueError(f'expected residual token ids of shape [b, h, w, {quantizer.num_quantizers}], '
+                         f'got {tuple(quant.shape)}')
+    if not residual and quant.dim() != 3:
         raise ValueError(f'expected token ids of shape [b, h, w], got {tuple(quant.shape)}')
     if not quant.is_cuda:
         raise VQBError('vector_quantization_b200 decodes CUDA (sm_100a) token ids only; there is no CPU fallback')
     if dtype not in (torch.float32, torch.bfloat16):
         raise TypeError(f'dtype must be float32 or bfloat16, got {dtype}')
-    b, h, w = quant.shape
+    b, h, w = quant.shape[:3]
     quantizer_memo = get_memo(memo, 'quantizer')
+    if residual:
+        bad = torch.zeros(1, dtype=torch.int32, device=quant.device) if check else None
+        z = ops.decode_residual_tokens([W.detach() for W in quantizer._weights()], quant.contiguous(), h * w, dtype, bad)
+        get_memo(quantizer_memo, 'decode')
+        if check:
+            _raise_bad_ids(int(bad.item()), quantizer.codebook_size)
+        return z, memo
     fsq = isinstance(quantizer, FiniteScalarQuantizer)
     hooked = any(quantizer._callbacks.overrides(hook) for hook in ('before_decode', 'after_decode'))
     if isinstance(quantizer, VectorQuantizer):
@@ -118,6 +146,13 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     return (z if z.dtype == dtype else z.to(dtype)), memo
 
 
+def _token_grid(quant: torch.Tensor, x_shape: Sequence[int]) -> tuple:
+    """(b, h, w) for one id per token; (b, h, w, L) for residual ids ([b, h, w, L], or L ids per token)."""
+    b, _, h, w = x_shape
+    depth = quant.numel() // max(b * h * w, 1)
+    return (b, h, w, depth) if (quant.dim() == 4 or depth != 1) else (b, h, w)
+
+
 def _raise_bad_ids(count: int, codebook_size: int) -> None:
     if count:
         raise IndexError(f'{count} token id(s) outside [0, {codebook_size}): not in the codebook')
@@ -127,9 +162,9 @@ def save_tokens(path: str | pathlib.Path, id_: Sequence[Any], category: torch.Te
                 x_shape: Sequence[int]) -> None:
     """`TokenizeCallback.after_run_iter` (runners/callbacks.py:40-53): torch.save of the `Tokens` dict
     {id_, category, tokens [b, h, w]}.  Compact ids are widened to int64 so that reference readers see the
-    dtype they expect; pass an int64 tensor to skip the conversion."""
-    b, _, h, w = x_shape
-    tokens = quant.reshape(b, h, w)
+    dtype they expect; pass an int64 tensor to skip the conversion.  Residual ids keep their trailing depth axis:
+    tokens [b, h, w, L]."""
+    tokens = quant.reshape(_token_grid(quant, x_shape))
     if tokens.dtype != torch.int64:
         tokens = tokens.to(torch.int32).to(torch.int64) if tokens.dtype == torch.uint16 else tokens.to(torch.int64)
     torch.save(dict(id_=id_, category=category, tokens=tokens.cpu()), str(path))
@@ -179,7 +214,6 @@ class TokenStreamWriter:
               x_shape: Sequence[int]) -> pathlib.Path:
         if self._error is not None:
             raise self._error
-        b, _, h, w = x_shape
         host = self._free.get()                                 # blocks only when `depth` writes are in flight
         flat = quant.reshape(-1)
         if host is None or host.numel() != flat.numel() or host.dtype != flat.dtype:
@@ -197,7 +231,7 @@ class TokenStreamWriter:
         else:
             host.copy_(flat)
         path = self.token_dir / f'{iter_}_{self.rank}.pth'
-        self._jobs.put((path, list(id_), category.detach().cpu(), host, event, (b, h, w)))
+        self._jobs.put((path, list(id_), category.detach().cpu(), host, event, _token_grid(quant, x_shape)))
         return path
 
     def close(self) -> None:
