@@ -283,6 +283,36 @@ int vqb_residual_backward_rows(const void* g_z, int g_dtype, const void* x, int 
                                const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
                                int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
 
+/* ---- grouped (product) quantization: G codebooks, group g quantizes channels [g*Dg, (g+1)*Dg) of every token ---- *
+ * Group g behaves exactly like its own vqb_gather_ste_loss / vqb_quantize_backward on the contiguous [N, Dg] slice
+ * x_g (same row geometry, same grid, its own partials and ticket), so every per-group result is bit for bit that of
+ * a standalone quantizer on x_g.  The per-group pointers travel BY VALUE in a vqb_residual_levels with L = G
+ * (W[g], gW[g], g[g][4]).
+ * Split: src [batch, G*Dg, hw] (NCHW latents; hw = 1 is token-major [N, D]) -> dst [G, batch*hw, Dg], the group-major
+ * copy whose group g is the contiguous x_g.  dtype VQB_F32 or VQB_BF16 (copied as is). */
+int vqb_split_groups(const void* src, int dtype, int64_t batch, int G, int Dg, int64_t hw, void* dst, void* stream);
+/* Every group's gather + straight-through + MSE terms in ONE launch (grid y = group).  xs: the split [G, N, Dg];
+ * quant / keys: group-major [G, N] (exactly one); writes quant_out[n*G + g] (optional; the [N, G] code layout),
+ * z = x_g + (W_g[q_g] - x_g) into channels [g*Dg, (g+1)*Dg) of z_out (token-major [N, G*Dg], or NCHW with z_hw > 0
+ * as in vqb_gather_ste_loss) and group g's four terms to mse4_out[4*g .. 4*g+4).  partials: G x
+ * vqb_loss_partials_count() floats, tickets: G zero-initialised (self-resetting) uint32. */
+int vqb_group_gather_ste_loss(const void* xs, int x_dtype, int64_t N, int Dg, const vqb_residual_levels* groups,
+                              int64_t K, const int64_t* quant, const unsigned long long* keys, int64_t* quant_out,
+                              float* z_out, int64_t z_hw, int want_norm_mse, float* mse4_out, float* partials,
+                              unsigned int* tickets, void* stream);
+/* Every group's backward in ONE launch: the closed form of vqb_quantize_backward per group with (x, W, quant) =
+ * (x_g, W_g, quant[:, g]).  gx channels [g*Dg, (g+1)*Dg) = g_z's + group g's commitment-role terms (x dtype; token-major
+ * [N, G*Dg], or NCHW for both g_z and gx with g_hw > 0); gW_g[q_g] += the codebook-role row (fp32 vector atomics).
+ * xs: the split [G, N, Dg] of the forward; quant: int64 [N, G]. */
+int vqb_group_backward(const void* g_z, int g_dtype, const void* xs, int x_dtype, const vqb_residual_levels* groups,
+                       int64_t K, const int64_t* quant, int64_t N, int Dg, int want_norm_mse, void* gx_out, int64_t g_hw,
+                       void* stream);
+/* The same with group g's codebook-gradient rows STORED to groups->gW[g] (fp32 [N, Dg] each; gx identical): their
+ * vqb_segment_sum_rows, group by group, is a deterministic gW_g. */
+int vqb_group_backward_rows(const void* g_z, int g_dtype, const void* xs, int x_dtype, const vqb_residual_levels* groups,
+                            int64_t K, const int64_t* quant, int64_t N, int Dg, int want_norm_mse, void* gx_out,
+                            int64_t g_hw, void* stream);
+
 /* ---- row l2-normalisation (NormalizeCallback.before_encode on x) ------------------------ *
  * vq/algorithms/vq/callbacks/normalize.py:24  — forward y = x / max(||x||, 1e-12); backward
  * gx = (gy - (gy.y) y) / max(||x||, 1e-12). */
@@ -393,6 +423,11 @@ int vqb_fsq_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t 
 int vqb_decode_residual_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw,
                                const vqb_residual_levels* levels, int64_t K, int D, void* z_out, int out_dtype,
                                int* bad_count, void* stream);
+/* The same for grouped codes: ids [batch * hw, G] (a token's G ids contiguous), z[b][g*Dg + d][s] = W_g[id_g][d].
+ * An id outside [0, K) in ANY group gives a NaN row (every channel) and counts the token once.  G = groups->L; only
+ * groups->L and groups->W are read. */
+int vqb_decode_group_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_residual_levels* groups,
+                            int64_t K, int Dg, void* z_out, int out_dtype, int* bad_count, void* stream);
 
 /* ---- compatibility mode: the materialised distance matrix ---------------------------------- *
  * out[n, k] = torch.cdist(x, W)[n, k]  (cosine = 0)         vq/algorithms/vq/distances.py:28-32

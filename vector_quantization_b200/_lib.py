@@ -90,6 +90,13 @@ SIGNATURES = {
                                       c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_residual_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
                                            c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_group_gather_ste_loss': (c_int, [c_void_p, c_int, c_int64, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
+                                          c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p,
+                                          c_void_p]),
+    'vqb_group_backward': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p, c_int64,
+                                   c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_group_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
+                                        c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_segment_chunk': (c_int64, []),
     'vqb_code_sort_scratch_bytes': (c_size_t, [c_int64, c_int64]),
     'vqb_code_sort': (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_size_t,
@@ -118,6 +125,9 @@ SIGNATURES = {
                                       c_void_p]),
     'vqb_decode_residual_tokens': (c_int, [c_void_p, c_int, c_int64, c_int64, POINTER(ResidualLevels), c_int64, c_int,
                                            c_void_p, c_int, c_void_p, c_void_p]),
+    'vqb_decode_group_tokens': (c_int, [c_void_p, c_int, c_int64, c_int64, POINTER(ResidualLevels), c_int64, c_int,
+                                        c_void_p, c_int, c_void_p, c_void_p]),
+    'vqb_split_groups': (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_int64, c_void_p, c_void_p]),
     'vqb_distance_matrix': (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     'vqb_comm_alloc': (c_int, [c_size_t, POINTER(c_void_p), POINTER(c_ubyte)]),
     'vqb_comm_open': (c_int, [POINTER(c_ubyte), POINTER(c_void_p)]),

@@ -80,6 +80,51 @@ __global__ void __launch_bounds__(256) transpose_last2_vec_kernel(const T* __res
   }
 }
 
+// ---- grouped quantization: latents -> one contiguous [N, Dg] token slice per group ---------------------------------
+// src [batch][G*Dg][hw] -> dst [G][batch*hw][Dg].  A block takes one band of kTile spatial positions of one image
+// (blockIdx.x) and strides over the channel tiles (blockIdx.y, gridDim.y); the loads run along hw, the stores along
+// the channels of a token, which are contiguous within a group.
+template <typename T>
+__global__ void __launch_bounds__(kTile * 8) split_groups_kernel(const T* __restrict__ src, int64_t hw,
+                                                                 int64_t bands_per_image, int D, int Dg, int64_t N,
+                                                                 T* __restrict__ dst) {
+  __shared__ T tile[kTile][kTile + 1];
+  const unsigned band = (unsigned)bands_per_image;   // the grid has fewer than 2^31 blocks: 32-bit division
+  const int64_t b = blockIdx.x / band;
+  const int64_t s0 = (int64_t)(blockIdx.x - (unsigned)b * band) * kTile;
+  const int tx = threadIdx.x, ty = threadIdx.y;
+  for (int c0 = blockIdx.y * kTile; c0 < D; c0 += gridDim.y * kTile) {
+#pragma unroll
+    for (int i = ty; i < kTile; i += 8) {
+      const int c = c0 + i;
+      const int64_t s = s0 + tx;
+      if (c < D && s < hw) tile[i][tx] = src[(b * D + c) * hw + s];
+    }
+    __syncthreads();
+#pragma unroll
+    for (int i = ty; i < kTile; i += 8) {
+      const int c = c0 + tx;
+      const int64_t s = s0 + i;
+      if (c < D && s < hw) {
+        const int g = c / Dg;
+        dst[((int64_t)g * N + b * hw + s) * Dg + (c - g * Dg)] = tile[tx][i];
+      }
+    }
+    __syncthreads();
+  }
+}
+
+// Token-major src [N][G*Dg] (hw = 1): element (or, with T = uint4, 16-byte vector) i of a row goes to its group's row.
+template <typename T>
+__global__ void split_groups_rows_kernel(const T* __restrict__ src, int64_t N, int D, int Dg, T* __restrict__ dst) {
+  const int64_t total = N * D;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t n = i / D;
+    const int c = (int)(i - n * D), g = c / Dg;
+    dst[((int64_t)g * N + n) * Dg + (c - g * Dg)] = src[i];
+  }
+}
+
 // ---- token ids -> NCHW latents (decode_from_quant, vq/tasks/image_reconstruction/models.py:97-108) ----------------
 // The transpose above with a different load stage: the "source row" of spatial position s is the codebook row of its
 // token id.  A row source provides
@@ -174,6 +219,44 @@ struct ResidualRowSource {   // RQ-VAE codes: token n's ids are ids[n*L .. n*L +
       }
     }
     return s;
+  }
+};
+
+template <typename TI>
+struct GroupRowSource {      // product codes: token n's ids are ids[n*G .. n*G + G); channel g*Dg + d = W_g[id_g][d]
+  const TI* __restrict__ ids;
+  const float* W[VQB_MAX_LEVELS];   // read through `book` (unrolled constant indices): the struct stays in the parameter bank
+  int G;
+  int64_t K;
+  int Dg;
+  int D;                     // G * Dg
+  bool vec;                  // Dg % 4 == 0 and every W_g 16-byte aligned: a quad lies inside one group
+  __device__ __forceinline__ int64_t code(int64_t n) const {   // n when all G ids are in [0, K), else -1
+    bool ok = true;
+#pragma unroll
+    for (int g = 0; g < VQB_MAX_LEVELS; ++g)
+      if (g < G) ok = ok && checked_id(ids, n * G + g, K) >= 0;
+    return ok ? n : -1;
+  }
+  __device__ __forceinline__ const float* book(int g) const {
+    const float* w = W[0];
+#pragma unroll
+    for (int k = 1; k < VQB_MAX_LEVELS; ++k)
+      if (k == g) w = W[k];
+    return w;
+  }
+  __device__ __forceinline__ float value(int64_t code, int c) const {   // channel c of the token's row
+    if (c >= D) return 0.f;
+    const int g = c / Dg;
+    return __ldg(book(g) + (int64_t)ids[code * G + g] * Dg + (c - g * Dg));
+  }
+  __device__ __forceinline__ float4 quad(int64_t code, int c) const {
+    if (code < 0) return make_float4(kNaN, kNaN, kNaN, kNaN);
+    if (vec) {
+      const int g = c / Dg;
+      return __ldg(reinterpret_cast<const float4*>(book(g) + (int64_t)ids[code * G + g] * Dg + (c - g * Dg)));
+    }
+    return make_float4(value(code, c), value(code, c + 1), value(code, c + 2), value(code, c + 3));
   }
 };
 
@@ -417,6 +500,75 @@ int vqb_decode_residual_tokens(const void* ids, int id_bytes, int64_t batch, int
   }
   VQB_RESIDUAL_SRC(int64_t)
 #undef VQB_RESIDUAL_SRC
+}
+
+int vqb_decode_group_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_residual_levels* lv,
+                            int64_t K, int Dg, void* z_out, int out_dtype, int* bad_count, void* stream) {
+  if (int e = check_decode_args("vqb_decode_group_tokens", ids, id_bytes, batch, hw, z_out, out_dtype)) return e;
+  VQB_REQUIRE(lv, "vqb_decode_group_tokens: null groups");
+  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "vqb_decode_group_tokens: G=%d outside [1, %d]", lv->L,
+              VQB_MAX_LEVELS);
+  VQB_REQUIRE(K >= 1 && Dg >= 1 && (int64_t)Dg * lv->L <= 0x7fffffff, "vqb_decode_group_tokens: bad codebook shape");
+  bool aligned = true;
+  for (int g = 0; g < lv->L; ++g) {
+    VQB_REQUIRE(lv->W[g], "vqb_decode_group_tokens: null codebook of group %d", g);
+    aligned = aligned && (uintptr_t)lv->W[g] % 16 == 0;
+  }
+  if (batch == 0 || hw == 0) return VQB_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = Dg * lv->L;
+  const bool vec = Dg % 4 == 0 && aligned;
+#define VQB_GROUP_SRC(TI_) \
+  GroupRowSource<TI_> src{(const TI_*)ids, {}, lv->L, K, Dg, D, vec};                                               \
+  for (int g = 0; g < lv->L; ++g) src.W[g] = lv->W[g];                                                              \
+  return launch_decode_tokens_for_width(src, batch, hw, D, z_out, out_dtype, bad_count, st);
+  if (id_bytes == 2) {
+    VQB_GROUP_SRC(uint16_t)
+  }
+  if (id_bytes == 4) {
+    VQB_GROUP_SRC(int32_t)
+  }
+  VQB_GROUP_SRC(int64_t)
+#undef VQB_GROUP_SRC
+}
+
+int vqb_split_groups(const void* src, int dtype, int64_t batch, int G, int Dg, int64_t hw, void* dst, void* stream) {
+  VQB_REQUIRE(src && dst, "vqb_split_groups: null pointer");
+  VQB_REQUIRE(src != dst, "vqb_split_groups: in-place split is not supported");
+  VQB_REQUIRE(dtype == VQB_F32 || dtype == VQB_BF16, "vqb_split_groups: dtype must be VQB_F32 or VQB_BF16");
+  VQB_REQUIRE(G >= 1 && G <= VQB_MAX_LEVELS, "vqb_split_groups: G=%d outside [1, %d]", G, VQB_MAX_LEVELS);
+  VQB_REQUIRE(Dg >= 1 && (int64_t)Dg * G <= 0x7fffffff && batch >= 0 && hw >= 1, "vqb_split_groups: bad shape");
+  if (batch == 0) return VQB_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = G * Dg, eb = dtype == VQB_F32 ? 4 : 2;
+  const int64_t N = batch * hw;
+  if (hw == 1) {
+    const int ve = 16 / eb;
+    const bool vec = Dg % ve == 0 && (uintptr_t)src % 16 == 0 && (uintptr_t)dst % 16 == 0;
+    const int64_t items = vec ? N * D / ve : N * D;
+    int64_t blocks = (items + 255) / 256;
+    if (blocks > (int64_t)sm_count() * 16) blocks = (int64_t)sm_count() * 16;
+    if (vec)
+      split_groups_rows_kernel<uint4><<<(unsigned)blocks, 256, 0, st>>>((const uint4*)src, N, D / ve, Dg / ve, (uint4*)dst);
+    else if (eb == 4)
+      split_groups_rows_kernel<uint32_t><<<(unsigned)blocks, 256, 0, st>>>((const uint32_t*)src, N, D, Dg, (uint32_t*)dst);
+    else
+      split_groups_rows_kernel<uint16_t><<<(unsigned)blocks, 256, 0, st>>>((const uint16_t*)src, N, D, Dg, (uint16_t*)dst);
+    VQB_LAUNCH_OK();
+    return VQB_OK;
+  }
+  const int64_t per_image = (hw + kTile - 1) / kTile, bands = per_image * batch;
+  VQB_REQUIRE(bands <= 0x7fffffff, "vqb_split_groups: too many tokens (batch * ceil(hw / %d) must be < 2^31)", kTile);
+  const int64_t ct = (D + kTile - 1) / kTile;
+  int64_t gy = ((int64_t)sm_count() * 16 + bands - 1) / bands;   // enough blocks for ~2 waves, as the transpose
+  gy = gy > ct ? ct : (gy < 1 ? 1 : gy);
+  const dim3 grid((unsigned)bands, (unsigned)gy), block(kTile, 8);
+  if (eb == 4)
+    split_groups_kernel<uint32_t><<<grid, block, 0, st>>>((const uint32_t*)src, hw, per_image, D, Dg, N, (uint32_t*)dst);
+  else
+    split_groups_kernel<uint16_t><<<grid, block, 0, st>>>((const uint16_t*)src, hw, per_image, D, Dg, N, (uint16_t*)dst);
+  VQB_LAUNCH_OK();
+  return VQB_OK;
 }
 
 int vqb_fsq_decode_tokens(const void* ids, int id_bytes, int64_t batch, int64_t hw, const vqb_fsq_params* p_host,

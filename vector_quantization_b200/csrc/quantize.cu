@@ -586,6 +586,202 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
   }
 }
 
+// ---- grouped quantization ------------------------------------------------------------------------------------------
+// quantize_forward_kernel (without token normalisation) for group g = blockIdx.y on its contiguous slice
+// xs + g*N*Dg: the same per-token arithmetic, grid (gridDim.x) and loss fold as a standalone launch on (N, Dg), with
+// group g's own partials and ticket.  z goes to channels [g*Dg, (g+1)*Dg) of the full-width output; the slice
+// stores stay inside the group because d0 < Dg and V divides Dg whenever V > 1.
+template <typename TX, int G, int V, int NV>
+__global__ void __launch_bounds__(256) group_forward_kernel(
+    const TX* __restrict__ xs, int64_t N, int Dg, const __grid_constant__ vqb_residual_levels lv, int64_t K,
+    const int64_t* __restrict__ quant, const unsigned long long* __restrict__ keys, int64_t* __restrict__ quant_out,
+    float* __restrict__ z_out, int64_t z_hw, int want_norm, float* __restrict__ mse4, float* __restrict__ partials,
+    unsigned int* __restrict__ tickets) {
+  __shared__ float sh[16];
+  pdl_wait();               // keys / codebooks come from the preceding launches of the step
+  pdl_launch_dependents();
+  const int grp = blockIdx.y, groups = lv.L;
+  const int64_t D = (int64_t)groups * Dg;
+  const TX* __restrict__ x = xs + grp * N * Dg;
+  const float* __restrict__ W = lv.W[grp];
+  const int64_t* __restrict__ gq = quant ? quant + grp * N : nullptr;
+  const unsigned long long* __restrict__ gk = keys ? keys + grp * N : nullptr;
+  float* __restrict__ zg = z_hw > 0 ? z_out + grp * Dg * z_hw : z_out + grp * Dg;
+  const int lane = threadIdx.x % G;
+  const int64_t rows_per_block = blockDim.x / G;
+  float sse = 0.f, sse_n = 0.f;
+  for (int64_t base = blockIdx.x * rows_per_block; base < N; base += (int64_t)gridDim.x * rows_per_block) {
+    const int64_t n_raw = base + threadIdx.x / G;  // warp-uniform trip count: shuffles need every lane
+    const bool valid = n_raw < N;
+    const int64_t n = valid ? n_raw : N - 1;
+    const int64_t q = row_index(gq, gk, n, 0, K);
+    const float* __restrict__ wrow = W + q * Dg;
+    const TX* __restrict__ xrow = x + n * Dg;
+    float xr[NV][V], wr[NV][V];
+    float sxx = 0.f, sww = 0.f;
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      if (d0 < Dg) {
+        load_slice<TX, V>(xrow, d0, Dg, xr[it]);
+        load_slice<float, V>(wrow, d0, Dg, wr[it]);
+      } else {
+#pragma unroll
+        for (int i = 0; i < V; ++i) xr[it][i] = wr[it][i] = 0.f;
+      }
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        sxx = fmaf(xr[it][i], xr[it][i], sxx);
+        sww = fmaf(wr[it][i], wr[it][i], sww);
+      }
+    }
+    float rdx = 1.f, rdw = 1.f;
+    if (want_norm) {
+      sxx = group_sum<G>(sxx);
+      sww = group_sum<G>(sww);
+      rdx = 1.f / fmaxf(sqrtf(sxx), kNormEps);
+      rdw = 1.f / fmaxf(sqrtf(sww), kNormEps);
+    }
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      float zr[V];
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        const float diff = __fsub_rn(wr[it][i], xr[it][i]);
+        zr[i] = __fadd_rn(xr[it][i], diff);  // ste value: x + (z - x)
+        if (valid) sse = fmaf(diff, diff, sse);
+        if (want_norm) {
+          const float dn = wr[it][i] * rdw - xr[it][i] * rdx;
+          if (valid) sse_n = fmaf(dn, dn, sse_n);
+        }
+      }
+      if (valid && d0 < Dg) {
+        if (z_hw > 0) store_slice_nchw<float, V>(zg, n, z_hw, d0, (int)D, zr);
+        else store_slice<float, V>(zg + n * D, d0, Dg, zr);
+      }
+    }
+    if (quant_out && valid && lane == 0) quant_out[n * groups + grp] = q;
+  }
+  finish_mse4(sse, sse_n, N, Dg, mse4 + 4 * grp, partials + (int64_t)grp * 2 * kMaxPartials, tickets + grp, sh);
+}
+
+// quantize_backward_kernel (without token normalisation) for group g = blockIdx.y: x_g from the split buffer,
+// W_g / gW_g / the four loss-gradient scalars from the group table, q_g = quant[n*G + g]; g_z and gx are the
+// full-width tensors at channel offset g*Dg.
+template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut>
+__global__ void __launch_bounds__(256) group_backward_kernel(
+    const TG* __restrict__ gz, const TX* __restrict__ xs, const __grid_constant__ vqb_residual_levels lv, int64_t K,
+    const int64_t* __restrict__ quant, int64_t N, int Dg, int want_norm, TX* __restrict__ gx, int64_t g_hw) {
+  pdl_wait();               // upstream gradients / indices come from the preceding launches
+  pdl_launch_dependents();
+  const int grp = blockIdx.y, groups = lv.L;
+  const int64_t D = (int64_t)groups * Dg;
+  const TX* __restrict__ x = xs + grp * N * Dg;
+  const float* __restrict__ W = lv.W[grp];
+  float* __restrict__ gW = lv.gW[grp];
+  const TG* __restrict__ gzg = g_hw > 0 ? gz + grp * Dg * g_hw : gz + grp * Dg;
+  TX* __restrict__ gxg = g_hw > 0 ? gx + grp * Dg * g_hw : gx + grp * Dg;
+  const int lane = threadIdx.x % G;
+  const int64_t rows_per_block = blockDim.x / G;
+  const float scale = 2.f / ((float)N * (float)Dg);
+  const float* __restrict__ g_cb = lv.g[grp][0];
+  const float* __restrict__ g_cm = lv.g[grp][1];
+  const float* __restrict__ g_cbn = lv.g[grp][2];
+  const float* __restrict__ g_cmn = lv.g[grp][3];
+  const float c_cb = g_cb ? *g_cb * scale : 0.f, c_cm = g_cm ? *g_cm * scale : 0.f;
+  const float c_cbn = (want_norm && g_cbn) ? *g_cbn * scale : 0.f, c_cmn = (want_norm && g_cmn) ? *g_cmn * scale : 0.f;
+  for (int64_t base = blockIdx.x * rows_per_block; base < N; base += (int64_t)gridDim.x * rows_per_block) {
+    const int64_t n_raw = base + threadIdx.x / G;
+    const bool valid = n_raw < N;
+    const int64_t n = valid ? n_raw : N - 1;
+    const int64_t q = row_index(quant, nullptr, n * groups + grp, 0, K);
+    const float* __restrict__ wrow = W + q * Dg;
+    const TX* __restrict__ xrow = x + n * Dg;
+    float yr[NV][V], wr[NV][V], gr[NV][V];
+    float sxx = 0.f, sww = 0.f;
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      if (d0 < Dg) {
+        load_slice<TX, V>(xrow, d0, Dg, yr[it]);
+        load_slice<float, V>(wrow, d0, Dg, wr[it]);
+        if (g_hw > 0) load_slice_nchw<TG, V>(gzg, n, g_hw, d0, (int)D, gr[it]);
+        else load_slice<TG, V>(gzg + n * D, d0, Dg, gr[it]);
+      } else {
+#pragma unroll
+        for (int i = 0; i < V; ++i) yr[it][i] = wr[it][i] = gr[it][i] = 0.f;
+      }
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        sxx = fmaf(yr[it][i], yr[it][i], sxx);
+        sww = fmaf(wr[it][i], wr[it][i], sww);
+      }
+    }
+    float dy = 1.f, dw = 1.f, uu = 0.f, vv = 0.f, uv = 0.f;
+    bool cy = false, cw = false;
+    if (want_norm) {
+      float syw = 0.f;
+#pragma unroll
+      for (int it = 0; it < NV; ++it)
+#pragma unroll
+        for (int i = 0; i < V; ++i) syw = fmaf(yr[it][i], wr[it][i], syw);
+      sxx = group_sum<G>(sxx);
+      sww = group_sum<G>(sww);
+      syw = group_sum<G>(syw);
+      const float ny = sqrtf(sxx), nw = sqrtf(sww);
+      cy = ny < kNormEps;
+      cw = nw < kNormEps;
+      dy = 1.f / fmaxf(ny, kNormEps);   // reciprocal norms
+      dw = 1.f / fmaxf(nw, kNormEps);
+      uu = sxx * dy * dy;
+      vv = sww * dw * dw;
+      uv = syw * dy * dw;
+    }
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      float gw[V];
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        const float yv = yr[it][i], wv = wr[it][i];
+        float g_y = gr[it][i] + c_cm * (yv - wv);
+        float g_w = c_cb * (wv - yv);
+        if (want_norm) {
+          const float u = yv * dy, v = wv * dw;
+          const float gu = c_cmn * (u - v), gu_dot_u = c_cmn * (uu - uv);
+          g_y += (gu - (cy ? 0.f : gu_dot_u * u)) * dy;
+          const float gv = c_cbn * (v - u), gv_dot_v = c_cbn * (vv - uv);
+          g_w += (gv - (cw ? 0.f : gv_dot_v * v)) * dw;
+        }
+        gr[it][i] = g_y;
+        gw[i] = g_w;
+      }
+      if constexpr (kRowsOut) {
+        if (valid && d0 < Dg) store_slice<float, V>(gW + n * Dg, d0, Dg, gw);
+      } else if (gW && valid && d0 < Dg) {
+        float* dst = gW + q * Dg + d0;
+        if constexpr (V == 8) {
+          atomicAdd(reinterpret_cast<float4*>(dst), make_float4(gw[0], gw[1], gw[2], gw[3]));
+          atomicAdd(reinterpret_cast<float4*>(dst + 4), make_float4(gw[4], gw[5], gw[6], gw[7]));
+        } else {
+#pragma unroll
+          for (int i = 0; i < V; ++i)
+            if (d0 + i < Dg) atomicAdd(dst + i, gw[i]);
+        }
+      }
+    }
+#pragma unroll
+    for (int it = 0; it < NV; ++it) {
+      const int d0 = (it * G + lane) * V;
+      if (valid && d0 < Dg) {
+        if (g_hw > 0) store_slice_nchw<TX, V>(gxg, n, g_hw, d0, (int)D, gr[it]);
+        else store_slice<TX, V>(gxg + n * D, d0, Dg, gr[it]);
+      }
+    }
+  }
+}
+
 __global__ void unpack_keys_kernel(const unsigned long long* __restrict__ keys, int64_t n, int64_t offset,
                                    int64_t* __restrict__ idx, float* __restrict__ score) {
   pdl_wait();               // PDL: inputs come from the preceding launches
@@ -838,6 +1034,92 @@ int vqb_residual_backward_rows(const void* gz, int g_dtype, const void* x, int x
                                int want_norm, void* gx, int64_t g_hw, void* stream) {
   return residual_backward_launch<true>("vqb_residual_backward_rows", gz, g_dtype, x, x_dtype, levels, K, quant, N, D,
                                         want_norm, gx, g_hw, stream);
+}
+
+int vqb_group_gather_ste_loss(const void* xs, int x_dtype, int64_t N, int Dg, const vqb_residual_levels* lv, int64_t K,
+                              const int64_t* quant, const unsigned long long* keys, int64_t* quant_out, float* z_out,
+                              int64_t z_hw, int want_norm, float* mse4, float* partials, unsigned int* tickets,
+                              void* stream) {
+  VQB_REQUIRE(z_hw >= 0 && (z_hw == 0 || N % z_hw == 0),
+              "vqb_group_gather_ste_loss: z_hw must divide N (tokens = images x h*w)");
+  VQB_REQUIRE(xs && lv && z_out && mse4 && partials && tickets, "vqb_group_gather_ste_loss: null pointer");
+  VQB_REQUIRE((quant != nullptr) != (keys != nullptr), "vqb_group_gather_ste_loss: pass exactly one of quant / keys");
+  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "vqb_group_gather_ste_loss: G=%d outside [1, %d]", lv->L,
+              VQB_MAX_LEVELS);
+  for (int g = 0; g < lv->L; ++g) VQB_REQUIRE(lv->W[g], "vqb_group_gather_ste_loss: null codebook of group %d", g);
+  VQB_REQUIRE(N >= 1 && Dg >= 1 && K >= 1, "vqb_group_gather_ste_loss: bad shape N=%lld Dg=%d K=%lld", (long long)N, Dg,
+              (long long)K);
+  RowGeom geom;
+  VQB_REQUIRE(row_geom(Dg, N, &geom),
+              "vqb_group_gather_ste_loss: Dg=%d unsupported (multiple of 8 up to 2048, or any Dg <= 256)", Dg);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int blocks = grid_for(N, 256 / geom.G);   // per group: the grid of vqb_gather_ste_loss on (N, Dg)
+  VQB_REQUIRE(blocks <= kMaxPartials, "vqb_group_gather_ste_loss: grid too large");
+  const dim3 grid((unsigned)blocks, (unsigned)lv->L);
+  bool launched = false;
+#define VQB_GROUP_FWD(TX_)                                                                                           \
+  VQB_DISPATCH_GEOM((launch_pdl(group_forward_kernel<TX_, G, V, NV>, grid, 256, 0, st, (const TX_*)xs, N, Dg, *lv, K, \
+      quant, keys, quant_out, z_out, z_hw, want_norm, mse4, partials, tickets)))
+  if (x_dtype == VQB_F32) {
+    VQB_GROUP_FWD(float)
+  } else if (x_dtype == VQB_BF16) {
+    VQB_GROUP_FWD(__nv_bfloat16)
+  }
+#undef VQB_GROUP_FWD
+  VQB_REQUIRE(launched, "vqb_group_gather_ste_loss: unsupported dtype/geometry");
+  VQB_LAUNCH_OK();
+  return VQB_OK;
+}
+
+}  // extern "C"
+
+template <bool kRowsOut>
+static int group_backward_launch(const char* fn, const void* gz, int g_dtype, const void* xs, int x_dtype,
+                                 const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int Dg,
+                                 int want_norm, void* gx, int64_t g_hw, void* stream) {
+  VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
+  VQB_REQUIRE(gz && xs && lv && quant && gx, "%s: null pointer", fn);
+  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "%s: G=%d outside [1, %d]", fn, lv->L, VQB_MAX_LEVELS);
+  for (int g = 0; g < lv->L; ++g) {
+    VQB_REQUIRE(lv->W[g], "%s: null codebook of group %d", fn, g);
+    VQB_REQUIRE(!kRowsOut || lv->gW[g], "%s: null gradient rows of group %d", fn, g);
+  }
+  VQB_REQUIRE(N >= 1 && Dg >= 1 && K >= 1, "%s: bad shape", fn);
+  RowGeom geom;
+  VQB_REQUIRE(row_geom(Dg, N, &geom), "%s: Dg=%d unsupported", fn, Dg);
+  cudaStream_t st = (cudaStream_t)stream;
+  const dim3 grid((unsigned)grid_for(N, 256 / geom.G), (unsigned)lv->L);
+  bool launched = false;
+#define VQB_GROUP_BWD(TX_, TG_)                                                                                       \
+  VQB_DISPATCH_GEOM((launch_pdl(group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>, grid, 256, 0, st,               \
+      (const TG_*)gz, (const TX_*)xs, *lv, K, quant, N, Dg, want_norm, (TX_*)gx, g_hw)))
+  if (x_dtype == VQB_F32 && g_dtype == VQB_F32) {
+    VQB_GROUP_BWD(float, float)
+  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_F32) {
+    VQB_GROUP_BWD(__nv_bfloat16, float)
+  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_BF16) {
+    VQB_GROUP_BWD(__nv_bfloat16, __nv_bfloat16)
+  }
+#undef VQB_GROUP_BWD
+  VQB_REQUIRE(launched, "%s: unsupported dtype/geometry", fn);
+  VQB_LAUNCH_OK();
+  return VQB_OK;
+}
+
+extern "C" {
+
+int vqb_group_backward(const void* gz, int g_dtype, const void* xs, int x_dtype, const vqb_residual_levels* groups,
+                       int64_t K, const int64_t* quant, int64_t N, int Dg, int want_norm, void* gx, int64_t g_hw,
+                       void* stream) {
+  return group_backward_launch<false>("vqb_group_backward", gz, g_dtype, xs, x_dtype, groups, K, quant, N, Dg,
+                                      want_norm, gx, g_hw, stream);
+}
+
+int vqb_group_backward_rows(const void* gz, int g_dtype, const void* xs, int x_dtype, const vqb_residual_levels* groups,
+                            int64_t K, const int64_t* quant, int64_t N, int Dg, int want_norm, void* gx, int64_t g_hw,
+                            void* stream) {
+  return group_backward_launch<true>("vqb_group_backward_rows", gz, g_dtype, xs, x_dtype, groups, K, quant, N, Dg,
+                                     want_norm, gx, g_hw, stream);
 }
 
 int vqb_unpack_keys(const unsigned long long* keys, int64_t n, int64_t offset, int64_t* idx, float* score,

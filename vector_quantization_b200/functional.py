@@ -443,6 +443,87 @@ def residual_quantize(levels, x: torch.Tensor, memos, want_norm: bool, *, nchw: 
     return z, quant, [tuple(flat[4 * l:4 * l + 4]) for l in range(len(levels))]
 
 
+@torch.no_grad()
+def group_encode(groups, xs: torch.Tensor, memos, *, keys: torch.Tensor | None = None, track_codebooks: bool = False):
+    """The group loop of a grouped quantizer: group g runs its own `encode` (before_encode -> assignment ->
+    after_encode, codebook updates included) on its token slice xs[g] ([G, N, Dg] from `ops.split_groups`), its
+    assignment writing the packed keys straight into row g of ONE [G, N] buffer (`keys`, whose rows must be
+    contiguous; allocated when None).  memos[g] becomes group g's memo.
+    -> (keys int64 [G, N], [CodebookRef per group] of the codebooks as the encodes left them (registered with the
+    group when track_codebooks))"""
+    G, N, _ = xs.shape
+    if keys is None:
+        keys = torch.empty((G, N), dtype=torch.int64, device=xs.device)
+    refs = []
+    for g, group in enumerate(groups):
+        memo = memos[g]
+        memo['_keys_out'] = keys[g]
+        memo['_lazy_unpack'] = group._callbacks.packed_keys_ok()
+        group.encode(xs[g], memo)     # int64 indices only when a training callback reads them; the keys stay valid
+        ref = CodebookRef(group._weight().detach())
+        if track_codebooks:
+            group._pending.add(ref)
+        refs.append(ref)
+    return keys, refs
+
+
+class _GroupedQuantize(torch.autograd.Function):
+    """Every group of a grouped quantizer as ONE node: forward = `ops.split_groups` + the group loop (`group_encode`) +
+    one `vqb_group_gather_ste_loss` launch; backward = one `vqb_group_backward` launch for all groups (+ per-group code
+    sort / segment sum under the deterministic flag).  x is the tokens [N, D] or the NCHW latents [b, D, h, w]; z and
+    gx have x's layout.  Outputs z, quant [N, G] and the 4 G MSE terms as separate 0-dim tensors (their upstream
+    gradients arrive as device scalars); memos[g] gets 'x' (the split slice xs[g]) and 'quant' (quant[:, g])."""
+
+    @staticmethod
+    def forward(ctx, x, groups, memos, want_norm, track, *Ws):
+        G = len(groups)
+        nchw = x.dim() == 4
+        hw = x.shape[2] * x.shape[3] if nchw else 0
+        xd = x.detach()
+        xs = xd.view(1, *xd.shape) if (G == 1 and not nchw) else ops.split_groups(xd, G)
+        N = xs.shape[1]
+        keys, refs = group_encode(groups, xs, memos, track_codebooks=track)
+        z = torch.empty(tuple(x.shape), dtype=torch.float32, device=x.device)
+        quant = torch.empty((N, G), dtype=torch.int64, device=x.device)
+        _, mse = ops.group_gather_ste_loss(xs, [r.tensor for r in refs], keys=keys, want_norm=want_norm, quant_out=quant,
+                                           z_out=z, z_hw=hw)
+        for g, memo in enumerate(memos):
+            memo.update(x=xs[g], quant=quant[:, g])
+        ctx.save_for_backward(xs, quant)
+        ctx.refs = refs
+        ctx.shape = tuple(x.shape)
+        ctx.hw = hw
+        ctx.want_norm = want_norm
+        ctx.set_materialize_grads(False)
+        ctx.mark_non_differentiable(quant)
+        return (z, quant) + tuple(mse.view(-1).unbind(0))
+
+    @staticmethod
+    def backward(ctx, gz, _gq, *g):
+        xs, quant = ctx.saved_tensors
+        G = xs.shape[0]
+        if gz is None:
+            gz = torch.zeros(ctx.shape, dtype=torch.float32, device=xs.device)
+        g4s = [[None if t is None else t.contiguous().float() for t in g[4 * i:4 * i + 4]] for i in range(G)]
+        need_gW = list(ctx.needs_input_grad[5:5 + G])
+        gx, gWs = ops.group_backward(gz.contiguous(), xs, [r.tensor for r in ctx.refs], quant, g4s,
+                                     want_norm=ctx.want_norm, need_gW=need_gW, g_hw=ctx.hw)
+        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, *gWs)
+
+
+def grouped_quantize(groups, x: torch.Tensor, memos, want_norm: bool):
+    """Grouped quantization of x (tokens [N, D] or latents [b, D, h, w]; fp32 / bf16) through `groups` (VectorQuantizer
+    modules sharing K and Dg = D / G), group g on channels [g*Dg, (g+1)*Dg).
+    -> (z fp32 in x's layout: value x_g + (W_g[q_g] - x_g) per group, gradient straight to x;  quant int64 [N, G];
+        mse: per group the four MSE terms (codebook, commitment, codebook-norm,
+        commitment-norm) of W_g[q_g] against x_g, 0-dim tensors whose gradients reach W_g and x)"""
+    Ws = [group._weight() for group in groups]
+    track = torch.is_grad_enabled() and (x.requires_grad or any(W.requires_grad for W in Ws))
+    out = _GroupedQuantize.apply(x.contiguous(), list(groups), memos, bool(want_norm), track, *Ws)
+    z, quant, flat = out[0], out[1], out[2:]
+    return z, quant, [tuple(flat[4 * i:4 * i + 4]) for i in range(len(groups))]
+
+
 class _FSQ(torch.autograd.Function):
 
     @staticmethod

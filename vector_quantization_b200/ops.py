@@ -22,6 +22,7 @@ __all__ = [
     'deterministic_enabled', 'segment_chunk', 'code_sort', 'segment_sum_rows',
     'kmeans_ema_update', 'gather_rows_by_key', 'cvq_update', 'embedding_gather', 'fsq_params', 'fsq_forward', 'fsq_backward',
     'fsq_decode', 'decode_tokens', 'fsq_decode_tokens', 'residual_step', 'residual_backward', 'decode_residual_tokens',
+    'split_groups', 'group_gather_ste_loss', 'group_backward', 'decode_group_tokens',
     'transpose_last2', 'compact_tokens', 'distance_matrix', 'comm_kmeans_ema_update', 'comm_cvq_update',
     'comm_allreduce_min_keys', 'comm_allreduce_sum_f32', 'BACKEND_TCGEN05', 'BACKEND_SIMT',
 ]
@@ -860,4 +861,120 @@ def decode_residual_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtyp
     p = _residual_levels(Ws)
     _call('vqb_decode_residual_tokens', lib.vqb_decode_residual_tokens, dev, _p(ids), id_bytes, b, hw, ctypes.byref(p),
           K, D, _p(z), _dt(z), _p(bad_count), _S)
+    return z
+
+
+# ---- grouped (product) quantization (csrc/quantize.cu, csrc/layout.cu) ---------------------------------------------
+
+
+def _group_codebooks(Ws) -> tuple[int, int]:
+    if not 1 <= len(Ws) <= MAX_LEVELS:
+        raise ValueError(f'grouped quantization takes 1..{MAX_LEVELS} groups, got {len(Ws)}')
+    return _codebooks(Ws)
+
+
+def split_groups(x: torch.Tensor, G: int) -> torch.Tensor:
+    """Latents [b, G*Dg, h, w] or tokens [N, G*Dg] (fp32 / bf16) -> [G, N, Dg] in one launch (vqb_split_groups): group g
+    is the contiguous token slice x_g, N = b*h*w tokens in `b h w` order."""
+    lib = _lib.load()
+    dev = _cuda(x)
+    if x.dim() not in (2, 4):
+        raise ValueError(f'expected latents [b, c, h, w] or tokens [N, c], got {tuple(x.shape)}')
+    if not 1 <= G <= MAX_LEVELS or x.shape[1] % G:
+        raise ValueError(f'{x.shape[1]} channels do not split into {G} groups (1 <= G <= {MAX_LEVELS})')
+    b, D = x.shape[0], x.shape[1]
+    hw = x.shape[2] * x.shape[3] if x.dim() == 4 else 1
+    out = torch.empty((G, b * hw, D // G), dtype=x.dtype, device=x.device)
+    _call('vqb_split_groups', lib.vqb_split_groups, dev, _p(x), _dt(x), b, G, D // G, hw, _p(out), _S)
+    return out
+
+
+def _group_loss_ws(device):
+    """Per-group partials + self-resetting tickets of the loss reduction (MAX_LEVELS groups), one set per
+    (device, stream) like `_loss_ws`."""
+    key = (device.index, torch.cuda.current_stream(device).cuda_stream, 'groups')
+    if key not in _WS:
+        lib = _lib.load()
+        _WS[key] = (torch.empty((MAX_LEVELS * int(lib.vqb_loss_partials_count()),), dtype=torch.float32, device=device),
+                    torch.zeros((MAX_LEVELS,), dtype=torch.int32, device=device))
+    return _WS[key]
+
+
+def group_gather_ste_loss(xs: torch.Tensor, Ws, *, quant: torch.Tensor | None = None, keys: torch.Tensor | None = None,
+                          want_norm: bool, quant_out: torch.Tensor | None = None, z_out: torch.Tensor | None = None,
+                          z_hw: int = 0):
+    """Every group's gather + STE + loss in one launch (vqb_group_gather_ste_loss).  xs: split tokens [G, N, Dg];
+    quant (int64) or keys (packed): group-major [G, N].  quant_out: optional int64 [N, G]; z_out: fp32 [N, G*Dg], or
+    NCHW [b, G*Dg, h, w] with z_hw = h*w (allocated token-major when None).  -> (z, mse fp32 [G, 4])"""
+    lib = _lib.load()
+    dev = _cuda(xs, quant, keys, quant_out, z_out, *Ws)
+    K, Dg = _group_codebooks(Ws)
+    G, N = len(Ws), xs.shape[1]
+    if xs.dim() != 3 or tuple(xs.shape) != (G, N, Dg):
+        raise ValueError(f'expected split tokens [{G}, N, {Dg}], got {tuple(xs.shape)}')
+    index = quant if quant is not None else keys
+    assert (quant is None) != (keys is None) and index.dtype == torch.int64 and index.shape == (G, N)
+    assert quant_out is None or (quant_out.dtype == torch.int64 and quant_out.shape == (N, G))
+    if z_out is None:
+        z_out = torch.empty((N, G * Dg), dtype=torch.float32, device=xs.device)
+    assert z_out.dtype == torch.float32 and z_out.numel() == N * G * Dg
+    mse = torch.empty((G, 4), dtype=torch.float32, device=xs.device)
+    partials, tickets = _group_loss_ws(xs.device)
+    p = _residual_levels(Ws)
+    _call('vqb_group_gather_ste_loss', lib.vqb_group_gather_ste_loss, dev, _p(xs), _dt(xs), N, Dg, ctypes.byref(p), K,
+          _p(quant), _p(keys), _p(quant_out), _p(z_out), z_hw, int(want_norm), _p(mse), _p(partials), _p(tickets), _S)
+    return z_out, mse
+
+
+def group_backward(g_z: torch.Tensor, xs: torch.Tensor, Ws, quant: torch.Tensor, g4s, *, want_norm: bool, need_gW,
+                   g_hw: int = 0, deterministic: bool | None = None):
+    """Backward of every group in one launch (vqb_group_backward).  g_z: fp32 (or bf16 with bf16 tokens) [N, G*Dg], or
+    NCHW with g_hw = h*w (gx then has g_z's NCHW shape); xs: the forward's split tokens [G, N, Dg]; quant: int64 [N, G];
+    g4s: per group four 0-dim fp32 device tensors / None; need_gW: per group bool.
+    deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, each gW_g is the segment sum of
+    the group's per-token rows (vqb_group_backward_rows + vqb_code_sort + vqb_segment_sum_rows, the contract of
+    quantize_backward).  -> (gx in xs's dtype with g_z's shape, [gW_g fp32 [K, Dg] or None])"""
+    lib = _lib.load()
+    G = len(Ws)
+    dev = _cuda(g_z, xs, quant, *Ws, *[g for g4 in g4s for g in g4])
+    K, Dg = _group_codebooks(Ws)
+    N = xs.shape[1]
+    assert tuple(xs.shape) == (G, N, Dg) and quant.dtype == torch.int64 and quant.shape == (N, G) and len(g4s) == G
+    assert g_z.numel() == N * G * Dg and all(g is None or g.dtype == torch.float32 for g4 in g4s for g in g4)
+    if not (g_z.dtype == torch.float32 or (g_z.dtype == torch.bfloat16 and xs.dtype == torch.bfloat16)):
+        g_z = g_z.float()
+    gx = torch.empty(g_z.shape, dtype=xs.dtype, device=xs.device)
+    gWs = [torch.zeros_like(W) if need else None for W, need in zip(Ws, need_gW)]
+    if any(need_gW) and deterministic_enabled(deterministic):
+        rows = _det_ws(xs.device, 'gw_rows', G * N * Dg, torch.float32).view(G, N, Dg)
+        p = _residual_levels(Ws, list(rows), g4s)
+        _call('vqb_group_backward_rows', lib.vqb_group_backward_rows, dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs),
+              ctypes.byref(p), K, _p(quant), N, Dg, int(want_norm), _p(gx), g_hw, _S)
+        by_group = quant.view(G, N) if G == 1 else transpose_last2(quant.view(1, N, G)).view(G, N)
+        for g, gW in enumerate(gWs):
+            if gW is not None:
+                order, offsets = _code_sort_ws(dev, N, K, by_group[g], None, 0)
+                _segment_sum(dev, rows[g], N, Dg, False, order, offsets, K, gW, None)
+        return gx, gWs
+    p = _residual_levels(Ws, gWs, g4s)
+    _call('vqb_group_backward', lib.vqb_group_backward, dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs), ctypes.byref(p), K,
+          _p(quant), N, Dg, int(want_norm), _p(gx), g_hw, _S)
+    return gx, gWs
+
+
+def decode_group_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtype = torch.float32,
+                        bad_count: torch.Tensor | None = None) -> torch.Tensor:
+    """Grouped token ids [b, h, w, G] (uint16 / int32 / int64; a token's G ids contiguous) -> z with channels
+    [g*Dg, (g+1)*Dg) = W_g[id_g], as [b, G*Dg, h, w] of `out_dtype`, in one launch (vqb_decode_group_tokens).  A token
+    with an id outside [0, K) in any group gives a NaN row and is counted once into `bad_count`."""
+    lib = _lib.load()
+    dev = _cuda(ids, bad_count, *Ws)
+    K, Dg = _group_codebooks(Ws)
+    G = len(Ws)
+    if ids.dim() < 2 or ids.shape[-1] != G:
+        raise ValueError(f'expected grouped token ids with a trailing group axis of {G}, got {tuple(ids.shape)}')
+    b, id_bytes, z = _decode_out(ids.select(-1, 0), hw, G * Dg, out_dtype, bad_count)
+    p = _residual_levels(Ws)
+    _call('vqb_decode_group_tokens', lib.vqb_decode_group_tokens, dev, _p(ids), id_bytes, b, hw, ctypes.byref(p), K, Dg,
+          _p(z), _dt(z), _p(bad_count), _S)
     return z

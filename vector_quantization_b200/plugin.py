@@ -13,7 +13,7 @@ from __future__ import annotations
 from . import anchors, callbacks, distances, losses, quantizers, registry
 
 QUANTIZERS = ['VectorQuantizer', 'VQGANQuantizer', 'VQKDQuantizer', 'ScalarQuantizer', 'FiniteScalarQuantizer',
-              'ResidualVectorQuantizer']
+              'ResidualVectorQuantizer', 'GroupedVectorQuantizer']
 CALLBACKS = ['ComposedCallback', 'NormalizeCallback', 'VQKDCallback', 'VQGAN_VQKDCallback', 'CVQVAECallback']
 LOSSES = ['CodebookLoss', 'CommitmentLoss', 'VQGANLoss', 'EntropyLoss']
 DISTANCES = ['L2Distance', 'CosineDistance']

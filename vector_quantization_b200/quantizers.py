@@ -23,7 +23,7 @@ from torch import nn
 
 from . import functional as Fq
 from . import ops, parallel
-from ._lib import VQBError
+from ._lib import MAX_LEVELS, VQBError
 from .callbacks import ComposedCallback
 from .distances import BaseDistance
 from .registry import (Config, InitRegistry, ModelRegistry, ModuleDict, VQITQuantizerCallbackRegistry,
@@ -31,7 +31,7 @@ from .registry import (Config, InitRegistry, ModelRegistry, ModuleDict, VQITQuan
                        build_module_dict, get_config)
 
 __all__ = ['BaseQuantizer', 'VectorQuantizer', 'VQGANQuantizer', 'VQKDQuantizer', 'ScalarQuantizer',
-           'FiniteScalarQuantizer', 'ResidualVectorQuantizer']
+           'FiniteScalarQuantizer', 'ResidualVectorQuantizer', 'GroupedVectorQuantizer']
 
 
 def get_memo(memo: dict, key: str) -> dict:
@@ -97,12 +97,13 @@ class BaseQuantizer(nn.Module):
     def encode(self, x: torch.Tensor, memo: dict):
         x = self._callbacks.before_encode(x, memo)
         enc = get_memo(memo, 'encode')
-        for flag in ('_normalize_codebook', '_normalize_x', '_lazy_unpack', '_zero_fill'):  # requests of the callbacks / forward
+        for flag in ('_normalize_codebook', '_normalize_x', '_lazy_unpack', '_zero_fill', '_keys_out'):  # requests of the callbacks / forward
             if flag in memo:
                 enc[flag] = memo[flag]
         memo.pop('_normalize_codebook', None)
         memo.pop('_lazy_unpack', None)
         memo.pop('_zero_fill', None)
+        memo.pop('_keys_out', None)
         quant, memo['encode'] = self._encode(x, enc)
         quant = self._callbacks.after_encode(x, quant, memo)
         memo['encode'].pop('_column_ctx', None)      # operands kept for the callbacks' column arg-min
@@ -239,7 +240,9 @@ class VectorQuantizer(BaseQuantizer):
         x = _check_tokens(x.detach(), self.embedding_dim)
         W = self._weight().data
         metric = self._distance.metric
-        keys = torch.empty((x.shape[0],), dtype=torch.int64, device=x.device)
+        keys = memo.pop('_keys_out', None)      # a caller's [N] int64 buffer (GroupedVectorQuantizer: a row of [G, N])
+        if keys is None:
+            keys = torch.empty((x.shape[0],), dtype=torch.int64, device=x.device)
         writeback = memo.pop('_normalize_codebook', False)
         if writeback:
             self.protect_saved_codebook()   # the codebook is normalised in place
@@ -448,6 +451,61 @@ class FiniteScalarQuantizer(ScalarQuantizer):
         return z, x.new_zeros([]), memo
 
 
+def _build_members(owner: BaseQuantizer, quantizer: Mapping, count, count_name: str, members: str) -> list:
+    """The member quantizers of a composed quantizer (ResidualVectorQuantizer levels, GroupedVectorQuantizer groups):
+    `count` copies of the `quantizer` node, each an ordinary VectorQuantizer / VQGANQuantizer.  Accepted: L2 or Cosine
+    distance, no callback or CVQVAECallback (NearestAnchor / CachedAnchor), CodebookLoss / CommitmentLoss / VQGANLoss.
+    Everything else raises a ValueError naming the offending item: callbacks that rewrite the tokens, callbacks that
+    hook decode or loss, compatibility mode, a count outside [1, 16], members that are not VectorQuantizer modules
+    (FSQ, or a composed quantizer: no nesting), and callbacks or losses on the composed node itself."""
+    name = type(owner).__name__
+    if isinstance(count, bool) or not isinstance(count, int) or not 1 <= count <= MAX_LEVELS:
+        raise ValueError(f'{name}: {count_name}={count!r} is outside [1, {MAX_LEVELS}]')
+    if list(owner._callbacks) or len(owner._losses):
+        raise ValueError(f'{name}: callbacks and losses belong to the {members[:-1]} config (`quantizer`), '
+                         f'not to the {name} node itself')
+    cls = VQITQuantizerRegistry.lookup(quantizer['type']) if isinstance(quantizer.get('type'), str) else None
+    if isinstance(cls, type) and not issubclass(cls, VectorQuantizer):
+        raise ValueError(f'{name}: the {members} must be VectorQuantizer modules, got {cls.__name__}')
+    built = []
+    for _ in range(count):
+        cfg = Config(copy.deepcopy(dict(quantizer)))
+        cfg['init_weights'] = None       # applied per member by init_weights (after the train / eval mode is set)
+        built.append(VQITQuantizerRegistry.build(cfg))
+    for member in built:
+        _check_member(name, member, members)
+    return built
+
+
+def _check_member(owner: str, member, members: str) -> None:
+    from .callbacks import BaseCallback, CVQVAECallback, NormalizeCallback
+    from .losses import CodebookLoss, CommitmentLoss, VQGANLoss
+    name = type(member).__name__
+    if not isinstance(member, VectorQuantizer):
+        raise ValueError(f'{owner}: the {members} must be VectorQuantizer modules, got {name}')
+    if member.materialize_distance:
+        raise ValueError(f'{owner}: materialize_distance (compatibility mode) is not supported')
+    for c in member._callbacks:
+        cname = type(c).__name__
+        if isinstance(c, NormalizeCallback):
+            raise ValueError(f'{owner}: callback {cname} rewrites the tokens; normalised {members} are not supported')
+        hooks = [h for h in ('before_decode', 'after_decode', 'before_loss', 'after_loss')
+                 if getattr(type(c), h) is not getattr(BaseCallback, h)]
+        if hooks:
+            raise ValueError(f'{owner}: callback {cname} hooks {", ".join(hooks)}; callbacks that '
+                             'hook decode or loss are not supported')
+        if not isinstance(c, CVQVAECallback):
+            raise ValueError(f'{owner}: callback {cname} is not supported ({members} take no callback '
+                             'or CVQVAECallback)')
+        if c._anchor.needs_distance:
+            raise ValueError(f'{owner}: {type(c._anchor).__name__} of {cname} reads the [N, K] '
+                             'distance matrix (compatibility mode), which is not supported')
+    for lname, loss in member._losses.items():
+        if not isinstance(loss, (CodebookLoss, CommitmentLoss, VQGANLoss)):
+            raise ValueError(f'{owner}: loss {lname!r} ({type(loss).__name__}) is not supported '
+                             '(CodebookLoss, CommitmentLoss and VQGANLoss are)')
+
+
 @VQITQuantizerRegistry.register_()
 class ResidualVectorQuantizer(BaseQuantizer):
     """Residual quantization (RQ-VAE): L codebooks code every token in turn, level l quantizing what the earlier levels
@@ -474,50 +532,7 @@ class ResidualVectorQuantizer(BaseQuantizer):
 
     def __init__(self, *args, num_quantizers: int, quantizer: Mapping, **kwargs) -> None:
         super().__init__(*args, **kwargs)
-        if isinstance(num_quantizers, bool) or not isinstance(num_quantizers, int) or \
-                not 1 <= num_quantizers <= self.MAX_LEVELS:
-            raise ValueError(f'ResidualVectorQuantizer: num_quantizers={num_quantizers!r} is outside [1, {self.MAX_LEVELS}]')
-        if list(self._callbacks) or len(self._losses):
-            raise ValueError('ResidualVectorQuantizer: callbacks and losses belong to the level config (`quantizer`), '
-                             'not to the residual quantizer itself')
-        levels = []
-        for _ in range(num_quantizers):
-            cfg = Config(copy.deepcopy(dict(quantizer)))
-            cfg['init_weights'] = None       # applied per level by init_weights (after the train / eval mode is set)
-            levels.append(VQITQuantizerRegistry.build(cfg))
-        for level in levels:
-            self._check_level(level)
-        self._quantizers = nn.ModuleList(levels)
-
-    @staticmethod
-    def _check_level(level) -> None:
-        from .callbacks import BaseCallback, CVQVAECallback, NormalizeCallback
-        from .losses import CodebookLoss, CommitmentLoss, VQGANLoss
-        name = type(level).__name__
-        if not isinstance(level, VectorQuantizer):
-            raise ValueError(f'ResidualVectorQuantizer: the levels must be VectorQuantizer modules, got {name}')
-        if level.materialize_distance:
-            raise ValueError('ResidualVectorQuantizer: materialize_distance (compatibility mode) is not supported')
-        for c in level._callbacks:
-            cname = type(c).__name__
-            if isinstance(c, NormalizeCallback):
-                raise ValueError(f'ResidualVectorQuantizer: callback {cname} rewrites the tokens; a residual of '
-                                 'normalised levels is not supported')
-            hooks = [h for h in ('before_decode', 'after_decode', 'before_loss', 'after_loss')
-                     if getattr(type(c), h) is not getattr(BaseCallback, h)]
-            if hooks:
-                raise ValueError(f'ResidualVectorQuantizer: callback {cname} hooks {", ".join(hooks)}; callbacks that '
-                                 'hook decode or loss are not supported')
-            if not isinstance(c, CVQVAECallback):
-                raise ValueError(f'ResidualVectorQuantizer: callback {cname} is not supported (levels take no callback '
-                                 'or CVQVAECallback)')
-            if c._anchor.needs_distance:
-                raise ValueError(f'ResidualVectorQuantizer: {type(c._anchor).__name__} of {cname} reads the [N, K] '
-                                 'distance matrix (compatibility mode), which is not supported')
-        for lname, loss in level._losses.items():
-            if not isinstance(loss, (CodebookLoss, CommitmentLoss, VQGANLoss)):
-                raise ValueError(f'ResidualVectorQuantizer: loss {lname!r} ({type(loss).__name__}) is not supported '
-                                 '(CodebookLoss, CommitmentLoss and VQGANLoss are)')
+        self._quantizers = nn.ModuleList(_build_members(self, quantizer, num_quantizers, 'num_quantizers', 'levels'))
 
     @property
     def quantizers(self) -> nn.ModuleList:
@@ -607,6 +622,155 @@ class ResidualVectorQuantizer(BaseQuantizer):
                 level_loss[name] = value
                 loss_memo[name] = value if l == 0 else loss_memo[name] + value
         for name in levels[0]._losses:
+            loss = loss_memo[name] if loss is None else loss + loss_memo[name]
+        if loss is None:
+            loss = mse[0][0].new_zeros([])
+        return z, loss, memo
+
+
+@VQITQuantizerRegistry.register_()
+class GroupedVectorQuantizer(BaseQuantizer):
+    """Grouped (product) quantization: the D channels of a token are split into G groups of Dg = D / G channels and
+    group g is quantized against its own codebook of K codes, so a token gets G ids (a joint code space of K^G).  Groups
+    are ordinary VectorQuantizer / VQGANQuantizer modules with embedding_dim = Dg, built from ONE config node
+    (`quantizer`) and stored as `_quantizers.{g}`; group g sees the column slice x_g = x[:, g*Dg:(g+1)*Dg] and behaves
+    exactly like its own VectorQuantizer on x_g.contiguous():
+
+        q_g = group_g.encode(x_g);  e_g = W_g[q_g]     (its callbacks run, CVQ-VAE update included: W_g after the step)
+        z[:, g*Dg:(g+1)*Dg] = x_g + (e_g - x_g)        (fp32 subtract, then add; no FMA)
+        loss[name] = (sum_g loss_{g,name}(e_g, x_g)) / G  (fp32 adds in group order, one division)
+
+    The unnormalised MSE terms thus average over all N * D elements, so a config's loss weights keep their meaning when a
+    width-D quantizer is split into groups; with mse.norm=True each group normalises its own sub-vector.  With G = 1 this
+    is VectorQuantizer.forward bit for bit.  forward / encode take tokens [N, D] or latents [b, D, h, w] (z then comes
+    back NCHW).  memo: 'x' (the input as given), 'quant' (int64 [N, G]), 'groups' (group g's own memo: x = its token
+    slice, encode, decode, loss), 'loss' (per loss name, the group mean).
+
+    Accepted and rejected configurations are those of ResidualVectorQuantizer (see `_build_members`), with
+    1 <= num_groups <= 16.  `init_weights` is applied to every group."""
+
+    def __init__(self, *args, num_groups: int, quantizer: Mapping, **kwargs) -> None:
+        super().__init__(*args, **kwargs)
+        self._quantizers = nn.ModuleList(_build_members(self, quantizer, num_groups, 'num_groups', 'groups'))
+
+    @property
+    def quantizers(self) -> nn.ModuleList:
+        return self._quantizers
+
+    @property
+    def num_groups(self) -> int:
+        return len(self._quantizers)
+
+    @property
+    def group_dim(self) -> int:
+        return self._quantizers[0].embedding_dim
+
+    @property
+    def embedding_dim(self) -> int:
+        return self.num_groups * self.group_dim
+
+    @property
+    def codebook_size(self) -> int:
+        """Codes per group."""
+        return self._quantizers[0].codebook_size
+
+    @property
+    def embeddings(self) -> torch.Tensor:
+        """[G, K, Dg] copy of the group codebooks."""
+        return torch.stack([group.embedding.weight.detach() for group in self._quantizers]).clone()
+
+    def _init_weights(self, config) -> bool:
+        for group in self._quantizers:
+            group.init_weights(Config(copy.deepcopy(dict(config))))
+        return False
+
+    def _weights(self) -> list:
+        return [group._weight() for group in self._quantizers]
+
+    def _want_norm(self) -> bool:
+        return self._quantizers[0]._loss_terms()
+
+    def _group_memos(self, memo: dict) -> list:
+        memo['groups'] = [dict() for _ in self._quantizers]
+        return memo['groups']
+
+    def _check_input(self, x: torch.Tensor) -> torch.Tensor:
+        """Tokens [N, D] or latents [b, D, h, w], fp32 / bf16 on the GPU."""
+        if x.dim() != 4:
+            return _check_tokens(x, self.embedding_dim)
+        if not x.is_cuda:
+            raise VQBError('vector_quantization_b200 quantizers run on CUDA (sm_100a) tensors only; no CPU fallback')
+        if x.shape[1] != self.embedding_dim:
+            raise ValueError(f'expected latents of shape [b, {self.embedding_dim}, h, w], got {tuple(x.shape)}')
+        if x.dtype not in (torch.float32, torch.bfloat16):
+            raise TypeError(f'latents must be float32 or bfloat16, got {x.dtype}')
+        return x.contiguous()
+
+    def _split(self, x: torch.Tensor) -> torch.Tensor:
+        x = self._check_input(x).detach()
+        if self.num_groups == 1 and x.dim() == 2:
+            return x.view(1, *x.shape)
+        return ops.split_groups(x, self.num_groups)
+
+    @torch.no_grad()
+    def encode(self, x: torch.Tensor, memo: dict):
+        """-> (x, quant int64 [N, G], memo); every group's callbacks run as in forward (codebook updates included)."""
+        xs = self._split(x)
+        G, N, _ = xs.shape
+        keys, _ = Fq.group_encode(list(self._quantizers), xs, self._group_memos(memo))
+        idx = ops.unpack_keys(keys.view(-1))
+        quant = idx.view(N, G) if G == 1 else ops.transpose_last2(idx.view(1, G, N)).view(N, G)
+        for g, group_memo in enumerate(memo['groups']):
+            group_memo.update(x=xs[g], quant=quant[:, g])
+        return x, quant, memo
+
+    @torch.no_grad()
+    def encode_compact(self, x: torch.Tensor, memo: dict) -> torch.Tensor:
+        """Tokenise-only encode: [G, N'] uint16 (K <= 65 536) or int32 ids straight from the packed assignment keys (N' = N
+        rounded up to 8; the first N columns are the ids); None when a group's training callback needs int64 indices
+        (then `encode` is the way)."""
+        if not all(group._callbacks.packed_keys_ok() for group in self._quantizers):
+            return None
+        xs = self._split(x)
+        G, N, _ = xs.shape
+        # rows padded to 8: every row starts 16-byte aligned, as vqb_compact_tokens reads and stores 16 bytes at a time
+        Np = (N + 7) // 8 * 8
+        keys = torch.empty((G, Np), dtype=torch.int64, device=xs.device)[:, :N]
+        out = torch.empty((G, Np), dtype=torch.uint16 if self.codebook_size <= 65536 else torch.int32, device=xs.device)
+        Fq.group_encode(list(self._quantizers), xs, self._group_memos(memo), keys=keys)
+        for g in range(G):
+            ops.compact_tokens(keys[g], self.codebook_size, out=out[g, :N])
+        return out
+
+    def decode(self, quant: torch.Tensor, memo: dict):
+        """quant [N, G] (or [..., G]; uint16 / int32 / int64) -> (z fp32 [..., D], memo): channels [g*Dg, (g+1)*Dg) =
+        W_g[q_g], one launch.  A token with an id outside [0, codebook_size) in any group decodes to NaN."""
+        if not quant.is_cuda:
+            raise VQBError('GroupedVectorQuantizer decodes CUDA tensors only; there is no CPU fallback')
+        lead = tuple(quant.shape[:-1])
+        flat = quant.contiguous().view(-1, quant.shape[-1])
+        z = ops.decode_group_tokens([W.detach() for W in self._weights()], flat, 1)
+        get_memo(memo, 'decode')
+        return z.view(*lead, self.embedding_dim), memo
+
+    def forward(self, x: torch.Tensor, memo: dict):
+        x = self._check_input(x)
+        groups = list(self._quantizers)
+        memos = self._group_memos(memo)
+        z, quant, mse = Fq.grouped_quantize(groups, x, memos, self._want_norm())
+        memo.update(x=x, quant=quant)
+        loss_memo = get_memo(memo, 'loss')
+        sums: dict = {}
+        for g, (group, group_memo) in enumerate(zip(groups, memos)):
+            group_memo['decode'] = get_memo(group_memo, 'decode')
+            group_loss = get_memo(group_memo, 'loss')
+            for name, module in group._losses.items():
+                value = module.from_mse4(mse[g])
+                group_loss[name] = value
+                sums[name] = value if g == 0 else sums[name] + value
+        loss = None
+        for name, total in sums.items():
+            loss_memo[name] = total / len(groups)
             loss = loss_memo[name] if loss is None else loss + loss_memo[name]
         if loss is None:
             loss = mse[0][0].new_zeros([])

@@ -18,7 +18,8 @@ import torch
 from . import functional as Fq
 from . import ops
 from ._lib import VQBError
-from .quantizers import FiniteScalarQuantizer, ResidualVectorQuantizer, VectorQuantizer, get_memo
+from .quantizers import (FiniteScalarQuantizer, GroupedVectorQuantizer, ResidualVectorQuantizer, VectorQuantizer,
+                         get_memo)
 
 __all__ = ['quantize', 'encode_to_quant', 'decode_from_quant', 'save_tokens', 'load_tokens', 'save_llamagen_codes', 'TokenStreamWriter']
 
@@ -26,9 +27,13 @@ __all__ = ['quantize', 'encode_to_quant', 'decode_from_quant', 'save_tokens', 'l
 def quantize(quantizer, x: torch.Tensor, memo: dict):
     """`BaseModel.quantize` (base.py:116-129): x [b, c, h, w] -> (z [b, c, h, w] contiguous, q_loss, memo) with
     memo['quantizer'] = the quantizer's memo (+ 'x_shape').  A ResidualVectorQuantizer always takes the fused layout: its
-    last residual step writes z NCHW."""
+    last residual step writes z NCHW.  A GroupedVectorQuantizer takes the latents themselves: one split launch makes
+    its group-major tokens and the group gather kernel writes z NCHW."""
     quantizer_memo = get_memo(memo, 'quantizer')
     quantizer_memo['x_shape'] = (b, c, h, w) = tuple(x.shape)
+    if isinstance(quantizer, GroupedVectorQuantizer) and x.is_cuda:
+        z, q_loss, memo['quantizer'] = quantizer(x, quantizer_memo)
+        return z, q_loss, memo
     fusable = isinstance(quantizer, ResidualVectorQuantizer) or (isinstance(quantizer, VectorQuantizer)
                                                                   and quantizer.can_fuse_nchw())
     if fusable and x.is_cuda:
@@ -52,9 +57,23 @@ def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = F
     compact=True is the tokenise-only variant: token ids come back as uint16 (K <= 65 536) or int32 straight
     from the packed assignment keys and memo['quantizer']['quant'] holds that compact tensor.
     A ResidualVectorQuantizer gives quant [b, h, w, L] (a token's L ids contiguous); with compact=True each level's
-    ids are compacted into a row of an [L, N] buffer and one transpose makes the [N, L] layout."""
+    ids are compacted into a row of an [L, N] buffer and one transpose makes the [N, L] layout.  A
+    GroupedVectorQuantizer gives quant [b, h, w, G] the same way (its encode reads the latents through one split
+    launch; memo['quantizer']['x'] is then the latents)."""
     quantizer_memo = get_memo(memo, 'quantizer')
     quantizer_memo['x_shape'] = (b, _, h, w) = tuple(x.shape)
+    if isinstance(quantizer, GroupedVectorQuantizer):
+        G = quantizer.num_groups
+        by_group = quantizer.encode_compact(x, quantizer_memo) if compact else None
+        if by_group is not None:
+            quant = by_group.view(-1, 1) if G == 1 else ops.transpose_last2(by_group.view(1, G, -1)).view(-1, G)
+            quant = quant[:b * h * w]
+        else:
+            _, quant, _ = quantizer.encode(x, quantizer_memo)
+            if compact:
+                quant = quant.to(torch.int32)
+        quantizer_memo.update(x=x, quant=quant)
+        return quant.view(b, h, w, G), memo
     rows = Fq.nchw_to_rows(x)
     if isinstance(quantizer, ResidualVectorQuantizer):
         L = quantizer.num_quantizers
@@ -87,7 +106,8 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     quant [b, h, w] -> (z [b, c, h, w] contiguous of `dtype`, memo) with memo['quantizer'] = the quantizer's memo as
     `quantizer.decode` leaves it.  quant is uint16, int32 or int64 on the GPU: what `encode_to_quant` (compact or not)
     and FSQ produce, or a `load_tokens` dump moved to the device.  The codebook is used as stored (no before_encode).
-    A ResidualVectorQuantizer takes quant [b, h, w, L] and decodes sum_l W_l[id_l] in one launch.
+    A ResidualVectorQuantizer takes quant [b, h, w, L] and decodes sum_l W_l[id_l] in one launch; a
+    GroupedVectorQuantizer takes quant [b, h, w, G] and decodes channel group g from W_g[id_g] in one launch.
 
     A VectorQuantizer or FiniteScalarQuantizer without before_decode / after_decode hooks decodes in ONE launch that
     reads the ids as they are and writes NCHW `dtype` directly.  Hooks, or a codebook that requires grad with grad
@@ -98,10 +118,14 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     IndexError with the number of such tokens.  check=False does not synchronise (safe inside a CUDA graph capture)
     and, on the one-launch path, decodes such tokens to NaN in every channel."""
     residual = isinstance(quantizer, ResidualVectorQuantizer)
+    grouped = isinstance(quantizer, GroupedVectorQuantizer)
     if residual and (quant.dim() != 4 or quant.shape[-1] != quantizer.num_quantizers):
         raise ValueError(f'expected residual token ids of shape [b, h, w, {quantizer.num_quantizers}], '
                          f'got {tuple(quant.shape)}')
-    if not residual and quant.dim() != 3:
+    if grouped and (quant.dim() != 4 or quant.shape[-1] != quantizer.num_groups):
+        raise ValueError(f'expected grouped token ids of shape [b, h, w, {quantizer.num_groups}], '
+                         f'got {tuple(quant.shape)}')
+    if not (residual or grouped) and quant.dim() != 3:
         raise ValueError(f'expected token ids of shape [b, h, w], got {tuple(quant.shape)}')
     if not quant.is_cuda:
         raise VQBError('vector_quantization_b200 decodes CUDA (sm_100a) token ids only; there is no CPU fallback')
@@ -109,9 +133,10 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
         raise TypeError(f'dtype must be float32 or bfloat16, got {dtype}')
     b, h, w = quant.shape[:3]
     quantizer_memo = get_memo(memo, 'quantizer')
-    if residual:
+    if residual or grouped:
         bad = torch.zeros(1, dtype=torch.int32, device=quant.device) if check else None
-        z = ops.decode_residual_tokens([W.detach() for W in quantizer._weights()], quant.contiguous(), h * w, dtype, bad)
+        decode = ops.decode_residual_tokens if residual else ops.decode_group_tokens
+        z = decode([W.detach() for W in quantizer._weights()], quant.contiguous(), h * w, dtype, bad)
         get_memo(quantizer_memo, 'decode')
         if check:
             _raise_bad_ids(int(bad.item()), quantizer.codebook_size)
@@ -147,7 +172,7 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
 
 
 def _token_grid(quant: torch.Tensor, x_shape: Sequence[int]) -> tuple:
-    """(b, h, w) for one id per token; (b, h, w, L) for residual ids ([b, h, w, L], or L ids per token)."""
+    """(b, h, w) for one id per token; (b, h, w, L) for residual or grouped ids ([b, h, w, L], or L ids per token)."""
     b, _, h, w = x_shape
     depth = quant.numel() // max(b * h * w, 1)
     return (b, h, w, depth) if (quant.dim() == 4 or depth != 1) else (b, h, w)
@@ -162,8 +187,8 @@ def save_tokens(path: str | pathlib.Path, id_: Sequence[Any], category: torch.Te
                 x_shape: Sequence[int]) -> None:
     """`TokenizeCallback.after_run_iter` (runners/callbacks.py:40-53): torch.save of the `Tokens` dict
     {id_, category, tokens [b, h, w]}.  Compact ids are widened to int64 so that reference readers see the
-    dtype they expect; pass an int64 tensor to skip the conversion.  Residual ids keep their trailing depth axis:
-    tokens [b, h, w, L]."""
+    dtype they expect; pass an int64 tensor to skip the conversion.  Residual and grouped ids keep their trailing
+    axis: tokens [b, h, w, L]."""
     tokens = quant.reshape(_token_grid(quant, x_shape))
     if tokens.dtype != torch.int64:
         tokens = tokens.to(torch.int32).to(torch.int64) if tokens.dtype == torch.uint16 else tokens.to(torch.int64)
