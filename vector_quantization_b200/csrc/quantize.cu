@@ -140,6 +140,112 @@ __device__ __forceinline__ int64_t row_index(const int64_t* __restrict__ quant,
   return q < 0 ? 0 : (q >= K ? K - 1 : q);  // never read out of bounds on a corrupt index
 }
 
+// ---- the per-token terms shared by the plain, residual and grouped kernels -----------------------------------------
+// The forward's reciprocal norms for the norm=True MSE term (1 ulp vs a true division), from the lane-partial sums of
+// squares of the token x and the codebook row z.
+template <int G>
+__device__ __forceinline__ void recip_norms(int want_norm, float sxx, float sww, float& rdx, float& rdw) {
+  rdx = 1.f;
+  rdw = 1.f;
+  if (want_norm) {
+    sxx = group_sum<G>(sxx);
+    sww = group_sum<G>(sww);
+    rdx = 1.f / fmaxf(sqrtf(sxx), kNormEps);
+    rdw = 1.f / fmaxf(sqrtf(sww), kNormEps);
+  }
+}
+
+// One element of the forward's MSE sums, with diff = __fsub_rn(z, x): sse += diff^2 and, with want_norm,
+// sse_n += (n(z) - n(x))^2, over valid tokens only.
+__device__ __forceinline__ void mse_term(float diff, float xv, float wv, float rdx, float rdw, bool valid, int want_norm,
+                                         float& sse, float& sse_n) {
+  if (valid) sse = fmaf(diff, diff, sse);
+  if (want_norm) {
+    const float dn = wv * rdw - xv * rdx;
+    if (valid) sse_n = fmaf(dn, dn, sse_n);
+  }
+}
+
+// The four loss-gradient coefficients c_* = g4[*] * scale of the backward (0 for an absent gradient, and for the
+// norm terms without want_norm); scale = 2 / (N D).
+struct LossCoefs {
+  float cb, cm, cbn, cmn;
+};
+__device__ __forceinline__ LossCoefs loss_coefs(const float* g_cb, const float* g_cm, const float* g_cbn,
+                                                const float* g_cmn, int want_norm, float scale) {
+  return {g_cb ? *g_cb * scale : 0.f, g_cm ? *g_cm * scale : 0.f, (want_norm && g_cbn) ? *g_cbn * scale : 0.f,
+          (want_norm && g_cmn) ? *g_cmn * scale : 0.f};
+}
+
+// The backward's norm=True terms of one token, from its y and z rows and their lane-partial sums of squares:
+// reciprocal norms dy = 1/|y|, dw = 1/|z|, the clamp flags cy, cw (norm below kNormEps: n() is then a plain scaling),
+// and uu = u.u, vv = v.v, uv = u.v with u = n(y), v = n(z).  Without want_norm: dy = dw = 1, the rest 0.
+struct NormTerms {
+  float dy = 1.f, dw = 1.f, uu = 0.f, vv = 0.f, uv = 0.f;
+  bool cy = false, cw = false;
+};
+template <int G, int V, int NV>
+__device__ __forceinline__ NormTerms norm_terms(int want_norm, const float (&yr)[NV][V], const float (&wr)[NV][V],
+                                                float syy, float sww) {
+  NormTerms t;
+  if (want_norm) {
+    float syw = 0.f;
+#pragma unroll
+    for (int it = 0; it < NV; ++it)
+#pragma unroll
+      for (int i = 0; i < V; ++i) syw = fmaf(yr[it][i], wr[it][i], syw);
+    syy = group_sum<G>(syy);
+    sww = group_sum<G>(sww);
+    syw = group_sum<G>(syw);
+    const float ny = sqrtf(syy), nw = sqrtf(sww);
+    t.cy = ny < kNormEps;
+    t.cw = nw < kNormEps;
+    t.dy = 1.f / fmaxf(ny, kNormEps);
+    t.dw = 1.f / fmaxf(nw, kNormEps);
+    t.uu = syy * t.dy * t.dy;
+    t.vv = sww * t.dw * t.dw;
+    t.uv = syw * t.dy * t.dw;
+  }
+  return t;
+}
+
+// One element of the backward term (formulas above quantize_backward_kernel) for (y, z) = (yv, wv): g holds g_zste on
+// entry and g_y on return.  Returns g_z, the codebook-row gradient.
+__device__ __forceinline__ float backward_term(float yv, float wv, float& g, const LossCoefs& c, const NormTerms& t,
+                                               int want_norm) {
+  float g_y = g + c.cm * (yv - wv);
+  float g_w = c.cb * (wv - yv);
+  if (want_norm) {
+    const float u = yv * t.dy, v = wv * t.dw;
+    const float gu = c.cmn * (u - v), gu_dot_u = c.cmn * (t.uu - t.uv);
+    g_y += (gu - (t.cy ? 0.f : gu_dot_u * u)) * t.dy;
+    const float gv = c.cbn * (v - u), gv_dot_v = c.cbn * (t.vv - t.uv);
+    g_w += (gv - (t.cw ? 0.f : gv_dot_v * v)) * t.dw;
+  }
+  g = g_y;
+  return g_w;
+}
+
+// One V-slice (elements d0.. of a D-wide row) of token n's codebook-row gradient: with kRowsOut stored to row n of gW
+// ([N, D] rows for the deterministic segment sum), else added to row q of gW when gW is given.
+template <bool kRowsOut, int V>
+__device__ __forceinline__ void emit_gw(float* gW, int64_t n, int64_t q, int D, int d0, bool valid,
+                                        const float (&gw)[V]) {
+  if constexpr (kRowsOut) {
+    if (valid && d0 < D) store_slice<float, V>(gW + n * D, d0, D, gw);
+  } else if (gW && valid && d0 < D) {
+    float* dst = gW + q * D + d0;
+    if constexpr (V == 8) {   // two red.global.add.v4.f32 instead of eight scalar atomics (the slice is 32-byte aligned)
+      atomicAdd(reinterpret_cast<float4*>(dst), make_float4(gw[0], gw[1], gw[2], gw[3]));
+      atomicAdd(reinterpret_cast<float4*>(dst + 4), make_float4(gw[4], gw[5], gw[6], gw[7]));
+    } else {
+#pragma unroll
+      for (int i = 0; i < V; ++i)
+        if (d0 + i < D) atomicAdd(dst + i, gw[i]);
+    }
+  }
+}
+
 // ---- forward -----------------------------------------------------------------------------------
 template <typename TX, int G, int V, int NV>
 __global__ void __launch_bounds__(256) quantize_forward_kernel(
@@ -191,13 +297,8 @@ __global__ void __launch_bounds__(256) quantize_forward_kernel(
         }
       sxx = s2;
     }
-    float rdx = 1.f, rdw = 1.f;  // reciprocal norms for the norm=True MSE term (1 ulp vs a true division)
-    if (want_norm) {
-      sxx = group_sum<G>(sxx);
-      sww = group_sum<G>(sww);
-      rdx = 1.f / fmaxf(sqrtf(sxx), kNormEps);
-      rdw = 1.f / fmaxf(sqrtf(sww), kNormEps);
-    }
+    float rdx, rdw;
+    recip_norms<G>(want_norm, sxx, sww, rdx, rdw);
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
       const int d0 = (it * G + lane) * V;
@@ -206,11 +307,7 @@ __global__ void __launch_bounds__(256) quantize_forward_kernel(
       for (int i = 0; i < V; ++i) {
         const float diff = __fsub_rn(wr[it][i], xr[it][i]);
         zr[i] = __fadd_rn(xr[it][i], diff);  // ste value: x + (z - x)
-        if (valid) sse = fmaf(diff, diff, sse);
-        if (want_norm) {
-          const float dn = wr[it][i] * rdw - xr[it][i] * rdx;
-          if (valid) sse_n = fmaf(dn, dn, sse_n);
-        }
+        mse_term(diff, xr[it][i], wr[it][i], rdx, rdw, valid, want_norm, sse, sse_n);
       }
       if (valid && d0 < D) {
         if (z_hw > 0) store_slice_nchw<float, V>(z_out, n, z_hw, d0, D, zr);   // z straight into the caller's NCHW layout
@@ -239,9 +336,7 @@ __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
   pdl_launch_dependents();
   const int lane = threadIdx.x % G;
   const int64_t rows_per_block = blockDim.x / G;
-  const float scale = 2.f / ((float)N * (float)D);
-  const float c_cb = g_cb ? *g_cb * scale : 0.f, c_cm = g_cm ? *g_cm * scale : 0.f;
-  const float c_cbn = (want_norm && g_cbn) ? *g_cbn * scale : 0.f, c_cmn = (want_norm && g_cmn) ? *g_cmn * scale : 0.f;
+  const LossCoefs c = loss_coefs(g_cb, g_cm, g_cbn, g_cmn, want_norm, 2.f / ((float)N * (float)D));
   for (int64_t base = blockIdx.x * rows_per_block; base < N; base += (int64_t)gridDim.x * rows_per_block) {
     const int64_t n_raw = base + threadIdx.x / G;
     const bool valid = n_raw < N;
@@ -287,26 +382,7 @@ __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
         }
       sxx = s2;
     }
-    float dy = 1.f, dw = 1.f, uu = 0.f, vv = 0.f, uv = 0.f;
-    bool cy = false, cw = false;
-    if (want_norm) {
-      float syw = 0.f;
-#pragma unroll
-      for (int it = 0; it < NV; ++it)
-#pragma unroll
-        for (int i = 0; i < V; ++i) syw = fmaf(yr[it][i], wr[it][i], syw);
-      sxx = group_sum<G>(sxx);
-      sww = group_sum<G>(sww);
-      syw = group_sum<G>(syw);
-      const float ny = sqrtf(sxx), nw = sqrtf(sww);
-      cy = ny < kNormEps;
-      cw = nw < kNormEps;
-      dy = 1.f / fmaxf(ny, kNormEps);   // from here on dy, dw hold the RECIPROCAL norms
-      dw = 1.f / fmaxf(nw, kNormEps);
-      uu = sxx * dy * dy;
-      vv = sww * dw * dw;
-      uv = syw * dy * dw;
-    }
+    const NormTerms t = norm_terms<G, V, NV>(want_norm, yr, wr, sxx, sww);
     // g_y (overwrites gr) and the codebook-row gradient
     float gy_dot_y = 0.f;
 #pragma unroll
@@ -315,33 +391,10 @@ __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
       float gw[V];
 #pragma unroll
       for (int i = 0; i < V; ++i) {
-        const float yv = yr[it][i], wv = wr[it][i];
-        float g_y = gr[it][i] + c_cm * (yv - wv);
-        float g_w = c_cb * (wv - yv);
-        if (want_norm) {
-          const float u = yv * dy, v = wv * dw;
-          const float gu = c_cmn * (u - v), gu_dot_u = c_cmn * (uu - uv);
-          g_y += (gu - (cy ? 0.f : gu_dot_u * u)) * dy;
-          const float gv = c_cbn * (v - u), gv_dot_v = c_cbn * (vv - uv);
-          g_w += (gv - (cw ? 0.f : gv_dot_v * v)) * dw;
-        }
-        gr[it][i] = g_y;
-        gy_dot_y = fmaf(g_y, yv, gy_dot_y);
-        gw[i] = g_w;
+        gw[i] = backward_term(yr[it][i], wr[it][i], gr[it][i], c, t, want_norm);
+        gy_dot_y = fmaf(gr[it][i], yr[it][i], gy_dot_y);
       }
-      if constexpr (kRowsOut) {
-        if (valid && d0 < D) store_slice<float, V>(gW + n * D, d0, D, gw);
-      } else if (gW && valid && d0 < D) {
-        float* dst = gW + q * D + d0;
-        if constexpr (V == 8) {   // two red.global.add.v4.f32 instead of eight scalar atomics (the slice is 32-byte aligned)
-          atomicAdd(reinterpret_cast<float4*>(dst), make_float4(gw[0], gw[1], gw[2], gw[3]));
-          atomicAdd(reinterpret_cast<float4*>(dst + 4), make_float4(gw[4], gw[5], gw[6], gw[7]));
-        } else {
-#pragma unroll
-          for (int i = 0; i < V; ++i)
-            if (d0 + i < D) atomicAdd(dst + i, gw[i]);
-        }
-      }
+      emit_gw<kRowsOut, V>(gW, n, q, D, d0, valid, gw);
     }
     if (normalize_x) {
       gy_dot_y = group_sum<G>(gy_dot_y);
@@ -406,16 +459,13 @@ __global__ void __launch_bounds__(256) residual_step_kernel(
         sww = fmaf(wr[it][i], wr[it][i], sww);
       }
     }
-    float rdr = 1.f, rdw = 1.f;
-    if (want_norm) {
-      srr = group_sum<G>(srr);
-      sww = group_sum<G>(sww);
-      rdr = 1.f / fmaxf(sqrtf(srr), kNormEps);
-      rdw = 1.f / fmaxf(sqrtf(sww), kNormEps);
-    }
+    float rdr, rdw;
+    recip_norms<G>(want_norm, srr, sww, rdr, rdw);
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
       const int d0 = (it * G + lane) * V;
+      // mse_term's arithmetic, written out: as a call, the compiler splits this slice loop on `last` instead of
+      // want_norm (G = 1, V = 8, NV = 2: 15 % more instructions and a stack frame with bf16 tokens)
 #pragma unroll
       for (int i = 0; i < V; ++i) {
         const float diff = __fsub_rn(wr[it][i], rr[it][i]);
@@ -495,12 +545,7 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
     }
 #pragma unroll 1
     for (int l = 0; l < L; ++l) {
-      const float* __restrict__ g_cb = lv.g[l][0];
-      const float* __restrict__ g_cm = lv.g[l][1];
-      const float* __restrict__ g_cbn = lv.g[l][2];
-      const float* __restrict__ g_cmn = lv.g[l][3];
-      const float c_cb = g_cb ? *g_cb * scale : 0.f, c_cm = g_cm ? *g_cm * scale : 0.f;
-      const float c_cbn = (want_norm && g_cbn) ? *g_cbn * scale : 0.f, c_cmn = (want_norm && g_cmn) ? *g_cmn * scale : 0.f;
+      const LossCoefs c = loss_coefs(lv.g[l][0], lv.g[l][1], lv.g[l][2], lv.g[l][3], want_norm, scale);
       const int64_t q = row_index(quant, nullptr, n * L + l, 0, K);
       const float* __restrict__ wrow = lv.W[l] + q * D;
       float* __restrict__ gW = lv.gW[l];
@@ -520,59 +565,17 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
           sww = fmaf(wr[it][i], wr[it][i], sww);
         }
       }
-      float dy = 1.f, dw = 1.f, uu = 0.f, vv = 0.f, uv = 0.f;
-      bool cy = false, cw = false;
-      if (want_norm) {
-        float syw = 0.f;
-#pragma unroll
-        for (int it = 0; it < NV; ++it)
-#pragma unroll
-          for (int i = 0; i < V; ++i) syw = fmaf(yr[it][i], wr[it][i], syw);
-        sxx = group_sum<G>(sxx);
-        sww = group_sum<G>(sww);
-        syw = group_sum<G>(syw);
-        const float ny = sqrtf(sxx), nw = sqrtf(sww);
-        cy = ny < kNormEps;
-        cw = nw < kNormEps;
-        dy = 1.f / fmaxf(ny, kNormEps);   // reciprocal norms
-        dw = 1.f / fmaxf(nw, kNormEps);
-        uu = sxx * dy * dy;
-        vv = sww * dw * dw;
-        uv = syw * dy * dw;
-      }
+      const NormTerms t = norm_terms<G, V, NV>(want_norm, yr, wr, sxx, sww);
 #pragma unroll
       for (int it = 0; it < NV; ++it) {
         const int d0 = (it * G + lane) * V;
         float gw[V];
 #pragma unroll
         for (int i = 0; i < V; ++i) {
-          const float yv = yr[it][i], wv = wr[it][i];
-          float g_y = gr[it][i] + c_cm * (yv - wv);
-          float g_w = c_cb * (wv - yv);
-          if (want_norm) {
-            const float u = yv * dy, v = wv * dw;
-            const float gu = c_cmn * (u - v), gu_dot_u = c_cmn * (uu - uv);
-            g_y += (gu - (cy ? 0.f : gu_dot_u * u)) * dy;
-            const float gv = c_cbn * (v - u), gv_dot_v = c_cbn * (vv - uv);
-            g_w += (gv - (cw ? 0.f : gv_dot_v * v)) * dw;
-          }
-          gr[it][i] = g_y;
-          gw[i] = g_w;
-          yr[it][i] = __fsub_rn(yv, wv);    // r_l
+          gw[i] = backward_term(yr[it][i], wr[it][i], gr[it][i], c, t, want_norm);
+          yr[it][i] = __fsub_rn(yr[it][i], wr[it][i]);    // r_l
         }
-        if constexpr (kRowsOut) {
-          if (valid && d0 < D) store_slice<float, V>(gW + n * D, d0, D, gw);
-        } else if (gW && valid && d0 < D) {
-          float* dst = gW + q * D + d0;
-          if constexpr (V == 8) {
-            atomicAdd(reinterpret_cast<float4*>(dst), make_float4(gw[0], gw[1], gw[2], gw[3]));
-            atomicAdd(reinterpret_cast<float4*>(dst + 4), make_float4(gw[4], gw[5], gw[6], gw[7]));
-          } else {
-#pragma unroll
-            for (int i = 0; i < V; ++i)
-              if (d0 + i < D) atomicAdd(dst + i, gw[i]);
-          }
-        }
+        emit_gw<kRowsOut, V>(gW, n, q, D, d0, valid, gw);
       }
     }
 #pragma unroll
@@ -635,13 +638,8 @@ __global__ void __launch_bounds__(256) group_forward_kernel(
         sww = fmaf(wr[it][i], wr[it][i], sww);
       }
     }
-    float rdx = 1.f, rdw = 1.f;
-    if (want_norm) {
-      sxx = group_sum<G>(sxx);
-      sww = group_sum<G>(sww);
-      rdx = 1.f / fmaxf(sqrtf(sxx), kNormEps);
-      rdw = 1.f / fmaxf(sqrtf(sww), kNormEps);
-    }
+    float rdx, rdw;
+    recip_norms<G>(want_norm, sxx, sww, rdx, rdw);
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
       const int d0 = (it * G + lane) * V;
@@ -650,11 +648,7 @@ __global__ void __launch_bounds__(256) group_forward_kernel(
       for (int i = 0; i < V; ++i) {
         const float diff = __fsub_rn(wr[it][i], xr[it][i]);
         zr[i] = __fadd_rn(xr[it][i], diff);  // ste value: x + (z - x)
-        if (valid) sse = fmaf(diff, diff, sse);
-        if (want_norm) {
-          const float dn = wr[it][i] * rdw - xr[it][i] * rdx;
-          if (valid) sse_n = fmaf(dn, dn, sse_n);
-        }
+        mse_term(diff, xr[it][i], wr[it][i], rdx, rdw, valid, want_norm, sse, sse_n);
       }
       if (valid && d0 < Dg) {
         if (z_hw > 0) store_slice_nchw<float, V>(zg, n, z_hw, d0, (int)D, zr);
@@ -685,12 +679,7 @@ __global__ void __launch_bounds__(256) group_backward_kernel(
   const int lane = threadIdx.x % G;
   const int64_t rows_per_block = blockDim.x / G;
   const float scale = 2.f / ((float)N * (float)Dg);
-  const float* __restrict__ g_cb = lv.g[grp][0];
-  const float* __restrict__ g_cm = lv.g[grp][1];
-  const float* __restrict__ g_cbn = lv.g[grp][2];
-  const float* __restrict__ g_cmn = lv.g[grp][3];
-  const float c_cb = g_cb ? *g_cb * scale : 0.f, c_cm = g_cm ? *g_cm * scale : 0.f;
-  const float c_cbn = (want_norm && g_cbn) ? *g_cbn * scale : 0.f, c_cmn = (want_norm && g_cmn) ? *g_cmn * scale : 0.f;
+  const LossCoefs c = loss_coefs(lv.g[grp][0], lv.g[grp][1], lv.g[grp][2], lv.g[grp][3], want_norm, scale);
   for (int64_t base = blockIdx.x * rows_per_block; base < N; base += (int64_t)gridDim.x * rows_per_block) {
     const int64_t n_raw = base + threadIdx.x / G;
     const bool valid = n_raw < N;
@@ -718,58 +707,14 @@ __global__ void __launch_bounds__(256) group_backward_kernel(
         sww = fmaf(wr[it][i], wr[it][i], sww);
       }
     }
-    float dy = 1.f, dw = 1.f, uu = 0.f, vv = 0.f, uv = 0.f;
-    bool cy = false, cw = false;
-    if (want_norm) {
-      float syw = 0.f;
-#pragma unroll
-      for (int it = 0; it < NV; ++it)
-#pragma unroll
-        for (int i = 0; i < V; ++i) syw = fmaf(yr[it][i], wr[it][i], syw);
-      sxx = group_sum<G>(sxx);
-      sww = group_sum<G>(sww);
-      syw = group_sum<G>(syw);
-      const float ny = sqrtf(sxx), nw = sqrtf(sww);
-      cy = ny < kNormEps;
-      cw = nw < kNormEps;
-      dy = 1.f / fmaxf(ny, kNormEps);   // reciprocal norms
-      dw = 1.f / fmaxf(nw, kNormEps);
-      uu = sxx * dy * dy;
-      vv = sww * dw * dw;
-      uv = syw * dy * dw;
-    }
+    const NormTerms t = norm_terms<G, V, NV>(want_norm, yr, wr, sxx, sww);
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
       const int d0 = (it * G + lane) * V;
       float gw[V];
 #pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const float yv = yr[it][i], wv = wr[it][i];
-        float g_y = gr[it][i] + c_cm * (yv - wv);
-        float g_w = c_cb * (wv - yv);
-        if (want_norm) {
-          const float u = yv * dy, v = wv * dw;
-          const float gu = c_cmn * (u - v), gu_dot_u = c_cmn * (uu - uv);
-          g_y += (gu - (cy ? 0.f : gu_dot_u * u)) * dy;
-          const float gv = c_cbn * (v - u), gv_dot_v = c_cbn * (vv - uv);
-          g_w += (gv - (cw ? 0.f : gv_dot_v * v)) * dw;
-        }
-        gr[it][i] = g_y;
-        gw[i] = g_w;
-      }
-      if constexpr (kRowsOut) {
-        if (valid && d0 < Dg) store_slice<float, V>(gW + n * Dg, d0, Dg, gw);
-      } else if (gW && valid && d0 < Dg) {
-        float* dst = gW + q * Dg + d0;
-        if constexpr (V == 8) {
-          atomicAdd(reinterpret_cast<float4*>(dst), make_float4(gw[0], gw[1], gw[2], gw[3]));
-          atomicAdd(reinterpret_cast<float4*>(dst + 4), make_float4(gw[4], gw[5], gw[6], gw[7]));
-        } else {
-#pragma unroll
-          for (int i = 0; i < V; ++i)
-            if (d0 + i < Dg) atomicAdd(dst + i, gw[i]);
-        }
-      }
+      for (int i = 0; i < V; ++i) gw[i] = backward_term(yr[it][i], wr[it][i], gr[it][i], c, t, want_norm);
+      emit_gw<kRowsOut, V>(gW, n, q, Dg, d0, valid, gw);
     }
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
@@ -861,6 +806,16 @@ using namespace vqb;
   VQB_GEOM_CASE(1, 1, 1, __VA_ARGS__) VQB_GEOM_CASE(1, 2, 1, __VA_ARGS__) VQB_GEOM_CASE(1, 4, 1, __VA_ARGS__)     \
   VQB_GEOM_CASE(1, 8, 1, __VA_ARGS__) VQB_GEOM_CASE(1, 16, 1, __VA_ARGS__) VQB_GEOM_CASE(1, 32, 1, __VA_ARGS__)   \
   VQB_GEOM_CASE(1, 32, 2, __VA_ARGS__) VQB_GEOM_CASE(1, 32, 4, __VA_ARGS__) VQB_GEOM_CASE(1, 32, 8, __VA_ARGS__)
+// the (x, upstream gradient) dtype pairs of the backward kernels, each launched by LAUNCH_(TX, TG); a bf16 upstream
+// gradient (autocast training) is read as is
+#define VQB_DISPATCH_BWD_DTYPES(LAUNCH_)                  \
+  if (x_dtype == VQB_F32 && g_dtype == VQB_F32) {         \
+    LAUNCH_(float, float)                                 \
+  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_F32) { \
+    LAUNCH_(__nv_bfloat16, float)                         \
+  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_BF16) { \
+    LAUNCH_(__nv_bfloat16, __nv_bfloat16)                 \
+  }
 
 extern "C" {
 
@@ -912,18 +867,12 @@ static int quantize_backward_launch(const void* gz, int g_dtype, const void* x, 
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = grid_for(N, 256 / geom.G);
   bool launched = false;
-  if (x_dtype == VQB_F32 && g_dtype == VQB_F32) {
-    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<float, float, G, V, NV, kRowsOut>, blocks, 256, 0, st,
-        (const float*)gz, (const float*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn, want_norm, (float*)gx, gW, g_hw)))
-  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_F32) {
-    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<__nv_bfloat16, float, G, V, NV, kRowsOut>, blocks, 256, 0, st,
-        (const float*)gz, (const __nv_bfloat16*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn, want_norm,
-        (__nv_bfloat16*)gx, gW, g_hw)))
-  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_BF16) {   // bf16 upstream gradient (autocast training): read as is
-    VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<__nv_bfloat16, __nv_bfloat16, G, V, NV, kRowsOut>, blocks, 256, 0, st,
-        (const __nv_bfloat16*)gz, (const __nv_bfloat16*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn,
-        want_norm, (__nv_bfloat16*)gx, gW, g_hw)))
-  }
+#define VQB_QUANTIZE_BWD(TX_, TG_)                                                                                     \
+  VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>, blocks, 256, 0, st,            \
+      (const TG_*)gz, (const TX_*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn, want_norm, (TX_*)gx, gW, \
+      g_hw)))
+  VQB_DISPATCH_BWD_DTYPES(VQB_QUANTIZE_BWD)
+#undef VQB_QUANTIZE_BWD
   VQB_REQUIRE(launched, "vqb_quantize_backward: unsupported dtype/geometry");
   VQB_LAUNCH_OK();
   return VQB_OK;
@@ -987,34 +936,34 @@ int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype,
 
 }  // extern "C"
 
-template <bool kRowsOut>
-static int residual_backward_launch(const char* fn, const void* gz, int g_dtype, const void* x, int x_dtype,
-                                    const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int D,
-                                    int want_norm, void* gx, int64_t g_hw, void* stream) {
+// The one-launch backward over the members of a vqb_residual_levels table: the levels of a residual chain
+// (residual_backward_kernel on tokens of width D) or the channel groups of a grouped quantizer (group_backward_kernel,
+// D the group width Dg, one grid row per group).  Messages name the members as "level" or "group".
+template <bool kGroups, bool kRowsOut>
+static int member_backward_launch(const char* fn, const void* gz, int g_dtype, const void* x, int x_dtype,
+                                  const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int D,
+                                  int want_norm, void* gx, int64_t g_hw, void* stream) {
+  const char* member = kGroups ? "of group" : "at level";
   VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
   VQB_REQUIRE(gz && x && lv && quant && gx, "%s: null pointer", fn);
-  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "%s: L=%d outside [1, %d]", fn, lv->L, VQB_MAX_LEVELS);
+  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "%s: %s=%d outside [1, %d]", fn, kGroups ? "G" : "L", lv->L,
+              VQB_MAX_LEVELS);
   for (int l = 0; l < lv->L; ++l) {
-    VQB_REQUIRE(lv->W[l], "%s: null codebook at level %d", fn, l);
-    VQB_REQUIRE(!kRowsOut || lv->gW[l], "%s: null gradient rows at level %d", fn, l);
+    VQB_REQUIRE(lv->W[l], "%s: null codebook %s %d", fn, member, l);
+    VQB_REQUIRE(!kRowsOut || lv->gW[l], "%s: null gradient rows %s %d", fn, member, l);
   }
   VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "%s: bad shape", fn);
   RowGeom geom;
-  VQB_REQUIRE(row_geom(D, N, &geom), "%s: D=%d unsupported", fn, D);
+  VQB_REQUIRE(row_geom(D, N, &geom), "%s: %s=%d unsupported", fn, kGroups ? "Dg" : "D", D);
   cudaStream_t st = (cudaStream_t)stream;
-  const int blocks = grid_for(N, 256 / geom.G);
+  const dim3 grid((unsigned)grid_for(N, 256 / geom.G), kGroups ? (unsigned)lv->L : 1u);
   bool launched = false;
-#define VQB_RESIDUAL_BWD(TX_, TG_)                                                                                      \
-  VQB_DISPATCH_GEOM((launch_pdl(residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>, blocks, 256, 0, st,             \
-      (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw)))
-  if (x_dtype == VQB_F32 && g_dtype == VQB_F32) {
-    VQB_RESIDUAL_BWD(float, float)
-  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_F32) {
-    VQB_RESIDUAL_BWD(__nv_bfloat16, float)
-  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_BF16) {
-    VQB_RESIDUAL_BWD(__nv_bfloat16, __nv_bfloat16)
-  }
-#undef VQB_RESIDUAL_BWD
+#define VQB_MEMBER_BWD(TX_, TG_)                                                                                      \
+  VQB_DISPATCH_GEOM((launch_pdl(kGroups ? group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>                          \
+                                        : residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>,                      \
+      grid, 256, 0, st, (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw)))
+  VQB_DISPATCH_BWD_DTYPES(VQB_MEMBER_BWD)
+#undef VQB_MEMBER_BWD
   VQB_REQUIRE(launched, "%s: unsupported dtype/geometry", fn);
   VQB_LAUNCH_OK();
   return VQB_OK;
@@ -1025,15 +974,15 @@ extern "C" {
 int vqb_residual_backward(const void* gz, int g_dtype, const void* x, int x_dtype, const vqb_residual_levels* levels,
                           int64_t K, const int64_t* quant, int64_t N, int D, int want_norm, void* gx, int64_t g_hw,
                           void* stream) {
-  return residual_backward_launch<false>("vqb_residual_backward", gz, g_dtype, x, x_dtype, levels, K, quant, N, D,
-                                         want_norm, gx, g_hw, stream);
+  return member_backward_launch<false, false>("vqb_residual_backward", gz, g_dtype, x, x_dtype, levels, K, quant, N, D,
+                                              want_norm, gx, g_hw, stream);
 }
 
 int vqb_residual_backward_rows(const void* gz, int g_dtype, const void* x, int x_dtype,
                                const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
                                int want_norm, void* gx, int64_t g_hw, void* stream) {
-  return residual_backward_launch<true>("vqb_residual_backward_rows", gz, g_dtype, x, x_dtype, levels, K, quant, N, D,
-                                        want_norm, gx, g_hw, stream);
+  return member_backward_launch<false, true>("vqb_residual_backward_rows", gz, g_dtype, x, x_dtype, levels, K, quant, N,
+                                             D, want_norm, gx, g_hw, stream);
 }
 
 int vqb_group_gather_ste_loss(const void* xs, int x_dtype, int64_t N, int Dg, const vqb_residual_levels* lv, int64_t K,
@@ -1071,55 +1020,18 @@ int vqb_group_gather_ste_loss(const void* xs, int x_dtype, int64_t N, int Dg, co
   return VQB_OK;
 }
 
-}  // extern "C"
-
-template <bool kRowsOut>
-static int group_backward_launch(const char* fn, const void* gz, int g_dtype, const void* xs, int x_dtype,
-                                 const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int Dg,
-                                 int want_norm, void* gx, int64_t g_hw, void* stream) {
-  VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
-  VQB_REQUIRE(gz && xs && lv && quant && gx, "%s: null pointer", fn);
-  VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "%s: G=%d outside [1, %d]", fn, lv->L, VQB_MAX_LEVELS);
-  for (int g = 0; g < lv->L; ++g) {
-    VQB_REQUIRE(lv->W[g], "%s: null codebook of group %d", fn, g);
-    VQB_REQUIRE(!kRowsOut || lv->gW[g], "%s: null gradient rows of group %d", fn, g);
-  }
-  VQB_REQUIRE(N >= 1 && Dg >= 1 && K >= 1, "%s: bad shape", fn);
-  RowGeom geom;
-  VQB_REQUIRE(row_geom(Dg, N, &geom), "%s: Dg=%d unsupported", fn, Dg);
-  cudaStream_t st = (cudaStream_t)stream;
-  const dim3 grid((unsigned)grid_for(N, 256 / geom.G), (unsigned)lv->L);
-  bool launched = false;
-#define VQB_GROUP_BWD(TX_, TG_)                                                                                       \
-  VQB_DISPATCH_GEOM((launch_pdl(group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>, grid, 256, 0, st,               \
-      (const TG_*)gz, (const TX_*)xs, *lv, K, quant, N, Dg, want_norm, (TX_*)gx, g_hw)))
-  if (x_dtype == VQB_F32 && g_dtype == VQB_F32) {
-    VQB_GROUP_BWD(float, float)
-  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_F32) {
-    VQB_GROUP_BWD(__nv_bfloat16, float)
-  } else if (x_dtype == VQB_BF16 && g_dtype == VQB_BF16) {
-    VQB_GROUP_BWD(__nv_bfloat16, __nv_bfloat16)
-  }
-#undef VQB_GROUP_BWD
-  VQB_REQUIRE(launched, "%s: unsupported dtype/geometry", fn);
-  VQB_LAUNCH_OK();
-  return VQB_OK;
-}
-
-extern "C" {
-
 int vqb_group_backward(const void* gz, int g_dtype, const void* xs, int x_dtype, const vqb_residual_levels* groups,
                        int64_t K, const int64_t* quant, int64_t N, int Dg, int want_norm, void* gx, int64_t g_hw,
                        void* stream) {
-  return group_backward_launch<false>("vqb_group_backward", gz, g_dtype, xs, x_dtype, groups, K, quant, N, Dg,
-                                      want_norm, gx, g_hw, stream);
+  return member_backward_launch<true, false>("vqb_group_backward", gz, g_dtype, xs, x_dtype, groups, K, quant, N, Dg,
+                                            want_norm, gx, g_hw, stream);
 }
 
 int vqb_group_backward_rows(const void* gz, int g_dtype, const void* xs, int x_dtype, const vqb_residual_levels* groups,
                             int64_t K, const int64_t* quant, int64_t N, int Dg, int want_norm, void* gx, int64_t g_hw,
                             void* stream) {
-  return group_backward_launch<true>("vqb_group_backward_rows", gz, g_dtype, xs, x_dtype, groups, K, quant, N, Dg,
-                                     want_norm, gx, g_hw, stream);
+  return member_backward_launch<true, true>("vqb_group_backward_rows", gz, g_dtype, xs, x_dtype, groups, K, quant, N,
+                                           Dg, want_norm, gx, g_hw, stream);
 }
 
 int vqb_unpack_keys(const unsigned long long* keys, int64_t n, int64_t offset, int64_t* idx, float* score,

@@ -413,8 +413,7 @@ def quantize_backward(g_z: torch.Tensor, x: torch.Tensor, W: torch.Tensor, quant
         _call('vqb_quantize_backward_rows', lib.vqb_quantize_backward_rows, dev, _p(g_z), _dt(g_z), _p(x), _dt(x),
               int(normalize_x), _p(W), K, _p(quant), N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm),
               _p(gx), _p(rows), g_hw, _S)
-        order, offsets = _code_sort_ws(dev, N, K, quant, None, 0)
-        _segment_sum(dev, rows, N, D, False, order, offsets, K, gW, None)
+        _segment_sum_members(dev, rows.view(1, N, D), quant, K, [gW])
         return gx, gW
     _call('vqb_quantize_backward', lib.vqb_quantize_backward, dev, _p(g_z), _dt(g_z), _p(x), _dt(x), int(normalize_x), _p(W),
           K, _p(quant), N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm), _p(gx), _p(gW),
@@ -510,6 +509,18 @@ def _segment_sum(dev, rows, N: int, D: int, normalize: bool, order, offsets, K: 
     scratch = _det_ws(dev, 'segment', int(lib.vqb_segment_sum_scratch_bytes(N, K, D)), torch.uint8)
     _call('vqb_segment_sum_rows', lib.vqb_segment_sum_rows, dev, _p(rows), _dt(rows), N, D, int(normalize), _p(order),
           _p(offsets), K, _p(out_sums), _p(out_counts), _p(scratch), scratch.numel(), _S)
+
+
+def _segment_sum_members(dev, rows, quant, K: int, gWs) -> None:
+    """The deterministic codebook gradients of M members (levels or groups) from their per-token rows [M, N, D]:
+    gWs[m] (a [K, D] tensor, or None to skip) += the segment sum of rows[m] over the tokens of each code, with the codes
+    of member m in column m of quant int64 [N, M] (or quant [N] when M == 1)."""
+    M, N, D = rows.shape
+    by_member = quant.view(M, N) if M == 1 else transpose_last2(quant.view(1, N, M)).view(M, N)
+    for m, gW in enumerate(gWs):
+        if gW is not None:
+            order, offsets = _code_sort_ws(dev, N, K, by_member[m], None, 0)
+            _segment_sum(dev, rows[m], N, D, False, order, offsets, K, gW, None)
 
 
 def code_sort(K: int, *, quant: torch.Tensor | None = None, keys: torch.Tensor | None = None,
@@ -834,11 +845,7 @@ def residual_backward(g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tenso
         p = _residual_levels(Ws, list(rows), g4s)
         _call('vqb_residual_backward_rows', lib.vqb_residual_backward_rows, dev, _p(g_z), _dt(g_z), _p(x), _dt(x),
               ctypes.byref(p), K, _p(quant), N, D, int(want_norm), _p(gx), g_hw, _S)
-        by_level = quant.view(L, N) if L == 1 else transpose_last2(quant.view(1, N, L)).view(L, N)
-        for l, gW in enumerate(gWs):
-            if gW is not None:
-                order, offsets = _code_sort_ws(dev, N, K, by_level[l], None, 0)
-                _segment_sum(dev, rows[l], N, D, False, order, offsets, K, gW, None)
+        _segment_sum_members(dev, rows, quant, K, gWs)
         return gx, gWs
     p = _residual_levels(Ws, gWs, g4s)
     _call('vqb_residual_backward', lib.vqb_residual_backward, dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K,
@@ -950,11 +957,7 @@ def group_backward(g_z: torch.Tensor, xs: torch.Tensor, Ws, quant: torch.Tensor,
         p = _residual_levels(Ws, list(rows), g4s)
         _call('vqb_group_backward_rows', lib.vqb_group_backward_rows, dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs),
               ctypes.byref(p), K, _p(quant), N, Dg, int(want_norm), _p(gx), g_hw, _S)
-        by_group = quant.view(G, N) if G == 1 else transpose_last2(quant.view(1, N, G)).view(G, N)
-        for g, gW in enumerate(gWs):
-            if gW is not None:
-                order, offsets = _code_sort_ws(dev, N, K, by_group[g], None, 0)
-                _segment_sum(dev, rows[g], N, Dg, False, order, offsets, K, gW, None)
+        _segment_sum_members(dev, rows, quant, K, gWs)
         return gx, gWs
     p = _residual_levels(Ws, gWs, g4s)
     _call('vqb_group_backward', lib.vqb_group_backward, dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs), ctypes.byref(p), K,
