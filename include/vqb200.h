@@ -243,6 +243,20 @@ int vqb_quantize_backward_rows(const void* g_zste, int g_dtype, const void* x, i
                                const float* g_codebook, const float* g_commitment,
                                const float* g_codebook_norm, const float* g_commitment_norm,
                                int want_norm_mse, void* gx_out, float* gW_rows, int64_t g_hw, void* stream);
+/* The rotation trick (Fifty et al., arXiv:2410.06424): vqb_quantize_backward / _rows with each token's g_zste first
+ * replaced by  g' = lambda R^T g_zste,  R the rotation taking y/|y| to e/|e| (y the token as quantized, e = W[q]),
+ * lambda = |e|/|y|;  a token with |y| or |e| below 1e-12 keeps g_zste.  gW is bit-identical to the unrotated entry
+ * points; only gx differs (DESIGN.md §4.9). */
+int vqb_quantize_backward_rotated(const void* g_zste, int g_dtype, const void* x, int x_dtype, int normalize_x,
+                                  const float* W, int64_t K, const int64_t* quant, int64_t N, int D,
+                                  const float* g_codebook, const float* g_commitment,
+                                  const float* g_codebook_norm, const float* g_commitment_norm,
+                                  int want_norm_mse, void* gx_out, float* gW_accum, int64_t g_hw, void* stream);
+int vqb_quantize_backward_rotated_rows(const void* g_zste, int g_dtype, const void* x, int x_dtype, int normalize_x,
+                                       const float* W, int64_t K, const int64_t* quant, int64_t N, int D,
+                                       const float* g_codebook, const float* g_commitment,
+                                       const float* g_codebook_norm, const float* g_commitment_norm,
+                                       int want_norm_mse, void* gx_out, float* gW_rows, int64_t g_hw, void* stream);
 
 /* ---- residual quantization (RQ-VAE: L codebooks, level l quantizes what levels 1..l-1 left over) ------------ *
  *   r_0 = x;  e_l = W_l[q_l];  zhat_1 = e_1, zhat_l = zhat_{l-1} + e_l;  r_l = r_{l-1} - e_l   (fp32 add / subtract,
@@ -312,6 +326,13 @@ int vqb_group_backward(const void* g_z, int g_dtype, const void* xs, int x_dtype
 int vqb_group_backward_rows(const void* g_z, int g_dtype, const void* xs, int x_dtype, const vqb_residual_levels* groups,
                             int64_t K, const int64_t* quant, int64_t N, int Dg, int want_norm_mse, void* gx_out,
                             int64_t g_hw, void* stream);
+/* vqb_group_backward / _rows with the rotation trick of vqb_quantize_backward_rotated, per group on (x_g, W_g[q_g]). */
+int vqb_group_backward_rotated(const void* g_z, int g_dtype, const void* xs, int x_dtype,
+                               const vqb_residual_levels* groups, int64_t K, const int64_t* quant, int64_t N, int Dg,
+                               int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
+int vqb_group_backward_rotated_rows(const void* g_z, int g_dtype, const void* xs, int x_dtype,
+                                    const vqb_residual_levels* groups, int64_t K, const int64_t* quant, int64_t N,
+                                    int Dg, int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
 
 /* ---- row l2-normalisation (NormalizeCallback.before_encode on x) ------------------------ *
  * vq/algorithms/vq/callbacks/normalize.py:24  — forward y = x / max(||x||, 1e-12); backward

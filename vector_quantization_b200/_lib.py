@@ -83,6 +83,12 @@ SIGNATURES = {
     'vqb_quantize_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p, c_int64,
                                            c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64,
                                            c_void_p]),
+    'vqb_quantize_backward_rotated': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p,
+                                              c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                              c_void_p, c_int64, c_void_p]),
+    'vqb_quantize_backward_rotated_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p,
+                                                   c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                                   c_void_p, c_void_p, c_int64, c_void_p]),
     'vqb_residual_step': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_int, c_void_p, c_int64, c_void_p, c_void_p,
                                   c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p,
                                   c_void_p, c_void_p, c_void_p]),
@@ -97,6 +103,10 @@ SIGNATURES = {
                                    c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_group_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
                                         c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_group_backward_rotated': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
+                                           c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_group_backward_rotated_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64,
+                                                c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_segment_chunk': (c_int64, []),
     'vqb_code_sort_scratch_bytes': (c_size_t, [c_int64, c_int64]),
     'vqb_code_sort': (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_size_t,

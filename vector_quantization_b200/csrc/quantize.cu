@@ -226,6 +226,54 @@ __device__ __forceinline__ float backward_term(float yv, float wv, float& g, con
   return g_w;
 }
 
+// The rotation trick (DESIGN.md §4.9) on one token's upstream gradient: gr <- lambda R^T g with a = |y|, b = |e|,
+// u = y / a, ehat = e / b, s = u + ehat, w = s / max(|s|, 1e-12), lambda = b / a and R = I - 2 w w^T + 2 ehat u^T, i.e.
+//   g' = lambda (g - 2 w (w.g) + 2 u (ehat.g))  =  lambda g - c_s s + c_y y
+// with c_s = 2 lambda (s.g) / max(|s|, 1e-12)^2 and c_y = 2 lambda (e.g) / (a b).  Group sums: |y|^2, |e|^2 (from the
+// lane partials syy, sww), y.g and e.g in one round; then |s|^2 summed from the per-element s (not the algebraic
+// 2 + 2 u.ehat, which cancels to noise for a nearly antipodal pair).  s and s.g are formed without FMA so that an exactly
+// antipodal pair (y = -e) gives s = 0 exactly, hence w = 0.  a or b below 1e-12: g unchanged (straight-through).
+template <int G, int V, int NV>
+__device__ __forceinline__ void rotate_grad(const float (&yr)[NV][V], const float (&wr)[NV][V], float (&gr)[NV][V],
+                                            float syy, float sww) {
+  float syg = 0.f, seg = 0.f;
+#pragma unroll
+  for (int it = 0; it < NV; ++it)
+#pragma unroll
+    for (int i = 0; i < V; ++i) {
+      syg = fmaf(yr[it][i], gr[it][i], syg);
+      seg = fmaf(wr[it][i], gr[it][i], seg);
+    }
+  syy = group_sum<G>(syy);
+  sww = group_sum<G>(sww);
+  syg = group_sum<G>(syg);
+  seg = group_sum<G>(seg);
+  const float a = sqrtf(syy), b = sqrtf(sww);
+  const bool rotate = a >= kNormEps && b >= kNormEps;   // uniform over the token's lanes, not over the warp
+  const float ra = rotate ? 1.f / a : 0.f, rb = rotate ? 1.f / b : 0.f;
+  float sss = 0.f;
+#pragma unroll
+  for (int it = 0; it < NV; ++it)
+#pragma unroll
+    for (int i = 0; i < V; ++i) {
+      const float s = __fadd_rn(__fmul_rn(yr[it][i], ra), __fmul_rn(wr[it][i], rb));
+      sss = fmaf(s, s, sss);
+    }
+  sss = group_sum<G>(sss);   // every lane of the warp takes part in the shuffles: the fallback returns only after them
+  if (!rotate) return;
+  const float lam = b * ra;
+  const float m = fmaxf(sqrtf(sss), kNormEps);
+  const float sg = __fadd_rn(__fmul_rn(syg, ra), __fmul_rn(seg, rb));
+  const float cs = 2.f * lam * sg / (m * m), cy = 2.f * lam * seg * ra * rb;
+#pragma unroll
+  for (int it = 0; it < NV; ++it)
+#pragma unroll
+    for (int i = 0; i < V; ++i) {
+      const float s = __fadd_rn(__fmul_rn(yr[it][i], ra), __fmul_rn(wr[it][i], rb));
+      gr[it][i] = fmaf(lam, gr[it][i], fmaf(cy, yr[it][i], -cs * s));
+    }
+}
+
 // One V-slice (elements d0.. of a D-wide row) of token n's codebook-row gradient: with kRowsOut stored to row n of gW
 // ([N, D] rows for the deterministic segment sum), else added to row q of gW when gW is given.
 template <bool kRowsOut, int V>
@@ -326,7 +374,8 @@ __global__ void __launch_bounds__(256) quantize_forward_kernel(
 //   g_z = c_cb (z - y) + J_n(z)^T [c_cbn (v - u)]                   -> atomically added to gW[q]
 //   g_x_in = J_n(x_in)^T g_y  when normalize_x, else g_y            J_n(a)^T g = (g - (g.n(a)) n(a)) / |a|
 // kRowsOut: store each token's g_z row to gW + n*D ([N, D] rows for the deterministic segment sum) instead of the atomics
-template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut = false>
+// kRotate: g_zste is first replaced by its rotation-trick form (rotate_grad, DESIGN.md §4.9); g_z is unchanged
+template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut = false, bool kRotate = false>
 __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
     const TG* __restrict__ gz, const TX* __restrict__ x, int normalize_x, const float* __restrict__ W, int64_t K,
     const int64_t* __restrict__ quant, int64_t N, int D, const float* __restrict__ g_cb,
@@ -383,6 +432,7 @@ __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
       sxx = s2;
     }
     const NormTerms t = norm_terms<G, V, NV>(want_norm, yr, wr, sxx, sww);
+    if constexpr (kRotate) rotate_grad<G, V, NV>(yr, wr, gr, sxx, sww);
     // g_y (overwrites gr) and the codebook-row gradient
     float gy_dot_y = 0.f;
 #pragma unroll
@@ -662,8 +712,8 @@ __global__ void __launch_bounds__(256) group_forward_kernel(
 
 // quantize_backward_kernel (without token normalisation) for group g = blockIdx.y: x_g from the split buffer,
 // W_g / gW_g / the four loss-gradient scalars from the group table, q_g = quant[n*G + g]; g_z and gx are the
-// full-width tensors at channel offset g*Dg.
-template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut>
+// full-width tensors at channel offset g*Dg.  kRotate as in quantize_backward_kernel.
+template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut, bool kRotate>
 __global__ void __launch_bounds__(256) group_backward_kernel(
     const TG* __restrict__ gz, const TX* __restrict__ xs, const __grid_constant__ vqb_residual_levels lv, int64_t K,
     const int64_t* __restrict__ quant, int64_t N, int Dg, int want_norm, TX* __restrict__ gx, int64_t g_hw) {
@@ -708,6 +758,7 @@ __global__ void __launch_bounds__(256) group_backward_kernel(
       }
     }
     const NormTerms t = norm_terms<G, V, NV>(want_norm, yr, wr, sxx, sww);
+    if constexpr (kRotate) rotate_grad<G, V, NV>(yr, wr, gr, sxx, sww);
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
       const int d0 = (it * G + lane) * V;
@@ -852,28 +903,29 @@ int vqb_gather_ste_loss(const void* x, int x_dtype, int64_t N, int D, int normal
 
 }  // extern "C"
 
-// kRowsOut selects the per-token-row variant (gW then points at fp32 [N, D] rows)
-template <bool kRowsOut>
+// kRowsOut selects the per-token-row variant (gW then points at fp32 [N, D] rows), kRotate the rotation trick
+template <bool kRowsOut, bool kRotate>
 static int quantize_backward_launch(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x, const float* W,
                                     int64_t K, const int64_t* quant, int64_t N, int D, const float* g_cb, const float* g_cm,
                                     const float* g_cbn, const float* g_cmn, int want_norm, void* gx, float* gW,
                                     int64_t g_hw, void* stream) {
-  VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "vqb_quantize_backward: g_hw must divide N");
-  VQB_REQUIRE(gz && x && W && quant && gx, "vqb_quantize_backward: null pointer");
-  VQB_REQUIRE(!kRowsOut || gW, "vqb_quantize_backward_rows: null gW_rows");
-  VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "vqb_quantize_backward: bad shape");
+  const char* fn = kRotate ? "vqb_quantize_backward_rotated" : "vqb_quantize_backward";
+  VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
+  VQB_REQUIRE(gz && x && W && quant && gx, "%s: null pointer", fn);
+  VQB_REQUIRE(!kRowsOut || gW, "%s_rows: null gW_rows", fn);
+  VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "%s: bad shape", fn);
   RowGeom geom;
-  VQB_REQUIRE(row_geom(D, N, &geom), "vqb_quantize_backward: D=%d unsupported", D);
+  VQB_REQUIRE(row_geom(D, N, &geom), "%s: D=%d unsupported", fn, D);
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = grid_for(N, 256 / geom.G);
   bool launched = false;
 #define VQB_QUANTIZE_BWD(TX_, TG_)                                                                                     \
-  VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>, blocks, 256, 0, st,            \
+  VQB_DISPATCH_GEOM((launch_pdl(quantize_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate>, blocks, 256, 0, st,   \
       (const TG_*)gz, (const TX_*)x, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn, want_norm, (TX_*)gx, gW, \
       g_hw)))
   VQB_DISPATCH_BWD_DTYPES(VQB_QUANTIZE_BWD)
 #undef VQB_QUANTIZE_BWD
-  VQB_REQUIRE(launched, "vqb_quantize_backward: unsupported dtype/geometry");
+  VQB_REQUIRE(launched, "%s: unsupported dtype/geometry", fn);
   VQB_LAUNCH_OK();
   return VQB_OK;
 }
@@ -884,16 +936,32 @@ int vqb_quantize_backward(const void* gz, int g_dtype, const void* x, int x_dtyp
                           const int64_t* quant, int64_t N, int D, const float* g_cb, const float* g_cm,
                           const float* g_cbn, const float* g_cmn, int want_norm, void* gx, float* gW, int64_t g_hw,
                           void* stream) {
-  return quantize_backward_launch<false>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn,
-                                         want_norm, gx, gW, g_hw, stream);
+  return quantize_backward_launch<false, false>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm,
+                                                g_cbn, g_cmn, want_norm, gx, gW, g_hw, stream);
 }
 
 int vqb_quantize_backward_rows(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x, const float* W,
                                int64_t K, const int64_t* quant, int64_t N, int D, const float* g_cb, const float* g_cm,
                                const float* g_cbn, const float* g_cmn, int want_norm, void* gx, float* gW_rows,
                                int64_t g_hw, void* stream) {
-  return quantize_backward_launch<true>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn, g_cmn,
-                                        want_norm, gx, gW_rows, g_hw, stream);
+  return quantize_backward_launch<true, false>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm,
+                                               g_cbn, g_cmn, want_norm, gx, gW_rows, g_hw, stream);
+}
+
+int vqb_quantize_backward_rotated(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x,
+                                  const float* W, int64_t K, const int64_t* quant, int64_t N, int D, const float* g_cb,
+                                  const float* g_cm, const float* g_cbn, const float* g_cmn, int want_norm, void* gx,
+                                  float* gW, int64_t g_hw, void* stream) {
+  return quantize_backward_launch<false, true>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm,
+                                               g_cbn, g_cmn, want_norm, gx, gW, g_hw, stream);
+}
+
+int vqb_quantize_backward_rotated_rows(const void* gz, int g_dtype, const void* x, int x_dtype, int normalize_x,
+                                       const float* W, int64_t K, const int64_t* quant, int64_t N, int D,
+                                       const float* g_cb, const float* g_cm, const float* g_cbn, const float* g_cmn,
+                                       int want_norm, void* gx, float* gW_rows, int64_t g_hw, void* stream) {
+  return quantize_backward_launch<true, true>(gz, g_dtype, x, x_dtype, normalize_x, W, K, quant, N, D, g_cb, g_cm, g_cbn,
+                                              g_cmn, want_norm, gx, gW_rows, g_hw, stream);
 }
 
 int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N, int D, const float* W,
@@ -938,11 +1006,13 @@ int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype,
 
 // The one-launch backward over the members of a vqb_residual_levels table: the levels of a residual chain
 // (residual_backward_kernel on tokens of width D) or the channel groups of a grouped quantizer (group_backward_kernel,
-// D the group width Dg, one grid row per group).  Messages name the members as "level" or "group".
-template <bool kGroups, bool kRowsOut>
+// D the group width Dg, one grid row per group).  Messages name the members as "level" or "group".  kRotate (groups
+// only): the rotation trick of group_backward_kernel.
+template <bool kGroups, bool kRowsOut, bool kRotate = false>
 static int member_backward_launch(const char* fn, const void* gz, int g_dtype, const void* x, int x_dtype,
                                   const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int D,
                                   int want_norm, void* gx, int64_t g_hw, void* stream) {
+  static_assert(kGroups || !kRotate, "residual levels have no rotated backward");
   const char* member = kGroups ? "of group" : "at level";
   VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
   VQB_REQUIRE(gz && x && lv && quant && gx, "%s: null pointer", fn);
@@ -959,7 +1029,7 @@ static int member_backward_launch(const char* fn, const void* gz, int g_dtype, c
   const dim3 grid((unsigned)grid_for(N, 256 / geom.G), kGroups ? (unsigned)lv->L : 1u);
   bool launched = false;
 #define VQB_MEMBER_BWD(TX_, TG_)                                                                                      \
-  VQB_DISPATCH_GEOM((launch_pdl(kGroups ? group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>                          \
+  VQB_DISPATCH_GEOM((launch_pdl(kGroups ? group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate>                 \
                                         : residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>,                      \
       grid, 256, 0, st, (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw)))
   VQB_DISPATCH_BWD_DTYPES(VQB_MEMBER_BWD)
@@ -1032,6 +1102,20 @@ int vqb_group_backward_rows(const void* gz, int g_dtype, const void* xs, int x_d
                             void* stream) {
   return member_backward_launch<true, true>("vqb_group_backward_rows", gz, g_dtype, xs, x_dtype, groups, K, quant, N,
                                            Dg, want_norm, gx, g_hw, stream);
+}
+
+int vqb_group_backward_rotated(const void* gz, int g_dtype, const void* xs, int x_dtype,
+                               const vqb_residual_levels* groups, int64_t K, const int64_t* quant, int64_t N, int Dg,
+                               int want_norm, void* gx, int64_t g_hw, void* stream) {
+  return member_backward_launch<true, false, true>("vqb_group_backward_rotated", gz, g_dtype, xs, x_dtype, groups, K,
+                                                   quant, N, Dg, want_norm, gx, g_hw, stream);
+}
+
+int vqb_group_backward_rotated_rows(const void* gz, int g_dtype, const void* xs, int x_dtype,
+                                    const vqb_residual_levels* groups, int64_t K, const int64_t* quant, int64_t N,
+                                    int Dg, int want_norm, void* gx, int64_t g_hw, void* stream) {
+  return member_backward_launch<true, true, true>("vqb_group_backward_rotated_rows", gz, g_dtype, xs, x_dtype, groups,
+                                                  K, quant, N, Dg, want_norm, gx, g_hw, stream);
 }
 
 int vqb_unpack_keys(const unsigned long long* keys, int64_t n, int64_t offset, int64_t* idx, float* score,

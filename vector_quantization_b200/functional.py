@@ -296,7 +296,7 @@ class _QuantizeSTELoss(torch.autograd.Function):
     back as four device scalars (no select_backward / stack kernels between the loss and our backward)."""
 
     @staticmethod
-    def forward(ctx, x, W, index, index_is_keys, key_offset, normalize_x, want_norm, ref, x_nchw):
+    def forward(ctx, x, W, index, index_is_keys, key_offset, normalize_x, want_norm, ref, x_nchw, rotate):
         # x_nchw: the caller's [b, c, h, w] latents of which `x` is the (detached) token-major copy: z is then written
         # straight into that layout and the backward reads / writes NCHW gradients (no transposes around the kernels)
         hw = 0 if x_nchw is None else x_nchw.shape[2] * x_nchw.shape[3]
@@ -311,7 +311,7 @@ class _QuantizeSTELoss(torch.autograd.Function):
             quant = index
         ctx.save_for_backward(x, quant)
         ctx.codebook = ref if ref is not None else CodebookRef(W.detach())
-        ctx.cfg = (normalize_x, want_norm)
+        ctx.cfg = (normalize_x, want_norm, rotate)
         ctx.set_materialize_grads(False)   # unused outputs arrive as None instead of freshly zero-filled tensors
         if xn is None:
             xn = x.detach()
@@ -323,29 +323,32 @@ class _QuantizeSTELoss(torch.autograd.Function):
     def backward(ctx, gz, g0, g1, g2, g3, _gq, _gxn):
         x, quant = ctx.saved_tensors
         W = ctx.codebook.tensor
-        normalize_x, want_norm = ctx.cfg
+        normalize_x, want_norm, rotate = ctx.cfg
         if gz is None:
             gz = torch.zeros(ctx.nchw or x.shape, dtype=torch.float32, device=x.device)
         g4 = [None if g is None else g.contiguous().float() for g in (g0, g1, g2, g3)]
         hw = 0 if ctx.nchw is None else ctx.nchw[2] * ctx.nchw[3]
         need_gx = ctx.needs_input_grad[0] or ctx.needs_input_grad[8]
         gx, gW = ops.quantize_backward(gz.contiguous(), x, W, quant, g4, normalize_x=normalize_x,
-                                       want_norm=want_norm, need_gW=ctx.needs_input_grad[1], g_hw=hw)
+                                       want_norm=want_norm, need_gW=ctx.needs_input_grad[1], g_hw=hw, rotate=rotate)
         if ctx.nchw is not None:     # the gradient belongs to the NCHW latents
-            return None, gW, None, None, None, None, None, None, (gx.view(ctx.nchw) if need_gx else None)
-        return (gx if need_gx else None), gW, None, None, None, None, None, None, None
+            return None, gW, None, None, None, None, None, None, (gx.view(ctx.nchw) if need_gx else None), None
+        return (gx if need_gx else None), gW, None, None, None, None, None, None, None, None
 
 
 def quantize_ste_loss(x: torch.Tensor, W: torch.Tensor, index: torch.Tensor, want_norm: bool, *,
                       index_is_keys: bool = False, key_offset: int = 0, normalize_x: bool = False,
-                      codebook_ref: CodebookRef | None = None, nchw: torch.Tensor | None = None):
+                      codebook_ref: CodebookRef | None = None, nchw: torch.Tensor | None = None,
+                      rotate: bool = False):
     """One kernel: [x' = F.normalize(x)] -> gather W[q] -> straight-through -> MSE terms.
+    rotate: the gradient of z reaches x' through the rotation trick (DESIGN.md §4.9) instead of straight through; the
+    values and the codebook gradient are unchanged.
     -> (z_ste [N,D] fp32: value x' + (W[q] - x'), gradient to x only;
         mse4 = (codebook, commitment, codebook(norm), commitment(norm)) as four 0-dim tensors;
         quant int64 [N] (unpacked from the keys when index_is_keys);  x' (detached; x itself if not normalised))"""
     z, m0, m1, m2, m3, quant, xn = _QuantizeSTELoss.apply(x.contiguous(), W, index, bool(index_is_keys),
                                                           int(key_offset), bool(normalize_x), bool(want_norm),
-                                                          codebook_ref, nchw)
+                                                          codebook_ref, nchw, bool(rotate))
     return z, (m0, m1, m2, m3), quant, xn
 
 
@@ -475,7 +478,7 @@ class _GroupedQuantize(torch.autograd.Function):
     gradients arrive as device scalars); memos[g] gets 'x' (the split slice xs[g]) and 'quant' (quant[:, g])."""
 
     @staticmethod
-    def forward(ctx, x, groups, memos, want_norm, track, *Ws):
+    def forward(ctx, x, groups, memos, want_norm, track, rotate, *Ws):
         G = len(groups)
         nchw = x.dim() == 4
         hw = x.shape[2] * x.shape[3] if nchw else 0
@@ -494,6 +497,7 @@ class _GroupedQuantize(torch.autograd.Function):
         ctx.shape = tuple(x.shape)
         ctx.hw = hw
         ctx.want_norm = want_norm
+        ctx.rotate = rotate
         ctx.set_materialize_grads(False)
         ctx.mark_non_differentiable(quant)
         return (z, quant) + tuple(mse.view(-1).unbind(0))
@@ -505,21 +509,22 @@ class _GroupedQuantize(torch.autograd.Function):
         if gz is None:
             gz = torch.zeros(ctx.shape, dtype=torch.float32, device=xs.device)
         g4s = [[None if t is None else t.contiguous().float() for t in g[4 * i:4 * i + 4]] for i in range(G)]
-        need_gW = list(ctx.needs_input_grad[5:5 + G])
+        need_gW = list(ctx.needs_input_grad[6:6 + G])
         gx, gWs = ops.group_backward(gz.contiguous(), xs, [r.tensor for r in ctx.refs], quant, g4s,
-                                     want_norm=ctx.want_norm, need_gW=need_gW, g_hw=ctx.hw)
-        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, *gWs)
+                                     want_norm=ctx.want_norm, need_gW=need_gW, g_hw=ctx.hw, rotate=ctx.rotate)
+        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, None, *gWs)
 
 
-def grouped_quantize(groups, x: torch.Tensor, memos, want_norm: bool):
+def grouped_quantize(groups, x: torch.Tensor, memos, want_norm: bool, *, rotate: bool = False):
     """Grouped quantization of x (tokens [N, D] or latents [b, D, h, w]; fp32 / bf16) through `groups` (VectorQuantizer
     modules sharing K and Dg = D / G), group g on channels [g*Dg, (g+1)*Dg).
     -> (z fp32 in x's layout: value x_g + (W_g[q_g] - x_g) per group, gradient straight to x;  quant int64 [N, G];
         mse: per group the four MSE terms (codebook, commitment, codebook-norm,
-        commitment-norm) of W_g[q_g] against x_g, 0-dim tensors whose gradients reach W_g and x)"""
+        commitment-norm) of W_g[q_g] against x_g, 0-dim tensors whose gradients reach W_g and x)
+    rotate: the gradient of z reaches x through the rotation trick of each group (DESIGN.md §4.9)"""
     Ws = [group._weight() for group in groups]
     track = torch.is_grad_enabled() and (x.requires_grad or any(W.requires_grad for W in Ws))
-    out = _GroupedQuantize.apply(x.contiguous(), list(groups), memos, bool(want_norm), track, *Ws)
+    out = _GroupedQuantize.apply(x.contiguous(), list(groups), memos, bool(want_norm), track, bool(rotate), *Ws)
     z, quant, flat = out[0], out[1], out[2:]
     return z, quant, [tuple(flat[4 * i:4 * i + 4]) for i in range(len(groups))]
 

@@ -392,11 +392,13 @@ def gather_ste_loss(x: torch.Tensor, W: torch.Tensor, *, quant: torch.Tensor | N
 
 def quantize_backward(g_z: torch.Tensor, x: torch.Tensor, W: torch.Tensor, quant: torch.Tensor, g4, *,
                       normalize_x: bool = False, want_norm: bool, need_gW: bool, g_hw: int = 0,
-                      deterministic: bool | None = None):
+                      deterministic: bool | None = None, rotate: bool = False):
     """g4: a float32 [4] tensor or a sequence of four 0-dim device tensors / None
     (codebook, commitment, codebook-norm, commitment-norm upstream gradients).
     deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, gW is the segment sum of the
-    per-token gradient rows (fixed association, see vqb_segment_sum_rows) instead of fp32 atomics.  gx is the same."""
+    per-token gradient rows (fixed association, see vqb_segment_sum_rows) instead of fp32 atomics.  gx is the same.
+    rotate: pass g_z to the tokens through the rotation trick (vqb_quantize_backward_rotated; DESIGN.md §4.9) instead of
+    straight through; gW is unchanged."""
     lib = _lib.load()
     if isinstance(g4, torch.Tensor):
         g4 = [g4[i] for i in range(4)]
@@ -410,14 +412,14 @@ def quantize_backward(g_z: torch.Tensor, x: torch.Tensor, W: torch.Tensor, quant
     gW = torch.zeros_like(W) if need_gW else None
     if need_gW and deterministic_enabled(deterministic):
         rows = _det_ws(x.device, 'gw_rows', N * D, torch.float32)
-        _call('vqb_quantize_backward_rows', lib.vqb_quantize_backward_rows, dev, _p(g_z), _dt(g_z), _p(x), _dt(x),
-              int(normalize_x), _p(W), K, _p(quant), N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm),
-              _p(gx), _p(rows), g_hw, _S)
+        name = 'vqb_quantize_backward_rotated_rows' if rotate else 'vqb_quantize_backward_rows'
+        _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), int(normalize_x), _p(W), K, _p(quant),
+              N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm), _p(gx), _p(rows), g_hw, _S)
         _segment_sum_members(dev, rows.view(1, N, D), quant, K, [gW])
         return gx, gW
-    _call('vqb_quantize_backward', lib.vqb_quantize_backward, dev, _p(g_z), _dt(g_z), _p(x), _dt(x), int(normalize_x), _p(W),
-          K, _p(quant), N, D, _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm), _p(gx), _p(gW),
-          g_hw, _S)
+    name = 'vqb_quantize_backward_rotated' if rotate else 'vqb_quantize_backward'
+    _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), int(normalize_x), _p(W), K, _p(quant), N, D,
+          _p(g4[0]), _p(g4[1]), _p(g4[2]), _p(g4[3]), int(want_norm), _p(gx), _p(gW), g_hw, _S)
     return gx, gW
 
 
@@ -934,13 +936,14 @@ def group_gather_ste_loss(xs: torch.Tensor, Ws, *, quant: torch.Tensor | None = 
 
 
 def group_backward(g_z: torch.Tensor, xs: torch.Tensor, Ws, quant: torch.Tensor, g4s, *, want_norm: bool, need_gW,
-                   g_hw: int = 0, deterministic: bool | None = None):
+                   g_hw: int = 0, deterministic: bool | None = None, rotate: bool = False):
     """Backward of every group in one launch (vqb_group_backward).  g_z: fp32 (or bf16 with bf16 tokens) [N, G*Dg], or
     NCHW with g_hw = h*w (gx then has g_z's NCHW shape); xs: the forward's split tokens [G, N, Dg]; quant: int64 [N, G];
     g4s: per group four 0-dim fp32 device tensors / None; need_gW: per group bool.
     deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, each gW_g is the segment sum of
     the group's per-token rows (vqb_group_backward_rows + vqb_code_sort + vqb_segment_sum_rows, the contract of
-    quantize_backward).  -> (gx in xs's dtype with g_z's shape, [gW_g fp32 [K, Dg] or None])"""
+    quantize_backward).  rotate: the rotation trick per group, as in quantize_backward.
+    -> (gx in xs's dtype with g_z's shape, [gW_g fp32 [K, Dg] or None])"""
     lib = _lib.load()
     G = len(Ws)
     dev = _cuda(g_z, xs, quant, *Ws, *[g for g4 in g4s for g in g4])
@@ -955,13 +958,15 @@ def group_backward(g_z: torch.Tensor, xs: torch.Tensor, Ws, quant: torch.Tensor,
     if any(need_gW) and deterministic_enabled(deterministic):
         rows = _det_ws(xs.device, 'gw_rows', G * N * Dg, torch.float32).view(G, N, Dg)
         p = _residual_levels(Ws, list(rows), g4s)
-        _call('vqb_group_backward_rows', lib.vqb_group_backward_rows, dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs),
-              ctypes.byref(p), K, _p(quant), N, Dg, int(want_norm), _p(gx), g_hw, _S)
+        name = 'vqb_group_backward_rotated_rows' if rotate else 'vqb_group_backward_rows'
+        _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs), ctypes.byref(p), K, _p(quant), N, Dg,
+              int(want_norm), _p(gx), g_hw, _S)
         _segment_sum_members(dev, rows, quant, K, gWs)
         return gx, gWs
     p = _residual_levels(Ws, gWs, g4s)
-    _call('vqb_group_backward', lib.vqb_group_backward, dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs), ctypes.byref(p), K,
-          _p(quant), N, Dg, int(want_norm), _p(gx), g_hw, _S)
+    name = 'vqb_group_backward_rotated' if rotate else 'vqb_group_backward'
+    _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs), ctypes.byref(p), K, _p(quant), N, Dg,
+          int(want_norm), _p(gx), g_hw, _S)
     return gx, gWs
 
 

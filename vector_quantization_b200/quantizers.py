@@ -24,7 +24,7 @@ from torch import nn
 from . import functional as Fq
 from . import ops, parallel
 from ._lib import MAX_LEVELS, VQBError
-from .callbacks import ComposedCallback
+from .callbacks import BaseCallback, ComposedCallback
 from .distances import BaseDistance
 from .registry import (Config, InitRegistry, ModelRegistry, ModuleDict, VQITQuantizerCallbackRegistry,
                        VQITQuantizerDistanceRegistry, VQITQuantizerLossRegistry, VQITQuantizerRegistry,
@@ -151,13 +151,26 @@ class BaseQuantizer(nn.Module):
 @VQITQuantizerRegistry.register_()
 class VectorQuantizer(BaseQuantizer):
     """distance -> arg-min -> (codebook update callbacks) -> gather -> losses -> straight-through, as three
-    kernel launches: pack+assign (tcgen05, no N x K matrix), [stats/update], fused gather+STE+loss."""
+    kernel launches: pack+assign (tcgen05, no N x K matrix), [stats/update], fused gather+STE+loss.
+
+    rotation_trick: the encoder gradient of z follows the rotation trick (Fifty et al., arXiv:2410.06424; DESIGN.md
+    §4.9) instead of the straight-through estimator.  z, the losses, the indices, the codebook updates and the codebook
+    gradient are unchanged; only the gradient reaching x differs.  Not available with callbacks that hook decode or
+    loss (they run the unfused template)."""
 
     def __init__(self, *args, embedding: nn.Embedding, distance: BaseDistance, precision: str = Fq.DEFAULT_PRECISION,
-                 materialize_distance: bool = False, **kwargs) -> None:
+                 materialize_distance: bool = False, rotation_trick: bool = False, **kwargs) -> None:
         super().__init__(*args, **kwargs)
         if precision not in Fq.PRECISION_PLANES:
             raise ValueError(f'precision must be one of {sorted(Fq.PRECISION_PLANES)}')
+        self.rotation_trick = bool(rotation_trick)
+        if self.rotation_trick:
+            for c in self._callbacks:
+                hooks = [h for h in ('before_decode', 'after_decode', 'before_loss', 'after_loss')
+                         if getattr(type(c), h) is not getattr(BaseCallback, h)]
+                if hooks:
+                    raise ValueError(f'{type(self).__name__}: rotation_trick is not supported with callback '
+                                     f'{type(c).__name__}, which hooks {", ".join(hooks)} (the unfused template path)')
         self._embedding = embedding
         self._distance = distance
         self.precision = precision
@@ -356,7 +369,8 @@ class VectorQuantizer(BaseQuantizer):
             if ref is not None:
                 self._pending.add(ref)
         z, mse4, quant, xn = Fq.quantize_ste_loss(x, W, index, self._loss_terms(), index_is_keys=lazy_unpack,
-                                                  normalize_x=normalize_x, codebook_ref=ref, nchw=nchw)
+                                                  normalize_x=normalize_x, codebook_ref=ref, nchw=nchw,
+                                                  rotate=self.rotation_trick)
         memo.update(x=xn if normalize_x else x, quant=quant)
         memo['decode'] = get_memo(memo, 'decode')
         loss_memo = get_memo(memo, 'loss')
@@ -485,6 +499,9 @@ def _check_member(owner: str, member, members: str) -> None:
         raise ValueError(f'{owner}: the {members} must be VectorQuantizer modules, got {name}')
     if member.materialize_distance:
         raise ValueError(f'{owner}: materialize_distance (compatibility mode) is not supported')
+    if members == 'levels' and member.rotation_trick:
+        raise ValueError(f'{owner}: rotation_trick is not supported for residual levels (one straight-through '
+                         'estimator spans the whole depth)')
     for c in member._callbacks:
         cname = type(c).__name__
         if isinstance(c, NormalizeCallback):
@@ -526,7 +543,8 @@ class ResidualVectorQuantizer(BaseQuantizer):
     Accepted: 1 <= L <= 16, L2 or Cosine distance, no callback or CVQVAECallback (NearestAnchor / CachedAnchor),
     CodebookLoss / CommitmentLoss / VQGANLoss with or without mse.norm.  Rejected with a ValueError: callbacks that
     rewrite the tokens (NormalizeCallback and its subclasses), callbacks that hook decode or loss, and compatibility
-    mode (EntropyLoss, MultinomialAnchor, materialize_distance).  `init_weights` is applied to every level."""
+    mode (EntropyLoss, MultinomialAnchor, materialize_distance), and rotation_trick=True.  `init_weights` is applied to
+    every level."""
 
     MAX_LEVELS = 16
 
@@ -647,7 +665,8 @@ class GroupedVectorQuantizer(BaseQuantizer):
     slice, encode, decode, loss), 'loss' (per loss name, the group mean).
 
     Accepted and rejected configurations are those of ResidualVectorQuantizer (see `_build_members`), with
-    1 <= num_groups <= 16.  `init_weights` is applied to every group."""
+    1 <= num_groups <= 16, except that the group config may set rotation_trick=True: every group then passes its
+    encoder gradient through the rotation trick (DESIGN.md §4.9).  `init_weights` is applied to every group."""
 
     def __init__(self, *args, num_groups: int, quantizer: Mapping, **kwargs) -> None:
         super().__init__(*args, **kwargs)
@@ -757,7 +776,7 @@ class GroupedVectorQuantizer(BaseQuantizer):
         x = self._check_input(x)
         groups = list(self._quantizers)
         memos = self._group_memos(memo)
-        z, quant, mse = Fq.grouped_quantize(groups, x, memos, self._want_norm())
+        z, quant, mse = Fq.grouped_quantize(groups, x, memos, self._want_norm(), rotate=groups[0].rotation_trick)
         memo.update(x=x, quant=quant)
         loss_memo = get_memo(memo, 'loss')
         sums: dict = {}
