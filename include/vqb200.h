@@ -296,6 +296,18 @@ int vqb_residual_backward(const void* g_z, int g_dtype, const void* x, int x_dty
 int vqb_residual_backward_rows(const void* g_z, int g_dtype, const void* x, int x_dtype,
                                const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
                                int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
+/* vqb_residual_backward / _rows with the rotation trick of vqb_quantize_backward_rotated over the whole depth, the
+ * stack's one straight-through estimator (DESIGN.md §4.7, §4.9).  Per token, in fp32 (bf16 tokens up-cast):
+ *   zhat_L = W_0[q_0] + W_1[q_1] + ... + W_{L-1}[q_{L-1}]   (round-to-nearest adds in level order: the forward's zhat)
+ *   g' = rotate(x, zhat_L, g_z)   (|x| or |zhat_L| below 1e-12: g' = g_z)
+ *   gx = g' + sum_l [commitment-role terms of level l]   (unchanged, level order)
+ * gW_l is bit-identical to the unrotated entry points; only gx differs. */
+int vqb_residual_backward_rotated(const void* g_z, int g_dtype, const void* x, int x_dtype,
+                                  const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
+                                  int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
+int vqb_residual_backward_rotated_rows(const void* g_z, int g_dtype, const void* x, int x_dtype,
+                                       const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N,
+                                       int D, int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
 
 /* ---- grouped (product) quantization: G codebooks, group g quantizes channels [g*Dg, (g+1)*Dg) of every token ---- *
  * Group g behaves exactly like its own vqb_gather_ste_loss / vqb_quantize_backward on the contiguous [N, Dg] slice

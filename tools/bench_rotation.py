@@ -2,13 +2,14 @@
 
     python tools/bench_rotation.py [--steps 30] [--warmup 5] [--rounds 3] [--out FILE]
 
-Training step = forward + backward of the quantizer, for four workloads (WORKLOADS) and three paths:
+Training step = forward + backward of the quantizer, for four single / grouped workloads (WORKLOADS), three
+residual ones (RVQ_WORKLOADS: those of tools/bench_rvq.py, the rotation over the whole depth) and three paths:
   a  rotation_trick=True: the rotation runs inside the one backward launch;
   b  rotation_trick=False: the straight-through step, as before;
   c  the module with the straight-through estimator plus eager rotation glue on its output
      (z = lambda R x with lambda, R from x and z.detach(), as in oracle/rotation.py): what users write today.
-Backward kernel alone: ops.quantize_backward / ops.group_backward with rotate on and off on the forward's saved
-tensors, each call between an L2 flush (a 256 MB write) and timed with CUDA events around the call only.
+Backward kernel alone: ops.quantize_backward / ops.group_backward / ops.residual_backward with rotate on and off on
+the forward's saved tensors, each call between an L2 flush (a 256 MB write) and timed with CUDA events around the call only.
 Timing: CUDA events around `steps` back-to-back calls after `warmup` calls, `rounds` rounds with the paths
 alternating, the median round reported.  Inputs rotate over enough seeded sets to exceed the 126 MB L2.
 Before timing, a and b run from the same codebooks on the same input: z, the loss and the indices must be bitwise
@@ -44,6 +45,18 @@ WORKLOADS = {
                     'VQGANQuantizer'),
     'gvq_vqgan_grid': ((64, 256, 16, 16), 4, 8192, 'L2', [], torch.float32, VQGAN_LOSS, 'VQGANQuantizer'),
 }
+CVQ = [dict(type='CVQVAECallback', anchor=dict(type='NearestAnchor'), ema=dict())]
+# ResidualVectorQuantizer(rotation_trick=...) over levels of `quantizer`; the fields of WORKLOADS with the number of
+# levels L in place of the groups
+RVQ_WORKLOADS = {
+    'rvq_rqvae_like': ((256, 256, 8, 8), 4, 16384, 'L2', [], torch.float32, VQGAN_LOSS, 'VQGANQuantizer'),
+    'rvq_vqgan_grid_cvq': ((64, 256, 16, 16), 4, 8192, 'Cosine', CVQ, torch.float32, VQGAN_LOSS, 'VQGANQuantizer'),
+    'rvq_small_d': ((256, 8, 16, 16), 8, 16384, 'L2', [], torch.float32, VQGAN_LOSS, 'VQGANQuantizer'),
+}
+
+
+def workload(name):
+    return WORKLOADS[name] if name in WORKLOADS else RVQ_WORKLOADS[name]
 
 
 def gpu_info() -> dict:
@@ -58,6 +71,8 @@ def gpu_info() -> dict:
 
 
 def build(name, dev, rotation_trick):
+    if name in RVQ_WORKLOADS:
+        return build_rvq(name, dev, rotation_trick)
     shape, G, K, dist, callbacks, _, losses, kind = WORKLOADS[name]
     D = shape[1]
     node = dict(type=kind, distance=dict(type=f'{dist}Distance'), callbacks=callbacks, losses=losses,
@@ -73,8 +88,23 @@ def build(name, dev, rotation_trick):
     return q
 
 
+def build_rvq(name, dev, rotation_trick):
+    """The residual workloads with the codebooks of tools/bench_rvq.py (level l at scale 0.6**l)."""
+    shape, L, K, dist, callbacks, _, losses, kind = RVQ_WORKLOADS[name]
+    D = shape[1]
+    node = dict(type=kind, distance=dict(type=f'{dist}Distance'), callbacks=callbacks, losses=losses,
+                embedding=dict(type='torch_nn_modules_sparse_Embedding', num_embeddings=K, embedding_dim=D))
+    q = vqb.build_quantizer(dict(type='ResidualVectorQuantizer', num_quantizers=L, quantizer=node,
+                                 rotation_trick=rotation_trick), training=True).to(dev)
+    g = torch.Generator().manual_seed(7)
+    with torch.no_grad():
+        for l, level in enumerate(q.quantizers):
+            level.embedding.weight.copy_(torch.randn(K, D, generator=g) * 0.6 ** l)
+    return q
+
+
 def inputs(name, dev):
-    shape, _, _, _, _, dtype, _, _ = WORKLOADS[name]
+    shape, _, _, _, _, dtype, _, _ = workload(name)
     g = torch.Generator().manual_seed(11)
     size = math.prod(shape) * (2 if dtype == torch.bfloat16 else 4)
     sets = max(2, math.ceil(2 * L2_BYTES / size))
@@ -126,21 +156,22 @@ def timed(fn, xs, steps, warmup):
 def backward_kernel_us(q, x, gz, rotate, reps, flush):
     """The backward launch alone (rotate on / off) on the forward's saved tensors, L2 flushed before each call."""
     captured = {}
-    real_qb, real_gb = ops.quantize_backward, ops.group_backward
+    names = ('quantize_backward', 'group_backward', 'residual_backward')
+    real = {n: getattr(ops, n) for n in names}
 
-    def grab_qb(*a, **kw):
-        captured.update(fn=real_qb, a=a, kw=kw)
-        return real_qb(*a, **kw)
+    def grab(fn):
+        def call(*a, **kw):
+            captured.update(fn=fn, a=a, kw=kw)
+            return fn(*a, **kw)
+        return call
 
-    def grab_gb(*a, **kw):
-        captured.update(fn=real_gb, a=a, kw=kw)
-        return real_gb(*a, **kw)
-
-    ops.quantize_backward, ops.group_backward = grab_qb, grab_gb
+    for n in names:
+        setattr(ops, n, grab(real[n]))
     try:
         step(q, x, gz)
     finally:
-        ops.quantize_backward, ops.group_backward = real_qb, real_gb
+        for n in names:
+            setattr(ops, n, real[n])
     fn, args, kw = captured['fn'], captured['a'], dict(captured['kw'], rotate=rotate)
     times = []
     for i in range(reps + 3):
@@ -156,9 +187,10 @@ def backward_kernel_us(q, x, gz, rotate, reps, flush):
 
 
 def run(name, dev, args) -> dict:
-    shape, G, K, dist, callbacks, dtype, _, kind = WORKLOADS[name]
-    rec = dict(workload=name, shape=list(shape), groups=G, K=K, distance=dist, quantizer=kind,
+    shape, G, K, dist, callbacks, dtype, _, kind = workload(name)
+    rec = dict(workload=name, shape=list(shape), K=K, distance=dist, quantizer=kind,
                callbacks=[c['type'] for c in callbacks], dtype=str(dtype).split('.')[-1])
+    rec['levels' if name in RVQ_WORKLOADS else 'groups'] = G
     xs, gz = inputs(name, dev)
     rec['input_sets'] = len(xs)
     qa, qb, qc = build(name, dev, True), build(name, dev, False), build(name, dev, False)
@@ -198,7 +230,7 @@ def main() -> None:
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--rounds', type=int, default=3)
     ap.add_argument('--out', type=str, default=None)
-    ap.add_argument('--workloads', nargs='*', default=list(WORKLOADS))
+    ap.add_argument('--workloads', nargs='*', default=list(WORKLOADS) + list(RVQ_WORKLOADS))
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit('bench_rotation.py measures on a CUDA device; none is available')

@@ -96,6 +96,10 @@ SIGNATURES = {
                                       c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_residual_backward_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
                                            c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_residual_backward_rotated': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64,
+                                              c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_residual_backward_rotated_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64,
+                                                   c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_group_gather_ste_loss': (c_int, [c_void_p, c_int, c_int64, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
                                           c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p,
                                           c_void_p]),

@@ -565,7 +565,9 @@ __global__ void __launch_bounds__(256) residual_step_kernel(
 // contributes quantize_backward_kernel's terms with (y, z) = (r_{l-1}, W_l[q_l]) (no token normalisation): its
 // commitment-role terms accumulate onto g_z in level order, its codebook-role row goes to gW_l (atomics, or the level's
 // [N, D] rows with kRowsOut).  The level table is a __grid_constant__ parameter: indexed in place, never copied.
-template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut>
+// kRotate: the rotation trick over the whole depth (DESIGN.md §4.9): before the level loop, g_z is replaced by
+// rotate_grad(x, zhat_L, g_z), with zhat_L = W_0[q_0] + ... + W_{L-1}[q_{L-1}] rebuilt in wr with the forward's adds.
+template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut, bool kRotate = false>
 __global__ void __launch_bounds__(256) residual_backward_kernel(
     const TG* __restrict__ gz, const TX* __restrict__ x, const __grid_constant__ vqb_residual_levels lv, int64_t K,
     const int64_t* __restrict__ quant, int64_t N, int D, int want_norm, TX* __restrict__ gx, int64_t g_hw) {
@@ -592,6 +594,36 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
 #pragma unroll
         for (int i = 0; i < V; ++i) yr[it][i] = gr[it][i] = 0.f;
       }
+    }
+    if constexpr (kRotate) {
+      // zhat_L into wr (the level loop reloads it): level 0's row, then each deeper row added in level order
+#pragma unroll 1
+      for (int l = 0; l < L; ++l) {
+        const int64_t q = row_index(quant, nullptr, n * L + l, 0, K);
+        const float* __restrict__ wrow = lv.W[l] + q * D;
+#pragma unroll
+        for (int it = 0; it < NV; ++it) {
+          const int d0 = (it * G + lane) * V;
+          float e[V];
+          if (d0 < D) {
+            load_slice<float, V>(wrow, d0, D, e);
+          } else {
+#pragma unroll
+            for (int i = 0; i < V; ++i) e[i] = 0.f;
+          }
+#pragma unroll
+          for (int i = 0; i < V; ++i) wr[it][i] = l == 0 ? e[i] : __fadd_rn(wr[it][i], e[i]);
+        }
+      }
+      float sxx = 0.f, sww = 0.f;
+#pragma unroll
+      for (int it = 0; it < NV; ++it)
+#pragma unroll
+        for (int i = 0; i < V; ++i) {
+          sxx = fmaf(yr[it][i], yr[it][i], sxx);
+          sww = fmaf(wr[it][i], wr[it][i], sww);
+        }
+      rotate_grad<G, V, NV>(yr, wr, gr, sxx, sww);
     }
 #pragma unroll 1
     for (int l = 0; l < L; ++l) {
@@ -1006,13 +1038,12 @@ int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype,
 
 // The one-launch backward over the members of a vqb_residual_levels table: the levels of a residual chain
 // (residual_backward_kernel on tokens of width D) or the channel groups of a grouped quantizer (group_backward_kernel,
-// D the group width Dg, one grid row per group).  Messages name the members as "level" or "group".  kRotate (groups
-// only): the rotation trick of group_backward_kernel.
+// D the group width Dg, one grid row per group).  Messages name the members as "level" or "group".  kRotate: the
+// rotation trick, per group (group_backward_kernel) or over the whole depth (residual_backward_kernel).
 template <bool kGroups, bool kRowsOut, bool kRotate = false>
 static int member_backward_launch(const char* fn, const void* gz, int g_dtype, const void* x, int x_dtype,
                                   const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int D,
                                   int want_norm, void* gx, int64_t g_hw, void* stream) {
-  static_assert(kGroups || !kRotate, "residual levels have no rotated backward");
   const char* member = kGroups ? "of group" : "at level";
   VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
   VQB_REQUIRE(gz && x && lv && quant && gx, "%s: null pointer", fn);
@@ -1030,7 +1061,7 @@ static int member_backward_launch(const char* fn, const void* gz, int g_dtype, c
   bool launched = false;
 #define VQB_MEMBER_BWD(TX_, TG_)                                                                                      \
   VQB_DISPATCH_GEOM((launch_pdl(kGroups ? group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate>                 \
-                                        : residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut>,                      \
+                                        : residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate>,             \
       grid, 256, 0, st, (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw)))
   VQB_DISPATCH_BWD_DTYPES(VQB_MEMBER_BWD)
 #undef VQB_MEMBER_BWD
@@ -1053,6 +1084,20 @@ int vqb_residual_backward_rows(const void* gz, int g_dtype, const void* x, int x
                                int want_norm, void* gx, int64_t g_hw, void* stream) {
   return member_backward_launch<false, true>("vqb_residual_backward_rows", gz, g_dtype, x, x_dtype, levels, K, quant, N,
                                              D, want_norm, gx, g_hw, stream);
+}
+
+int vqb_residual_backward_rotated(const void* gz, int g_dtype, const void* x, int x_dtype,
+                                  const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
+                                  int want_norm, void* gx, int64_t g_hw, void* stream) {
+  return member_backward_launch<false, false, true>("vqb_residual_backward_rotated", gz, g_dtype, x, x_dtype, levels, K,
+                                                    quant, N, D, want_norm, gx, g_hw, stream);
+}
+
+int vqb_residual_backward_rotated_rows(const void* gz, int g_dtype, const void* x, int x_dtype,
+                                       const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N,
+                                       int D, int want_norm, void* gx, int64_t g_hw, void* stream) {
+  return member_backward_launch<false, true, true>("vqb_residual_backward_rotated_rows", gz, g_dtype, x, x_dtype, levels,
+                                                   K, quant, N, D, want_norm, gx, g_hw, stream);
 }
 
 int vqb_group_gather_ste_loss(const void* xs, int x_dtype, int64_t N, int Dg, const vqb_residual_levels* lv, int64_t K,

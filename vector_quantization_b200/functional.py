@@ -401,7 +401,7 @@ class _ResidualQuantize(torch.autograd.Function):
     device scalars)."""
 
     @staticmethod
-    def forward(ctx, x, x_nchw, levels, memos, want_norm, track, *Ws):
+    def forward(ctx, x, x_nchw, levels, memos, want_norm, track, rotate, *Ws):
         N, D = x.shape
         L = len(levels)
         hw = 0 if x_nchw is None else x_nchw.shape[2] * x_nchw.shape[3]
@@ -413,6 +413,7 @@ class _ResidualQuantize(torch.autograd.Function):
         ctx.refs = refs
         ctx.nchw = None if x_nchw is None else tuple(x_nchw.shape)
         ctx.want_norm = want_norm
+        ctx.rotate = rotate
         ctx.set_materialize_grads(False)
         ctx.mark_non_differentiable(quant)
         return (z, quant) + tuple(mse.view(-1).unbind(0))
@@ -424,24 +425,27 @@ class _ResidualQuantize(torch.autograd.Function):
         if gz is None:
             gz = torch.zeros(ctx.nchw or x.shape, dtype=torch.float32, device=x.device)
         g4s = [[None if t is None else t.contiguous().float() for t in g[4 * l:4 * l + 4]] for l in range(L)]
-        need_gW = list(ctx.needs_input_grad[6:6 + L])
+        need_gW = list(ctx.needs_input_grad[7:7 + L])
         hw = 0 if ctx.nchw is None else ctx.nchw[2] * ctx.nchw[3]
         gx, gWs = ops.residual_backward(gz.contiguous(), x, [r.tensor for r in ctx.refs], quant, g4s,
-                                        want_norm=ctx.want_norm, need_gW=need_gW, g_hw=hw)
+                                        want_norm=ctx.want_norm, need_gW=need_gW, g_hw=hw, rotate=ctx.rotate)
         if ctx.nchw is not None:     # the gradient belongs to the NCHW latents
-            return (None, gx.view(ctx.nchw) if ctx.needs_input_grad[1] else None, None, None, None, None, *gWs)
-        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, None, *gWs)
+            return (None, gx.view(ctx.nchw) if ctx.needs_input_grad[1] else None, None, None, None, None, None, *gWs)
+        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, None, None, *gWs)
 
 
-def residual_quantize(levels, x: torch.Tensor, memos, want_norm: bool, *, nchw: torch.Tensor | None = None):
+def residual_quantize(levels, x: torch.Tensor, memos, want_norm: bool, *, nchw: torch.Tensor | None = None,
+                      rotate: bool = False):
     """Residual quantization of x [N, D] (fp32 / bf16) through `levels` (VectorQuantizer modules sharing K and D).
     -> (z fp32 [N, D] (or NCHW like `nchw`): value x + (zhat_L - x), gradient straight to x;
         quant int64 [N, L];  mse: per level the four MSE terms (codebook, commitment, codebook-norm,
-        commitment-norm) of e_l against r_{l-1}, 0-dim tensors whose gradients reach W_l and, through r_{l-1}, x)"""
+        commitment-norm) of e_l against r_{l-1}, 0-dim tensors whose gradients reach W_l and, through r_{l-1}, x)
+    rotate: the gradient of z reaches x through the rotation trick from x to zhat_L, one rotation over the whole
+    depth (DESIGN.md §4.9), instead of straight through; the values and the codebook gradients are unchanged."""
     Ws = [level._weight() for level in levels]
     track = torch.is_grad_enabled() and (x.requires_grad or (nchw is not None and nchw.requires_grad)
                                          or any(W.requires_grad for W in Ws))
-    out = _ResidualQuantize.apply(x.contiguous(), nchw, list(levels), memos, bool(want_norm), track, *Ws)
+    out = _ResidualQuantize.apply(x.contiguous(), nchw, list(levels), memos, bool(want_norm), track, bool(rotate), *Ws)
     z, quant, flat = out[0], out[1], out[2:]
     return z, quant, [tuple(flat[4 * l:4 * l + 4]) for l in range(len(levels))]
 

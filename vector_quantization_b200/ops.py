@@ -824,13 +824,15 @@ def residual_step(r: torch.Tensor, x: torch.Tensor, W: torch.Tensor, mse4: torch
 
 
 def residual_backward(g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tensor, g4s, *, want_norm: bool,
-                      need_gW, g_hw: int = 0, deterministic: bool | None = None):
+                      need_gW, g_hw: int = 0, deterministic: bool | None = None, rotate: bool = False):
     """Backward of the whole residual depth in one launch (vqb_residual_backward).  Ws: the L codebooks as used by the
     forward; quant: int64 [N, L]; g4s: per level four 0-dim fp32 device tensors / None (codebook, commitment,
     codebook-norm, commitment-norm upstream gradients); need_gW: per level bool.
     deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, each gW_l is the segment sum of
     the level's per-token rows (vqb_residual_backward_rows + vqb_code_sort + vqb_segment_sum_rows, the contract of
-    quantize_backward).  -> (gx in x's dtype, [gW_l fp32 [K, D] or None])"""
+    quantize_backward).  rotate: g_z reaches x through the rotation trick from x to zhat_L, over the whole depth
+    (vqb_residual_backward_rotated; DESIGN.md §4.9); gW is unchanged.
+    -> (gx in x's dtype, [gW_l fp32 [K, D] or None])"""
     lib = _lib.load()
     L = len(Ws)
     dev = _cuda(g_z, x, quant, *Ws, *[g for g4 in g4s for g in g4])
@@ -845,13 +847,15 @@ def residual_backward(g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tenso
     if any(need_gW) and deterministic_enabled(deterministic):
         rows = _det_ws(x.device, 'gw_rows', L * N * D, torch.float32).view(L, N, D)
         p = _residual_levels(Ws, list(rows), g4s)
-        _call('vqb_residual_backward_rows', lib.vqb_residual_backward_rows, dev, _p(g_z), _dt(g_z), _p(x), _dt(x),
-              ctypes.byref(p), K, _p(quant), N, D, int(want_norm), _p(gx), g_hw, _S)
+        name = 'vqb_residual_backward_rotated_rows' if rotate else 'vqb_residual_backward_rows'
+        _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K, _p(quant), N, D,
+              int(want_norm), _p(gx), g_hw, _S)
         _segment_sum_members(dev, rows, quant, K, gWs)
         return gx, gWs
     p = _residual_levels(Ws, gWs, g4s)
-    _call('vqb_residual_backward', lib.vqb_residual_backward, dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K,
-          _p(quant), N, D, int(want_norm), _p(gx), g_hw, _S)
+    name = 'vqb_residual_backward_rotated' if rotate else 'vqb_residual_backward'
+    _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K, _p(quant), N, D,
+          int(want_norm), _p(gx), g_hw, _S)
     return gx, gWs
 
 

@@ -501,7 +501,8 @@ def _check_member(owner: str, member, members: str) -> None:
         raise ValueError(f'{owner}: materialize_distance (compatibility mode) is not supported')
     if members == 'levels' and member.rotation_trick:
         raise ValueError(f'{owner}: rotation_trick is not supported for residual levels (one straight-through '
-                         'estimator spans the whole depth)')
+                         'estimator spans the whole depth); set rotation_trick=True on the ResidualVectorQuantizer '
+                         'node instead')
     for c in member._callbacks:
         cname = type(c).__name__
         if isinstance(c, NormalizeCallback):
@@ -540,16 +541,22 @@ class ResidualVectorQuantizer(BaseQuantizer):
     L = 1 this is VectorQuantizer.forward bit for bit.  memo: 'x' (the tokens), 'quant' (int64 [N, L]), 'levels'
     (level l's own memo: x = r_{l-1}, encode, decode, loss), 'loss' (per loss name, the sum over the levels).
 
+    rotation_trick: that one estimator follows the rotation trick from x to zhat_L (Fifty et al., arXiv:2410.06424;
+    DESIGN.md §4.9): x receives lambda R^T g instead of g, plus the levels' commitment terms as before.  z, the losses,
+    the indices, the codebook updates and the codebook gradients are unchanged; with L = 1 the gradient is that of a
+    rotated VectorQuantizer bit for bit.  The key belongs to this node; in the level config it is rejected.
+
     Accepted: 1 <= L <= 16, L2 or Cosine distance, no callback or CVQVAECallback (NearestAnchor / CachedAnchor),
     CodebookLoss / CommitmentLoss / VQGANLoss with or without mse.norm.  Rejected with a ValueError: callbacks that
     rewrite the tokens (NormalizeCallback and its subclasses), callbacks that hook decode or loss, and compatibility
-    mode (EntropyLoss, MultinomialAnchor, materialize_distance), and rotation_trick=True.  `init_weights` is applied to
-    every level."""
+    mode (EntropyLoss, MultinomialAnchor, materialize_distance), and rotation_trick=True in the level config.
+    `init_weights` is applied to every level."""
 
     MAX_LEVELS = 16
 
-    def __init__(self, *args, num_quantizers: int, quantizer: Mapping, **kwargs) -> None:
+    def __init__(self, *args, num_quantizers: int, quantizer: Mapping, rotation_trick: bool = False, **kwargs) -> None:
         super().__init__(*args, **kwargs)
+        self.rotation_trick = bool(rotation_trick)
         self._quantizers = nn.ModuleList(_build_members(self, quantizer, num_quantizers, 'num_quantizers', 'levels'))
 
     @property
@@ -628,7 +635,8 @@ class ResidualVectorQuantizer(BaseQuantizer):
         nchw = memo.pop('_nchw', None)     # tokenizer.quantize: x is the token-major copy of these [b, c, h, w] latents
         levels = list(self._quantizers)
         memos = self._level_memos(memo)
-        z, quant, mse = Fq.residual_quantize(levels, x, memos, self._want_norm(), nchw=nchw)
+        z, quant, mse = Fq.residual_quantize(levels, x, memos, self._want_norm(), nchw=nchw,
+                                             rotate=self.rotation_trick)
         memo.update(x=x, quant=quant)
         loss_memo = get_memo(memo, 'loss')
         loss = None
