@@ -352,6 +352,18 @@ def quantize_ste_loss(x: torch.Tensor, W: torch.Tensor, index: torch.Tensor, wan
     return z, (m0, m1, m2, m3), quant, xn
 
 
+def _encode_member(member, x: torch.Tensor, memo: dict, track_codebooks: bool):
+    """member.encode(x) keeping the packed assignment keys unless a training callback reads int64 indices, then a
+    CodebookRef of the codebook as that encode left it (registered with the member when track_codebooks).
+    -> (keys or indices, whether they are keys, ref)"""
+    lazy = memo['_lazy_unpack'] = member._callbacks.packed_keys_ok()
+    _, index, _ = member.encode(x, memo)
+    ref = CodebookRef(member._weight().detach())
+    if track_codebooks:
+        member._pending.add(ref)
+    return index, lazy, ref
+
+
 @torch.no_grad()
 def residual_levels(levels, x: torch.Tensor, memos, want_norm: bool, *, quant_out: torch.Tensor | None = None,
                     z_out: torch.Tensor | None = None, z_hw: int = 0, compact_out: torch.Tensor | None = None,
@@ -371,13 +383,7 @@ def residual_levels(levels, x: torch.Tensor, memos, want_norm: bool, *, quant_ou
     r = x
     for l, level in enumerate(levels):
         memo = memos[l]
-        lazy = level._callbacks.packed_keys_ok()
-        memo['_lazy_unpack'] = lazy
-        _, index, memo = level.encode(r, memo)
-        W = level._weight().detach()
-        ref = CodebookRef(W)
-        if track_codebooks:
-            level._pending.add(ref)
+        index, lazy, ref = _encode_member(level, r, memo, track_codebooks)
         refs.append(ref)
         last = l == L - 1
         if compact_out is not None:
@@ -385,33 +391,30 @@ def residual_levels(levels, x: torch.Tensor, memos, want_norm: bool, *, quant_ou
             ops.compact_tokens(index, level.codebook_size, out=compact_out[l])
         r_out = None if last else torch.empty((N, D), dtype=torch.float32, device=x.device)
         if not (last and z_out is None and quant_out is None):
-            ops.residual_step(r, x, W, mse[l], level=l, L=L, quant=None if lazy else index, keys=index if lazy else None,
-                              quant_out=quant_out, zhat=zhat, r_out=r_out, z_out=z_out if last else None, z_hw=z_hw,
-                              want_norm=want_norm)
+            ops.residual_step(r, x, ref.tensor, mse[l], level=l, L=L, quant=None if lazy else index,
+                              keys=index if lazy else None, quant_out=quant_out, zhat=zhat, r_out=r_out,
+                              z_out=z_out if last else None, z_hw=z_hw, want_norm=want_norm)
         memo['x'] = r
         memo['quant'] = quant_out[:, l] if quant_out is not None else index
         r = r_out
     return mse, refs
 
 
-class _ResidualQuantize(torch.autograd.Function):
-    """The whole depth of a residual quantizer as ONE node: forward = the level loop (`residual_levels`), backward = one
-    `vqb_residual_backward` launch for all levels (+ per-level code sort / segment sum under the deterministic flag).
-    Outputs z, quant [N, L] and the 4 L MSE terms as separate 0-dim tensors (their upstream gradients arrive as
-    device scalars)."""
+class _ComposedQuantize(torch.autograd.Function):
+    """The part shared by the nodes of the composed quantizers (residual levels, groups): all M members in ONE node,
+    whose backward is one launch for all of them (`ctx.backward_op`: ops.residual_backward or ops.group_backward, + per
+    member code sort / segment sum under the deterministic flag).  A node's inputs are the tensor that receives gx first
+    and the M codebooks last; its outputs are z, quant [N, M] and the 4·M MSE terms as separate 0-dim tensors (their
+    upstream gradients arrive as device scalars)."""
 
     @staticmethod
-    def forward(ctx, x, x_nchw, levels, memos, want_norm, track, rotate, *Ws):
-        N, D = x.shape
-        L = len(levels)
-        hw = 0 if x_nchw is None else x_nchw.shape[2] * x_nchw.shape[3]
-        z = torch.empty(tuple(x_nchw.shape) if x_nchw is not None else (N, D), dtype=torch.float32, device=x.device)
-        quant = torch.empty((N, L), dtype=torch.int64, device=x.device)
-        mse, refs = residual_levels(levels, x, memos, want_norm, quant_out=quant, z_out=z, z_hw=hw,
-                                    track_codebooks=track)
+    def _save(ctx, backward_op, x, quant, refs, z, hw, mse, want_norm, rotate):
+        """Record what the backward needs (x: the tokens the backward kernel reads) -> the node's outputs."""
         ctx.save_for_backward(x, quant)
+        ctx.backward_op = backward_op
         ctx.refs = refs
-        ctx.nchw = None if x_nchw is None else tuple(x_nchw.shape)
+        ctx.shape = tuple(z.shape)
+        ctx.hw = hw
         ctx.want_norm = want_norm
         ctx.rotate = rotate
         ctx.set_materialize_grads(False)
@@ -421,17 +424,39 @@ class _ResidualQuantize(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gz, _gq, *g):
         x, quant = ctx.saved_tensors
-        L = quant.shape[1]
+        M = quant.shape[1]
         if gz is None:
-            gz = torch.zeros(ctx.nchw or x.shape, dtype=torch.float32, device=x.device)
-        g4s = [[None if t is None else t.contiguous().float() for t in g[4 * l:4 * l + 4]] for l in range(L)]
-        need_gW = list(ctx.needs_input_grad[7:7 + L])
-        hw = 0 if ctx.nchw is None else ctx.nchw[2] * ctx.nchw[3]
-        gx, gWs = ops.residual_backward(gz.contiguous(), x, [r.tensor for r in ctx.refs], quant, g4s,
-                                        want_norm=ctx.want_norm, need_gW=need_gW, g_hw=hw, rotate=ctx.rotate)
-        if ctx.nchw is not None:     # the gradient belongs to the NCHW latents
-            return (None, gx.view(ctx.nchw) if ctx.needs_input_grad[1] else None, None, None, None, None, None, *gWs)
-        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, None, None, *gWs)
+            gz = torch.zeros(ctx.shape, dtype=torch.float32, device=x.device)
+        g4s = [[None if t is None else t.contiguous().float() for t in g[4 * m:4 * m + 4]] for m in range(M)]
+        gx, gWs = ctx.backward_op(gz.contiguous(), x, [r.tensor for r in ctx.refs], quant, g4s, want_norm=ctx.want_norm,
+                                  need_gW=list(ctx.needs_input_grad[-M:]), g_hw=ctx.hw, rotate=ctx.rotate)
+        rest = (None,) * (len(ctx.needs_input_grad) - M - 1)
+        return (gx if ctx.needs_input_grad[0] else None, *rest, *gWs)
+
+
+def _quantize_composed(node, members, inputs: tuple, memos, want_norm: bool, rotate: bool):
+    """node.apply(*inputs, members, memos, want_norm, track, rotate, *codebooks) -> (z, quant, per member its four
+    MSE terms)."""
+    Ws = [member._weight() for member in members]
+    track = torch.is_grad_enabled() and any([t.requires_grad for t in inputs + tuple(Ws)])
+    out = node.apply(*inputs, list(members), memos, bool(want_norm), track, bool(rotate), *Ws)
+    z, quant, flat = out[0], out[1], out[2:]
+    return z, quant, [tuple(flat[4 * m:4 * m + 4]) for m in range(len(members))]
+
+
+class _ResidualQuantize(_ComposedQuantize):
+    """The whole depth of a residual quantizer: forward = the level loop (`residual_levels`).  x receives gx: the
+    tokens [N, D], or the NCHW latents of which `rows` is the token-major copy (z and gx are then NCHW)."""
+
+    @staticmethod
+    def forward(ctx, x, rows, levels, memos, want_norm, track, rotate, *Ws):
+        N = rows.shape[0]
+        hw = x.shape[2] * x.shape[3] if x.dim() == 4 else 0
+        z = torch.empty(tuple(x.shape), dtype=torch.float32, device=x.device)
+        quant = torch.empty((N, len(levels)), dtype=torch.int64, device=x.device)
+        mse, refs = residual_levels(levels, rows, memos, want_norm, quant_out=quant, z_out=z, z_hw=hw,
+                                    track_codebooks=track)
+        return _ComposedQuantize._save(ctx, ops.residual_backward, rows, quant, refs, z, hw, mse, want_norm, rotate)
 
 
 def residual_quantize(levels, x: torch.Tensor, memos, want_norm: bool, *, nchw: torch.Tensor | None = None,
@@ -442,12 +467,8 @@ def residual_quantize(levels, x: torch.Tensor, memos, want_norm: bool, *, nchw: 
         commitment-norm) of e_l against r_{l-1}, 0-dim tensors whose gradients reach W_l and, through r_{l-1}, x)
     rotate: the gradient of z reaches x through the rotation trick from x to zhat_L, one rotation over the whole
     depth (DESIGN.md §4.9), instead of straight through; the values and the codebook gradients are unchanged."""
-    Ws = [level._weight() for level in levels]
-    track = torch.is_grad_enabled() and (x.requires_grad or (nchw is not None and nchw.requires_grad)
-                                         or any(W.requires_grad for W in Ws))
-    out = _ResidualQuantize.apply(x.contiguous(), nchw, list(levels), memos, bool(want_norm), track, bool(rotate), *Ws)
-    z, quant, flat = out[0], out[1], out[2:]
-    return z, quant, [tuple(flat[4 * l:4 * l + 4]) for l in range(len(levels))]
+    x = x.contiguous()
+    return _quantize_composed(_ResidualQuantize, levels, (x if nchw is None else nchw, x), memos, want_norm, rotate)
 
 
 @torch.no_grad()
@@ -463,23 +484,16 @@ def group_encode(groups, xs: torch.Tensor, memos, *, keys: torch.Tensor | None =
         keys = torch.empty((G, N), dtype=torch.int64, device=xs.device)
     refs = []
     for g, group in enumerate(groups):
-        memo = memos[g]
-        memo['_keys_out'] = keys[g]
-        memo['_lazy_unpack'] = group._callbacks.packed_keys_ok()
-        group.encode(xs[g], memo)     # int64 indices only when a training callback reads them; the keys stay valid
-        ref = CodebookRef(group._weight().detach())
-        if track_codebooks:
-            group._pending.add(ref)
-        refs.append(ref)
+        memos[g]['_keys_out'] = keys[g]
+        # int64 indices only when a training callback reads them; the keys stay valid
+        refs.append(_encode_member(group, xs[g], memos[g], track_codebooks)[2])
     return keys, refs
 
 
-class _GroupedQuantize(torch.autograd.Function):
-    """Every group of a grouped quantizer as ONE node: forward = `ops.split_groups` + the group loop (`group_encode`) +
-    one `vqb_group_gather_ste_loss` launch; backward = one `vqb_group_backward` launch for all groups (+ per-group code
-    sort / segment sum under the deterministic flag).  x is the tokens [N, D] or the NCHW latents [b, D, h, w]; z and
-    gx have x's layout.  Outputs z, quant [N, G] and the 4 G MSE terms as separate 0-dim tensors (their upstream
-    gradients arrive as device scalars); memos[g] gets 'x' (the split slice xs[g]) and 'quant' (quant[:, g])."""
+class _GroupedQuantize(_ComposedQuantize):
+    """Every group of a grouped quantizer: forward = `ops.split_groups` + the group loop (`group_encode`) + one
+    `vqb_group_gather_ste_loss` launch.  x is the tokens [N, D] or the NCHW latents [b, D, h, w]; z and gx have x's
+    layout.  memos[g] gets 'x' (the split slice xs[g]) and 'quant' (quant[:, g])."""
 
     @staticmethod
     def forward(ctx, x, groups, memos, want_norm, track, rotate, *Ws):
@@ -496,27 +510,7 @@ class _GroupedQuantize(torch.autograd.Function):
                                            z_out=z, z_hw=hw)
         for g, memo in enumerate(memos):
             memo.update(x=xs[g], quant=quant[:, g])
-        ctx.save_for_backward(xs, quant)
-        ctx.refs = refs
-        ctx.shape = tuple(x.shape)
-        ctx.hw = hw
-        ctx.want_norm = want_norm
-        ctx.rotate = rotate
-        ctx.set_materialize_grads(False)
-        ctx.mark_non_differentiable(quant)
-        return (z, quant) + tuple(mse.view(-1).unbind(0))
-
-    @staticmethod
-    def backward(ctx, gz, _gq, *g):
-        xs, quant = ctx.saved_tensors
-        G = xs.shape[0]
-        if gz is None:
-            gz = torch.zeros(ctx.shape, dtype=torch.float32, device=xs.device)
-        g4s = [[None if t is None else t.contiguous().float() for t in g[4 * i:4 * i + 4]] for i in range(G)]
-        need_gW = list(ctx.needs_input_grad[6:6 + G])
-        gx, gWs = ops.group_backward(gz.contiguous(), xs, [r.tensor for r in ctx.refs], quant, g4s,
-                                     want_norm=ctx.want_norm, need_gW=need_gW, g_hw=ctx.hw, rotate=ctx.rotate)
-        return (gx if ctx.needs_input_grad[0] else None, None, None, None, None, None, *gWs)
+        return _ComposedQuantize._save(ctx, ops.group_backward, xs, quant, refs, z, hw, mse, want_norm, rotate)
 
 
 def grouped_quantize(groups, x: torch.Tensor, memos, want_norm: bool, *, rotate: bool = False):
@@ -526,11 +520,7 @@ def grouped_quantize(groups, x: torch.Tensor, memos, want_norm: bool, *, rotate:
         mse: per group the four MSE terms (codebook, commitment, codebook-norm,
         commitment-norm) of W_g[q_g] against x_g, 0-dim tensors whose gradients reach W_g and x)
     rotate: the gradient of z reaches x through the rotation trick of each group (DESIGN.md §4.9)"""
-    Ws = [group._weight() for group in groups]
-    track = torch.is_grad_enabled() and (x.requires_grad or any(W.requires_grad for W in Ws))
-    out = _GroupedQuantize.apply(x.contiguous(), list(groups), memos, bool(want_norm), track, bool(rotate), *Ws)
-    z, quant, flat = out[0], out[1], out[2:]
-    return z, quant, [tuple(flat[4 * i:4 * i + 4]) for i in range(len(groups))]
+    return _quantize_composed(_GroupedQuantize, groups, (x.contiguous(),), memos, want_norm, rotate)
 
 
 class _FSQ(torch.autograd.Function):

@@ -780,8 +780,9 @@ def fsq_decode_tokens(ids: torch.Tensor, p: FSQParams, hw: int, out_dtype: torch
 
 
 def _residual_levels(Ws, gWs=None, g4s=None) -> ResidualLevels:
-    """The vqb_residual_levels struct (host memory, copied by value into the kernel parameters)."""
-    if not 1 <= len(Ws) <= MAX_LEVELS:
+    """The vqb_residual_levels struct (host memory, copied by value into the kernel parameters) of the members of a
+    composed quantizer: residual levels, or groups with L = G."""
+    if not 1 <= len(Ws) <= MAX_LEVELS:      # the struct's fixed arrays; the launches check the count in `_codebooks`
         raise ValueError(f'residual quantization takes 1..{MAX_LEVELS} levels, got {len(Ws)}')
     p = ResidualLevels()
     p.L = len(Ws)
@@ -796,12 +797,67 @@ def _residual_levels(Ws, gWs=None, g4s=None) -> ResidualLevels:
     return p
 
 
-def _codebooks(Ws) -> tuple[int, int]:
+def _codebooks(Ws, members: str) -> tuple[int, int]:
+    """(K, D) of the codebooks of a composed quantizer's members (`members`: 'levels' or 'groups'): 1..MAX_LEVELS
+    float32 tensors of one shape [K, D]."""
+    if not 1 <= len(Ws) <= MAX_LEVELS:
+        raise ValueError(f'composed quantization takes 1..{MAX_LEVELS} {members}, got {len(Ws)}')
     K, D = Ws[0].shape
     for W in Ws:
         if W.dtype != torch.float32 or tuple(W.shape) != (K, D):
-            raise TypeError(f'every level codebook must be a float32 [{K}, {D}] tensor, got {W.dtype} {tuple(W.shape)}')
+            raise TypeError(f'every {members[:-1]} codebook must be a float32 [{K}, {D}] tensor, got {W.dtype} '
+                            f'{tuple(W.shape)}')
     return K, D
+
+
+def _group_codebooks(Ws) -> tuple[int, int]:
+    return _codebooks(Ws, 'groups')
+
+
+def _members_backward(name: str, members: str, g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tensor, g4s, *,
+                      want_norm: bool, need_gW, g_hw: int, deterministic: bool | None, rotate: bool):
+    """The one-launch backward of M members: entry point `name` (vqb_residual_backward, vqb_group_backward) or its
+    _rotated / _rows variants.  x: the tokens the kernel reads ([N, D], or split [M, N, D]) -> (gx in x's dtype with
+    g_z's shape, [gW_m fp32 [K, D] or None])"""
+    lib = _lib.load()
+    M = len(Ws)
+    dev = _cuda(g_z, x, quant, *Ws, *[g for g4 in g4s for g in g4])
+    K, D = _codebooks(Ws, members)
+    N = quant.shape[0]
+    assert tuple(x.shape) in ((N, D), (M, N, D)) and g_z.numel() == x.numel() and len(g4s) == M
+    assert quant.dtype == torch.int64 and quant.shape == (N, M)
+    assert all(g is None or g.dtype == torch.float32 for g4 in g4s for g in g4)
+    if not (g_z.dtype == torch.float32 or (g_z.dtype == torch.bfloat16 and x.dtype == torch.bfloat16)):
+        g_z = g_z.float()
+    gx = torch.empty_like(g_z, dtype=x.dtype)
+    gWs = [torch.zeros_like(W) if need else None for W, need in zip(Ws, need_gW)]
+    rows = None
+    if any(need_gW) and deterministic_enabled(deterministic):
+        rows = _det_ws(x.device, 'gw_rows', M * N * D, torch.float32).view(M, N, D)
+    name += ('_rotated' if rotate else '') + ('_rows' if rows is not None else '')
+    p = _residual_levels(Ws, gWs if rows is None else list(rows), g4s)
+    _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K, _p(quant), N, D,
+          int(want_norm), _p(gx), g_hw, _S)
+    if rows is not None:
+        _segment_sum_members(dev, rows, quant, K, gWs)
+    return gx, gWs
+
+
+def _decode_members(name: str, members: str, Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtype, bad_count, *,
+                    side_by_side: bool) -> torch.Tensor:
+    """The one-launch decode (entry point `name`) of token ids [..., M] (a token's M ids contiguous) into [b, C, h, w]:
+    C = M·D when the members' rows sit side by side (groups), D when they are summed (levels)."""
+    lib = _lib.load()
+    dev = _cuda(ids, bad_count, *Ws)
+    K, D = _codebooks(Ws, members)
+    M = len(Ws)
+    if ids.dim() < 2 or ids.shape[-1] != M:
+        raise ValueError(f'expected token ids with a trailing axis of {M} {members}, got {tuple(ids.shape)}')
+    b, id_bytes, z = _decode_out(ids.select(-1, 0), hw, M * D if side_by_side else D, out_dtype, bad_count)
+    p = _residual_levels(Ws)
+    _call(name, getattr(lib, name), dev, _p(ids), id_bytes, b, hw, ctypes.byref(p), K, D, _p(z), _dt(z),
+          _p(bad_count), _S)
+    return z
 
 
 def residual_step(r: torch.Tensor, x: torch.Tensor, W: torch.Tensor, mse4: torch.Tensor, *, level: int, L: int,
@@ -825,38 +881,17 @@ def residual_step(r: torch.Tensor, x: torch.Tensor, W: torch.Tensor, mse4: torch
 
 def residual_backward(g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tensor, g4s, *, want_norm: bool,
                       need_gW, g_hw: int = 0, deterministic: bool | None = None, rotate: bool = False):
-    """Backward of the whole residual depth in one launch (vqb_residual_backward).  Ws: the L codebooks as used by the
-    forward; quant: int64 [N, L]; g4s: per level four 0-dim fp32 device tensors / None (codebook, commitment,
-    codebook-norm, commitment-norm upstream gradients); need_gW: per level bool.
+    """Backward of the whole residual depth in one launch (vqb_residual_backward).  g_z: fp32 (or bf16 with bf16
+    tokens) [N, D], or NCHW with g_hw = h*w; Ws: the L codebooks as used by the forward; quant: int64 [N, L]; g4s: per
+    level four 0-dim fp32 device tensors / None (codebook, commitment, codebook-norm, commitment-norm upstream
+    gradients); need_gW: per level bool.
     deterministic: None follows torch.are_deterministic_algorithms_enabled(); when on, each gW_l is the segment sum of
     the level's per-token rows (vqb_residual_backward_rows + vqb_code_sort + vqb_segment_sum_rows, the contract of
     quantize_backward).  rotate: g_z reaches x through the rotation trick from x to zhat_L, over the whole depth
     (vqb_residual_backward_rotated; DESIGN.md §4.9); gW is unchanged.
-    -> (gx in x's dtype, [gW_l fp32 [K, D] or None])"""
-    lib = _lib.load()
-    L = len(Ws)
-    dev = _cuda(g_z, x, quant, *Ws, *[g for g4 in g4s for g in g4])
-    K, D = _codebooks(Ws)
-    N = x.shape[0]
-    assert x.shape[1] == D and quant.dtype == torch.int64 and quant.shape == (N, L) and len(g4s) == L
-    assert all(g is None or g.dtype == torch.float32 for g4 in g4s for g in g4)
-    if not (g_z.dtype == torch.float32 or (g_z.dtype == torch.bfloat16 and x.dtype == torch.bfloat16)):
-        g_z = g_z.float()
-    gx = torch.empty_like(x)
-    gWs = [torch.zeros_like(W) if need else None for W, need in zip(Ws, need_gW)]
-    if any(need_gW) and deterministic_enabled(deterministic):
-        rows = _det_ws(x.device, 'gw_rows', L * N * D, torch.float32).view(L, N, D)
-        p = _residual_levels(Ws, list(rows), g4s)
-        name = 'vqb_residual_backward_rotated_rows' if rotate else 'vqb_residual_backward_rows'
-        _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K, _p(quant), N, D,
-              int(want_norm), _p(gx), g_hw, _S)
-        _segment_sum_members(dev, rows, quant, K, gWs)
-        return gx, gWs
-    p = _residual_levels(Ws, gWs, g4s)
-    name = 'vqb_residual_backward_rotated' if rotate else 'vqb_residual_backward'
-    _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K, _p(quant), N, D,
-          int(want_norm), _p(gx), g_hw, _S)
-    return gx, gWs
+    -> (gx in x's dtype with g_z's shape, [gW_l fp32 [K, D] or None])"""
+    return _members_backward('vqb_residual_backward', 'levels', g_z, x, Ws, quant, g4s, want_norm=want_norm,
+                             need_gW=need_gW, g_hw=g_hw, deterministic=deterministic, rotate=rotate)
 
 
 def decode_residual_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtype = torch.float32,
@@ -864,26 +899,11 @@ def decode_residual_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtyp
     """Residual token ids [b, h, w, L] (uint16 / int32 / int64; a token's L ids contiguous) -> z = sum_l W_l[id_l]
     (level order, fp32 adds) as [b, D, h, w] of `out_dtype`, in one launch (vqb_decode_residual_tokens).  A token with
     an id outside [0, K) at any level gives a NaN row and is counted once into `bad_count`."""
-    lib = _lib.load()
-    dev = _cuda(ids, bad_count, *Ws)
-    K, D = _codebooks(Ws)
-    L = len(Ws)
-    if ids.dim() < 2 or ids.shape[-1] != L:
-        raise ValueError(f'expected residual token ids with a trailing depth axis of {L}, got {tuple(ids.shape)}')
-    b, id_bytes, z = _decode_out(ids.select(-1, 0), hw, D, out_dtype, bad_count)
-    p = _residual_levels(Ws)
-    _call('vqb_decode_residual_tokens', lib.vqb_decode_residual_tokens, dev, _p(ids), id_bytes, b, hw, ctypes.byref(p),
-          K, D, _p(z), _dt(z), _p(bad_count), _S)
-    return z
+    return _decode_members('vqb_decode_residual_tokens', 'levels', Ws, ids, hw, out_dtype, bad_count,
+                           side_by_side=False)
 
 
 # ---- grouped (product) quantization (csrc/quantize.cu, csrc/layout.cu) ---------------------------------------------
-
-
-def _group_codebooks(Ws) -> tuple[int, int]:
-    if not 1 <= len(Ws) <= MAX_LEVELS:
-        raise ValueError(f'grouped quantization takes 1..{MAX_LEVELS} groups, got {len(Ws)}')
-    return _codebooks(Ws)
 
 
 def split_groups(x: torch.Tensor, G: int) -> torch.Tensor:
@@ -948,30 +968,8 @@ def group_backward(g_z: torch.Tensor, xs: torch.Tensor, Ws, quant: torch.Tensor,
     the group's per-token rows (vqb_group_backward_rows + vqb_code_sort + vqb_segment_sum_rows, the contract of
     quantize_backward).  rotate: the rotation trick per group, as in quantize_backward.
     -> (gx in xs's dtype with g_z's shape, [gW_g fp32 [K, Dg] or None])"""
-    lib = _lib.load()
-    G = len(Ws)
-    dev = _cuda(g_z, xs, quant, *Ws, *[g for g4 in g4s for g in g4])
-    K, Dg = _group_codebooks(Ws)
-    N = xs.shape[1]
-    assert tuple(xs.shape) == (G, N, Dg) and quant.dtype == torch.int64 and quant.shape == (N, G) and len(g4s) == G
-    assert g_z.numel() == N * G * Dg and all(g is None or g.dtype == torch.float32 for g4 in g4s for g in g4)
-    if not (g_z.dtype == torch.float32 or (g_z.dtype == torch.bfloat16 and xs.dtype == torch.bfloat16)):
-        g_z = g_z.float()
-    gx = torch.empty(g_z.shape, dtype=xs.dtype, device=xs.device)
-    gWs = [torch.zeros_like(W) if need else None for W, need in zip(Ws, need_gW)]
-    if any(need_gW) and deterministic_enabled(deterministic):
-        rows = _det_ws(xs.device, 'gw_rows', G * N * Dg, torch.float32).view(G, N, Dg)
-        p = _residual_levels(Ws, list(rows), g4s)
-        name = 'vqb_group_backward_rotated_rows' if rotate else 'vqb_group_backward_rows'
-        _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs), ctypes.byref(p), K, _p(quant), N, Dg,
-              int(want_norm), _p(gx), g_hw, _S)
-        _segment_sum_members(dev, rows, quant, K, gWs)
-        return gx, gWs
-    p = _residual_levels(Ws, gWs, g4s)
-    name = 'vqb_group_backward_rotated' if rotate else 'vqb_group_backward'
-    _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(xs), _dt(xs), ctypes.byref(p), K, _p(quant), N, Dg,
-          int(want_norm), _p(gx), g_hw, _S)
-    return gx, gWs
+    return _members_backward('vqb_group_backward', 'groups', g_z, xs, Ws, quant, g4s, want_norm=want_norm,
+                             need_gW=need_gW, g_hw=g_hw, deterministic=deterministic, rotate=rotate)
 
 
 def decode_group_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtype = torch.float32,
@@ -979,14 +977,5 @@ def decode_group_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtype =
     """Grouped token ids [b, h, w, G] (uint16 / int32 / int64; a token's G ids contiguous) -> z with channels
     [g*Dg, (g+1)*Dg) = W_g[id_g], as [b, G*Dg, h, w] of `out_dtype`, in one launch (vqb_decode_group_tokens).  A token
     with an id outside [0, K) in any group gives a NaN row and is counted once into `bad_count`."""
-    lib = _lib.load()
-    dev = _cuda(ids, bad_count, *Ws)
-    K, Dg = _group_codebooks(Ws)
-    G = len(Ws)
-    if ids.dim() < 2 or ids.shape[-1] != G:
-        raise ValueError(f'expected grouped token ids with a trailing group axis of {G}, got {tuple(ids.shape)}')
-    b, id_bytes, z = _decode_out(ids.select(-1, 0), hw, G * Dg, out_dtype, bad_count)
-    p = _residual_levels(Ws)
-    _call('vqb_decode_group_tokens', lib.vqb_decode_group_tokens, dev, _p(ids), id_bytes, b, hw, ctypes.byref(p), K, Dg,
-          _p(z), _dt(z), _p(bad_count), _S)
-    return z
+    return _decode_members('vqb_decode_group_tokens', 'groups', Ws, ids, hw, out_dtype, bad_count,
+                           side_by_side=True)

@@ -465,67 +465,158 @@ class FiniteScalarQuantizer(ScalarQuantizer):
         return z, x.new_zeros([]), memo
 
 
-def _build_members(owner: BaseQuantizer, quantizer: Mapping, count, count_name: str, members: str) -> list:
-    """The member quantizers of a composed quantizer (ResidualVectorQuantizer levels, GroupedVectorQuantizer groups):
-    `count` copies of the `quantizer` node, each an ordinary VectorQuantizer / VQGANQuantizer.  Accepted: L2 or Cosine
-    distance, no callback or CVQVAECallback (NearestAnchor / CachedAnchor), CodebookLoss / CommitmentLoss / VQGANLoss.
-    Everything else raises a ValueError naming the offending item: callbacks that rewrite the tokens, callbacks that
-    hook decode or loss, compatibility mode, a count outside [1, 16], members that are not VectorQuantizer modules
-    (FSQ, or a composed quantizer: no nesting), and callbacks or losses on the composed node itself."""
-    name = type(owner).__name__
-    if isinstance(count, bool) or not isinstance(count, int) or not 1 <= count <= MAX_LEVELS:
-        raise ValueError(f'{name}: {count_name}={count!r} is outside [1, {MAX_LEVELS}]')
-    if list(owner._callbacks) or len(owner._losses):
-        raise ValueError(f'{name}: callbacks and losses belong to the {members[:-1]} config (`quantizer`), '
-                         f'not to the {name} node itself')
-    cls = VQITQuantizerRegistry.lookup(quantizer['type']) if isinstance(quantizer.get('type'), str) else None
-    if isinstance(cls, type) and not issubclass(cls, VectorQuantizer):
-        raise ValueError(f'{name}: the {members} must be VectorQuantizer modules, got {cls.__name__}')
-    built = []
-    for _ in range(count):
-        cfg = Config(copy.deepcopy(dict(quantizer)))
-        cfg['init_weights'] = None       # applied per member by init_weights (after the train / eval mode is set)
-        built.append(VQITQuantizerRegistry.build(cfg))
-    for member in built:
-        _check_member(name, member, members)
-    return built
+class _ComposedQuantizer(BaseQuantizer):
+    """What ResidualVectorQuantizer and GroupedVectorQuantizer share.  M ordinary VectorQuantizer / VQGANQuantizer
+    members are built from ONE config node (`quantizer`) and stored as `_quantizers.{i}`; each runs its own `encode`,
+    one autograd node and one backward launch serve all of them, and one launch decodes.  The base owns the members
+    (their checks, properties, codebooks and memos under memo[_members]), `decode`, the gate and buffer of
+    `encode_compact` and the loss memo.  A subclass decides the input layout (`_check_input`, `encode`,
+    `_encode_compact`), the node and the place of the rotation key (`_quantize`), the decode kernel (`_decode_ids`) and
+    the reduction of the member losses (`_loss_mean`).
 
+    Accepted members: L2 or Cosine distance, no callback or CVQVAECallback (NearestAnchor / CachedAnchor),
+    CodebookLoss / CommitmentLoss / VQGANLoss.  Everything else raises a ValueError naming the offending item: callbacks
+    that rewrite the tokens, callbacks that hook decode or loss, compatibility mode, a count outside [1, 16], members
+    that are not VectorQuantizer modules (FSQ, or a composed quantizer: no nesting), and callbacks or losses on the
+    composed node itself.  `init_weights` is applied to every member."""
 
-def _check_member(owner: str, member, members: str) -> None:
-    from .callbacks import BaseCallback, CVQVAECallback, NormalizeCallback
-    from .losses import CodebookLoss, CommitmentLoss, VQGANLoss
-    name = type(member).__name__
-    if not isinstance(member, VectorQuantizer):
-        raise ValueError(f'{owner}: the {members} must be VectorQuantizer modules, got {name}')
-    if member.materialize_distance:
-        raise ValueError(f'{owner}: materialize_distance (compatibility mode) is not supported')
-    if members == 'levels' and member.rotation_trick:
-        raise ValueError(f'{owner}: rotation_trick is not supported for residual levels (one straight-through '
-                         'estimator spans the whole depth); set rotation_trick=True on the ResidualVectorQuantizer '
-                         'node instead')
-    for c in member._callbacks:
-        cname = type(c).__name__
-        if isinstance(c, NormalizeCallback):
-            raise ValueError(f'{owner}: callback {cname} rewrites the tokens; normalised {members} are not supported')
-        hooks = [h for h in ('before_decode', 'after_decode', 'before_loss', 'after_loss')
-                 if getattr(type(c), h) is not getattr(BaseCallback, h)]
-        if hooks:
-            raise ValueError(f'{owner}: callback {cname} hooks {", ".join(hooks)}; callbacks that '
-                             'hook decode or loss are not supported')
-        if not isinstance(c, CVQVAECallback):
-            raise ValueError(f'{owner}: callback {cname} is not supported ({members} take no callback '
-                             'or CVQVAECallback)')
-        if c._anchor.needs_distance:
-            raise ValueError(f'{owner}: {type(c._anchor).__name__} of {cname} reads the [N, K] '
-                             'distance matrix (compatibility mode), which is not supported')
-    for lname, loss in member._losses.items():
-        if not isinstance(loss, (CodebookLoss, CommitmentLoss, VQGANLoss)):
-            raise ValueError(f'{owner}: loss {lname!r} ({type(loss).__name__}) is not supported '
-                             '(CodebookLoss, CommitmentLoss and VQGANLoss are)')
+    MAX_LEVELS = MAX_LEVELS
+    _members = ''               # 'levels' / 'groups': the memo key of the member memos, and the noun of the messages
+    _rotation_on_node = False   # rotation_trick is a key of this node; the member config may not set it
+    _loss_mean = False          # the loss of a name is the mean over the members (groups), not their sum (levels)
+
+    def _build_members(self, quantizer: Mapping, count, count_name: str) -> nn.ModuleList:
+        name = type(self).__name__
+        if isinstance(count, bool) or not isinstance(count, int) or not 1 <= count <= MAX_LEVELS:
+            raise ValueError(f'{name}: {count_name}={count!r} is outside [1, {MAX_LEVELS}]')
+        if list(self._callbacks) or len(self._losses):
+            raise ValueError(f'{name}: callbacks and losses belong to the {self._members[:-1]} config (`quantizer`), '
+                             f'not to the {name} node itself')
+        cls = VQITQuantizerRegistry.lookup(quantizer['type']) if isinstance(quantizer.get('type'), str) else None
+        if isinstance(cls, type) and not issubclass(cls, VectorQuantizer):
+            raise ValueError(f'{name}: the {self._members} must be VectorQuantizer modules, got {cls.__name__}')
+        built = []
+        for _ in range(count):
+            cfg = Config(copy.deepcopy(dict(quantizer)))
+            cfg['init_weights'] = None       # applied per member by init_weights (after the train / eval mode is set)
+            built.append(VQITQuantizerRegistry.build(cfg))
+        for member in built:
+            self._check_member(member)
+        return nn.ModuleList(built)
+
+    def _check_member(self, member) -> None:
+        from .callbacks import BaseCallback, CVQVAECallback, NormalizeCallback
+        from .losses import CodebookLoss, CommitmentLoss, VQGANLoss
+        owner, members, name = type(self).__name__, self._members, type(member).__name__
+        if not isinstance(member, VectorQuantizer):
+            raise ValueError(f'{owner}: the {members} must be VectorQuantizer modules, got {name}')
+        if member.materialize_distance:
+            raise ValueError(f'{owner}: materialize_distance (compatibility mode) is not supported')
+        if self._rotation_on_node and member.rotation_trick:
+            raise ValueError(f'{owner}: rotation_trick is not supported for residual levels (one straight-through '
+                             f'estimator spans the whole depth); set rotation_trick=True on the {owner} node instead')
+        for c in member._callbacks:
+            cname = type(c).__name__
+            if isinstance(c, NormalizeCallback):
+                raise ValueError(f'{owner}: callback {cname} rewrites the tokens; normalised {members} are not supported')
+            hooks = [h for h in ('before_decode', 'after_decode', 'before_loss', 'after_loss')
+                     if getattr(type(c), h) is not getattr(BaseCallback, h)]
+            if hooks:
+                raise ValueError(f'{owner}: callback {cname} hooks {", ".join(hooks)}; callbacks that '
+                                 'hook decode or loss are not supported')
+            if not isinstance(c, CVQVAECallback):
+                raise ValueError(f'{owner}: callback {cname} is not supported ({members} take no callback '
+                                 'or CVQVAECallback)')
+            if c._anchor.needs_distance:
+                raise ValueError(f'{owner}: {type(c._anchor).__name__} of {cname} reads the [N, K] '
+                                 'distance matrix (compatibility mode), which is not supported')
+        for lname, loss in member._losses.items():
+            if not isinstance(loss, (CodebookLoss, CommitmentLoss, VQGANLoss)):
+                raise ValueError(f'{owner}: loss {lname!r} ({type(loss).__name__}) is not supported '
+                                 '(CodebookLoss, CommitmentLoss and VQGANLoss are)')
+
+    @property
+    def quantizers(self) -> nn.ModuleList:
+        return self._quantizers
+
+    @property
+    def codebook_size(self) -> int:
+        """Codes per member."""
+        return self._quantizers[0].codebook_size
+
+    @property
+    def embeddings(self) -> torch.Tensor:
+        """[M, K, Dm] copy of the member codebooks."""
+        return torch.stack([member.embedding.weight.detach() for member in self._quantizers]).clone()
+
+    def _init_weights(self, config) -> bool:
+        for member in self._quantizers:
+            member.init_weights(Config(copy.deepcopy(dict(config))))
+        return False
+
+    def _weights(self) -> list:
+        return [member._weight() for member in self._quantizers]
+
+    def _want_norm(self) -> bool:
+        return self._quantizers[0]._loss_terms()
+
+    def _member_memos(self, memo: dict) -> list:
+        memo[self._members] = [dict() for _ in self._quantizers]
+        return memo[self._members]
+
+    def _check_input(self, x: torch.Tensor) -> torch.Tensor:
+        return _check_tokens(x, self.embedding_dim)
+
+    @torch.no_grad()
+    def encode_compact(self, x: torch.Tensor, memo: dict) -> torch.Tensor:
+        """Tokenise-only encode: [M, N'] uint16 (K <= 65 536) or int32 ids straight from the packed assignment keys (N' = N
+        rounded up to 8; the first N columns are the ids); None when a member's training callback needs int64 indices
+        (then `encode` is the way)."""
+        if not all(member._callbacks.packed_keys_ok() for member in self._quantizers):
+            return None
+        return self._encode_compact(x, self._member_memos(memo))
+
+    def _compact_out(self, N: int, device) -> torch.Tensor:
+        # rows padded to 8 ids: every row starts 16-byte aligned, as vqb_compact_tokens reads and stores 16 bytes at a time
+        return torch.empty((len(self._quantizers), (N + 7) // 8 * 8),
+                           dtype=torch.uint16 if self.codebook_size <= 65536 else torch.int32, device=device)
+
+    def decode(self, quant: torch.Tensor, memo: dict):
+        """quant [N, M] (or [..., M]; uint16 / int32 / int64) -> (z fp32 [..., embedding_dim], memo) in one launch (see
+        `_decode_ids`).  A token with an id outside [0, codebook_size) in any member decodes to NaN."""
+        if not quant.is_cuda:
+            raise VQBError(f'{type(self).__name__} decodes CUDA tensors only; there is no CPU fallback')
+        lead = tuple(quant.shape[:-1])
+        z = self._decode_ids(quant.contiguous().view(-1, quant.shape[-1]), 1)
+        get_memo(memo, 'decode')
+        return z.view(*lead, self.embedding_dim), memo
+
+    def forward(self, x: torch.Tensor, memo: dict):
+        x = self._check_input(x)
+        members = list(self._quantizers)
+        memos = self._member_memos(memo)
+        z, quant, mse = self._quantize(x, members, memos, memo)
+        memo.update(x=x, quant=quant)
+        loss_memo = get_memo(memo, 'loss')
+        sums: dict = {}
+        for m, (member, member_memo) in enumerate(zip(members, memos)):
+            member_memo['decode'] = get_memo(member_memo, 'decode')
+            member_loss = get_memo(member_memo, 'loss')
+            for name, module in member._losses.items():
+                value = module.from_mse4(mse[m])
+                member_loss[name] = value
+                sums[name] = value if m == 0 else sums[name] + value
+        loss = None
+        for name, total in sums.items():
+            loss_memo[name] = total / len(members) if self._loss_mean else total
+            loss = loss_memo[name] if loss is None else loss + loss_memo[name]
+        if loss is None:
+            loss = mse[0][0].new_zeros([])
+        return z, loss, memo
 
 
 @VQITQuantizerRegistry.register_()
-class ResidualVectorQuantizer(BaseQuantizer):
+class ResidualVectorQuantizer(_ComposedQuantizer):
     """Residual quantization (RQ-VAE): L codebooks code every token in turn, level l quantizing what the earlier levels
     left over.  Levels are ordinary VectorQuantizer / VQGANQuantizer modules built from ONE config node (`quantizer`),
     stored as `_quantizers.{l}`; level l runs its own `encode` (before_encode -> assignment -> after_encode, codebook
@@ -546,22 +637,16 @@ class ResidualVectorQuantizer(BaseQuantizer):
     the indices, the codebook updates and the codebook gradients are unchanged; with L = 1 the gradient is that of a
     rotated VectorQuantizer bit for bit.  The key belongs to this node; in the level config it is rejected.
 
-    Accepted: 1 <= L <= 16, L2 or Cosine distance, no callback or CVQVAECallback (NearestAnchor / CachedAnchor),
-    CodebookLoss / CommitmentLoss / VQGANLoss with or without mse.norm.  Rejected with a ValueError: callbacks that
-    rewrite the tokens (NormalizeCallback and its subclasses), callbacks that hook decode or loss, and compatibility
-    mode (EntropyLoss, MultinomialAnchor, materialize_distance), and rotation_trick=True in the level config.
-    `init_weights` is applied to every level."""
+    Accepted and rejected level configurations: see `_ComposedQuantizer`, with 1 <= L <= 16 and mse.norm on or off;
+    rotation_trick=True in the level config is rejected too."""
 
-    MAX_LEVELS = 16
+    _members = 'levels'
+    _rotation_on_node = True
 
     def __init__(self, *args, num_quantizers: int, quantizer: Mapping, rotation_trick: bool = False, **kwargs) -> None:
         super().__init__(*args, **kwargs)
         self.rotation_trick = bool(rotation_trick)
-        self._quantizers = nn.ModuleList(_build_members(self, quantizer, num_quantizers, 'num_quantizers', 'levels'))
-
-    @property
-    def quantizers(self) -> nn.ModuleList:
-        return self._quantizers
+        self._quantizers = self._build_members(quantizer, num_quantizers, 'num_quantizers')
 
     @property
     def num_quantizers(self) -> int:
@@ -571,91 +656,30 @@ class ResidualVectorQuantizer(BaseQuantizer):
     def embedding_dim(self) -> int:
         return self._quantizers[0].embedding_dim
 
-    @property
-    def codebook_size(self) -> int:
-        """Codes per level."""
-        return self._quantizers[0].codebook_size
-
-    @property
-    def embeddings(self) -> torch.Tensor:
-        """[L, K, D] copy of the level codebooks."""
-        return torch.stack([level.embedding.weight.detach() for level in self._quantizers]).clone()
-
-    def _init_weights(self, config) -> bool:
-        for level in self._quantizers:
-            level.init_weights(Config(copy.deepcopy(dict(config))))
-        return False
-
-    def _weights(self) -> list:
-        return [level._weight() for level in self._quantizers]
-
-    def _want_norm(self) -> bool:
-        return self._quantizers[0]._loss_terms()
-
-    def _level_memos(self, memo: dict) -> list:
-        memo['levels'] = [dict() for _ in self._quantizers]
-        return memo['levels']
-
     @torch.no_grad()
     def encode(self, x: torch.Tensor, memo: dict):
         """-> (x, quant int64 [N, L], memo); every level's callbacks run as in forward (codebook updates included)."""
-        x = _check_tokens(x, self.embedding_dim)
+        x = self._check_input(x)
         quant = torch.empty((x.shape[0], self.num_quantizers), dtype=torch.int64, device=x.device)
-        Fq.residual_levels(list(self._quantizers), x, self._level_memos(memo), self._want_norm(), quant_out=quant)
+        Fq.residual_levels(list(self._quantizers), x, self._member_memos(memo), self._want_norm(), quant_out=quant)
         return x, quant, memo
 
-    @torch.no_grad()
-    def encode_compact(self, x: torch.Tensor, memo: dict) -> torch.Tensor:
-        """Tokenise-only encode: [L, N'] uint16 (K <= 65 536) or int32 ids straight from the packed assignment keys (N' = N
-        rounded up to 8; the first N columns are the ids); None when a level's training callback needs int64 indices
-        (then `encode` is the way)."""
-        if not all(level._callbacks.packed_keys_ok() for level in self._quantizers):
-            return None
-        x = _check_tokens(x, self.embedding_dim)
-        N = x.shape[0]
-        # rows padded to 8 ids: every row starts 16-byte aligned, as vqb_compact_tokens stores 16 bytes at a time
-        out = torch.empty((self.num_quantizers, (N + 7) // 8 * 8),
-                          dtype=torch.uint16 if self.codebook_size <= 65536 else torch.int32, device=x.device)
-        Fq.residual_levels(list(self._quantizers), x, self._level_memos(memo), self._want_norm(), compact_out=out[:, :N])
+    def _encode_compact(self, x: torch.Tensor, memos: list) -> torch.Tensor:
+        x = self._check_input(x)
+        out = self._compact_out(x.shape[0], x.device)
+        Fq.residual_levels(list(self._quantizers), x, memos, self._want_norm(), compact_out=out[:, :x.shape[0]])
         return out
 
-    def decode(self, quant: torch.Tensor, memo: dict):
-        """quant [N, L] (or [..., L]; uint16 / int32 / int64) -> (zhat fp32 [..., D], memo): sum_l W_l[q_l] in level order,
-        one launch.  A token with an id outside [0, codebook_size) at any level decodes to NaN."""
-        if not quant.is_cuda:
-            raise VQBError('ResidualVectorQuantizer decodes CUDA tensors only; there is no CPU fallback')
-        lead = tuple(quant.shape[:-1])
-        flat = quant.contiguous().view(-1, quant.shape[-1])
-        z = ops.decode_residual_tokens([W.detach() for W in self._weights()], flat, 1)
-        get_memo(memo, 'decode')
-        return z.view(*lead, self.embedding_dim), memo
+    def _decode_ids(self, ids: torch.Tensor, hw: int, dtype: torch.dtype = torch.float32, bad_count=None):
+        """ids [b*h*w, L] -> sum_l W_l[id_l] in level order, [b, D, h, w] of `dtype`."""
+        return ops.decode_residual_tokens(self._weights(), ids, hw, dtype, bad_count)
 
-    def forward(self, x: torch.Tensor, memo: dict):
-        x = _check_tokens(x, self.embedding_dim)
+    def _quantize(self, x: torch.Tensor, levels: list, memos: list, memo: dict):
         nchw = memo.pop('_nchw', None)     # tokenizer.quantize: x is the token-major copy of these [b, c, h, w] latents
-        levels = list(self._quantizers)
-        memos = self._level_memos(memo)
-        z, quant, mse = Fq.residual_quantize(levels, x, memos, self._want_norm(), nchw=nchw,
-                                             rotate=self.rotation_trick)
-        memo.update(x=x, quant=quant)
-        loss_memo = get_memo(memo, 'loss')
-        loss = None
-        for l, (level, level_memo) in enumerate(zip(levels, memos)):
-            level_memo['decode'] = get_memo(level_memo, 'decode')
-            level_loss = get_memo(level_memo, 'loss')
-            for name, module in level._losses.items():
-                value = module.from_mse4(mse[l])
-                level_loss[name] = value
-                loss_memo[name] = value if l == 0 else loss_memo[name] + value
-        for name in levels[0]._losses:
-            loss = loss_memo[name] if loss is None else loss + loss_memo[name]
-        if loss is None:
-            loss = mse[0][0].new_zeros([])
-        return z, loss, memo
-
+        return Fq.residual_quantize(levels, x, memos, self._want_norm(), nchw=nchw, rotate=self.rotation_trick)
 
 @VQITQuantizerRegistry.register_()
-class GroupedVectorQuantizer(BaseQuantizer):
+class GroupedVectorQuantizer(_ComposedQuantizer):
     """Grouped (product) quantization: the D channels of a token are split into G groups of Dg = D / G channels and
     group g is quantized against its own codebook of K codes, so a token gets G ids (a joint code space of K^G).  Groups
     are ordinary VectorQuantizer / VQGANQuantizer modules with embedding_dim = Dg, built from ONE config node
@@ -672,17 +696,16 @@ class GroupedVectorQuantizer(BaseQuantizer):
     back NCHW).  memo: 'x' (the input as given), 'quant' (int64 [N, G]), 'groups' (group g's own memo: x = its token
     slice, encode, decode, loss), 'loss' (per loss name, the group mean).
 
-    Accepted and rejected configurations are those of ResidualVectorQuantizer (see `_build_members`), with
+    Accepted and rejected configurations are those of ResidualVectorQuantizer (see `_ComposedQuantizer`), with
     1 <= num_groups <= 16, except that the group config may set rotation_trick=True: every group then passes its
-    encoder gradient through the rotation trick (DESIGN.md §4.9).  `init_weights` is applied to every group."""
+    encoder gradient through the rotation trick (DESIGN.md §4.9)."""
+
+    _members = 'groups'
+    _loss_mean = True
 
     def __init__(self, *args, num_groups: int, quantizer: Mapping, **kwargs) -> None:
         super().__init__(*args, **kwargs)
-        self._quantizers = nn.ModuleList(_build_members(self, quantizer, num_groups, 'num_groups', 'groups'))
-
-    @property
-    def quantizers(self) -> nn.ModuleList:
-        return self._quantizers
+        self._quantizers = self._build_members(quantizer, num_groups, 'num_groups')
 
     @property
     def num_groups(self) -> int:
@@ -695,31 +718,6 @@ class GroupedVectorQuantizer(BaseQuantizer):
     @property
     def embedding_dim(self) -> int:
         return self.num_groups * self.group_dim
-
-    @property
-    def codebook_size(self) -> int:
-        """Codes per group."""
-        return self._quantizers[0].codebook_size
-
-    @property
-    def embeddings(self) -> torch.Tensor:
-        """[G, K, Dg] copy of the group codebooks."""
-        return torch.stack([group.embedding.weight.detach() for group in self._quantizers]).clone()
-
-    def _init_weights(self, config) -> bool:
-        for group in self._quantizers:
-            group.init_weights(Config(copy.deepcopy(dict(config))))
-        return False
-
-    def _weights(self) -> list:
-        return [group._weight() for group in self._quantizers]
-
-    def _want_norm(self) -> bool:
-        return self._quantizers[0]._loss_terms()
-
-    def _group_memos(self, memo: dict) -> list:
-        memo['groups'] = [dict() for _ in self._quantizers]
-        return memo['groups']
 
     def _check_input(self, x: torch.Tensor) -> torch.Tensor:
         """Tokens [N, D] or latents [b, D, h, w], fp32 / bf16 on the GPU."""
@@ -744,61 +742,27 @@ class GroupedVectorQuantizer(BaseQuantizer):
         """-> (x, quant int64 [N, G], memo); every group's callbacks run as in forward (codebook updates included)."""
         xs = self._split(x)
         G, N, _ = xs.shape
-        keys, _ = Fq.group_encode(list(self._quantizers), xs, self._group_memos(memo))
+        memos = self._member_memos(memo)
+        keys, _ = Fq.group_encode(list(self._quantizers), xs, memos)
         idx = ops.unpack_keys(keys.view(-1))
         quant = idx.view(N, G) if G == 1 else ops.transpose_last2(idx.view(1, G, N)).view(N, G)
-        for g, group_memo in enumerate(memo['groups']):
+        for g, group_memo in enumerate(memos):
             group_memo.update(x=xs[g], quant=quant[:, g])
         return x, quant, memo
 
-    @torch.no_grad()
-    def encode_compact(self, x: torch.Tensor, memo: dict) -> torch.Tensor:
-        """Tokenise-only encode: [G, N'] uint16 (K <= 65 536) or int32 ids straight from the packed assignment keys (N' = N
-        rounded up to 8; the first N columns are the ids); None when a group's training callback needs int64 indices
-        (then `encode` is the way)."""
-        if not all(group._callbacks.packed_keys_ok() for group in self._quantizers):
-            return None
+    def _encode_compact(self, x: torch.Tensor, memos: list) -> torch.Tensor:
         xs = self._split(x)
         G, N, _ = xs.shape
-        # rows padded to 8: every row starts 16-byte aligned, as vqb_compact_tokens reads and stores 16 bytes at a time
-        Np = (N + 7) // 8 * 8
-        keys = torch.empty((G, Np), dtype=torch.int64, device=xs.device)[:, :N]
-        out = torch.empty((G, Np), dtype=torch.uint16 if self.codebook_size <= 65536 else torch.int32, device=xs.device)
-        Fq.group_encode(list(self._quantizers), xs, self._group_memos(memo), keys=keys)
+        out = self._compact_out(N, xs.device)
+        keys = torch.empty(out.shape, dtype=torch.int64, device=xs.device)[:, :N]
+        Fq.group_encode(list(self._quantizers), xs, memos, keys=keys)
         for g in range(G):
             ops.compact_tokens(keys[g], self.codebook_size, out=out[g, :N])
         return out
 
-    def decode(self, quant: torch.Tensor, memo: dict):
-        """quant [N, G] (or [..., G]; uint16 / int32 / int64) -> (z fp32 [..., D], memo): channels [g*Dg, (g+1)*Dg) =
-        W_g[q_g], one launch.  A token with an id outside [0, codebook_size) in any group decodes to NaN."""
-        if not quant.is_cuda:
-            raise VQBError('GroupedVectorQuantizer decodes CUDA tensors only; there is no CPU fallback')
-        lead = tuple(quant.shape[:-1])
-        flat = quant.contiguous().view(-1, quant.shape[-1])
-        z = ops.decode_group_tokens([W.detach() for W in self._weights()], flat, 1)
-        get_memo(memo, 'decode')
-        return z.view(*lead, self.embedding_dim), memo
+    def _decode_ids(self, ids: torch.Tensor, hw: int, dtype: torch.dtype = torch.float32, bad_count=None):
+        """ids [b*h*w, G] -> channels [g*Dg, (g+1)*Dg) = W_g[id_g], [b, D, h, w] of `dtype`."""
+        return ops.decode_group_tokens(self._weights(), ids, hw, dtype, bad_count)
 
-    def forward(self, x: torch.Tensor, memo: dict):
-        x = self._check_input(x)
-        groups = list(self._quantizers)
-        memos = self._group_memos(memo)
-        z, quant, mse = Fq.grouped_quantize(groups, x, memos, self._want_norm(), rotate=groups[0].rotation_trick)
-        memo.update(x=x, quant=quant)
-        loss_memo = get_memo(memo, 'loss')
-        sums: dict = {}
-        for g, (group, group_memo) in enumerate(zip(groups, memos)):
-            group_memo['decode'] = get_memo(group_memo, 'decode')
-            group_loss = get_memo(group_memo, 'loss')
-            for name, module in group._losses.items():
-                value = module.from_mse4(mse[g])
-                group_loss[name] = value
-                sums[name] = value if g == 0 else sums[name] + value
-        loss = None
-        for name, total in sums.items():
-            loss_memo[name] = total / len(groups)
-            loss = loss_memo[name] if loss is None else loss + loss_memo[name]
-        if loss is None:
-            loss = mse[0][0].new_zeros([])
-        return z, loss, memo
+    def _quantize(self, x: torch.Tensor, groups: list, memos: list, memo: dict):
+        return Fq.grouped_quantize(groups, x, memos, self._want_norm(), rotate=groups[0].rotation_trick)

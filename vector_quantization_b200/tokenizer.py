@@ -19,7 +19,7 @@ from . import functional as Fq
 from . import ops
 from ._lib import VQBError
 from .quantizers import (FiniteScalarQuantizer, GroupedVectorQuantizer, ResidualVectorQuantizer, VectorQuantizer,
-                         get_memo)
+                         _ComposedQuantizer, get_memo)
 
 __all__ = ['quantize', 'encode_to_quant', 'decode_from_quant', 'save_tokens', 'load_tokens', 'save_llamagen_codes', 'TokenStreamWriter']
 
@@ -57,35 +57,26 @@ def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = F
     compact=True is the tokenise-only variant: token ids come back as uint16 (K <= 65 536) or int32 straight
     from the packed assignment keys and memo['quantizer']['quant'] holds that compact tensor.
     A ResidualVectorQuantizer gives quant [b, h, w, L] (a token's L ids contiguous); with compact=True each level's
-    ids are compacted into a row of an [L, N] buffer and one transpose makes the [N, L] layout.  A
+    ids are compacted into a row of an [L, N] buffer and one transpose (none when L = 1) makes the [N, L] layout.  A
     GroupedVectorQuantizer gives quant [b, h, w, G] the same way (its encode reads the latents through one split
     launch; memo['quantizer']['x'] is then the latents)."""
     quantizer_memo = get_memo(memo, 'quantizer')
     quantizer_memo['x_shape'] = (b, _, h, w) = tuple(x.shape)
-    if isinstance(quantizer, GroupedVectorQuantizer):
-        G = quantizer.num_groups
-        by_group = quantizer.encode_compact(x, quantizer_memo) if compact else None
-        if by_group is not None:
-            quant = by_group.view(-1, 1) if G == 1 else ops.transpose_last2(by_group.view(1, G, -1)).view(-1, G)
+    if isinstance(quantizer, _ComposedQuantizer):
+        M = len(quantizer.quantizers)
+        # a GroupedVectorQuantizer reads the latents through one split launch; residual levels read token-major rows
+        x = x if isinstance(quantizer, GroupedVectorQuantizer) else Fq.nchw_to_rows(x)
+        by_member = quantizer.encode_compact(x, quantizer_memo) if compact else None
+        if by_member is not None:
+            quant = by_member.view(-1, 1) if M == 1 else ops.transpose_last2(by_member.view(1, M, -1)).view(-1, M)
             quant = quant[:b * h * w]
         else:
-            _, quant, _ = quantizer.encode(x, quantizer_memo)
+            x, quant, _ = quantizer.encode(x, quantizer_memo)
             if compact:
                 quant = quant.to(torch.int32)
         quantizer_memo.update(x=x, quant=quant)
-        return quant.view(b, h, w, G), memo
+        return quant.view(b, h, w, M), memo
     rows = Fq.nchw_to_rows(x)
-    if isinstance(quantizer, ResidualVectorQuantizer):
-        L = quantizer.num_quantizers
-        by_level = quantizer.encode_compact(rows, quantizer_memo) if compact else None
-        if by_level is not None:
-            quant = ops.transpose_last2(by_level.view(1, L, -1)).view(-1, L)[:b * h * w]
-        else:
-            rows, quant, _ = quantizer.encode(rows, quantizer_memo)
-            if compact:
-                quant = quant.to(torch.int32)
-        quantizer_memo.update(x=rows, quant=quant)
-        return quant.view(b, h, w, L), memo
     # keep the packed keys (no int64 unpack launch) unless a training callback consumes the indices in after_encode
     lazy = compact and isinstance(quantizer, VectorQuantizer) and quantizer._callbacks.packed_keys_ok()
     if lazy:
@@ -117,15 +108,11 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     An id outside [0, codebook_size) is an error: with check=True (one 4-byte device-to-host read) it raises
     IndexError with the number of such tokens.  check=False does not synchronise (safe inside a CUDA graph capture)
     and, on the one-launch path, decodes such tokens to NaN in every channel."""
-    residual = isinstance(quantizer, ResidualVectorQuantizer)
-    grouped = isinstance(quantizer, GroupedVectorQuantizer)
-    if residual and (quant.dim() != 4 or quant.shape[-1] != quantizer.num_quantizers):
-        raise ValueError(f'expected residual token ids of shape [b, h, w, {quantizer.num_quantizers}], '
-                         f'got {tuple(quant.shape)}')
-    if grouped and (quant.dim() != 4 or quant.shape[-1] != quantizer.num_groups):
-        raise ValueError(f'expected grouped token ids of shape [b, h, w, {quantizer.num_groups}], '
-                         f'got {tuple(quant.shape)}')
-    if not (residual or grouped) and quant.dim() != 3:
+    composed = isinstance(quantizer, _ComposedQuantizer)
+    if composed and (quant.dim() != 4 or quant.shape[-1] != len(quantizer.quantizers)):
+        raise ValueError(f'expected {type(quantizer).__name__} token ids of shape '
+                         f'[b, h, w, {len(quantizer.quantizers)}], got {tuple(quant.shape)}')
+    if not composed and quant.dim() != 3:
         raise ValueError(f'expected token ids of shape [b, h, w], got {tuple(quant.shape)}')
     if not quant.is_cuda:
         raise VQBError('vector_quantization_b200 decodes CUDA (sm_100a) token ids only; there is no CPU fallback')
@@ -133,10 +120,9 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
         raise TypeError(f'dtype must be float32 or bfloat16, got {dtype}')
     b, h, w = quant.shape[:3]
     quantizer_memo = get_memo(memo, 'quantizer')
-    if residual or grouped:
+    if composed:
         bad = torch.zeros(1, dtype=torch.int32, device=quant.device) if check else None
-        decode = ops.decode_residual_tokens if residual else ops.decode_group_tokens
-        z = decode([W.detach() for W in quantizer._weights()], quant.contiguous(), h * w, dtype, bad)
+        z = quantizer._decode_ids(quant.contiguous(), h * w, dtype, bad)
         get_memo(quantizer_memo, 'decode')
         if check:
             _raise_bad_ids(int(bad.item()), quantizer.codebook_size)
