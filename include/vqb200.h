@@ -308,6 +308,35 @@ int vqb_residual_backward_rotated(const void* g_z, int g_dtype, const void* x, i
 int vqb_residual_backward_rotated_rows(const void* g_z, int g_dtype, const void* x, int x_dtype,
                                        const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N,
                                        int D, int want_norm_mse, void* gx_out, int64_t g_hw, void* stream);
+/* Quantizer dropout (DESIGN.md §4.10): the entry points above with a per-token depth.  Token n is coded by its first
+ * d_n = depth[n / depth_hw] levels (int32; depth_hw = h*w for one depth per image, 1 for one per token; values outside
+ * [1, L] are clamped to it, there is no host check).  Assignment is unchanged: q_l and r_l exist at every level.
+ *   step:      zhat adds e_l, and the level's mse4 sums take the token, only when level < d_n (mse4 keeps the 1/(N*D)
+ *              denominator); z = x + (zhat_{d_n} - x).
+ *   backward:  levels l >= d_n add nothing to gx and nothing to gW_l (the _rows variants store zero rows for them);
+ *              the _rotated variants rotate towards zhat_{d_n}.
+ * With every depth = L the results are bit for bit those of the entry points without _depth. */
+int vqb_residual_step_depth(const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N, int D,
+                            const float* W, int64_t K, const int64_t* quant, const unsigned long long* keys,
+                            int64_t key_index_offset, int64_t* quant_out, int L, int level, float* zhat, float* r_out,
+                            float* z_out, int64_t z_hw, int want_norm_mse, float* mse4_out, float* partials,
+                            unsigned int* ticket, const int32_t* depth, int64_t depth_hw, void* stream);
+int vqb_residual_backward_depth(const void* g_z, int g_dtype, const void* x, int x_dtype,
+                                const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
+                                int want_norm_mse, void* gx_out, int64_t g_hw, const int32_t* depth, int64_t depth_hw,
+                                void* stream);
+int vqb_residual_backward_depth_rows(const void* g_z, int g_dtype, const void* x, int x_dtype,
+                                     const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N,
+                                     int D, int want_norm_mse, void* gx_out, int64_t g_hw, const int32_t* depth,
+                                     int64_t depth_hw, void* stream);
+int vqb_residual_backward_depth_rotated(const void* g_z, int g_dtype, const void* x, int x_dtype,
+                                        const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N,
+                                        int D, int want_norm_mse, void* gx_out, int64_t g_hw, const int32_t* depth,
+                                        int64_t depth_hw, void* stream);
+int vqb_residual_backward_depth_rotated_rows(const void* g_z, int g_dtype, const void* x, int x_dtype,
+                                             const vqb_residual_levels* levels, int64_t K, const int64_t* quant,
+                                             int64_t N, int D, int want_norm_mse, void* gx_out, int64_t g_hw,
+                                             const int32_t* depth, int64_t depth_hw, void* stream);
 
 /* ---- grouped (product) quantization: G codebooks, group g quantizes channels [g*Dg, (g+1)*Dg) of every token ---- *
  * Group g behaves exactly like its own vqb_gather_ste_loss / vqb_quantize_backward on the contiguous [N, Dg] slice

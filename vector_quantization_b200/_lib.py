@@ -100,6 +100,21 @@ SIGNATURES = {
                                               c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     'vqb_residual_backward_rotated_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64,
                                                    c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    'vqb_residual_step_depth': (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_int, c_void_p, c_int64, c_void_p,
+                                        c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int64,
+                                        c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    'vqb_residual_backward_depth': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64,
+                                            c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p, c_int64,
+                                            c_void_p]),
+    'vqb_residual_backward_depth_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64,
+                                                 c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p, c_int64,
+                                                 c_void_p]),
+    'vqb_residual_backward_depth_rotated': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels), c_int64,
+                                                    c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p,
+                                                    c_int64, c_void_p]),
+    'vqb_residual_backward_depth_rotated_rows': (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(ResidualLevels),
+                                                         c_int64, c_void_p, c_int64, c_int, c_int, c_void_p, c_int64,
+                                                         c_void_p, c_int64, c_void_p]),
     'vqb_group_gather_ste_loss': (c_int, [c_void_p, c_int, c_int64, c_int, POINTER(ResidualLevels), c_int64, c_void_p,
                                           c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p,
                                           c_void_p]),

@@ -140,6 +140,13 @@ __device__ __forceinline__ int64_t row_index(const int64_t* __restrict__ quant,
   return q < 0 ? 0 : (q >= K ? K - 1 : q);  // never read out of bounds on a corrupt index
 }
 
+// The depth d_n of token n under quantizer dropout: depth[n / depth_hw] (one entry per image, or per token with
+// depth_hw = 1), clamped to [1, L].
+__device__ __forceinline__ int token_depth(const int32_t* __restrict__ depth, int64_t n, int64_t depth_hw, int L) {
+  const int d = depth[n / depth_hw];
+  return d < 1 ? 1 : (d > L ? L : d);
+}
+
 // ---- the per-token terms shared by the plain, residual and grouped kernels -----------------------------------------
 // The forward's reciprocal norms for the norm=True MSE term (1 ulp vs a true division), from the lane-partial sums of
 // squares of the token x and the codebook row z.
@@ -470,13 +477,15 @@ __global__ void __launch_bounds__(256, 4) quantize_backward_kernel(
 // One level of the residual chain (see vqb_residual_step): the per-token work of quantize_forward_kernel with (x, W[q])
 // = (r_{l-1}, W_l[q_l]), plus the running sum zhat and the next residual.  Every sum is an explicit round-to-nearest
 // add / subtract, so the backward can recompute r_{l-1} bit for bit.  TR: the dtype of r_{l-1} (TX at level 0).
-template <typename TX, typename TR, int G, int V, int NV>
+// kDepth: token n is coded by its first d_n = depth[n / depth_hw] levels (clamped to [1, L]; DESIGN.md §4.10): at a
+// level l >= d_n the token adds nothing to zhat or to the loss sums, while q_l and r_l are still written.
+template <typename TX, typename TR, int G, int V, int NV, bool kDepth = false>
 __global__ void __launch_bounds__(256) residual_step_kernel(
     const TR* __restrict__ r_in, const TX* __restrict__ x, int64_t N, int D, const float* __restrict__ W, int64_t K,
     const int64_t* __restrict__ quant, const unsigned long long* __restrict__ keys, int64_t key_offset,
     int64_t* __restrict__ quant_out, int L, int level, float* __restrict__ zhat, float* __restrict__ r_out,
     float* __restrict__ z_out, int64_t z_hw, int want_norm, float* __restrict__ mse4, float* __restrict__ partials,
-    unsigned int* __restrict__ ticket) {
+    unsigned int* __restrict__ ticket, const int32_t* __restrict__ depth, int64_t depth_hw) {
   __shared__ float sh[16];
   pdl_wait();               // keys / codebook / previous level come from the preceding launches
   pdl_launch_dependents();
@@ -489,6 +498,7 @@ __global__ void __launch_bounds__(256) residual_step_kernel(
     const bool valid = n_raw < N;
     const int64_t n = valid ? n_raw : N - 1;
     const int64_t q = row_index(quant, keys, n, key_offset, K);
+    const bool active = !kDepth || level < token_depth(depth, n, depth_hw, L);
     const float* __restrict__ wrow = W + q * D;
     const TR* __restrict__ rrow = r_in + n * D;
     float rr[NV][V], wr[NV][V];
@@ -519,10 +529,10 @@ __global__ void __launch_bounds__(256) residual_step_kernel(
 #pragma unroll
       for (int i = 0; i < V; ++i) {
         const float diff = __fsub_rn(wr[it][i], rr[it][i]);
-        if (valid) sse = fmaf(diff, diff, sse);
+        if (valid && active) sse = fmaf(diff, diff, sse);
         if (want_norm) {
           const float dn = wr[it][i] * rdw - rr[it][i] * rdr;
-          if (valid) sse_n = fmaf(dn, dn, sse_n);
+          if (valid && active) sse_n = fmaf(dn, dn, sse_n);
         }
       }
       if (valid && d0 < D) {
@@ -530,7 +540,7 @@ __global__ void __launch_bounds__(256) residual_step_kernel(
         if (level > 0 && zhat) {
           load_slice<float, V>(zhat + n * D, d0, D, h);
 #pragma unroll
-          for (int i = 0; i < V; ++i) h[i] = __fadd_rn(h[i], wr[it][i]);
+          for (int i = 0; i < V; ++i) h[i] = active ? __fadd_rn(h[i], wr[it][i]) : h[i];
         } else {
 #pragma unroll
           for (int i = 0; i < V; ++i) h[i] = wr[it][i];
@@ -539,7 +549,7 @@ __global__ void __launch_bounds__(256) residual_step_kernel(
           float rn[V];
 #pragma unroll
           for (int i = 0; i < V; ++i) rn[i] = __fsub_rn(rr[it][i], wr[it][i]);
-          if (zhat) store_slice<float, V>(zhat + n * D, d0, D, h);
+          if (zhat && active) store_slice<float, V>(zhat + n * D, d0, D, h);
           store_slice<float, V>(r_out + n * D, d0, D, rn);
         } else if (z_out) {
           float xv[V], zr[V];
@@ -567,10 +577,14 @@ __global__ void __launch_bounds__(256) residual_step_kernel(
 // [N, D] rows with kRowsOut).  The level table is a __grid_constant__ parameter: indexed in place, never copied.
 // kRotate: the rotation trick over the whole depth (DESIGN.md §4.9): before the level loop, g_z is replaced by
 // rotate_grad(x, zhat_L, g_z), with zhat_L = W_0[q_0] + ... + W_{L-1}[q_{L-1}] rebuilt in wr with the forward's adds.
-template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut, bool kRotate = false>
+// kDepth: token n is coded by its first d_n levels (token_depth; DESIGN.md §4.10): the levels l >= d_n add nothing to
+// g_z and store zero gradient rows (kRowsOut) or none (atomics), and the rotation goes to zhat_{d_n}.  The level loop
+// keeps its trip count L for every lane (norm_terms shuffles across the row's lanes); the inactive levels are masked.
+template <typename TX, typename TG, int G, int V, int NV, bool kRowsOut, bool kRotate = false, bool kDepth = false>
 __global__ void __launch_bounds__(256) residual_backward_kernel(
     const TG* __restrict__ gz, const TX* __restrict__ x, const __grid_constant__ vqb_residual_levels lv, int64_t K,
-    const int64_t* __restrict__ quant, int64_t N, int D, int want_norm, TX* __restrict__ gx, int64_t g_hw) {
+    const int64_t* __restrict__ quant, int64_t N, int D, int want_norm, TX* __restrict__ gx, int64_t g_hw,
+    const int32_t* __restrict__ depth, int64_t depth_hw) {
   pdl_wait();               // upstream gradients / indices come from the preceding launches
   pdl_launch_dependents();
   const int lane = threadIdx.x % G;
@@ -582,6 +596,7 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
     const bool valid = n_raw < N;
     const int64_t n = valid ? n_raw : N - 1;
     const TX* __restrict__ xrow = x + n * D;
+    const int dn = kDepth ? token_depth(depth, n, depth_hw, L) : L;
     float yr[NV][V], wr[NV][V], gr[NV][V];   // r_{l-1}, W_l[q_l], the running token gradient
 #pragma unroll
     for (int it = 0; it < NV; ++it) {
@@ -596,9 +611,10 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
       }
     }
     if constexpr (kRotate) {
-      // zhat_L into wr (the level loop reloads it): level 0's row, then each deeper row added in level order
+      // zhat_{d_n} into wr (the level loop reloads it): level 0's row, then each deeper row added in level order (no
+      // shuffle in this loop: its trip count may differ between the rows of a warp)
 #pragma unroll 1
-      for (int l = 0; l < L; ++l) {
+      for (int l = 0; l < dn; ++l) {
         const int64_t q = row_index(quant, nullptr, n * L + l, 0, K);
         const float* __restrict__ wrow = lv.W[l] + q * D;
 #pragma unroll
@@ -628,14 +644,15 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
 #pragma unroll 1
     for (int l = 0; l < L; ++l) {
       const LossCoefs c = loss_coefs(lv.g[l][0], lv.g[l][1], lv.g[l][2], lv.g[l][3], want_norm, scale);
-      const int64_t q = row_index(quant, nullptr, n * L + l, 0, K);
+      const bool active = !kDepth || l < dn;   // inactive levels read no row: r_l is not needed past d_n
+      const int64_t q = active ? row_index(quant, nullptr, n * L + l, 0, K) : 0;
       const float* __restrict__ wrow = lv.W[l] + q * D;
       float* __restrict__ gW = lv.gW[l];
       float sxx = 0.f, sww = 0.f;
 #pragma unroll
       for (int it = 0; it < NV; ++it) {
         const int d0 = (it * G + lane) * V;
-        if (d0 < D) {
+        if (d0 < D && active) {
           load_slice<float, V>(wrow, d0, D, wr[it]);
         } else {
 #pragma unroll
@@ -654,10 +671,13 @@ __global__ void __launch_bounds__(256) residual_backward_kernel(
         float gw[V];
 #pragma unroll
         for (int i = 0; i < V; ++i) {
-          gw[i] = backward_term(yr[it][i], wr[it][i], gr[it][i], c, t, want_norm);
+          float g = gr[it][i];
+          const float gwi = backward_term(yr[it][i], wr[it][i], g, c, t, want_norm);
+          gw[i] = active ? gwi : 0.f;
+          gr[it][i] = active ? g : gr[it][i];
           yr[it][i] = __fsub_rn(yr[it][i], wr[it][i]);    // r_l
         }
-        emit_gw<kRowsOut, V>(gW, n, q, D, d0, valid, gw);
+        emit_gw<kRowsOut, V>(gW, n, q, D, d0, valid && (kRowsOut || active), gw);   // _rows: zero rows when inactive
       }
     }
 #pragma unroll
@@ -996,31 +1016,38 @@ int vqb_quantize_backward_rotated_rows(const void* gz, int g_dtype, const void* 
                                               g_cmn, want_norm, gx, gW_rows, g_hw, stream);
 }
 
-int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N, int D, const float* W,
-                      int64_t K, const int64_t* quant, const unsigned long long* keys, int64_t key_index_offset,
-                      int64_t* quant_out, int L, int level, float* zhat, float* r_out, float* z_out, int64_t z_hw,
-                      int want_norm, float* mse4, float* partials, unsigned int* ticket, void* stream) {
-  VQB_REQUIRE(z_hw >= 0 && (z_hw == 0 || N % z_hw == 0), "vqb_residual_step: z_hw must divide N (tokens = images x h*w)");
-  VQB_REQUIRE(r_in && x && W && mse4 && partials && ticket, "vqb_residual_step: null pointer");
-  VQB_REQUIRE((quant != nullptr) != (keys != nullptr), "vqb_residual_step: pass exactly one of quant / keys");
-  VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "vqb_residual_step: bad shape N=%lld D=%d K=%lld", (long long)N, D, (long long)K);
-  VQB_REQUIRE(L >= 1 && L <= VQB_MAX_LEVELS && level >= 0 && level < L, "vqb_residual_step: level %d of L=%d (L <= %d)",
-              level, L, VQB_MAX_LEVELS);
-  VQB_REQUIRE((r_out != nullptr) == (level < L - 1), "vqb_residual_step: r_out is required below the last level, and "
-              "must be NULL at the last one");
+}  // extern "C"
+
+// kDepth: the per-token depths of quantizer dropout (vqb_residual_step_depth)
+template <bool kDepth>
+static int residual_step_launch(const char* fn, const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N,
+                                int D, const float* W, int64_t K, const int64_t* quant, const unsigned long long* keys,
+                                int64_t key_index_offset, int64_t* quant_out, int L, int level, float* zhat,
+                                float* r_out, float* z_out, int64_t z_hw, int want_norm, float* mse4, float* partials,
+                                unsigned int* ticket, const int32_t* depth, int64_t depth_hw, void* stream) {
+  VQB_REQUIRE(z_hw >= 0 && (z_hw == 0 || N % z_hw == 0), "%s: z_hw must divide N (tokens = images x h*w)", fn);
+  VQB_REQUIRE(r_in && x && W && mse4 && partials && ticket, "%s: null pointer", fn);
+  VQB_REQUIRE(!kDepth || depth, "%s: null depth", fn);
+  VQB_REQUIRE(!kDepth || (depth_hw >= 1 && N % depth_hw == 0), "%s: depth_hw must divide N (tokens = images x h*w)", fn);
+  VQB_REQUIRE((quant != nullptr) != (keys != nullptr), "%s: pass exactly one of quant / keys", fn);
+  VQB_REQUIRE(N >= 1 && D >= 1 && K >= 1, "%s: bad shape N=%lld D=%d K=%lld", fn, (long long)N, D, (long long)K);
+  VQB_REQUIRE(L >= 1 && L <= VQB_MAX_LEVELS && level >= 0 && level < L, "%s: level %d of L=%d (L <= %d)", fn, level, L,
+              VQB_MAX_LEVELS);
+  VQB_REQUIRE((r_out != nullptr) == (level < L - 1), "%s: r_out is required below the last level, and must be NULL "
+              "at the last one", fn);
   VQB_REQUIRE(level == 0 ? (r_in == x && r_dtype == x_dtype) : r_dtype == VQB_F32,
-              "vqb_residual_step: r_in is x at level 0 and an fp32 residual after");
-  VQB_REQUIRE(z_out == nullptr || level == 0 || zhat, "vqb_residual_step: z needs zhat (the levels' running sum)");
+              "%s: r_in is x at level 0 and an fp32 residual after", fn);
+  VQB_REQUIRE(z_out == nullptr || level == 0 || zhat, "%s: z needs zhat (the levels' running sum)", fn);
   RowGeom geom;
-  VQB_REQUIRE(row_geom(D, N, &geom), "vqb_residual_step: D=%d unsupported (multiple of 8 up to 2048, or any D <= 256)", D);
+  VQB_REQUIRE(row_geom(D, N, &geom), "%s: D=%d unsupported (multiple of 8 up to 2048, or any D <= 256)", fn, D);
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = grid_for(N, 256 / geom.G);
-  VQB_REQUIRE(blocks <= kMaxPartials, "vqb_residual_step: grid too large");
+  VQB_REQUIRE(blocks <= kMaxPartials, "%s: grid too large", fn);
   bool launched = false;
 #define VQB_RESIDUAL_STEP(TX_, TR_)                                                                                   \
-  VQB_DISPATCH_GEOM((launch_pdl(residual_step_kernel<TX_, TR_, G, V, NV>, blocks, 256, 0, st, (const TR_*)r_in,        \
-      (const TX_*)x, N, D, W, K, quant, keys, key_index_offset, quant_out, L, level, zhat, r_out, z_out, z_hw,        \
-      want_norm, mse4, partials, ticket)))
+  VQB_DISPATCH_GEOM((launch_pdl(residual_step_kernel<TX_, TR_, G, V, NV, kDepth>, blocks, 256, 0, st,                \
+      (const TR_*)r_in, (const TX_*)x, N, D, W, K, quant, keys, key_index_offset, quant_out, L, level, zhat, r_out,   \
+      z_out, z_hw, want_norm, mse4, partials, ticket, depth, depth_hw)))
   if (x_dtype == VQB_F32 && r_dtype == VQB_F32) {
     VQB_RESIDUAL_STEP(float, float)
   } else if (x_dtype == VQB_BF16 && r_dtype == VQB_BF16) {
@@ -1029,9 +1056,30 @@ int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype,
     VQB_RESIDUAL_STEP(__nv_bfloat16, float)
   }
 #undef VQB_RESIDUAL_STEP
-  VQB_REQUIRE(launched, "vqb_residual_step: unsupported dtype/geometry");
+  VQB_REQUIRE(launched, "%s: unsupported dtype/geometry", fn);
   VQB_LAUNCH_OK();
   return VQB_OK;
+}
+
+extern "C" {
+
+int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N, int D, const float* W,
+                      int64_t K, const int64_t* quant, const unsigned long long* keys, int64_t key_index_offset,
+                      int64_t* quant_out, int L, int level, float* zhat, float* r_out, float* z_out, int64_t z_hw,
+                      int want_norm, float* mse4, float* partials, unsigned int* ticket, void* stream) {
+  return residual_step_launch<false>("vqb_residual_step", r_in, r_dtype, x, x_dtype, N, D, W, K, quant, keys,
+                                     key_index_offset, quant_out, L, level, zhat, r_out, z_out, z_hw, want_norm, mse4,
+                                     partials, ticket, nullptr, 1, stream);
+}
+
+int vqb_residual_step_depth(const void* r_in, int r_dtype, const void* x, int x_dtype, int64_t N, int D,
+                            const float* W, int64_t K, const int64_t* quant, const unsigned long long* keys,
+                            int64_t key_index_offset, int64_t* quant_out, int L, int level, float* zhat, float* r_out,
+                            float* z_out, int64_t z_hw, int want_norm, float* mse4, float* partials,
+                            unsigned int* ticket, const int32_t* depth, int64_t depth_hw, void* stream) {
+  return residual_step_launch<true>("vqb_residual_step_depth", r_in, r_dtype, x, x_dtype, N, D, W, K, quant, keys,
+                                    key_index_offset, quant_out, L, level, zhat, r_out, z_out, z_hw, want_norm, mse4,
+                                    partials, ticket, depth, depth_hw, stream);
 }
 
 }  // extern "C"
@@ -1040,13 +1088,18 @@ int vqb_residual_step(const void* r_in, int r_dtype, const void* x, int x_dtype,
 // (residual_backward_kernel on tokens of width D) or the channel groups of a grouped quantizer (group_backward_kernel,
 // D the group width Dg, one grid row per group).  Messages name the members as "level" or "group".  kRotate: the
 // rotation trick, per group (group_backward_kernel) or over the whole depth (residual_backward_kernel).
-template <bool kGroups, bool kRowsOut, bool kRotate = false>
+// kDepth (levels only): the per-token depths of quantizer dropout, depth[n / depth_hw].
+template <bool kGroups, bool kRowsOut, bool kRotate = false, bool kDepth = false>
 static int member_backward_launch(const char* fn, const void* gz, int g_dtype, const void* x, int x_dtype,
                                   const vqb_residual_levels* lv, int64_t K, const int64_t* quant, int64_t N, int D,
-                                  int want_norm, void* gx, int64_t g_hw, void* stream) {
+                                  int want_norm, void* gx, int64_t g_hw, void* stream, const int32_t* depth = nullptr,
+                                  int64_t depth_hw = 1) {
+  static_assert(!(kGroups && kDepth), "quantizer dropout is a residual feature");
   const char* member = kGroups ? "of group" : "at level";
   VQB_REQUIRE(g_hw >= 0 && (g_hw == 0 || N % g_hw == 0), "%s: g_hw must divide N", fn);
   VQB_REQUIRE(gz && x && lv && quant && gx, "%s: null pointer", fn);
+  VQB_REQUIRE(!kDepth || depth, "%s: null depth", fn);
+  VQB_REQUIRE(!kDepth || (depth_hw >= 1 && N % depth_hw == 0), "%s: depth_hw must divide N", fn);
   VQB_REQUIRE(lv->L >= 1 && lv->L <= VQB_MAX_LEVELS, "%s: %s=%d outside [1, %d]", fn, kGroups ? "G" : "L", lv->L,
               VQB_MAX_LEVELS);
   for (int l = 0; l < lv->L; ++l) {
@@ -1060,9 +1113,13 @@ static int member_backward_launch(const char* fn, const void* gz, int g_dtype, c
   const dim3 grid((unsigned)grid_for(N, 256 / geom.G), kGroups ? (unsigned)lv->L : 1u);
   bool launched = false;
 #define VQB_MEMBER_BWD(TX_, TG_)                                                                                      \
-  VQB_DISPATCH_GEOM((launch_pdl(kGroups ? group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate>                 \
-                                        : residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate>,             \
-      grid, 256, 0, st, (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw)))
+  if constexpr (kGroups) {                                                                                             \
+    VQB_DISPATCH_GEOM((launch_pdl(group_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate>, grid, 256, 0, st,      \
+        (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw)))                               \
+  } else {                                                                                                             \
+    VQB_DISPATCH_GEOM((launch_pdl(residual_backward_kernel<TX_, TG_, G, V, NV, kRowsOut, kRotate, kDepth>, grid, 256,  \
+        0, st, (const TG_*)gz, (const TX_*)x, *lv, K, quant, N, D, want_norm, (TX_*)gx, g_hw, depth, depth_hw)))      \
+  }
   VQB_DISPATCH_BWD_DTYPES(VQB_MEMBER_BWD)
 #undef VQB_MEMBER_BWD
   VQB_REQUIRE(launched, "%s: unsupported dtype/geometry", fn);
@@ -1098,6 +1155,42 @@ int vqb_residual_backward_rotated_rows(const void* gz, int g_dtype, const void* 
                                        int D, int want_norm, void* gx, int64_t g_hw, void* stream) {
   return member_backward_launch<false, true, true>("vqb_residual_backward_rotated_rows", gz, g_dtype, x, x_dtype, levels,
                                                    K, quant, N, D, want_norm, gx, g_hw, stream);
+}
+
+int vqb_residual_backward_depth(const void* gz, int g_dtype, const void* x, int x_dtype,
+                                const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N, int D,
+                                int want_norm, void* gx, int64_t g_hw, const int32_t* depth, int64_t depth_hw,
+                                void* stream) {
+  return member_backward_launch<false, false, false, true>("vqb_residual_backward_depth", gz, g_dtype, x, x_dtype,
+                                                           levels, K, quant, N, D, want_norm, gx, g_hw, stream, depth,
+                                                           depth_hw);
+}
+
+int vqb_residual_backward_depth_rows(const void* gz, int g_dtype, const void* x, int x_dtype,
+                                     const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N,
+                                     int D, int want_norm, void* gx, int64_t g_hw, const int32_t* depth,
+                                     int64_t depth_hw, void* stream) {
+  return member_backward_launch<false, true, false, true>("vqb_residual_backward_depth_rows", gz, g_dtype, x, x_dtype,
+                                                          levels, K, quant, N, D, want_norm, gx, g_hw, stream, depth,
+                                                          depth_hw);
+}
+
+int vqb_residual_backward_depth_rotated(const void* gz, int g_dtype, const void* x, int x_dtype,
+                                        const vqb_residual_levels* levels, int64_t K, const int64_t* quant, int64_t N,
+                                        int D, int want_norm, void* gx, int64_t g_hw, const int32_t* depth,
+                                        int64_t depth_hw, void* stream) {
+  return member_backward_launch<false, false, true, true>("vqb_residual_backward_depth_rotated", gz, g_dtype, x,
+                                                          x_dtype, levels, K, quant, N, D, want_norm, gx, g_hw, stream,
+                                                          depth, depth_hw);
+}
+
+int vqb_residual_backward_depth_rotated_rows(const void* gz, int g_dtype, const void* x, int x_dtype,
+                                             const vqb_residual_levels* levels, int64_t K, const int64_t* quant,
+                                             int64_t N, int D, int want_norm, void* gx, int64_t g_hw,
+                                             const int32_t* depth, int64_t depth_hw, void* stream) {
+  return member_backward_launch<false, true, true, true>("vqb_residual_backward_depth_rotated_rows", gz, g_dtype, x,
+                                                         x_dtype, levels, K, quant, N, D, want_norm, gx, g_hw, stream,
+                                                         depth, depth_hw);
 }
 
 int vqb_group_gather_ste_loss(const void* xs, int x_dtype, int64_t N, int Dg, const vqb_residual_levels* lv, int64_t K,

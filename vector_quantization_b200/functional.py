@@ -367,13 +367,15 @@ def _encode_member(member, x: torch.Tensor, memo: dict, track_codebooks: bool):
 @torch.no_grad()
 def residual_levels(levels, x: torch.Tensor, memos, want_norm: bool, *, quant_out: torch.Tensor | None = None,
                     z_out: torch.Tensor | None = None, z_hw: int = 0, compact_out: torch.Tensor | None = None,
-                    track_codebooks: bool = False):
+                    track_codebooks: bool = False, depth: torch.Tensor | None = None, depth_hw: int = 1):
     """The level loop of a residual quantizer: level l runs its own `encode` (before_encode -> assignment ->
     after_encode, codebook updates included) on r_{l-1}, then ONE `vqb_residual_step` launch gathers W_l[q_l] from the
     codebook as that encode left it, writes the [N, L] indices, the running sum and r_l, and at the last level
     z = x + (zhat_L - x).  memos[l] becomes level l's memo (x = r_{l-1}, quant = its indices).
     compact_out: uint16 / int32 [L, N]: the compact ids of every level, straight from its packed assignment keys (every
     level must then accept packed keys: no training callback reads the indices).
+    depth: quantizer dropout (DESIGN.md §4.10): int32 depths, token n coded by its first depth[n // depth_hw] levels
+    (zhat, z and the MSE terms); every level still encodes every token.
     -> (mse fp32 [L, 4], [CodebookRef per level] (registered with the level when track_codebooks))"""
     N, D = x.shape
     L = len(levels)
@@ -393,7 +395,8 @@ def residual_levels(levels, x: torch.Tensor, memos, want_norm: bool, *, quant_ou
         if not (last and z_out is None and quant_out is None):
             ops.residual_step(r, x, ref.tensor, mse[l], level=l, L=L, quant=None if lazy else index,
                               keys=index if lazy else None, quant_out=quant_out, zhat=zhat, r_out=r_out,
-                              z_out=z_out if last else None, z_hw=z_hw, want_norm=want_norm)
+                              z_out=z_out if last else None, z_hw=z_hw, want_norm=want_norm, depth=depth,
+                              depth_hw=depth_hw)
         memo['x'] = r
         memo['quant'] = quant_out[:, l] if quant_out is not None else index
         r = r_out
@@ -408,9 +411,11 @@ class _ComposedQuantize(torch.autograd.Function):
     upstream gradients arrive as device scalars)."""
 
     @staticmethod
-    def _save(ctx, backward_op, x, quant, refs, z, hw, mse, want_norm, rotate):
-        """Record what the backward needs (x: the tokens the backward kernel reads) -> the node's outputs."""
-        ctx.save_for_backward(x, quant)
+    def _save(ctx, backward_op, x, quant, refs, z, hw, mse, want_norm, rotate, depth=None, depth_hw=1):
+        """Record what the backward needs (x: the tokens the backward kernel reads; depth: the per-token depths of a
+        residual node under quantizer dropout) -> the node's outputs."""
+        ctx.save_for_backward(x, quant, depth)
+        ctx.depth_hw = depth_hw
         ctx.backward_op = backward_op
         ctx.refs = refs
         ctx.shape = tuple(z.shape)
@@ -423,13 +428,14 @@ class _ComposedQuantize(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gz, _gq, *g):
-        x, quant = ctx.saved_tensors
+        x, quant, depth = ctx.saved_tensors
         M = quant.shape[1]
         if gz is None:
             gz = torch.zeros(ctx.shape, dtype=torch.float32, device=x.device)
         g4s = [[None if t is None else t.contiguous().float() for t in g[4 * m:4 * m + 4]] for m in range(M)]
+        dropout = {} if depth is None else dict(depth=depth, depth_hw=ctx.depth_hw)
         gx, gWs = ctx.backward_op(gz.contiguous(), x, [r.tensor for r in ctx.refs], quant, g4s, want_norm=ctx.want_norm,
-                                  need_gW=list(ctx.needs_input_grad[-M:]), g_hw=ctx.hw, rotate=ctx.rotate)
+                                  need_gW=list(ctx.needs_input_grad[-M:]), g_hw=ctx.hw, rotate=ctx.rotate, **dropout)
         rest = (None,) * (len(ctx.needs_input_grad) - M - 1)
         return (gx if ctx.needs_input_grad[0] else None, *rest, *gWs)
 
@@ -438,7 +444,7 @@ def _quantize_composed(node, members, inputs: tuple, memos, want_norm: bool, rot
     """node.apply(*inputs, members, memos, want_norm, track, rotate, *codebooks) -> (z, quant, per member its four
     MSE terms)."""
     Ws = [member._weight() for member in members]
-    track = torch.is_grad_enabled() and any([t.requires_grad for t in inputs + tuple(Ws)])
+    track = torch.is_grad_enabled() and any([t.requires_grad for t in inputs + tuple(Ws) if t is not None])
     out = node.apply(*inputs, list(members), memos, bool(want_norm), track, bool(rotate), *Ws)
     z, quant, flat = out[0], out[1], out[2:]
     return z, quant, [tuple(flat[4 * m:4 * m + 4]) for m in range(len(members))]
@@ -446,29 +452,36 @@ def _quantize_composed(node, members, inputs: tuple, memos, want_norm: bool, rot
 
 class _ResidualQuantize(_ComposedQuantize):
     """The whole depth of a residual quantizer: forward = the level loop (`residual_levels`).  x receives gx: the
-    tokens [N, D], or the NCHW latents of which `rows` is the token-major copy (z and gx are then NCHW)."""
+    tokens [N, D], or the NCHW latents of which `rows` is the token-major copy (z and gx are then NCHW).  depth: None, or
+    the int32 depths of quantizer dropout, one per image of the NCHW latents or one per token."""
 
     @staticmethod
-    def forward(ctx, x, rows, levels, memos, want_norm, track, rotate, *Ws):
+    def forward(ctx, x, rows, depth, levels, memos, want_norm, track, rotate, *Ws):
         N = rows.shape[0]
         hw = x.shape[2] * x.shape[3] if x.dim() == 4 else 0
+        depth_hw = N // depth.numel() if depth is not None else 1
         z = torch.empty(tuple(x.shape), dtype=torch.float32, device=x.device)
         quant = torch.empty((N, len(levels)), dtype=torch.int64, device=x.device)
         mse, refs = residual_levels(levels, rows, memos, want_norm, quant_out=quant, z_out=z, z_hw=hw,
-                                    track_codebooks=track)
-        return _ComposedQuantize._save(ctx, ops.residual_backward, rows, quant, refs, z, hw, mse, want_norm, rotate)
+                                    track_codebooks=track, depth=depth, depth_hw=depth_hw)
+        return _ComposedQuantize._save(ctx, ops.residual_backward, rows, quant, refs, z, hw, mse, want_norm, rotate,
+                                       depth, depth_hw)
 
 
 def residual_quantize(levels, x: torch.Tensor, memos, want_norm: bool, *, nchw: torch.Tensor | None = None,
-                      rotate: bool = False):
+                      rotate: bool = False, depth: torch.Tensor | None = None):
     """Residual quantization of x [N, D] (fp32 / bf16) through `levels` (VectorQuantizer modules sharing K and D).
     -> (z fp32 [N, D] (or NCHW like `nchw`): value x + (zhat_L - x), gradient straight to x;
         quant int64 [N, L];  mse: per level the four MSE terms (codebook, commitment, codebook-norm,
         commitment-norm) of e_l against r_{l-1}, 0-dim tensors whose gradients reach W_l and, through r_{l-1}, x)
     rotate: the gradient of z reaches x through the rotation trick from x to zhat_L, one rotation over the whole
-    depth (DESIGN.md §4.9), instead of straight through; the values and the codebook gradients are unchanged."""
+    depth (DESIGN.md §4.9), instead of straight through; the values and the codebook gradients are unchanged.
+    depth: quantizer dropout (DESIGN.md §4.10): int32 depths d, one per image of `nchw` or one per token of x; token n
+    is then coded by its first d_n levels: zhat_{d_n} in z, the MSE terms and both gradients of level l only from the
+    tokens with l < d_n.  The encodes (assignment, callbacks, indices) still run on every token at every level."""
     x = x.contiguous()
-    return _quantize_composed(_ResidualQuantize, levels, (x if nchw is None else nchw, x), memos, want_norm, rotate)
+    return _quantize_composed(_ResidualQuantize, levels, (x if nchw is None else nchw, x, depth), memos, want_norm,
+                              rotate)
 
 
 @torch.no_grad()

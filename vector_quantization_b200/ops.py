@@ -815,13 +815,14 @@ def _group_codebooks(Ws) -> tuple[int, int]:
 
 
 def _members_backward(name: str, members: str, g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tensor, g4s, *,
-                      want_norm: bool, need_gW, g_hw: int, deterministic: bool | None, rotate: bool):
+                      want_norm: bool, need_gW, g_hw: int, deterministic: bool | None, rotate: bool,
+                      depth: torch.Tensor | None = None, depth_hw: int = 1):
     """The one-launch backward of M members: entry point `name` (vqb_residual_backward, vqb_group_backward) or its
-    _rotated / _rows variants.  x: the tokens the kernel reads ([N, D], or split [M, N, D]) -> (gx in x's dtype with
-    g_z's shape, [gW_m fp32 [K, D] or None])"""
+    _depth (levels only) / _rotated / _rows variants.  x: the tokens the kernel reads ([N, D], or split [M, N, D]) ->
+    (gx in x's dtype with g_z's shape, [gW_m fp32 [K, D] or None])"""
     lib = _lib.load()
     M = len(Ws)
-    dev = _cuda(g_z, x, quant, *Ws, *[g for g4 in g4s for g in g4])
+    dev = _cuda(g_z, x, quant, depth, *Ws, *[g for g4 in g4s for g in g4])
     K, D = _codebooks(Ws, members)
     N = quant.shape[0]
     assert tuple(x.shape) in ((N, D), (M, N, D)) and g_z.numel() == x.numel() and len(g4s) == M
@@ -834,10 +835,12 @@ def _members_backward(name: str, members: str, g_z: torch.Tensor, x: torch.Tenso
     rows = None
     if any(need_gW) and deterministic_enabled(deterministic):
         rows = _det_ws(x.device, 'gw_rows', M * N * D, torch.float32).view(M, N, D)
+    name += '_depth' if depth is not None else ''
     name += ('_rotated' if rotate else '') + ('_rows' if rows is not None else '')
     p = _residual_levels(Ws, gWs if rows is None else list(rows), g4s)
+    extra = () if depth is None else (_p(_depths(depth, N, depth_hw)), depth_hw)
     _call(name, getattr(lib, name), dev, _p(g_z), _dt(g_z), _p(x), _dt(x), ctypes.byref(p), K, _p(quant), N, D,
-          int(want_norm), _p(gx), g_hw, _S)
+          int(want_norm), _p(gx), g_hw, *extra, _S)
     if rows is not None:
         _segment_sum_members(dev, rows, quant, K, gWs)
     return gx, gWs
@@ -860,27 +863,44 @@ def _decode_members(name: str, members: str, Ws, ids: torch.Tensor, hw: int, out
     return z
 
 
+def _depths(depth: torch.Tensor, N: int, depth_hw: int) -> torch.Tensor:
+    """Checks the per-token depths of quantizer dropout: int32 [N / depth_hw] (one per image of depth_hw tokens, or one
+    per token with depth_hw = 1).  Their values are not checked: the kernels clamp them to [1, L]."""
+    if depth.dtype != torch.int32:
+        raise TypeError(f'depth must be an int32 tensor, got {depth.dtype}')
+    if depth_hw < 1 or N % depth_hw or depth.numel() != N // depth_hw:
+        raise ValueError(f'depth has {depth.numel()} entries; {N} tokens with depth_hw = {depth_hw} need {N // max(depth_hw, 1)}')
+    return depth
+
+
 def residual_step(r: torch.Tensor, x: torch.Tensor, W: torch.Tensor, mse4: torch.Tensor, *, level: int, L: int,
                   quant: torch.Tensor | None = None, keys: torch.Tensor | None = None, key_offset: int = 0,
                   quant_out: torch.Tensor | None = None, zhat: torch.Tensor | None = None,
                   r_out: torch.Tensor | None = None, z_out: torch.Tensor | None = None, z_hw: int = 0,
-                  want_norm: bool = False) -> None:
+                  want_norm: bool = False, depth: torch.Tensor | None = None, depth_hw: int = 1) -> None:
     """One level of the residual chain (vqb_residual_step), into the caller's buffers: quant_out int64 [N, L]
     (column `level`), zhat fp32 [N, D], r_out fp32 [N, D] (None at the last level), z_out fp32 [N, D] or NCHW
-    (last level only), mse4 fp32 [4] (this level's terms).  r is x at level 0 and the previous r_out after."""
+    (last level only), mse4 fp32 [4] (this level's terms).  r is x at level 0 and the previous r_out after.
+    depth: quantizer dropout (vqb_residual_step_depth; DESIGN.md §4.10): int32 depths, token n taking
+    depth[n // depth_hw]; the level adds to zhat and to mse4 only the tokens whose depth exceeds `level`."""
     lib = _lib.load()
-    dev = _cuda(r, x, W, mse4, quant, keys, quant_out, zhat, r_out, z_out)
+    dev = _cuda(r, x, W, mse4, quant, keys, quant_out, zhat, r_out, z_out, depth)
     assert W.dtype == torch.float32 and (quant is None) != (keys is None) and mse4.dtype == torch.float32
     assert quant_out is None or (quant_out.dtype == torch.int64 and quant_out.shape == (x.shape[0], L))
     N, D = x.shape
     partials, ticket = _loss_ws(x.device)
-    _call('vqb_residual_step', lib.vqb_residual_step, dev, _p(r), _dt(r), _p(x), _dt(x), N, D, _p(W), W.shape[0],
-          _p(quant), _p(keys), key_offset, _p(quant_out), L, level, _p(zhat), _p(r_out), _p(z_out), z_hw,
-          int(want_norm), _p(mse4), _p(partials), _p(ticket), _S)
+    args = (_p(r), _dt(r), _p(x), _dt(x), N, D, _p(W), W.shape[0], _p(quant), _p(keys), key_offset, _p(quant_out), L,
+            level, _p(zhat), _p(r_out), _p(z_out), z_hw, int(want_norm), _p(mse4), _p(partials), _p(ticket))
+    if depth is None:
+        _call('vqb_residual_step', lib.vqb_residual_step, dev, *args, _S)
+    else:
+        _call('vqb_residual_step_depth', lib.vqb_residual_step_depth, dev, *args, _p(_depths(depth, N, depth_hw)),
+              depth_hw, _S)
 
 
 def residual_backward(g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tensor, g4s, *, want_norm: bool,
-                      need_gW, g_hw: int = 0, deterministic: bool | None = None, rotate: bool = False):
+                      need_gW, g_hw: int = 0, deterministic: bool | None = None, rotate: bool = False,
+                      depth: torch.Tensor | None = None, depth_hw: int = 1):
     """Backward of the whole residual depth in one launch (vqb_residual_backward).  g_z: fp32 (or bf16 with bf16
     tokens) [N, D], or NCHW with g_hw = h*w; Ws: the L codebooks as used by the forward; quant: int64 [N, L]; g4s: per
     level four 0-dim fp32 device tensors / None (codebook, commitment, codebook-norm, commitment-norm upstream
@@ -889,9 +909,13 @@ def residual_backward(g_z: torch.Tensor, x: torch.Tensor, Ws, quant: torch.Tenso
     the level's per-token rows (vqb_residual_backward_rows + vqb_code_sort + vqb_segment_sum_rows, the contract of
     quantize_backward).  rotate: g_z reaches x through the rotation trick from x to zhat_L, over the whole depth
     (vqb_residual_backward_rotated; DESIGN.md §4.9); gW is unchanged.
+    depth: quantizer dropout (the vqb_residual_backward_depth variants; DESIGN.md §4.10): int32 depths as in
+    residual_step; levels at or past a token's depth add nothing to its gx or to gW_l, and the rotation goes to the
+    token's zhat_{d_n}.
     -> (gx in x's dtype with g_z's shape, [gW_l fp32 [K, D] or None])"""
     return _members_backward('vqb_residual_backward', 'levels', g_z, x, Ws, quant, g4s, want_norm=want_norm,
-                             need_gW=need_gW, g_hw=g_hw, deterministic=deterministic, rotate=rotate)
+                             need_gW=need_gW, g_hw=g_hw, deterministic=deterministic, rotate=rotate, depth=depth,
+                             depth_hw=depth_hw)
 
 
 def decode_residual_tokens(Ws, ids: torch.Tensor, hw: int, out_dtype: torch.dtype = torch.float32,

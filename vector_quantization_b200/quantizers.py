@@ -560,8 +560,9 @@ class _ComposedQuantizer(BaseQuantizer):
     def _want_norm(self) -> bool:
         return self._quantizers[0]._loss_terms()
 
-    def _member_memos(self, memo: dict) -> list:
-        memo[self._members] = [dict() for _ in self._quantizers]
+    def _member_memos(self, memo: dict, count: int | None = None) -> list:
+        """One fresh memo per member (the first `count` members when given)."""
+        memo[self._members] = [dict() for _ in range(len(self._quantizers) if count is None else count)]
         return memo[self._members]
 
     def _check_input(self, x: torch.Tensor) -> torch.Tensor:
@@ -576,9 +577,9 @@ class _ComposedQuantizer(BaseQuantizer):
             return None
         return self._encode_compact(x, self._member_memos(memo))
 
-    def _compact_out(self, N: int, device) -> torch.Tensor:
+    def _compact_out(self, N: int, device, count: int | None = None) -> torch.Tensor:
         # rows padded to 8 ids: every row starts 16-byte aligned, as vqb_compact_tokens reads and stores 16 bytes at a time
-        return torch.empty((len(self._quantizers), (N + 7) // 8 * 8),
+        return torch.empty((len(self._quantizers) if count is None else count, (N + 7) // 8 * 8),
                            dtype=torch.uint16 if self.codebook_size <= 65536 else torch.int32, device=device)
 
     def decode(self, quant: torch.Tensor, memo: dict):
@@ -637,15 +638,33 @@ class ResidualVectorQuantizer(_ComposedQuantizer):
     the indices, the codebook updates and the codebook gradients are unchanged; with L = 1 the gradient is that of a
     rotated VectorQuantizer bit for bit.  The key belongs to this node; in the level config it is rejected.
 
+    quantizer_dropout = p in [0, 1] (SoundStream, EnCodec, DAC; DESIGN.md §4.10): in training, each forward draws a
+    depth d per sample on the device (a sample is an image under `tokenizer.quantize`, a token for [N, D] input): the
+    first floor(S * p) of the S samples get d uniform in {1, ..., L}, the others d = L.  A sample is then coded by its
+    first d levels only: z = x + (zhat_d - x), and level l's loss terms and gradients take only the tokens with l < d
+    (the loss keeps its 1 / (N * D) scale).  Every level still encodes every token, so the indices, the callbacks'
+    codebook updates and their statistics are those of the same step without dropout.  memo['depth'] holds the int32
+    depths of the step.  With p = 0 or in eval mode the step is the one without dropout.
+
+    encode / encode_compact(..., num_quantizers=n) run only the first n levels (truncated codes [N, n]).
+
     Accepted and rejected level configurations: see `_ComposedQuantizer`, with 1 <= L <= 16 and mse.norm on or off;
-    rotation_trick=True in the level config is rejected too."""
+    rotation_trick=True and quantizer_dropout in the level config are rejected too."""
 
     _members = 'levels'
     _rotation_on_node = True
 
-    def __init__(self, *args, num_quantizers: int, quantizer: Mapping, rotation_trick: bool = False, **kwargs) -> None:
+    def __init__(self, *args, num_quantizers: int, quantizer: Mapping, rotation_trick: bool = False,
+                 quantizer_dropout: float = 0.0, **kwargs) -> None:
         super().__init__(*args, **kwargs)
+        name = type(self).__name__
+        if isinstance(quantizer_dropout, bool) or not isinstance(quantizer_dropout, (int, float)) \
+                or not 0.0 <= quantizer_dropout <= 1.0:
+            raise ValueError(f'{name}: quantizer_dropout={quantizer_dropout!r} must be a float in [0, 1]')
+        if 'quantizer_dropout' in quantizer:
+            raise ValueError(f'{name}: quantizer_dropout is not a level key; set it on the {name} node')
         self.rotation_trick = bool(rotation_trick)
+        self.quantizer_dropout = float(quantizer_dropout)
         self._quantizers = self._build_members(quantizer, num_quantizers, 'num_quantizers')
 
     @property
@@ -656,27 +675,64 @@ class ResidualVectorQuantizer(_ComposedQuantizer):
     def embedding_dim(self) -> int:
         return self._quantizers[0].embedding_dim
 
+    def num_levels(self, num_quantizers: int | None = None) -> int:
+        """The depth n of truncated codes: `num_quantizers` checked against [1, L], or L when None."""
+        L = self.num_quantizers
+        if num_quantizers is None:
+            return L
+        if isinstance(num_quantizers, bool) or not isinstance(num_quantizers, int) or not 1 <= num_quantizers <= L:
+            raise ValueError(f'{type(self).__name__}: num_quantizers={num_quantizers!r} is outside [1, {L}]')
+        return num_quantizers
+
     @torch.no_grad()
-    def encode(self, x: torch.Tensor, memo: dict):
-        """-> (x, quant int64 [N, L], memo); every level's callbacks run as in forward (codebook updates included)."""
+    def encode(self, x: torch.Tensor, memo: dict, *, num_quantizers: int | None = None):
+        """-> (x, quant int64 [N, n], memo) with n = num_quantizers (L when None): the first n levels run as in forward
+        (callbacks and codebook updates included); the levels past n do not run at all."""
+        n = self.num_levels(num_quantizers)
         x = self._check_input(x)
-        quant = torch.empty((x.shape[0], self.num_quantizers), dtype=torch.int64, device=x.device)
-        Fq.residual_levels(list(self._quantizers), x, self._member_memos(memo), self._want_norm(), quant_out=quant)
+        quant = torch.empty((x.shape[0], n), dtype=torch.int64, device=x.device)
+        Fq.residual_levels(list(self._quantizers)[:n], x, self._member_memos(memo, n), self._want_norm(), quant_out=quant)
         return x, quant, memo
 
+    @torch.no_grad()
+    def encode_compact(self, x: torch.Tensor, memo: dict, *, num_quantizers: int | None = None) -> torch.Tensor:
+        """`_ComposedQuantizer.encode_compact` over the first n = num_quantizers levels (all L when None): [n, N']."""
+        n = self.num_levels(num_quantizers)
+        if not all(level._callbacks.packed_keys_ok() for level in list(self._quantizers)[:n]):
+            return None
+        return self._encode_compact(x, self._member_memos(memo, n))
+
     def _encode_compact(self, x: torch.Tensor, memos: list) -> torch.Tensor:
+        """The compact ids of the first len(memos) levels."""
         x = self._check_input(x)
-        out = self._compact_out(x.shape[0], x.device)
-        Fq.residual_levels(list(self._quantizers), x, memos, self._want_norm(), compact_out=out[:, :x.shape[0]])
+        out = self._compact_out(x.shape[0], x.device, len(memos))
+        Fq.residual_levels(list(self._quantizers)[:len(memos)], x, memos, self._want_norm(),
+                           compact_out=out[:, :x.shape[0]])
         return out
 
-    def _decode_ids(self, ids: torch.Tensor, hw: int, dtype: torch.dtype = torch.float32, bad_count=None):
-        """ids [b*h*w, L] -> sum_l W_l[id_l] in level order, [b, D, h, w] of `dtype`."""
-        return ops.decode_residual_tokens(self._weights(), ids, hw, dtype, bad_count)
+    def _decode_ids(self, ids: torch.Tensor, hw: int, dtype: torch.dtype = torch.float32, bad_count=None,
+                    num_quantizers: int | None = None):
+        """ids [b*h*w, n] -> sum_{l<n} W_l[id_l] in level order, [b, D, h, w] of `dtype`; n = num_quantizers (L when
+        None)."""
+        return ops.decode_residual_tokens(self._weights()[:self.num_levels(num_quantizers)], ids, hw, dtype, bad_count)
+
+    def draw_depths(self, samples: int, device) -> torch.Tensor:
+        """The depths of one dropout step, int32 [samples], drawn on `device` with torch's CUDA generator (no host
+        synchronisation; capturable in a CUDA graph): the first floor(samples * p) uniform in {1, ..., L}, the rest L."""
+        L = self.num_quantizers
+        depth = torch.full((samples,), L, dtype=torch.int32, device=device)
+        truncated = int(samples * self.quantizer_dropout)
+        if truncated:
+            depth[:truncated].random_(1, L + 1)
+        return depth
 
     def _quantize(self, x: torch.Tensor, levels: list, memos: list, memo: dict):
         nchw = memo.pop('_nchw', None)     # tokenizer.quantize: x is the token-major copy of these [b, c, h, w] latents
-        return Fq.residual_quantize(levels, x, memos, self._want_norm(), nchw=nchw, rotate=self.rotation_trick)
+        dropout = {}        # without dropout: today's call
+        if self.training and self.quantizer_dropout > 0:
+            dropout['depth'] = memo['depth'] = self.draw_depths(x.shape[0] if nchw is None else nchw.shape[0], x.device)
+        return Fq.residual_quantize(levels, x, memos, self._want_norm(), nchw=nchw, rotate=self.rotation_trick,
+                                    **dropout)
 
 @VQITQuantizerRegistry.register_()
 class GroupedVectorQuantizer(_ComposedQuantizer):

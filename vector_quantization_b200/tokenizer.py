@@ -50,8 +50,18 @@ def quantize(quantizer, x: torch.Tensor, memo: dict):
     return Fq.rows_to_nchw(z, b, c, h, w), q_loss, memo
 
 
+def _truncation(quantizer, num_quantizers: int | None) -> dict:
+    """The keyword that truncates a ResidualVectorQuantizer's codes to its first `num_quantizers` levels ({} for None)."""
+    if num_quantizers is None:
+        return {}
+    if not isinstance(quantizer, ResidualVectorQuantizer):
+        raise ValueError(f'num_quantizers truncates ResidualVectorQuantizer codes; {type(quantizer).__name__} has none')
+    return dict(num_quantizers=quantizer.num_levels(num_quantizers))
+
+
 @torch.no_grad()
-def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = False):
+def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = False,
+                    num_quantizers: int | None = None):
     """`BaseModel.encode_to_quant` after the encoder (base.py:131-146): x [b, c, h, w] -> (quant [b, h, w], memo);
     memo['quantizer'] gets 'x_shape', 'x' (token-major, after the callbacks) and 'quant' ([b*h*w] int64).
     compact=True is the tokenise-only variant: token ids come back as uint16 (K <= 65 536) or int32 straight
@@ -59,19 +69,22 @@ def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = F
     A ResidualVectorQuantizer gives quant [b, h, w, L] (a token's L ids contiguous); with compact=True each level's
     ids are compacted into a row of an [L, N] buffer and one transpose (none when L = 1) makes the [N, L] layout.  A
     GroupedVectorQuantizer gives quant [b, h, w, G] the same way (its encode reads the latents through one split
-    launch; memo['quantizer']['x'] is then the latents)."""
+    launch; memo['quantizer']['x'] is then the latents).
+    num_quantizers=n (ResidualVectorQuantizer only, 1 <= n <= L): truncated codes [b, h, w, n] from the first n levels;
+    the levels past n do not run."""
+    truncate = _truncation(quantizer, num_quantizers)
     quantizer_memo = get_memo(memo, 'quantizer')
     quantizer_memo['x_shape'] = (b, _, h, w) = tuple(x.shape)
     if isinstance(quantizer, _ComposedQuantizer):
-        M = len(quantizer.quantizers)
+        M = truncate.get('num_quantizers', len(quantizer.quantizers))
         # a GroupedVectorQuantizer reads the latents through one split launch; residual levels read token-major rows
         x = x if isinstance(quantizer, GroupedVectorQuantizer) else Fq.nchw_to_rows(x)
-        by_member = quantizer.encode_compact(x, quantizer_memo) if compact else None
+        by_member = quantizer.encode_compact(x, quantizer_memo, **truncate) if compact else None
         if by_member is not None:
             quant = by_member.view(-1, 1) if M == 1 else ops.transpose_last2(by_member.view(1, M, -1)).view(-1, M)
             quant = quant[:b * h * w]
         else:
-            x, quant, _ = quantizer.encode(x, quantizer_memo)
+            x, quant, _ = quantizer.encode(x, quantizer_memo, **truncate)
             if compact:
                 quant = quant.to(torch.int32)
         quantizer_memo.update(x=x, quant=quant)
@@ -92,13 +105,15 @@ def encode_to_quant(quantizer, x: torch.Tensor, memo: dict, *, compact: bool = F
 
 
 def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torch.dtype = torch.float32,
-                      check: bool = True):
+                      check: bool = True, num_quantizers: int | None = None):
     """`decode_from_quant` before the decoder (vq/tasks/image_reconstruction/models.py:97-108): token ids
     quant [b, h, w] -> (z [b, c, h, w] contiguous of `dtype`, memo) with memo['quantizer'] = the quantizer's memo as
     `quantizer.decode` leaves it.  quant is uint16, int32 or int64 on the GPU: what `encode_to_quant` (compact or not)
     and FSQ produce, or a `load_tokens` dump moved to the device.  The codebook is used as stored (no before_encode).
     A ResidualVectorQuantizer takes quant [b, h, w, L] and decodes sum_l W_l[id_l] in one launch; a
     GroupedVectorQuantizer takes quant [b, h, w, G] and decodes channel group g from W_g[id_g] in one launch.
+    num_quantizers=n (ResidualVectorQuantizer only, 1 <= n <= L): truncated codes [b, h, w, n], decoded as the sum of
+    the first n levels, sum_{l<n} W_l[id_l], in the same one launch.
 
     A VectorQuantizer or FiniteScalarQuantizer without before_decode / after_decode hooks decodes in ONE launch that
     reads the ids as they are and writes NCHW `dtype` directly.  Hooks, or a codebook that requires grad with grad
@@ -108,10 +123,12 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     An id outside [0, codebook_size) is an error: with check=True (one 4-byte device-to-host read) it raises
     IndexError with the number of such tokens.  check=False does not synchronise (safe inside a CUDA graph capture)
     and, on the one-launch path, decodes such tokens to NaN in every channel."""
+    truncate = _truncation(quantizer, num_quantizers)
     composed = isinstance(quantizer, _ComposedQuantizer)
-    if composed and (quant.dim() != 4 or quant.shape[-1] != len(quantizer.quantizers)):
+    M = truncate.get('num_quantizers', len(quantizer.quantizers) if composed else 1)
+    if composed and (quant.dim() != 4 or quant.shape[-1] != M):
         raise ValueError(f'expected {type(quantizer).__name__} token ids of shape '
-                         f'[b, h, w, {len(quantizer.quantizers)}], got {tuple(quant.shape)}')
+                         f'[b, h, w, {M}], got {tuple(quant.shape)}')
     if not composed and quant.dim() != 3:
         raise ValueError(f'expected token ids of shape [b, h, w], got {tuple(quant.shape)}')
     if not quant.is_cuda:
@@ -122,7 +139,7 @@ def decode_from_quant(quantizer, quant: torch.Tensor, memo: dict, *, dtype: torc
     quantizer_memo = get_memo(memo, 'quantizer')
     if composed:
         bad = torch.zeros(1, dtype=torch.int32, device=quant.device) if check else None
-        z = quantizer._decode_ids(quant.contiguous(), h * w, dtype, bad)
+        z = quantizer._decode_ids(quant.contiguous(), h * w, dtype, bad, **truncate)
         get_memo(quantizer_memo, 'decode')
         if check:
             _raise_bad_ids(int(bad.item()), quantizer.codebook_size)
